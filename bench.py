@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the DiTTo-TTS denoiser hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -22,7 +22,10 @@ Workloads (BASELINE.json configs):
                (packed, unpadded), balanced by cost over the N GPUs; value counts VALID frames
 
 value   = latent frames / s per denoising step = (frames of all utterances on all GPUs) / (time of one step), inputs
-          resident in HBM.  The K-step job is repeated inside the timed region until >= 1 s has elapsed (`repeats`).
+          resident in HBM.  The timed region is one K-step job: exactly K = --steps steps after the W warm-up steps.
+--dump-outputs DIR writes, after the timed region, the final latents of that job on rank 0 (what sample_latents returns)
+          as DIR/latents.npy, float32 [frames, 768]: all frames, or a fixed seeded sample of DUMP_ROWS frames in frame order
+          when there are more.  Weights, inputs and the job's noise seed are fixed, so two builds compare row for row.
 e2e     = the same metric through the public API (DiTTOSampler.sample_latents) starting from PINNED HOST text embeddings
           and x_T and ending with the final latents back in host memory; copies are inside the timed region.
 roofline= the dominant kernel class timed live with CUDA events on the launching stream (library profiler, eager steps
@@ -40,7 +43,6 @@ import argparse
 import atexit
 import hashlib
 import json
-import math
 import os
 import statistics
 import subprocess
@@ -54,7 +56,7 @@ sys.path.insert(0, ROOT)
 HIDDEN, LAYERS, HEADS, TIME_DIM = 768, 5, 1, 256
 FRAMES_10S, TEXT_LEN, GUIDANCE = 750, 64, 3.0
 C4_UTTERANCES = 256
-MIN_TIMED_MS = 1000.0
+DUMP_ROWS = 16384   # 48 MiB of float32 frames at H = 768: a --dump-outputs directory stays under 64 MB
 
 
 def forward_flops(T, S):
@@ -310,7 +312,7 @@ class UniformJob:
     """B utterances of T frames / S tokens on this rank: the product's own stepping (one CUDA-graph replay per step)."""
 
     def __init__(self, torch, D, model, sampler, B, T, S, K, dev, seed):
-        self.torch, self.B, self.T, self.S, self.K, self.dev = torch, B, T, S, K, dev
+        self.torch, self.B, self.T, self.S, self.K, self.dev, self.seed = torch, B, T, S, K, dev, seed
         self.sampler = sampler
         g = torch.Generator().manual_seed(seed)
         self.text_host = torch.randn(B, S, HIDDEN, generator=g).pin_memory()
@@ -325,7 +327,7 @@ class UniformJob:
         self.launches_per_step = self.graph.launches_per_step
 
     def reset(self):
-        self.graph.reset(self.x0, self.K - 1)
+        self.graph.reset(self.x0, self.K - 1, self.seed)
 
     def step(self):
         self.graph.replay()
@@ -358,7 +360,7 @@ class RaggedJob:
     def __init__(self, torch, D, model, sampler, total, world, rank, K, dev, seed):
         from ditto_tts_b200 import parallel
         from ditto_tts_b200.ragged import RaggedBatch, RaggedStepGraph
-        self.torch, self.K, self.dev, self.sampler = torch, K, dev, sampler
+        self.torch, self.K, self.dev, self.sampler, self.seed = torch, K, dev, sampler, seed
         T_all, S_all = parallel.c5_lengths(total)
         mine = parallel.balance_by_cost(T_all, world, S_all)[rank]
         self.T = [T_all[i] for i in mine]
@@ -377,7 +379,7 @@ class RaggedJob:
         self.groups = len(self.rb.groups)
 
     def reset(self):
-        self.graph.reset(self.x0, self.K - 1)
+        self.graph.reset(self.x0, self.K - 1, self.seed)
 
     def step(self):
         self.graph.replay()
@@ -407,30 +409,38 @@ class RaggedJob:
                    "ditto_p_sample_ragged_rng")
 
 
-def timed_job(torch, job, K, W, barrier, min_ms=MIN_TIMED_MS):
-    """W warm-up steps, then the K-step job repeated until >= min_ms: -> (ms_total, repeats, wall t0, wall t1)."""
+def timed_job(torch, job, K, W, barrier):
+    """W warm-up steps (a fresh job every K steps, so that t never runs below 0), then one K-step job between two CUDA
+    events: -> (ms, wall t0, wall t1)."""
+    for i in range(W):
+        if i % K == 0:
+            job.reset()
+        job.step()
     job.reset()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    e0.record()
-    for _ in range(W):
-        job.step()
-    e1.record()
-    torch.cuda.synchronize()
-    est = max(e0.elapsed_time(e1) / max(W, 1), 1e-3)
-    repeats = max(1, int(math.ceil(min_ms / (est * K))))
-    job.reset()
     barrier()
     t_wall0 = time.perf_counter()
     e0.record()
-    for _ in range(repeats):
-        job.reset()
-        for _ in range(K):
-            job.step()
+    for _ in range(K):
+        job.step()
     e1.record()
     barrier()
     t_wall1 = time.perf_counter()
-    return e0.elapsed_time(e1), repeats, t_wall0, t_wall1
+    return e0.elapsed_time(e1), t_wall0, t_wall1
+
+
+def dump_outputs(out_dir, x):
+    """DIR/latents.npy: the latents `x` as float32 rows [frames, H]; above DUMP_ROWS frames, a fixed seeded sample of
+    DUMP_ROWS of them in frame order (the same frames on every run).  -> what the JSON line reports about the dump."""
+    import numpy as np
+    import torch
+    rows = x.detach().reshape(-1, x.shape[-1]).float().cpu()
+    n = rows.shape[0]
+    if n > DUMP_ROWS:
+        rows = rows[torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "latents.npy"), rows.numpy())
+    return {"dir": out_dir, "latents": list(rows.shape), "frames_total": n}
 
 
 def run_ours(args):
@@ -467,8 +477,9 @@ def run_ours(args):
         job = RaggedJob(torch, D, model, sampler, spec["total"], world, rank, K, dev, 1 + rank)
 
     # ---------------- device-resident loop (metric `value`) ----------------
-    ms_total, repeats, t_wall0, t_wall1 = timed_job(torch, job, K, W, barrier)
+    ms_total, t_wall0, t_wall1 = timed_job(torch, job, K, W, barrier)
     finite = bool(torch.isfinite(job.result()).all())
+    dumped = dump_outputs(args.dump_outputs, job.result()) if args.dump_outputs and rank == 0 else None
     clock_summary = clocks.summary(t_wall0, t_wall1)
 
     # ---------------- end to end through the public API, host buffers ----------------
@@ -485,7 +496,7 @@ def run_ours(args):
     # The profiled steps must see the clock the timed region saw: ~1.2 s of back-to-back graph replays first (the SM clock
     # sags to the power-capped level again after the host-side pause of the e2e copy), then the eager steps with no gap;
     # the clock samples of exactly that window choose the roofline denominator.
-    ms_step_est = ms_total / (K * repeats)
+    ms_step_est = ms_total / K
     job.reset()
     for i in range(max(1, min(5000, int(1200.0 / max(ms_step_est, 1e-3))))):
         if i % K == 0:
@@ -507,9 +518,9 @@ def run_ours(args):
     c2 = None
     if world == 1 and args.workload == "c4" and not args.no_c2:
         job2 = UniformJob(torch, D, model, sampler, 16, FRAMES_10S, TEXT_LEN, K, dev, 101)
-        ms2, rep2, w0, w1 = timed_job(torch, job2, K, W, barrier)
+        ms2, w0, w1 = timed_job(torch, job2, K, W, barrier)
         ck2 = clocks.summary(w0, w1)
-        ms2_step = ms2 / (K * rep2)
+        ms2_step = ms2 / K
         job2.e2e_once()
         barrier()
         f0.record()
@@ -517,7 +528,7 @@ def run_ours(args):
         f1.record()
         barrier()
         c2 = {"workload": workload_spec("c2", 1)["text"], "value": job2.frames / (ms2_step / 1e3), "unit": "frames/s",
-              "ms_per_step": ms2_step, "repeats": rep2, "timed_ms": ms2,
+              "ms_per_step": ms2_step, "timed_ms": ms2,
               "algorithmic_tflops": job2.flops_step / (ms2_step / 1e3) / 1e12,
               "e2e_value": job2.frames * K / (f0.elapsed_time(f1) / 1e3),
               "rtf_10s_utterance_batch_latency": ms2_step * K / 1e3 / 10.0,
@@ -527,8 +538,7 @@ def run_ours(args):
     single = None
     if world == 1 and args.workload == "c4" and not args.no_c2:
         job1 = UniformJob(torch, D, model, sampler, 1, FRAMES_10S, TEXT_LEN, K, dev, 201)
-        ms1, rep1, _, _ = timed_job(torch, job1, K, W, barrier, min_ms=300.0)
-        ms1_job = ms1 / rep1
+        ms1_job, _, _ = timed_job(torch, job1, K, W, barrier)
         job1.e2e_once()
         barrier()
         f0.record()
@@ -536,7 +546,7 @@ def run_ours(args):
         f1.record()
         barrier()
         single = {"workload": f"one 10 s utterance (B=1, T={FRAMES_10S}, S={TEXT_LEN}), {K}-step CFG sampling", "job_latency_ms": ms1_job,
-                  "rtf": ms1_job / 1e3 / 10.0, "ms_per_step": ms1_job / K, "repeats": rep1,
+                  "rtf": ms1_job / 1e3 / 10.0, "ms_per_step": ms1_job / K,
                   "e2e_latency_ms": f0.elapsed_time(f1), "e2e_rtf": f0.elapsed_time(f1) / 1e3 / 10.0,
                   "launches_per_step": int(job1.launches_per_step)}
         del job1
@@ -566,7 +576,7 @@ def run_ours(args):
 
     if rank == 0:
         peaks = load_peaks()
-        ms_step = ms_total / (K * repeats)
+        ms_step = ms_total / K
         value = frames_all / (ms_step / 1e3)
         peak_kind, peak = choose_peak(peaks, prof_clocks if prof_clocks.get("sm_mhz") else clock_summary)
         tot_prof_ms = sum(v["ms"] for v in prof.values()) or 1.0
@@ -606,7 +616,7 @@ def run_ours(args):
         extra = {"length_groups_rank0": job.groups, "valid_frames_total": frames_all} if spec["kind"] == "ragged" else None
         line = {
             "metric": "latent frames/sec per denoising step", "value": value, "unit": "frames/s", "n_gpus": world,
-            "steps": K, "warmup": W, "repeats": repeats, "timed_ms": ms_total, "ms_per_step": ms_step, "higher_is_better": True,
+            "steps": K, "warmup": W, "timed_ms": ms_total, "ms_per_step": ms_step, "higher_is_better": True,
             "scaling": spec["scaling"], "vs_baseline": None, "dtype": args.precision, "data": "synthetic",
             "config": workload_config(args, spec, world, extra),
             "rtf": {"job_latency_s": ms_step * K / 1e3, "rtf_10s_utterance": ms_step * K / 1e3 / 10.0,
@@ -616,7 +626,7 @@ def run_ours(args):
             "e2e": {"value": frames_all * K / (ms_e2e / 1e3), "unit": "frames/s", "h2d_bytes_per_step": h2d / K,
                     "d2h_bytes_per_step": d2h / K, "ms_total": ms_e2e,
                     "api": "DiTTOSampler.sample_latents(text_emb, x_init) from pinned host tensors, final latents to host; one K-step job"},
-            "gpu_launches": int(job.launches_per_step * K * repeats), "launches_per_step": int(job.launches_per_step),
+            "gpu_launches": int(job.launches_per_step * K), "launches_per_step": int(job.launches_per_step),
             "stepping": "cuda-graph replay per step (libditto_b200 kernels only)", "clocks": clock_summary,
             "outputs_finite": finite, "output_gather_ms": gather_ms,
         }
@@ -624,12 +634,15 @@ def run_ours(args):
             line["c2"] = c2
         if single is not None:
             line["rtf"]["single_utterance"] = single
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
 
 
 def main():
+    sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
@@ -639,7 +652,11 @@ def main():
     ap.add_argument("--batch", type=int, default=None, help="utterances per GPU (overrides the workload's count)")
     ap.add_argument("--precision", choices=["bf16", "fp32"], default="bf16")
     ap.add_argument("--no-c2", action="store_true", help="skip the C2 side measurement of the single-GPU c4 run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the final latents of the timed job to DIR/latents.npy (float32, at most DUMP_ROWS frames)")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("bench.py: --steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
@@ -653,6 +670,8 @@ def main():
                    "--workload", args.workload, "--precision", args.precision]
             if args.batch:
                 cmd += ["--batch", str(args.batch)]
+            if args.dump_outputs:
+                cmd += ["--dump-outputs", args.dump_outputs]
             raise SystemExit(subprocess.call(cmd))
         run_ours(args)
 

@@ -30,7 +30,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from make_golden import build_reference, import_reference, reference_sampler  # noqa: E402
 from oracle import ditto_oracle as O  # noqa: E402
 
-STRIDE = 5
+STRIDE = 50   # keeps the file under 1 MB
 W = 3.0
 STEPS = 50
 # name, input seed, T, S

@@ -1,7 +1,12 @@
-"""Host-side pieces of bench.py that run without a GPU: the work model and the clock-sample window."""
+"""Host-side pieces of bench.py that run without a GPU: the work model, the clock-sample window, the timed-step count
+and the output dump."""
 import importlib.util
 import json
 import os
+import types
+
+import numpy as np
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
@@ -83,3 +88,57 @@ def test_per_class_roofline_picks_the_longer_bound():
     assert abs(out["tc_gemm.glu"]["achieved"] - 1000.0) < 1e-6 and abs(out["tc_gemm.glu"]["frac"] - 1000.0 / 1400.0) < 1e-3
     assert out["adaln_ln"]["bound"] == "hbm" and abs(out["adaln_ln"]["frac"] - 5000.0 / 6500.0) < 1e-3
     assert all(0.0 < v["frac"] <= 1.0 for v in out.values())
+
+
+def test_timed_region_is_exactly_steps_of_one_job():
+    """--steps K: K steps between the two CUDA events, after the W warm-up steps; no step runs past t = 0."""
+    log = []
+
+    class Event:
+        def __init__(self, enable_timing):
+            pass
+
+        def record(self):
+            log.append("event")
+
+        def elapsed_time(self, other):
+            return 12.5
+
+    class Job:
+        def __init__(self, K):
+            self.K, self.t = K, None
+
+        def reset(self):
+            self.t = self.K - 1
+
+        def step(self):
+            assert self.t is not None and self.t >= 0
+            self.t -= 1
+            log.append("step")
+
+    fake_torch = types.SimpleNamespace(cuda=types.SimpleNamespace(Event=Event))
+    for K, W in ((7, 3), (2, 5), (50, 0), (1, 1)):
+        log.clear()
+        ms, t0, t1 = bench.timed_job(fake_torch, Job(K), K, W, lambda: None)
+        assert ms == 12.5 and t0 <= t1
+        assert log.count("event") == 2 and log.count("step") == W + K
+        first = log.index("event")
+        assert log[first + 1:] == ["step"] * K + ["event"]
+
+
+def test_dump_outputs_writes_float32_latents_within_budget(tmp_path):
+    """Small outputs are written whole; large ones as the same seeded sample of frames on every call, under 64 MB."""
+    x = torch.randn(2, 5, 768)
+    info = bench.dump_outputs(str(tmp_path / "small"), x)
+    got = np.load(tmp_path / "small" / "latents.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, x.reshape(-1, 768).numpy())
+    assert info["latents"] == [10, 768] and info["frames_total"] == 10
+    big = torch.randn(3, 6000, 768)
+    bench.dump_outputs(str(tmp_path / "a"), big)
+    bench.dump_outputs(str(tmp_path / "b"), big)
+    a, b = np.load(tmp_path / "a" / "latents.npy"), np.load(tmp_path / "b" / "latents.npy")
+    assert a.shape == (bench.DUMP_ROWS, 768) and np.array_equal(a, b)
+    assert os.path.getsize(tmp_path / "a" / "latents.npy") < 64e6
+    rows = big.reshape(-1, 768).numpy()
+    idx = [int(np.flatnonzero((rows == r).all(1))[0]) for r in a[:50]]
+    assert idx == sorted(idx)                                   # frames kept in frame order

@@ -90,6 +90,10 @@ def test_c5_three_utterances_sampled_together_vs_per_utterance_reference(dev, tr
         assert rel(rec[-1][i][::stride], torch.from_numpy(traj[f"{n}::eps_last_sub"])[0]) <= BAR[precision], n
         e = rel(outs[i][::stride], torch.from_numpy(traj[f"{n}::final_sub"])[0])
         assert e <= BAR[precision], (n, e)
+        # norms of the full tensors: every frame, not only the stored ones
+        assert abs(float(outs[i].double().norm()) / traj[f"{n}::norms"][2] - 1.0) <= BAR[precision], n
+        norms = np.array([float(r[i].double().norm()) for r in rec])
+        assert np.allclose(norms, traj[f"{n}::eps_norms"], rtol=BAR[precision]), n
     graph_outs = s.sample_latents_ragged(texts, lengths, x_init=xs, noise=noises)      # CUDA-graph stepping, same noise
     for a, b in zip(graph_outs, outs):
         assert rel(a, b) <= 1e-6

@@ -248,9 +248,11 @@ def test_reference_sampler_loop_tiny(dev, golden, precision):
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
 def test_cfg_50_steps_vs_reference_trajectory(dev, golden, precision):
     """Full 50-step CFG sampling (w = 3, uncond = zero text) on the default model, B=2, T=96: first and last
-    per-step eps_hat and the final latent against the trajectory computed with the reference forward."""
+    per-step eps_hat and the final latent (every `stride`-th frame, plus the norms of the full tensors) against the
+    trajectory computed with the reference forward."""
     c = golden("cfg_traj.npz")
     B, T, S, iseed, wseed, steps = [int(v) for v in c["meta"]]
+    stride = int(c["stride"][0])
     cfg = O.OracleConfig(768, 5, 1, 256, 768, steps)
     sd = O.make_state_dict(cfg, wseed)
     x, text, noise = O.make_inputs(B, T, S, cfg, iseed, steps_noise=steps)
@@ -258,9 +260,10 @@ def test_cfg_50_steps_vs_reference_trajectory(dev, golden, precision):
     rec = []
     out = s.sample_latents(text.to(dev), x_init=x.to(dev), noise=noise.to(dev), record=rec)
     assert len(rec) == steps
-    assert rel(rec[0], torch.from_numpy(c["eps_first"])) <= BAR[precision]
-    assert rel(rec[-1], torch.from_numpy(c["eps_last"])) <= BAR[precision]
-    assert rel(out, torch.from_numpy(c["final"])) <= BAR[precision]
+    assert rel(rec[0][:, ::stride], torch.from_numpy(c["eps_first"])) <= BAR[precision]
+    assert rel(rec[-1][:, ::stride], torch.from_numpy(c["eps_last"])) <= BAR[precision]
+    assert rel(out[:, ::stride], torch.from_numpy(c["final"])) <= BAR[precision]
+    assert abs(float(out.double().norm()) / float(c["final_norm"][0]) - 1.0) <= BAR[precision]
     norms = np.array([float(e.double().norm()) for e in rec])
     assert np.allclose(norms, c["eps_norms"], rtol=BAR[precision])
 

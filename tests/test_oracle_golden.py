@@ -91,17 +91,20 @@ def test_full_size_forward(golden, name):
 
 def test_cfg_trajectory_endpoints(golden):
     """50-step CFG (w=3, uncond = zero text) on the default model: first/last eps_hat and final latent
-    of the reference-forward trajectory.  The oracle runs the same loop (2 forwards per step)."""
+    of the reference-forward trajectory (every `stride`-th frame, plus the norms of the full tensors).
+    The oracle runs the same loop (2 forwards per step)."""
     g = golden("cfg_traj.npz")
     B, T, S, iseed, wseed, steps = [int(v) for v in g["meta"]]
+    stride = int(g["stride"][0])
     cfg = O.OracleConfig(768, 5, 1, 256, 768, steps)
     sd = O.make_state_dict(cfg, seed=wseed)
     x, text, noise = O.make_inputs(B, T, S, cfg, seed=iseed, steps_noise=steps)
     rec = []
     final = O.sample_latents(sd, cfg, text, x, noise, guidance_scale=float(g["w"][0]), record=rec)
-    assert O.rel_l2(rec[0], torch.from_numpy(g["eps_first"])) <= FP32_BAR
+    assert O.rel_l2(rec[0][:, ::stride], torch.from_numpy(g["eps_first"])) <= FP32_BAR
     # chaotic growth of the latent (rms ~1e5 after 50 steps) amplifies fp32 re-association noise
-    assert O.rel_l2(rec[-1], torch.from_numpy(g["eps_last"])) <= 1e-4
-    assert O.rel_l2(final, torch.from_numpy(g["final"])) <= 1e-4
+    assert O.rel_l2(rec[-1][:, ::stride], torch.from_numpy(g["eps_last"])) <= 1e-4
+    assert O.rel_l2(final[:, ::stride], torch.from_numpy(g["final"])) <= 1e-4
+    assert float(final.double().norm()) == pytest.approx(float(g["final_norm"][0]), rel=1e-4)
     norms = np.array([float(e.double().norm()) for e in rec])
     assert np.allclose(norms, g["eps_norms"], rtol=1e-4)
