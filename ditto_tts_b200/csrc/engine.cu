@@ -487,7 +487,10 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
     DITTO_CUDA(cudaMemcpyAsync(w.h, x, static_cast<size_t>(M) * H * sizeof(float), cudaMemcpyDeviceToDevice, st));
     const char* nw = stage == 2 ? "norm2.weight" : stage == 3 ? "norm3.weight" : "norm1.weight";     // DiT.py:105 / :143 / :152
     const char* nb = stage == 2 ? "norm2.bias" : stage == 3 ? "norm3.bias" : "norm1.bias";
-    DITTO_TRY(launch_layernorm(w.h, e->LW(l_begin, nw), e->LW(l_begin, nb), w.u, b16, M, H, st));
+    // cross-attention alone with norm2 folded into the text context (K Wq diag(gamma2), score bias with beta2): there are no
+    // row statistics from a self-attention before it, so the query operand is the normalised row without the affine part
+    const bool affine = !(stage == 2 && fold_ln_active(e, g0.S));
+    DITTO_TRY(launch_layernorm(w.h, affine ? e->LW(l_begin, nw) : nullptr, affine ? e->LW(l_begin, nb) : nullptr, w.u, b16, M, H, st));
   }
   // AdaLN + LN1 of block 0 (+ bf16 copy of x for proj_in)                 DiTTO.py:86, DiT.py:25-40,105
   DITTO_TRY(fork.begin(block_only ? 0 : ng));
@@ -561,7 +564,7 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
         bf16* ug = u + grp.row0 * H;
         float* hg = w.h + grp.row0 * H;
         // norm2 deferred for this group (context built with the gamma2-folded K): whole-model DITTO_F_DEFER_LN, or norm2 only
-        const bool dln2 = dln ? dln2_all : fold_ln_active(e, S);
+        const bool dln2 = dln ? dln2_all : fold_ln_active(e, S) && do_self;   // the row statistics come from the self-attention
         float2* lnstat_g = w.lnstat ? w.lnstat + grp.row0 * std::max(w.ln_parts_h, w.ln_parts_attn) : nullptr;
         if (!do_self) {
           // stand-alone cross-attention / MLP section: u already holds that section's LayerNorm of the input
