@@ -48,6 +48,7 @@ SIGNATURES = {
     "ditto_engine_load_weight": (_I32, [_P, C.c_char_p, _P, _I64, _P]),
     "ditto_engine_load_schedule": (_I32, [_P, _P, _P, _P, _I64, _P]),
     "ditto_engine_load_update_table": (_I32, [_P, _P, _I64, _P]),
+    "ditto_engine_load_multistep_table": (_I32, [_P, _P, _I64, _P]),
     "ditto_engine_finalize": (_I32, [_P, _P]),
     "ditto_text_context_bytes": (_I64, [_P, _I64, _I64]),
     "ditto_workspace_bytes": (_I64, [_P, _I64, _I64, _I64]),
@@ -58,11 +59,18 @@ SIGNATURES = {
     "ditto_p_sample_rng": (_I32, [_P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _I64, _I32, _P]),
     "ditto_cfg_ddpm_update_rng": (_I32, [_P, _P, _P, _P, _P, _P, _I64, _F, _P, _I64, _I64, _I32, _P]),
     "ditto_randn": (_I32, [_P, _I64, _P, _I64, _P]),
+    "ditto_cfg_multistep_update": (_I32, [_P, _P, _P, _P, _P, _P, _F, _P, _P, _I64, _I64, _P]),
+    "ditto_cfg_multistep_update_rng": (_I32, [_P, _P, _P, _P, _P, _P, _I64, _F, _P, _P, _I64, _I64, _I32, _P]),
+    "ditto_p_sample_multistep": (_I32, [_P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _P]),
+    "ditto_p_sample_multistep_rng": (_I32, [_P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _I32, _P]),
     "ditto_q_sample": (_I32, [_P, _P, _P, _P, _P, _I64, _I64, _P]),
     "ditto_workspace_bytes_ragged": (_I64, [_P, C.POINTER(SeqGroup), _I64]),
     "ditto_forward_ragged": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _P, _I64, _P]),
     "ditto_p_sample_ragged": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _I32, _F, _P, _P, _P, _I64, _P]),
     "ditto_p_sample_ragged_rng": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _I32, _F, _P, _P, _P, _I64, _I32, _P]),
+    "ditto_p_sample_ragged_multistep": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _I32, _F, _P, _P, _P, _P, _I64, _P]),
+    "ditto_p_sample_ragged_multistep_rng": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _I32, _F, _P, _P, _P, _P, _I64, _I32,
+                                                   _P]),
     "ditto_dit_block": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),
     "ditto_attn_self": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),
     "ditto_attn_cross": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),

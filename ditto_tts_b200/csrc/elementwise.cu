@@ -689,6 +689,26 @@ __device__ __forceinline__ float4 philox_normal4(unsigned long long seed, unsign
   return make_float4(m0 * c0, m0 * s0, m1 * c1, m1 * s1);
 }
 
+// `advance` of the in-kernel-noise update kernels: called by every block after its last read of rng / t
+__device__ __forceinline__ void last_block_advances(unsigned long long* rng, int64_t* t, int64_t n_t, unsigned long long draw) {
+  // every thread of every block has read rng / t before its block takes a ticket; the block holding the last ticket owns them
+  __shared__ int s_last;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    const unsigned long long tk = atomicAdd(rng + 2, 1ull);
+    s_last = tk == static_cast<unsigned long long>(gridDim.x) - 1ull;
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  for (int64_t i = threadIdx.x; i < n_t; i += blockDim.x) t[i] -= 1;
+  if (threadIdx.x == 0) {
+    rng[1] = draw + 1ull;
+    rng[2] = 0ull;
+  }
+}
+
 __global__ void __launch_bounds__(256)
     cfg_ddpm_update_rng_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
                                unsigned long long* rng, int64_t* t, int64_t n_t, const float* __restrict__ coef, int steps, float w,
@@ -710,23 +730,7 @@ __global__ void __launch_bounds__(256)
     out[i] = make_float4(ddpm_update(xv.x, e.x, zv.x, c1, c2, c3), ddpm_update(xv.y, e.y, zv.y, c1, c2, c3),
                          ddpm_update(xv.z, e.z, zv.z, c1, c2, c3), ddpm_update(xv.w, e.w, zv.w, c1, c2, c3));
   }
-  if (!advance) return;
-  // every thread of every block has read rng / t before its block takes a ticket; the block holding the last ticket owns them
-  __shared__ int s_last;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    __threadfence();
-    const unsigned long long tk = atomicAdd(rng + 2, 1ull);
-    s_last = tk == static_cast<unsigned long long>(gridDim.x) - 1ull;
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  for (int64_t i = threadIdx.x; i < n_t; i += blockDim.x) t[i] -= 1;
-  if (threadIdx.x == 0) {
-    rng[1] = draw + 1ull;
-    rng[2] = 0ull;
-  }
+  if (advance) last_block_advances(rng, t, n_t, draw);
 }
 
 int launch_cfg_ddpm_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t, int64_t n_t,
@@ -742,6 +746,121 @@ int launch_cfg_ddpm_update_rng(const float* eps_c, const float* eps_u, const flo
                                                      reinterpret_cast<const float4*>(x), rng, t, n_t, coef, steps, w,
                                                      reinterpret_cast<float4*>(out), elems_per_seq / 4, total_vec, elem_offset / 4,
                                                      advance ? 1 : 0);
+  DITTO_LAUNCH_CHECK();
+  return 0;
+}
+
+// =====================================================================================================
+// CFG combine + multistep update (DPM-Solver++(2M), Lu et al. 2022 Alg. 2, and its SDE variant), one pass:
+//   x_out = c1 (x - c2 eps) + c3 z + c4 hist        hist <- d1 (x - d2 eps)   (the x0 prediction of this step)
+//   coef_ms[t] = {c1, c2, c3, c4, d1, d2}, computed on the host (schedules.dpmpp_2m_coef).
+// The first term is ddpm_update with the same roundings, the history term one more fma; a row with c4 == 0 (first-order
+// steps) neither reads hist nor adds the term, so x_out is bit-identical to cfg_ddpm_update_kernel with (c1, c2, c3) and
+// whatever hist held before the first step (uninitialised, NaN) cannot reach it.  c4 is uniform per sequence (one row per
+// t[seq]), so the branch does not diverge inside a sequence's vectors.  x_out may alias x and hist is updated in place:
+// every thread reads its elements before it writes them.  +8 B / element over the DDPM kernel (hist read + write).
+// =====================================================================================================
+__device__ __forceinline__ float x0_pred(float x, float e, float d1, float d2) { return __fmul_rn(d1, __fmaf_rn(-d2, e, x)); }
+
+// one row of the table; the hist read is issued together with the other loads of the element (before the noise is drawn),
+// predicated on c4 so that first-order rows never touch it
+struct MultistepRow {
+  float c1, c2, c3, c4, d1, d2;
+};
+__device__ __forceinline__ MultistepRow multistep_row(const float* __restrict__ coef, const int64_t* t, int64_t seq, int steps) {
+  int64_t tt = t[seq];
+  tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
+  const float* r = coef + tt * 6;
+  return MultistepRow{r[0], r[1], r[2], r[3], r[4], r[5]};
+}
+__device__ __forceinline__ float4 multistep_hist(const float4* __restrict__ hist, int64_t i, float c4) {
+  return c4 != 0.f ? hist[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+__device__ __forceinline__ void multistep_store(const MultistepRow& c, float4 xv, float4 e, float4 zv, float4 h,
+                                                float4* __restrict__ out, float4* __restrict__ hist, int64_t i) {
+  float4 o = make_float4(ddpm_update(xv.x, e.x, zv.x, c.c1, c.c2, c.c3), ddpm_update(xv.y, e.y, zv.y, c.c1, c.c2, c.c3),
+                         ddpm_update(xv.z, e.z, zv.z, c.c1, c.c2, c.c3), ddpm_update(xv.w, e.w, zv.w, c.c1, c.c2, c.c3));
+  if (c.c4 != 0.f)
+    o = make_float4(__fmaf_rn(c.c4, h.x, o.x), __fmaf_rn(c.c4, h.y, o.y), __fmaf_rn(c.c4, h.z, o.z), __fmaf_rn(c.c4, h.w, o.w));
+  hist[i] = make_float4(x0_pred(xv.x, e.x, c.d1, c.d2), x0_pred(xv.y, e.y, c.d1, c.d2), x0_pred(xv.z, e.z, c.d1, c.d2),
+                        x0_pred(xv.w, e.w, c.d1, c.d2));
+  out[i] = o;
+}
+
+__global__ void __launch_bounds__(256)
+    cfg_multistep_update_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
+                                const float4* __restrict__ z, const int64_t* __restrict__ t, const float* __restrict__ coef,
+                                int steps, float w, float4* __restrict__ out, float4* __restrict__ hist, int64_t vec_per_seq,
+                                int64_t total_vec) {
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const MultistepRow c = multistep_row(coef, t, i / vec_per_seq, steps);
+    float4 e = eps_c[i];
+    if (eps_u != nullptr) {
+      const float4 u = eps_u[i];
+      e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
+    }
+    const float4 xv = x[i];
+    const float4 zv = z != nullptr ? z[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 h = multistep_hist(hist, i, c.c4);
+    multistep_store(c, xv, e, zv, h, out, hist, i);
+  }
+}
+
+int launch_cfg_multistep_update(const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
+                                const float* coef, int steps, float w, float* out, float* hist, int64_t B, int64_t elems_per_seq,
+                                cudaStream_t st) {
+  DITTO_REQUIRE(elems_per_seq % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_multistep_update: elems_per_seq % 4");
+  const int64_t total_vec = B * elems_per_seq / 4;
+  if (total_vec == 0) return 0;
+  const int64_t want = ceil_div(total_vec, 256 * 4);
+  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
+  ProfScope prof(PC_CFG_UPDATE, st, 0.0, static_cast<double>(total_vec) * 16 * (5 + (eps_u ? 1 : 0) + (z ? 1 : 0)));
+  cfg_multistep_update_kernel<<<blocks, 256, 0, st>>>(
+      reinterpret_cast<const float4*>(eps_c), reinterpret_cast<const float4*>(eps_u), reinterpret_cast<const float4*>(x),
+      reinterpret_cast<const float4*>(z), t, coef, steps, w, reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(hist),
+      elems_per_seq / 4, total_vec);
+  DITTO_LAUNCH_CHECK();
+  return 0;
+}
+
+// the same with the noise drawn in the kernel: Philox stream, element offsets and `advance` bookkeeping exactly as
+// cfg_ddpm_update_rng_kernel (the normals equal ditto_randn's at the same {seed, draw})
+__global__ void __launch_bounds__(256)
+    cfg_multistep_update_rng_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
+                                    unsigned long long* rng, int64_t* t, int64_t n_t, const float* __restrict__ coef, int steps,
+                                    float w, float4* __restrict__ out, float4* __restrict__ hist, int64_t vec_per_seq,
+                                    int64_t total_vec, int64_t vec_offset, int advance) {
+  const unsigned long long seed = rng[0], draw = rng[1];
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const MultistepRow c = multistep_row(coef, t, i / vec_per_seq, steps);
+    float4 e = eps_c[i];
+    if (eps_u != nullptr) {
+      const float4 u = eps_u[i];
+      e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
+    }
+    const float4 xv = x[i];
+    const float4 h = multistep_hist(hist, i, c.c4);
+    const float4 zv = philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i));
+    multistep_store(c, xv, e, zv, h, out, hist, i);
+  }
+  if (advance) last_block_advances(rng, t, n_t, draw);
+}
+
+int launch_cfg_multistep_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t,
+                                    int64_t n_t, const float* coef, int steps, float w, float* out, float* hist, int64_t B,
+                                    int64_t elems_per_seq, int64_t elem_offset, bool advance, cudaStream_t st) {
+  DITTO_REQUIRE(elems_per_seq % 4 == 0 && elem_offset % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_multistep_update_rng: elems_per_seq % 4");
+  const int64_t total_vec = B * elems_per_seq / 4;
+  if (total_vec == 0) return advance ? launch_step_advance(rng, t, n_t, st) : 0;
+  const int64_t want = ceil_div(total_vec, 256 * 4);
+  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
+  ProfScope prof(PC_CFG_UPDATE, st, 0.0, static_cast<double>(total_vec) * 16 * (5 + (eps_u ? 1 : 0)));
+  cfg_multistep_update_rng_kernel<<<blocks, 256, 0, st>>>(
+      reinterpret_cast<const float4*>(eps_c), reinterpret_cast<const float4*>(eps_u), reinterpret_cast<const float4*>(x), rng, t,
+      n_t, coef, steps, w, reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(hist), elems_per_seq / 4, total_vec,
+      elem_offset / 4, advance ? 1 : 0);
   DITTO_LAUNCH_CHECK();
   return 0;
 }

@@ -107,6 +107,7 @@ struct ditto_engine {
   std::map<std::string, float*> w;          // device fp32 copies (owned)
   std::vector<void*> owned;                 // everything else cudaMalloc'ed by the engine
   float *time_table = nullptr, *rope_cos = nullptr, *rope_sin = nullptr, *rope_freq = nullptr, *coef = nullptr, *qs_buf = nullptr;
+  float* coef_ms = nullptr;  // [steps, 6] multistep update table (ditto_engine_load_multistep_table); null until loaded
   bf16 *w_in16 = nullptr, *w_out16 = nullptr;
   bf16* w_out_p4 = nullptr;   // proj_out rows in the perm4 order of gemm_resid_ln.cu (fc2_ln engines)
   std::vector<LayerPack> layers;
@@ -959,6 +960,15 @@ int32_t ditto_engine_load_update_table(ditto_engine_t* e, const float* coef, int
   return 0;
 }
 
+int32_t ditto_engine_load_multistep_table(ditto_engine_t* e, const float* coef6, int64_t steps, void* stream) {
+  DITTO_REQUIRE(e && coef6, DITTO_E_BADARG, "load_multistep_table: null argument");
+  DITTO_REQUIRE(steps == e->steps, DITTO_E_BADARG, "load_multistep_table: steps != diffusion_steps");
+  DITTO_REQUIRE(e->have_schedule, DITTO_E_STATE, "load_multistep_table: call ditto_engine_load_schedule first");
+  if (!e->coef_ms) DITTO_TRY(dev_alloc(e, reinterpret_cast<void**>(&e->coef_ms), sizeof(float) * 6 * steps));
+  DITTO_CUDA(cudaMemcpyAsync(e->coef_ms, coef6, sizeof(float) * 6 * steps, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
 int32_t ditto_engine_finalize(ditto_engine_t* e, void* stream) {
   DITTO_REQUIRE(e, DITTO_E_BADARG, "finalize: null engine");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1225,9 +1235,30 @@ int32_t ditto_cfg_ddpm_update(ditto_engine_t* e, const float* eps_c, const float
                                 static_cast<cudaStream_t>(stream));
 }
 
-int32_t ditto_p_sample(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
-                       float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
-                       int64_t workspace_bytes, void* stream) {
+// the update of one sampler step: the [steps, 3] DDPM-form table, or (hist != null) the [steps, 6] multistep table
+static int launch_update(const ditto_engine* e, const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
+                         float w, float* x_out, float* hist, int64_t B, int64_t per, cudaStream_t st) {
+  if (hist) return launch_cfg_multistep_update(eps_c, eps_u, x, z, t, e->coef_ms, e->steps, w, x_out, hist, B, per, st);
+  return launch_cfg_ddpm_update(eps_c, eps_u, x, z, t, e->coef, e->steps, w, x_out, B, per, st);
+}
+static int launch_update_rng(const ditto_engine* e, const float* eps_c, const float* eps_u, const float* x, uint64_t* rng, int64_t* t,
+                             int64_t n_t, float w, float* x_out, float* hist, int64_t B, int64_t per, int64_t elem_offset, bool advance,
+                             cudaStream_t st) {
+  unsigned long long* r = reinterpret_cast<unsigned long long*>(rng);
+  if (hist)
+    return launch_cfg_multistep_update_rng(eps_c, eps_u, x, r, t, n_t, e->coef_ms, e->steps, w, x_out, hist, B, per, elem_offset, advance, st);
+  return launch_cfg_ddpm_update_rng(eps_c, eps_u, x, r, t, n_t, e->coef, e->steps, w, x_out, B, per, elem_offset, advance, st);
+}
+// what every multistep entry point checks on top of its DDPM-form twin
+static int require_multistep(const ditto_engine* e, const float* hist, const char* what) {
+  DITTO_REQUIRE(e && hist, DITTO_E_BADARG, std::string(what) + ": null argument (hist)");
+  DITTO_REQUIRE(e->coef_ms, DITTO_E_STATE, std::string(what) + ": no multistep table loaded (ditto_engine_load_multistep_table)");
+  return 0;
+}
+
+static int32_t p_sample_impl(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
+                             float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
+                             void* workspace, int64_t workspace_bytes, void* stream) {
   DITTO_REQUIRE(e && x && ctx && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample: null argument");
   DITTO_REQUIRE(e->finalized && e->have_schedule && !e->blocks_only, DITTO_E_STATE, "p_sample: engine not finalized / schedule not loaded");
   DITTO_REQUIRE(B > 0 && T > 0 && S > 0 && T <= e->maxT, DITTO_E_BADARG, "p_sample: bad sizes");
@@ -1235,13 +1266,25 @@ int32_t ditto_p_sample(ditto_engine_t* e, const float* x, const void* ctx, const
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DITTO_TRY(forward_impl(e, x, B, ctx, t, n, T, S, eps_scratch, workspace, workspace_bytes, st));
   const int64_t per = T * e->H;
-  return launch_cfg_ddpm_update(eps_scratch, guided ? eps_scratch + B * per : nullptr, x, z, t, e->coef, e->steps, guidance_scale, x_out,
-                                B, per, st);
+  return launch_update(e, eps_scratch, guided ? eps_scratch + B * per : nullptr, x, z, t, guidance_scale, x_out, hist, B, per, st);
 }
 
-int32_t ditto_p_sample_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
-                           float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
-                           int64_t workspace_bytes, int32_t advance, void* stream) {
+int32_t ditto_p_sample(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
+                       float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
+                       int64_t workspace_bytes, void* stream) {
+  return p_sample_impl(e, x, ctx, t, z, guided, guidance_scale, B, T, S, eps_scratch, x_out, nullptr, workspace, workspace_bytes, stream);
+}
+
+int32_t ditto_p_sample_multistep(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
+                                 float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
+                                 void* workspace, int64_t workspace_bytes, void* stream) {
+  DITTO_TRY(require_multistep(e, hist, "p_sample_multistep"));
+  return p_sample_impl(e, x, ctx, t, z, guided, guidance_scale, B, T, S, eps_scratch, x_out, hist, workspace, workspace_bytes, stream);
+}
+
+static int32_t p_sample_rng_impl(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
+                                 float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
+                                 void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
   DITTO_REQUIRE(e && x && ctx && t && rng && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_rng: null argument");
   DITTO_REQUIRE(e->finalized && e->have_schedule && !e->blocks_only, DITTO_E_STATE, "p_sample_rng: engine not finalized / schedule not loaded");
   DITTO_REQUIRE(B > 0 && T > 0 && S > 0 && T <= e->maxT, DITTO_E_BADARG, "p_sample_rng: bad sizes");
@@ -1249,8 +1292,23 @@ int32_t ditto_p_sample_rng(ditto_engine_t* e, const float* x, const void* ctx, i
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DITTO_TRY(forward_impl(e, x, B, ctx, t, n, T, S, eps_scratch, workspace, workspace_bytes, st));
   const int64_t per = T * e->H;
-  return launch_cfg_ddpm_update_rng(eps_scratch, guided ? eps_scratch + B * per : nullptr, x, reinterpret_cast<unsigned long long*>(rng), t, n,
-                                    e->coef, e->steps, guidance_scale, x_out, B, per, 0, advance != 0, st);
+  return launch_update_rng(e, eps_scratch, guided ? eps_scratch + B * per : nullptr, x, rng, t, n, guidance_scale, x_out, hist, B, per, 0,
+                           advance != 0, st);
+}
+
+int32_t ditto_p_sample_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
+                           float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
+                           int64_t workspace_bytes, int32_t advance, void* stream) {
+  return p_sample_rng_impl(e, x, ctx, t, rng, guided, guidance_scale, B, T, S, eps_scratch, x_out, nullptr, workspace, workspace_bytes,
+                           advance, stream);
+}
+
+int32_t ditto_p_sample_multistep_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
+                                     float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
+                                     void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
+  DITTO_TRY(require_multistep(e, hist, "p_sample_multistep_rng"));
+  return p_sample_rng_impl(e, x, ctx, t, rng, guided, guidance_scale, B, T, S, eps_scratch, x_out, hist, workspace, workspace_bytes,
+                           advance, stream);
 }
 
 int32_t ditto_cfg_ddpm_update_rng(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, uint64_t* rng, int64_t* t,
@@ -1261,6 +1319,25 @@ int32_t ditto_cfg_ddpm_update_rng(ditto_engine_t* e, const float* eps_c, const f
   DITTO_REQUIRE(B >= 0 && elems_per_seq >= 0 && n_t >= B, DITTO_E_BADARG, "cfg_ddpm_update_rng: bad sizes");
   return launch_cfg_ddpm_update_rng(eps_c, eps_u, x, reinterpret_cast<unsigned long long*>(rng), t, n_t, e->coef, e->steps, guidance_scale,
                                     x_out, B, elems_per_seq, 0, advance != 0, static_cast<cudaStream_t>(stream));
+}
+
+int32_t ditto_cfg_multistep_update(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
+                                   const int64_t* t, float guidance_scale, float* x_out, float* hist, int64_t B, int64_t elems_per_seq,
+                                   void* stream) {
+  DITTO_REQUIRE(e && eps_c && x && t && x_out, DITTO_E_BADARG, "cfg_multistep_update: null argument");
+  DITTO_REQUIRE(B >= 0 && elems_per_seq >= 0, DITTO_E_BADARG, "cfg_multistep_update: negative size");
+  DITTO_TRY(require_multistep(e, hist, "cfg_multistep_update"));
+  return launch_update(e, eps_c, eps_u, x, z, t, guidance_scale, x_out, hist, B, elems_per_seq, static_cast<cudaStream_t>(stream));
+}
+
+int32_t ditto_cfg_multistep_update_rng(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, uint64_t* rng,
+                                       int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist, int64_t B,
+                                       int64_t elems_per_seq, int32_t advance, void* stream) {
+  DITTO_REQUIRE(e && eps_c && x && t && rng && x_out, DITTO_E_BADARG, "cfg_multistep_update_rng: null argument");
+  DITTO_REQUIRE(B >= 0 && elems_per_seq >= 0 && n_t >= B, DITTO_E_BADARG, "cfg_multistep_update_rng: bad sizes");
+  DITTO_TRY(require_multistep(e, hist, "cfg_multistep_update_rng"));
+  return launch_update_rng(e, eps_c, eps_u, x, rng, t, n_t, guidance_scale, x_out, hist, B, elems_per_seq, 0, advance != 0,
+                           static_cast<cudaStream_t>(stream));
 }
 
 int32_t ditto_randn(const uint64_t* rng, int64_t elem_offset, float* out, int64_t n, void* stream) {
@@ -1306,9 +1383,9 @@ int32_t ditto_forward_ragged(ditto_engine_t* e, const float* x, const ditto_seq_
   return forward_impl(e, x, t, gs.data(), static_cast<int>(gs.size()), out, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
-int32_t ditto_p_sample_ragged(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, const int64_t* t,
-                              const float* z, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, void* workspace,
-                              int64_t workspace_bytes, void* stream) {
+static int32_t p_sample_ragged_impl(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, const int64_t* t,
+                                    const float* z, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, float* hist,
+                                    void* workspace, int64_t workspace_bytes, void* stream) {
   DITTO_REQUIRE(e && x && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_ragged: null argument");
   DITTO_REQUIRE(e->finalized && e->have_schedule, DITTO_E_STATE, "p_sample_ragged: engine not finalized / schedule not loaded");
   std::vector<SeqGroup> gs;
@@ -1326,16 +1403,32 @@ int32_t ditto_p_sample_ragged(ditto_engine_t* e, const float* x, const ditto_seq
     const SeqGroup& g = gs[gi];
     const int64_t per = g.T * H;
     const float* ec = eps_scratch + g.row0 * H;
-    DITTO_TRY(launch_cfg_ddpm_update(ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, z ? z + g.xrow0 * H : nullptr, t + g.seq0,
-                                     e->coef, e->steps, guidance_scale, x_out + g.xrow0 * H, g.n_x, per, fork.stream(static_cast<int>(gi))));
+    DITTO_TRY(launch_update(e, ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, z ? z + g.xrow0 * H : nullptr, t + g.seq0,
+                            guidance_scale, x_out + g.xrow0 * H, hist ? hist + g.xrow0 * H : nullptr, g.n_x, per,
+                            fork.stream(static_cast<int>(gi))));
   }
   DITTO_TRY(fork.end());
   return 0;
 }
 
-int32_t ditto_p_sample_ragged_rng(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
-                                  uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, void* workspace,
-                                  int64_t workspace_bytes, int32_t advance, void* stream) {
+int32_t ditto_p_sample_ragged(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, const int64_t* t,
+                              const float* z, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, void* workspace,
+                              int64_t workspace_bytes, void* stream) {
+  return p_sample_ragged_impl(e, x, groups, n_groups, t, z, guided, guidance_scale, eps_scratch, x_out, nullptr, workspace,
+                              workspace_bytes, stream);
+}
+
+int32_t ditto_p_sample_ragged_multistep(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
+                                        const int64_t* t, const float* z, int32_t guided, float guidance_scale, float* eps_scratch,
+                                        float* x_out, float* hist, void* workspace, int64_t workspace_bytes, void* stream) {
+  DITTO_TRY(require_multistep(e, hist, "p_sample_ragged_multistep"));
+  return p_sample_ragged_impl(e, x, groups, n_groups, t, z, guided, guidance_scale, eps_scratch, x_out, hist, workspace,
+                              workspace_bytes, stream);
+}
+
+static int32_t p_sample_ragged_rng_impl(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
+                                        uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out,
+                                        float* hist, void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
   DITTO_REQUIRE(e && x && t && rng && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_ragged_rng: null argument");
   DITTO_REQUIRE(e->finalized && e->have_schedule && !e->blocks_only, DITTO_E_STATE, "p_sample_ragged_rng: engine not finalized / schedule not loaded");
   std::vector<SeqGroup> gs;
@@ -1357,13 +1450,29 @@ int32_t ditto_p_sample_ragged_rng(ditto_engine_t* e, const float* x, const ditto
     const int64_t per = g.T * H;
     const float* ec = eps_scratch + g.row0 * H;
     // element offset = position in the packed latent buffer: every element of the batch draws its own normal
-    DITTO_TRY(launch_cfg_ddpm_update_rng(ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, reinterpret_cast<unsigned long long*>(rng),
-                                         t + g.seq0, g.n, e->coef, e->steps, guidance_scale, x_out + g.xrow0 * H, g.n_x, per, g.xrow0 * H,
-                                         false, fork.stream(static_cast<int>(gi))));
+    DITTO_TRY(launch_update_rng(e, ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, rng, t + g.seq0, g.n, guidance_scale,
+                                x_out + g.xrow0 * H, hist ? hist + g.xrow0 * H : nullptr, g.n_x, per, g.xrow0 * H, false,
+                                fork.stream(static_cast<int>(gi))));
   }
   DITTO_TRY(fork.end());
   if (advance) DITTO_TRY(launch_step_advance(reinterpret_cast<unsigned long long*>(rng), t, n_t, st));
   return 0;
+}
+
+int32_t ditto_p_sample_ragged_rng(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
+                                  uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, void* workspace,
+                                  int64_t workspace_bytes, int32_t advance, void* stream) {
+  return p_sample_ragged_rng_impl(e, x, groups, n_groups, t, rng, guided, guidance_scale, eps_scratch, x_out, nullptr, workspace,
+                                  workspace_bytes, advance, stream);
+}
+
+int32_t ditto_p_sample_ragged_multistep_rng(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
+                                            int64_t* t, uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch,
+                                            float* x_out, float* hist, void* workspace, int64_t workspace_bytes, int32_t advance,
+                                            void* stream) {
+  DITTO_TRY(require_multistep(e, hist, "p_sample_ragged_multistep_rng"));
+  return p_sample_ragged_rng_impl(e, x, groups, n_groups, t, rng, guided, guidance_scale, eps_scratch, x_out, hist, workspace,
+                                  workspace_bytes, advance, stream);
 }
 
 // ---- block-level operators (the reference's component signatures, src/components/DiT.py) -----------------------------

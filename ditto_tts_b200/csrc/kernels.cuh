@@ -64,6 +64,14 @@ int launch_cfg_ddpm_update(const float* eps_c, const float* eps_u, const float* 
 int launch_cfg_ddpm_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t, int64_t n_t,
                                const float* coef, int steps, float w, float* out, int64_t B, int64_t elems_per_seq,
                                int64_t elem_offset, bool advance, cudaStream_t st);
+// multistep (DPM-Solver++(2M)) form: coef [steps, 6] = {c1, c2, c3, c4, d1, d2}; x_out = c1 (x - c2 eps) + c3 z + c4 hist,
+// then hist <- d1 (x - d2 eps); hist [B, elems_per_seq] is read only on rows with c4 != 0
+int launch_cfg_multistep_update(const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
+                                const float* coef, int steps, float w, float* out, float* hist, int64_t B, int64_t elems_per_seq,
+                                cudaStream_t st);
+int launch_cfg_multistep_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t,
+                                    int64_t n_t, const float* coef, int steps, float w, float* out, float* hist, int64_t B,
+                                    int64_t elems_per_seq, int64_t elem_offset, bool advance, cudaStream_t st);
 int launch_step_advance(unsigned long long* rng, int64_t* t, int64_t n_t, cudaStream_t st);
 int launch_randn(const unsigned long long* rng, int64_t elem_offset, float* out, int64_t n, cudaStream_t st);
 int launch_rope_angles(const float* t, const float* pos, float* out, int64_t batch, int T, int heads, int d, cudaStream_t st);

@@ -147,9 +147,16 @@ class RaggedBatch:
                        "ditto_forward_ragged")
         return out
 
-    def p_sample(self, x_packed, t_seq, z_packed, w: float, eps: torch.Tensor, x_out: torch.Tensor, ws=None):
+    def p_sample(self, x_packed, t_seq, z_packed, w: float, eps: torch.Tensor, x_out: torch.Tensor, ws=None, hist=None):
+        """One sampler step; ``hist`` (packed like x): the multistep update (ditto_p_sample_ragged_multistep)."""
         ws = self.workspace() if ws is None else ws
         with torch.cuda.device(self.device):
+            if hist is not None:
+                _lib.check(_lib.load().ditto_p_sample_ragged_multistep(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
+                                                                       _ptr(t_seq), _ptr(z_packed), 1 if self.guided else 0, float(w),
+                                                                       _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(ws), ws.numel(),
+                                                                       _stream()), "ditto_p_sample_ragged_multistep")
+                return
             _lib.check(_lib.load().ditto_p_sample_ragged(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
                                                          _ptr(t_seq), _ptr(z_packed), 1 if self.guided else 0, float(w),
                                                          _ptr(eps), _ptr(x_out), _ptr(ws), ws.numel(), _stream()),
@@ -157,12 +164,14 @@ class RaggedBatch:
 
 
 class RaggedStepGraph:
-    """One sampler iteration over a ragged batch as a CUDA graph (noise draw, forward, CFG + update, t decrement)."""
+    """One sampler iteration over a ragged batch as a CUDA graph (noise draw, forward, CFG + update, t decrement).  With
+    ``multistep`` the update is DPM-Solver++(2M)'s and the graph owns its ``hist`` buffer (packed like x)."""
 
-    def __init__(self, batch: RaggedBatch, w: float, draw_noise: bool):
+    def __init__(self, batch: RaggedBatch, w: float, draw_noise: bool, multistep: bool = False):
         self.batch, self.w, self.draw_noise = batch, w, draw_noise
         dev = batch.device
         self.x = torch.zeros((batch.x_rows, batch.H), dtype=torch.float32, device=dev)
+        self.hist = torch.zeros_like(self.x) if multistep else None
         self.z = None if draw_noise else torch.zeros_like(self.x)
         self.rng = torch.zeros((4,), dtype=torch.int64, device=dev)
         self._ctx_ptrs = [c.data_ptr() for c in batch._ctx]
@@ -185,12 +194,18 @@ class RaggedStepGraph:
         b = self.batch
         if self.draw_noise:   # noise drawn inside the per-group update kernels, bookkeeping in a one-block kernel after them
             with torch.cuda.device(b.device):
+                if self.hist is not None:
+                    _lib.check(_lib.load().ditto_p_sample_ragged_multistep_rng(
+                        b.model.engine(), _ptr(self.x), b.c_groups, len(b.groups), _ptr(self.t), _ptr(self.rng), 1 if b.guided else 0,
+                        float(self.w), _ptr(self.eps), _ptr(self.x), _ptr(self.hist), _ptr(self.ws), self.ws.numel(), 1, _stream()),
+                        "ditto_p_sample_ragged_multistep_rng")
+                    return
                 _lib.check(_lib.load().ditto_p_sample_ragged_rng(b.model.engine(), _ptr(self.x), b.c_groups, len(b.groups), _ptr(self.t),
                                                                  _ptr(self.rng), 1 if b.guided else 0, float(self.w), _ptr(self.eps),
                                                                  _ptr(self.x), _ptr(self.ws), self.ws.numel(), 1, _stream()),
                            "ditto_p_sample_ragged_rng")
             return
-        b.p_sample(self.x, self.t, self.z, self.w, self.eps, self.x, ws=self.ws)
+        b.p_sample(self.x, self.t, self.z, self.w, self.eps, self.x, ws=self.ws, hist=self.hist)
         self.t.sub_(1)
 
     def valid_for(self, batch: "RaggedBatch") -> bool:
@@ -204,6 +219,8 @@ class RaggedStepGraph:
     def reset(self, x_packed: torch.Tensor, t_start: int, seed: Optional[int] = None):
         self.x.copy_(x_packed)
         self.t.fill_(t_start)
+        if self.hist is not None:
+            self.hist.zero_()
         if self.draw_noise:
             if seed is None:
                 seed = int(torch.randint(0, 2 ** 62, (1,)).item())

@@ -6,6 +6,8 @@ argument meaning -- plus the classifier-free-guidance extension BASELINE.json as
 (eps = eps_u + w (eps_c - eps_u), unconditional branch = zero text embedding unless supplied).
 One sampler iteration is a single C-ABI call (ditto_p_sample): the 2B-sequence forward and the fused
 CFG-combine + update kernel; the text K/V and modulation vectors are built once per utterance batch.
+``method="dpmpp_2m"`` (DPM-Solver++(2M), schedules.dpmpp_2m_coef) also carries the previous step's x0 prediction in a
+device buffer ``hist`` that the update kernel reads and rewrites (ditto_p_sample_multistep).
 """
 from __future__ import annotations
 
@@ -29,7 +31,8 @@ class StepGraph:
     supplied by the caller that same kernel draws it (Philox, ``ditto_p_sample_rng``) and, as its last act, decrements
     the device-resident step index ``t`` and bumps the draw counter -- so the host issues ONE launch per denoising step
     instead of ~70 and the graph contains kernels of libditto_b200 only.  All buffers the graph touches are owned here
-    (or pinned by reference) so that the captured pointers stay valid."""
+    (or pinned by reference) so that the captured pointers stay valid.  A multistep sampler's graph also owns ``hist``, the
+    x0 prediction one step carries to the next (zero-filled by ``reset``)."""
 
     def __init__(self, sampler: "DiTTOSampler", B: int, T: int, S: int, guided: bool, w: float, ctx: torch.Tensor,
                  draw_noise: bool, device):
@@ -41,6 +44,7 @@ class StepGraph:
         # caller-supplied noise lands here; drawn noise never touches HBM
         self.z = None if draw_noise else torch.zeros((B, T, H), dtype=torch.float32, device=device)
         self.rng = torch.zeros((4,), dtype=torch.int64, device=device)   # {seed, draw counter, ticket, -} of ditto_p_sample_rng
+        self.hist = torch.zeros((B, T, H), dtype=torch.float32, device=device) if sampler.multistep else None
         self.eps = torch.empty((n, T, H), dtype=torch.float32, device=device)
         self.t = torch.zeros((n,), dtype=torch.int64, device=device)
         self.ctx = ctx
@@ -64,13 +68,21 @@ class StepGraph:
     def _step(self, sampler):
         if self.draw_noise:   # drawn every step incl. t = 0, like the reference's randn_like (SpeechGenerator.py:145)
             m = self._sampler_model
+            lib = _lib.load()
             with torch.cuda.device(self.x.device):
-                _lib.check(_lib.load().ditto_p_sample_rng(m.engine(), _ptr(self.x), _ptr(self.ctx), _ptr(self.t), _ptr(self.rng),
-                                                          1 if self.guided else 0, float(self.w), self.B, self.T, self.S,
-                                                          _ptr(self.eps), _ptr(self.x), _ptr(self.ws), self.ws.numel(), 1, _stream()),
+                if self.hist is not None:
+                    _lib.check(lib.ditto_p_sample_multistep_rng(m.engine(), _ptr(self.x), _ptr(self.ctx), _ptr(self.t), _ptr(self.rng),
+                                                                1 if self.guided else 0, float(self.w), self.B, self.T, self.S,
+                                                                _ptr(self.eps), _ptr(self.x), _ptr(self.hist), _ptr(self.ws),
+                                                                self.ws.numel(), 1, _stream()), "ditto_p_sample_multistep_rng")
+                    return
+                _lib.check(lib.ditto_p_sample_rng(m.engine(), _ptr(self.x), _ptr(self.ctx), _ptr(self.t), _ptr(self.rng),
+                                                  1 if self.guided else 0, float(self.w), self.B, self.T, self.S,
+                                                  _ptr(self.eps), _ptr(self.x), _ptr(self.ws), self.ws.numel(), 1, _stream()),
                            "ditto_p_sample_rng")
             return
-        sampler._p_sample_raw(self.x, self.ctx, self.t, self.z, self.guided, self.w, self.S, self.eps, self.x, ws=self.ws)
+        sampler._p_sample_raw(self.x, self.ctx, self.t, self.z, self.guided, self.w, self.S, self.eps, self.x, ws=self.ws,
+                              hist=self.hist)
         self.t.sub_(1)
 
     def valid_for(self, ctx: torch.Tensor, ws: torch.Tensor) -> bool:
@@ -79,6 +91,8 @@ class StepGraph:
     def reset(self, x_init: torch.Tensor, t_start: int, seed: Optional[int] = None):
         self.x.copy_(x_init)
         self.t.fill_(t_start)
+        if self.hist is not None:
+            self.hist.zero_()
         if self.draw_noise:   # fresh seed per sampling job (from torch's CPU generator: torch.manual_seed makes runs repeatable)
             if seed is None:
                 seed = int(torch.randint(0, 2 ** 62, (1,)).item())
@@ -90,12 +104,14 @@ class StepGraph:
 
 class DiTTOSampler:
     """``method`` / ``num_steps`` / ``eta`` / ``schedule_scale`` select the sampler variants of SURVEY.md 8f row 4
-    (schedules.py); the defaults are the reference's sampler: DDPM over every timestep of the cosine schedule."""
+    (schedules.py); the defaults are the reference's sampler: DDPM over every timestep of the cosine schedule.
+    ``method="dpmpp_2m"`` is the second-order multistep DPM-Solver++(2M) (eta = 0) or its SDE variant (eta = 1), e.g.
+    ``DiTTOSampler(model, 5.0, method="dpmpp_2m", num_steps=16)``; it has state across steps, so ``p_sample`` refuses it."""
 
     def __init__(self, model: DiTTO, guidance_scale: Optional[float] = None, *, method: str = "ddpm",
                  num_steps: Optional[int] = None, eta: float = 0.0, schedule_scale: Optional[float] = None):
-        if method not in ("ddpm", "ddim"):
-            raise ValueError("method must be 'ddpm' or 'ddim'")
+        if method not in ("ddpm", "ddim", "dpmpp_2m"):
+            raise ValueError("method must be 'ddpm', 'ddim' or 'dpmpp_2m'")
         self.model = model
         self.guidance_scale = guidance_scale
         self.method, self.eta, self.schedule_scale = method, float(eta), schedule_scale
@@ -108,13 +124,17 @@ class DiTTOSampler:
         self.num_steps = steps if num_steps is None else int(num_steps)
         # model timesteps visited, descending (the reference: reversed(range(DIFFUSION_STEPS)), SpeechGenerator.py:161)
         self.timesteps = schedules.spaced_timesteps(steps, self.num_steps)
-        self.update_table = None
-        if method == "ddim" or self.num_steps != steps:
-            acp64 = torch.cumprod(1.0 - self.betas.to(torch.float64), dim=0)
-            taus = self.timesteps.tolist()
+        self.update_table = None        # [steps, 3] DDPM-form table (ditto_engine_load_update_table)
+        self.multistep_table = None     # [steps, 6] multistep table (ditto_engine_load_multistep_table)
+        self.multistep = method == "dpmpp_2m"
+        acp64 = torch.cumprod(1.0 - self.betas.to(torch.float64), dim=0)
+        taus = self.timesteps.tolist()
+        if self.multistep:
+            self.multistep_table = schedules.coef_table(steps, taus, schedules.dpmpp_2m_coef(acp64, taus, eta))
+        elif method == "ddim" or self.num_steps != steps:
             coef = schedules.ddim_coef(acp64, taus, eta) if method == "ddim" else schedules.ddpm_coef(acp64, taus)
             self.update_table = schedules.coef_table(steps, taus, coef)
-        self._variant = self.update_table is not None or schedule_scale is not None
+        self._variant = self.update_table is not None or self.multistep or schedule_scale is not None
         self._tau_dev = None
         # captured step graphs pin x / eps / a private memory pool (hundreds of MB at B = 16, T = 750) and TTS serving sees a
         # new predicted length on almost every request: keep the few most recently used shapes only
@@ -132,6 +152,8 @@ class DiTTOSampler:
         m.load_schedule(self.betas, self.alphas, self.alphas_cumprod, owner=owner)
         if self.update_table is not None:
             m.load_update_table(self.update_table)
+        if self.multistep_table is not None:
+            m.load_multistep_table(self.multistep_table)
         m._schedule_engine = m._engine
 
     def _taus(self, device):
@@ -149,13 +171,18 @@ class DiTTOSampler:
             text_emb = torch.cat([text_emb, null], dim=0)  # [cond(B); uncond(B)]
         return self.model.text_context(text_emb, name="sampler_ctx", T_hint=T)
 
-    def _p_sample_raw(self, x, ctx, t_n, z, guided, w, S, eps, x_out, ws=None):
+    def _p_sample_raw(self, x, ctx, t_n, z, guided, w, S, eps, x_out, ws=None, hist=None):
         m = self.model
         B, T, H = x.shape
         n = 2 * B if guided else B
         with torch.cuda.device(x.device):
             if ws is None:
                 ws = m.workspace(n, T, S)
+            if hist is not None:
+                _lib.check(_lib.load().ditto_p_sample_multistep(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), 1 if guided else 0,
+                                                                float(w), B, T, S, _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(ws),
+                                                                ws.numel(), _stream()), "ditto_p_sample_multistep")
+                return
             _lib.check(_lib.load().ditto_p_sample(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), 1 if guided else 0,
                                                   float(w), B, T, S, _ptr(eps), _ptr(x_out), _ptr(ws), ws.numel(),
                                                   _stream()), "ditto_p_sample")
@@ -179,7 +206,11 @@ class DiTTOSampler:
     @torch.no_grad()
     def p_sample(self, x, t, text_emb, noise=None, guidance_scale=None, null_text_emb=None):
         """One reverse step (reference: __p_sample, SpeechGenerator.py:131-147).  ``noise`` replaces the
-        reference's in-place ``torch.randn_like(x)``; when omitted it is drawn the same way."""
+        reference's in-place ``torch.randn_like(x)``; when omitted it is drawn the same way.  Not for ``dpmpp_2m``: its
+        update needs the previous step's x0 prediction, which only sample_latents(_ragged) carries from step to step."""
+        if self.multistep:
+            raise DittoError("p_sample: method 'dpmpp_2m' is a multistep solver and has state across steps; "
+                             "use sample_latents / sample_latents_ragged")
         w = self.guidance_scale if guidance_scale is None else guidance_scale
         guided = w is not None
         x = _need_cuda_f32("x", x)
@@ -255,6 +286,7 @@ class DiTTOSampler:
         eps = torch.empty((n, T, H), dtype=torch.float32, device=dev)
         x_next = torch.empty_like(x)
         z_buf = None if noise is not None else torch.empty_like(x)
+        hist = torch.empty_like(x) if self.multistep else None   # first step is first order: never read before written
         for i, t_val in enumerate(taus):
             if noise is not None:
                 z = noise[t_val]
@@ -263,7 +295,7 @@ class DiTTOSampler:
                 z = z.contiguous()
             else:
                 z = z_buf.normal_(generator=generator)  # drawn every step incl. t = 0, as the reference does
-            self._p_sample_raw(x, ctx, t_all[i], z, guided, w if guided else 0.0, S, eps, x_next)
+            self._p_sample_raw(x, ctx, t_all[i], z, guided, w if guided else 0.0, S, eps, x_next, hist=hist)
             if record is not None:
                 record.append((eps[B:] + w * (eps[:B] - eps[B:])).clone() if guided else eps.clone())
             x, x_next = x_next, x
@@ -305,7 +337,7 @@ class DiTTOSampler:
             wv, draw = (w if guided else 0.0), zs is None
             g = cached[1].get((float(wv), draw)) if cached is not None else None
             if g is None or not g.valid_for(rb):
-                g = RaggedStepGraph(rb, wv, draw)
+                g = RaggedStepGraph(rb, wv, draw, multistep=self.multistep)
                 if cached is None:
                     while len(self._ragged_graphs) >= self.max_cached_graphs:
                         self._ragged_graphs.popitem(last=False)
@@ -326,10 +358,11 @@ class DiTTOSampler:
         eps = torch.empty((rb.seq_rows, H), dtype=torch.float32, device=dev)
         x_next = torch.empty_like(x)
         z_buf = torch.empty_like(x)
+        hist = torch.empty_like(x) if self.multistep else None
         for t_val in taus:
             t_seq = torch.full((rb.n_seq,), t_val, dtype=torch.int64, device=dev)
             z = zs[t_val] if zs is not None else z_buf.normal_()
-            rb.p_sample(x, t_seq, z, w if guided else 0.0, eps, x_next)
+            rb.p_sample(x, t_seq, z, w if guided else 0.0, eps, x_next, hist=hist)
             if record is not None:
                 record.append(rb.unpack_eps(eps, w))
             x, x_next = x_next, x

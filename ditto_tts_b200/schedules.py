@@ -17,7 +17,10 @@ CFG scale 5.0, noise-schedule scale-shift 0.3, PDF p.25 Fig. 6):
   * ``ddpm_coef``             -- ancestral sampling (sigma^2 = beta', the reference's choice) over a sub-sequence;
                                  over *all* timesteps it reproduces the reference's table;
   * ``ddim_coef``             -- DDIM with stochasticity eta (eta = 0: deterministic);
-  * ``shifted_cosine_betas``  -- the cosine schedule with its SNR multiplied by scale^2 (logSNR shift 2 log scale).
+  * ``shifted_cosine_betas``  -- the cosine schedule with its SNR multiplied by scale^2 (logSNR shift 2 log scale);
+  * ``dpmpp_2m_coef``         -- DPM-Solver++(2M) (Lu et al. 2022, "DPM-Solver++", Alg. 2) and its SDE variant: a second-order
+                                 multistep update that also carries the previous step's x0 prediction (a [diffusion_steps, 6]
+                                 table for ``ditto_engine_load_multistep_table``).
 """
 from __future__ import annotations
 
@@ -25,7 +28,7 @@ from typing import Sequence
 
 import torch
 
-__all__ = ["spaced_timesteps", "ddpm_coef", "ddim_coef", "shifted_cosine_betas", "coef_table"]
+__all__ = ["spaced_timesteps", "ddpm_coef", "ddim_coef", "dpmpp_2m_coef", "shifted_cosine_betas", "coef_table"]
 
 
 def spaced_timesteps(train_steps: int, num_steps: int) -> torch.Tensor:
@@ -75,6 +78,52 @@ def ddim_coef(alphas_cumprod: torch.Tensor, taus: Sequence[int], eta: float = 0.
     return torch.stack([c1, c2, sigma], dim=1)
 
 
+def dpmpp_2m_coef(alphas_cumprod: torch.Tensor, taus: Sequence[int], eta: float = 0.0) -> torch.Tensor:
+    """DPM-Solver++(2M) over the visited timesteps tau_0 > ... > tau_{K-1}, with stochasticity eta in [0, 1] (0: the ODE
+    solver of Lu et al. 2022, Alg. 2; 1: the "midpoint" 2M-SDE, rewritten for the VP process).  With
+    alpha_i = sqrt(abar_{tau_i}), sigma_i = sqrt(1 - abar_{tau_i}), abar_K = 1, lambda_i = log(alpha_i / sigma_i),
+    h_i = lambda_{i+1} - lambda_i, the step is
+
+        x0_i    = (x_i - sigma_i eps_i) / alpha_i
+        D_i     = x0_i                                        i == 0 or i == K-1 (first order)
+                = x0_i + (x0_i - x0_{i-1}) / (2 r_i),         r_i = h_{i-1} / h_i, otherwise
+        x_{i+1} = (sigma_{i+1}/sigma_i) e^{-eta h_i} x_i + alpha_{i+1} (1 - e^{-(1+eta) h_i}) D_i
+                  + sigma_{i+1} sqrt(1 - e^{-2 eta h_i}) z
+
+    and the last one returns x0_{K-1} without noise.  Rewritten for the device kernel as
+
+        x_out = c1 (x - c2 eps) + c3 z + c4 hist,     hist <- d1 (x - d2 eps)   (= x0_i, read by the next step)
+
+    with k = 1/(2 r_i) (0 on first-order steps), phi = alpha_{i+1} (1 - e^{-(1+eta) h}), rho = (sigma_{i+1}/sigma_i) e^{-eta h}:
+    c1 = rho + phi (1+k) / alpha_i, c2 = phi (1+k) sigma_i / (alpha_i c1), c3 = sigma_{i+1} sqrt(1 - e^{-2 eta h}),
+    c4 = -phi k, d1 = 1/alpha_i, d2 = sigma_i.  The first and last rows have c4 = 0; the last row equals DDIM's.  A
+    first-order step equals ``ddim_coef`` at eta = 0 and eta = 1; for 0 < eta < 1 the two families inject noise
+    differently (DDIM's eta scales its sigma_t, this one the exponent) and are different samplers.
+    Returns float64 [len(taus), 6]."""
+    eta = float(eta)
+    if not 0.0 <= eta <= 1.0:
+        raise ValueError("dpmpp_2m_coef: eta must be in [0, 1]")
+    taus, a_t, a_p = _acp_pairs(alphas_cumprod, taus)
+    al, sg = a_t.sqrt(), (1.0 - a_t).sqrt()
+    out = torch.zeros((len(taus), 6), dtype=torch.float64)
+    out[:, 4], out[:, 5] = 1.0 / al, sg
+    out[-1, 0], out[-1, 1] = (a_p[-1] / a_t[-1]).sqrt(), sg[-1]      # x_K = x0_{K-1}: DDIM's last row
+    if len(taus) > 1:
+        a, s, a1, s1 = al[:-1], sg[:-1], a_p[:-1].sqrt(), (1.0 - a_p[:-1]).sqrt()
+        lam = (al / sg).log()
+        h = lam[1:] - lam[:-1]                                           # h_i, i < K-1
+        k = torch.zeros_like(h)
+        k[1:] = h[1:] / (2.0 * h[:-1])                                   # 1 / (2 r_i) on the second-order steps
+        phi = a1 * -torch.expm1(-(1.0 + eta) * h)
+        rho = s1 / s * torch.exp(-eta * h)
+        c1 = rho + phi * (1.0 + k) / a
+        out[:-1, 0] = c1
+        out[:-1, 1] = phi * (1.0 + k) * s / (a * c1)
+        out[:-1, 2] = s1 * (-torch.expm1(-2.0 * eta * h)).sqrt()
+        out[:-1, 3] = -phi * k
+    return out
+
+
 def shifted_cosine_betas(timesteps: int, scale: float, s: float = 0.008) -> torch.Tensor:
     """DiTTO.cosine_beta_schedule (DiTTO.py:96-104) with the signal-to-noise ratio of every level multiplied by scale^2
     (abar' = scale^2 abar / (scale^2 abar + 1 - abar)); scale = 1 returns the reference's betas (same clip)."""
@@ -88,8 +137,13 @@ def shifted_cosine_betas(timesteps: int, scale: float, s: float = 0.008) -> torc
 
 
 def coef_table(diffusion_steps: int, taus: Sequence[int], coef: torch.Tensor) -> torch.Tensor:
-    """Scatter per-visited-step rows into the engine's [diffusion_steps, 3] fp32 table (unvisited rows: identity)."""
-    tab = torch.zeros((diffusion_steps, 3), dtype=torch.float32)
+    """Scatter per-visited-step rows into the engine's [diffusion_steps, 3] fp32 table, or its [diffusion_steps, 6] multistep
+    table for 6-column rows (unvisited rows: identity, c1 = d1 = 1)."""
+    if coef.dim() != 2 or coef.shape[1] not in (3, 6):
+        raise ValueError("coef_table: rows must have 3 or 6 columns")
+    tab = torch.zeros((diffusion_steps, coef.shape[1]), dtype=torch.float32)
     tab[:, 0] = 1.0
+    if coef.shape[1] == 6:
+        tab[:, 4] = 1.0
     tab[torch.as_tensor([int(t) for t in taus])] = coef.to(torch.float32)
     return tab

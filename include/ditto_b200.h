@@ -111,6 +111,13 @@ int32_t ditto_engine_load_schedule(ditto_engine_t* e, const float* betas, const 
  * also expresses DDIM(eta) and DDPM over a strided sub-sequence of timesteps (rows that are never visited may hold
  * anything).  The host computes the rows (ditto_tts_b200/schedules.py); load_schedule restores the reference's table. */
 int32_t ditto_engine_load_update_table(ditto_engine_t* e, const float* coef, int64_t steps, void* stream);
+/* Multistep sampler (DPM-Solver++(2M), Lu et al. 2022 Alg. 2; eta > 0: its SDE variant).  coef6 [diffusion_steps, 6] fp32
+ * (device), row t = {c1, c2, c3, c4, d1, d2} of
+ *     x_out = c1 (x - c2 eps) + c3 z + c4 hist        hist <- d1 (x - d2 eps)   (= the x0 prediction of the step)
+ * where hist carries the previous step's x0 prediction across steps (and CUDA-graph replays).  Rows with c4 == 0 (first-
+ * order steps) do not read hist.  Held in its own engine buffer, next to the DDPM-form table, until replaced; the host
+ * computes it (schedules.dpmpp_2m_coef).  DITTO_E_STATE without a loaded schedule, DITTO_E_BADARG if steps != diffusion_steps. */
+int32_t ditto_engine_load_multistep_table(ditto_engine_t* e, const float* coef6, int64_t steps, void* stream);
 /* Pack weights (bf16 copies, interleaved [fc1;gate], permuted QKV), build the per-step modulation table
  * time_mlp(SiLU(time_embed(t_embedding))) [steps, 2H] (DiTTO.py:75-76 + DiT.py:30) and the RoPE cos/sin
  * tables (DiT.py:46-59).  Synchronises the stream. */
@@ -167,6 +174,25 @@ int32_t ditto_cfg_ddpm_update_rng(ditto_engine_t* e, const float* eps_c, const f
  * (elem_offset % 4 == 0, out 16-B aligned): stand-alone randn on the library's stream of numbers; parity tests. */
 int32_t ditto_randn(const uint64_t* rng, int64_t elem_offset, float* out, int64_t n, void* stream);
 
+/* Multistep forms of the four calls above: the same arguments plus hist [B, T, H] (ragged: packed like x, [sum n_x*T, H]),
+ * read on second-order rows and overwritten with this step's x0 prediction; the update reads ditto_engine_load_multistep_table's
+ * table (DITTO_E_STATE before one was loaded).  One launch per step, like their DDPM-form twins; x_out may alias x.  A row
+ * with c4 == 0 gives x_out bit-identical to ditto_cfg_ddpm_update(_rng) with (c1, c2, c3). */
+int32_t ditto_cfg_multistep_update(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x,
+                                   const float* z, const int64_t* t, float guidance_scale, float* x_out, float* hist,
+                                   int64_t B, int64_t elems_per_seq, void* stream);
+int32_t ditto_cfg_multistep_update_rng(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, uint64_t* rng,
+                                       int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist, int64_t B,
+                                       int64_t elems_per_seq, int32_t advance, void* stream);
+int32_t ditto_p_sample_multistep(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z,
+                                 int32_t guided, float guidance_scale, int64_t B, int64_t T, int64_t S,
+                                 float* eps_scratch, float* x_out, float* hist, void* workspace, int64_t workspace_bytes,
+                                 void* stream);
+int32_t ditto_p_sample_multistep_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng,
+                                     int32_t guided, float guidance_scale, int64_t B, int64_t T, int64_t S,
+                                     float* eps_scratch, float* x_out, float* hist, void* workspace,
+                                     int64_t workspace_bytes, int32_t advance, void* stream);
+
 /* DiTTO.q_sample (DiTTO.py:106-126) with the reference's betas-as-alphas_cumprod buffer. */
 int32_t ditto_q_sample(ditto_engine_t* e, const float* x_start, const float* noise, const int64_t* t,
                        float* out, int64_t B, int64_t elems_per_seq, void* stream);
@@ -199,6 +225,15 @@ int32_t ditto_p_sample_ragged(ditto_engine_t* e, const float* x, const ditto_seq
 int32_t ditto_p_sample_ragged_rng(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
                                   int64_t* t, uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch,
                                   float* x_out, void* workspace, int64_t workspace_bytes, int32_t advance, void* stream);
+/* Multistep forms of the two ragged calls (hist packed like x; each group's update runs on its fork stream). */
+int32_t ditto_p_sample_ragged_multistep(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
+                                        const int64_t* t, const float* z, int32_t guided, float guidance_scale,
+                                        float* eps_scratch, float* x_out, float* hist, void* workspace,
+                                        int64_t workspace_bytes, void* stream);
+int32_t ditto_p_sample_ragged_multistep_rng(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
+                                            int64_t* t, uint64_t* rng, int32_t guided, float guidance_scale,
+                                            float* eps_scratch, float* x_out, float* hist, void* workspace,
+                                            int64_t workspace_bytes, int32_t advance, void* stream);
 
 /* ---- block-level operators: the component signatures of src/components/DiT.py ------------------------------- */
 /* DiT.forward(x, text_emb, time_emb, rotary_pos) (DiT.py:100-157) for block `layer` of the engine: x [n_seq, T, H] -> out
