@@ -49,6 +49,7 @@ SIGNATURES = {
     "ditto_engine_load_schedule": (_I32, [_P, _P, _P, _P, _I64, _P]),
     "ditto_engine_load_update_table": (_I32, [_P, _P, _I64, _P]),
     "ditto_engine_load_multistep_table": (_I32, [_P, _P, _I64, _P]),
+    "ditto_engine_load_known_table": (_I32, [_P, _P, _I64, _P]),
     "ditto_engine_finalize": (_I32, [_P, _P]),
     "ditto_text_context_bytes": (_I64, [_P, _I64, _I64]),
     "ditto_workspace_bytes": (_I64, [_P, _I64, _I64, _I64]),
@@ -63,6 +64,8 @@ SIGNATURES = {
     "ditto_cfg_multistep_update_rng": (_I32, [_P, _P, _P, _P, _P, _P, _I64, _F, _P, _P, _I64, _I64, _I32, _P]),
     "ditto_p_sample_multistep": (_I32, [_P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _P]),
     "ditto_p_sample_multistep_rng": (_I32, [_P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _I32, _P]),
+    "ditto_cfg_update_known": (_I32, [_P, _P, _P, _P, _P, _P, _P, _I64, _F, _P, _P, _P, _P, _I64, _I64, _I32, _P]),
+    "ditto_p_sample_known": (_I32, [_P, _P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _P, _P, _P, _I64, _I32, _P]),
     "ditto_q_sample": (_I32, [_P, _P, _P, _P, _P, _I64, _I64, _P]),
     "ditto_workspace_bytes_ragged": (_I64, [_P, C.POINTER(SeqGroup), _I64]),
     "ditto_forward_ragged": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _P, _I64, _P]),
@@ -71,6 +74,8 @@ SIGNATURES = {
     "ditto_p_sample_ragged_multistep": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _I32, _F, _P, _P, _P, _P, _I64, _P]),
     "ditto_p_sample_ragged_multistep_rng": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _I32, _F, _P, _P, _P, _P, _I64, _I32,
                                                    _P]),
+    "ditto_p_sample_ragged_known": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _P, _I32, _F, _P, _P, _P, _P, _P, _P, _I64,
+                                           _I32, _P]),
     "ditto_dit_block": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),
     "ditto_attn_self": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),
     "ditto_attn_cross": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),

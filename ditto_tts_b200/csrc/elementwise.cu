@@ -1,5 +1,7 @@
 // HBM-bound kernels of the DiT denoiser hot path: LayerNorm / AdaLN, RoPE, softmax, gated activation,
 // CFG-combine + DDPM update, q_sample, casts and weight packing.  All coalesced + 128-bit vectorised.
+#include <vector>
+
 #include "kernels.cuh"
 
 namespace ditto {
@@ -861,6 +863,128 @@ int launch_cfg_multistep_update_rng(const float* eps_c, const float* eps_u, cons
       reinterpret_cast<const float4*>(eps_c), reinterpret_cast<const float4*>(eps_u), reinterpret_cast<const float4*>(x), rng, t,
       n_t, coef, steps, w, reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(hist), elems_per_seq / 4, total_vec,
       elem_offset / 4, advance ? 1 : 0);
+  DITTO_LAUNCH_CHECK();
+  return 0;
+}
+
+// =====================================================================================================
+// CFG combine + update with known frames (replacement conditioning: a speech prompt or an infilled span; the imputation
+// of Song et al. 2021, score SDE, i.e. RePaint without its resampling loop), one pass.  A frame flagged in `mask` is
+// the known latent p re-noised to the level of this step's output,
+//     x_out = a p + s z,   coef_known[t] = {a, s} = {sqrt(abar_next), sqrt(1 - abar_next)}   (last visited step: {1, 0} -> p)
+// with z the normal the update draws (or is given) for that element, so the draw counter and its bookkeeping are those of
+// the plain update.  Every other frame takes the DDPM-form (MULTISTEP = false) or multistep update through the same device
+// helpers as cfg_ddpm_update(_rng)_kernel / cfg_multistep_update(_rng)_kernel, so it rounds exactly as they do.  A frame is
+// H/4 consecutive float4s (6 warps at H = 768), so the branch is uniform per warp when H % 128 == 0.  A known frame reads
+// the mask byte, p and (supplied noise) z -- no eps, x or hist -- and leaves hist as it was: 8 B / element with drawn noise
+// (12 with supplied z) against 16-28 B for an unknown one.  All loads are issued before the noise is drawn.
+// =====================================================================================================
+__device__ __forceinline__ float known_value(float p, float z, float a, float s) { return __fmaf_rn(s, z, __fmul_rn(a, p)); }
+
+template <bool MULTISTEP, bool RNG>
+__global__ void __launch_bounds__(256)
+    cfg_update_known_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
+                            const float4* __restrict__ z, unsigned long long* rng, int64_t* t, int64_t n_t,
+                            const float* __restrict__ coef, const float* __restrict__ coef_known, int steps, float w,
+                            float4* __restrict__ out, float4* __restrict__ hist, const float4* __restrict__ known,
+                            const uint8_t* __restrict__ mask, int64_t vec_per_seq, int64_t vec_per_frame, int64_t total_vec,
+                            int64_t vec_offset, int advance) {
+  unsigned long long seed = 0ull, draw = 0ull;
+  if (RNG) {
+    seed = rng[0];
+    draw = rng[1];
+  }
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int64_t seq = i / vec_per_seq;
+    if (mask[i / vec_per_frame] != 0) {
+      int64_t tt = t[seq];
+      tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
+      const float a = coef_known[tt * 2 + 0], s = coef_known[tt * 2 + 1];
+      const float4 pv = known[i];
+      const float4 zv = RNG ? philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i)) : z[i];
+      out[i] = make_float4(known_value(pv.x, zv.x, a, s), known_value(pv.y, zv.y, a, s), known_value(pv.z, zv.z, a, s),
+                           known_value(pv.w, zv.w, a, s));
+      continue;
+    }
+    if (MULTISTEP) {
+      const MultistepRow c = multistep_row(coef, t, seq, steps);
+      float4 e = eps_c[i];
+      if (eps_u != nullptr) {
+        const float4 u = eps_u[i];
+        e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
+      }
+      const float4 xv = x[i];
+      float4 zv = RNG ? make_float4(0.f, 0.f, 0.f, 0.f) : z[i];
+      const float4 h = multistep_hist(hist, i, c.c4);
+      if (RNG) zv = philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i));
+      multistep_store(c, xv, e, zv, h, out, hist, i);
+    } else {
+      int64_t tt = t[seq];
+      tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
+      const float c1 = coef[tt * 3 + 0], c2 = coef[tt * 3 + 1], c3 = coef[tt * 3 + 2];
+      float4 e = eps_c[i];
+      if (eps_u != nullptr) {
+        const float4 u = eps_u[i];
+        e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
+      }
+      const float4 xv = x[i];
+      const float4 zv = RNG ? philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i)) : z[i];
+      out[i] = make_float4(ddpm_update(xv.x, e.x, zv.x, c1, c2, c3), ddpm_update(xv.y, e.y, zv.y, c1, c2, c3),
+                           ddpm_update(xv.z, e.z, zv.z, c1, c2, c3), ddpm_update(xv.w, e.w, zv.w, c1, c2, c3));
+    }
+  }
+  if (RNG && advance) last_block_advances(rng, t, n_t, draw);
+}
+
+// known frames of mask[0, n) for the profiler's byte count; only while profiling (which synchronises anyway and is never
+// captured), so a step graph never sees the copy
+static int64_t profiled_known_frames(const uint8_t* mask, int64_t n, cudaStream_t st) {
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if (!g_prof_enabled || cudaStreamIsCapturing(st, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) return 0;
+  std::vector<uint8_t> h(static_cast<size_t>(n));
+  if (cudaMemcpyAsync(h.data(), mask, static_cast<size_t>(n), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+      cudaStreamSynchronize(st) != cudaSuccess)
+    return 0;
+  int64_t k = 0;
+  for (uint8_t v : h) k += v != 0;
+  return k;
+}
+
+int launch_cfg_update_known(const float* eps_c, const float* eps_u, const float* x, const float* z, unsigned long long* rng, int64_t* t,
+                            int64_t n_t, const float* coef, const float* coef_known, int steps, float w, float* out, float* hist,
+                            const float* known, const uint8_t* mask, int64_t B, int64_t T, int64_t H, int64_t elem_offset, bool advance,
+                            cudaStream_t st) {
+  DITTO_REQUIRE(H % 4 == 0 && elem_offset % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_update_known: H % 4 and element offset % 4");
+  const bool draw = rng != nullptr, ms = hist != nullptr;
+  const int64_t vec_per_frame = H / 4, total_vec = B * T * vec_per_frame;
+  if (total_vec == 0) return (draw && advance) ? launch_step_advance(rng, t, n_t, st) : 0;
+  const int64_t want = ceil_div(total_vec, 256 * 4);
+  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
+  // bytes moved: 16 B per float4 of every stream a frame touches, plus one mask byte per frame
+  const int64_t known_vec = profiled_known_frames(mask, B * T, st) * vec_per_frame;
+  const double unknown_streams = (ms ? 5 : 3) + (eps_u ? 1 : 0) + (draw ? 0 : 1), known_streams = 2 + (draw ? 0 : 1);
+  ProfScope prof(PC_CFG_UPDATE, st, 0.0,
+                 16.0 * (static_cast<double>(total_vec - known_vec) * unknown_streams + static_cast<double>(known_vec) * known_streams) +
+                     static_cast<double>(B * T));
+  const float4 *ec = reinterpret_cast<const float4*>(eps_c), *eu = reinterpret_cast<const float4*>(eps_u);
+  const float4 *xv = reinterpret_cast<const float4*>(x), *zv = reinterpret_cast<const float4*>(z);
+  const float4* kv = reinterpret_cast<const float4*>(known);
+  float4 *o = reinterpret_cast<float4*>(out), *h = reinterpret_cast<float4*>(hist);
+  const int64_t vps = T * vec_per_frame, voff = elem_offset / 4;
+  const int adv = advance ? 1 : 0;
+  if (ms && draw)
+    cfg_update_known_kernel<true, true><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv, mask,
+                                                                vps, vec_per_frame, total_vec, voff, adv);
+  else if (ms)
+    cfg_update_known_kernel<true, false><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv, mask,
+                                                                 vps, vec_per_frame, total_vec, voff, adv);
+  else if (draw)
+    cfg_update_known_kernel<false, true><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv, mask,
+                                                                 vps, vec_per_frame, total_vec, voff, adv);
+  else
+    cfg_update_known_kernel<false, false><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv,
+                                                                  mask, vps, vec_per_frame, total_vec, voff, adv);
   DITTO_LAUNCH_CHECK();
   return 0;
 }

@@ -108,6 +108,7 @@ struct ditto_engine {
   std::vector<void*> owned;                 // everything else cudaMalloc'ed by the engine
   float *time_table = nullptr, *rope_cos = nullptr, *rope_sin = nullptr, *rope_freq = nullptr, *coef = nullptr, *qs_buf = nullptr;
   float* coef_ms = nullptr;  // [steps, 6] multistep update table (ditto_engine_load_multistep_table); null until loaded
+  float* coef_known = nullptr;  // [steps, 2] re-noising table of known frames (ditto_engine_load_known_table); null until loaded
   bf16 *w_in16 = nullptr, *w_out16 = nullptr;
   bf16* w_out_p4 = nullptr;   // proj_out rows in the perm4 order of gemm_resid_ln.cu (fc2_ln engines)
   std::vector<LayerPack> layers;
@@ -969,6 +970,15 @@ int32_t ditto_engine_load_multistep_table(ditto_engine_t* e, const float* coef6,
   return 0;
 }
 
+int32_t ditto_engine_load_known_table(ditto_engine_t* e, const float* coef2, int64_t steps, void* stream) {
+  DITTO_REQUIRE(e && coef2, DITTO_E_BADARG, "load_known_table: null argument");
+  DITTO_REQUIRE(steps == e->steps, DITTO_E_BADARG, "load_known_table: steps != diffusion_steps");
+  DITTO_REQUIRE(e->have_schedule, DITTO_E_STATE, "load_known_table: call ditto_engine_load_schedule first");
+  if (!e->coef_known) DITTO_TRY(dev_alloc(e, reinterpret_cast<void**>(&e->coef_known), sizeof(float) * 2 * steps));
+  DITTO_CUDA(cudaMemcpyAsync(e->coef_known, coef2, sizeof(float) * 2 * steps, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
+  return 0;
+}
+
 int32_t ditto_engine_finalize(ditto_engine_t* e, void* stream) {
   DITTO_REQUIRE(e, DITTO_E_BADARG, "finalize: null engine");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1340,6 +1350,53 @@ int32_t ditto_cfg_multistep_update_rng(ditto_engine_t* e, const float* eps_c, co
                            static_cast<cudaStream_t>(stream));
 }
 
+// ---- known frames (speech prompt / infilling) -----------------------------------------------------------
+// what every known-frame entry point checks before it launches anything
+static int require_known(const ditto_engine* e, const float* z, const uint64_t* rng, const float* hist, const float* known,
+                         const uint8_t* known_mask, int32_t advance, const char* what) {
+  const std::string w(what);
+  DITTO_REQUIRE(e && known && known_mask, DITTO_E_BADARG, w + ": null argument (known / known_mask)");
+  DITTO_REQUIRE((z == nullptr) != (rng == nullptr), DITTO_E_BADARG, w + ": exactly one of z / rng (known frames need the step's noise)");
+  DITTO_REQUIRE(!advance || rng, DITTO_E_BADARG, w + ": advance needs rng (in-kernel noise)");
+  DITTO_REQUIRE(e->have_schedule, DITTO_E_STATE, w + ": schedule not loaded");
+  DITTO_REQUIRE(e->coef_known, DITTO_E_STATE, w + ": no known table loaded (ditto_engine_load_known_table)");
+  DITTO_REQUIRE(!hist || e->coef_ms, DITTO_E_STATE, w + ": no multistep table loaded (ditto_engine_load_multistep_table)");
+  return 0;
+}
+// the update of one step with known frames: the DDPM-form table, or (hist != null) the multistep table
+static int launch_update_known(const ditto_engine* e, const float* eps_c, const float* eps_u, const float* x, const float* z, uint64_t* rng,
+                               int64_t* t, int64_t n_t, float w, float* x_out, float* hist, const float* known, const uint8_t* mask,
+                               int64_t B, int64_t T, int64_t elem_offset, bool advance, cudaStream_t st) {
+  return launch_cfg_update_known(eps_c, eps_u, x, z, reinterpret_cast<unsigned long long*>(rng), t, n_t, hist ? e->coef_ms : e->coef,
+                                 e->coef_known, e->steps, w, x_out, hist, known, mask, B, T, e->H, elem_offset, advance, st);
+}
+
+int32_t ditto_cfg_update_known(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z, uint64_t* rng,
+                               int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist, const float* known,
+                               const uint8_t* known_mask, int64_t B, int64_t T, int32_t advance, void* stream) {
+  DITTO_REQUIRE(e && eps_c && x && t && x_out, DITTO_E_BADARG, "cfg_update_known: null argument");
+  DITTO_REQUIRE(B >= 0 && T >= 0 && (!rng || n_t >= B), DITTO_E_BADARG, "cfg_update_known: bad sizes");
+  DITTO_TRY(require_known(e, z, rng, hist, known, known_mask, advance, "cfg_update_known"));
+  return launch_update_known(e, eps_c, eps_u, x, z, rng, t, n_t, guidance_scale, x_out, hist, known, known_mask, B, T, 0, advance != 0,
+                             static_cast<cudaStream_t>(stream));
+}
+
+int32_t ditto_p_sample_known(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, const float* z, uint64_t* rng, int32_t guided,
+                             float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
+                             const float* known, const uint8_t* known_mask, void* workspace, int64_t workspace_bytes, int32_t advance,
+                             void* stream) {
+  DITTO_REQUIRE(e && x && ctx && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_known: null argument");
+  DITTO_REQUIRE(e->finalized && !e->blocks_only, DITTO_E_STATE, "p_sample_known: engine not finalized");
+  DITTO_REQUIRE(B > 0 && T > 0 && S > 0 && T <= e->maxT, DITTO_E_BADARG, "p_sample_known: bad sizes");
+  DITTO_TRY(require_known(e, z, rng, hist, known, known_mask, advance, "p_sample_known"));
+  const int64_t n = guided ? 2 * B : B;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  DITTO_TRY(forward_impl(e, x, B, ctx, t, n, T, S, eps_scratch, workspace, workspace_bytes, st));
+  const int64_t per = T * e->H;
+  return launch_update_known(e, eps_scratch, guided ? eps_scratch + B * per : nullptr, x, z, rng, t, n, guidance_scale, x_out, hist, known,
+                             known_mask, B, T, 0, advance != 0, st);
+}
+
 int32_t ditto_randn(const uint64_t* rng, int64_t elem_offset, float* out, int64_t n, void* stream) {
   DITTO_REQUIRE(rng && out && n >= 0 && elem_offset >= 0, DITTO_E_BADARG, "randn: bad argument");
   return launch_randn(reinterpret_cast<const unsigned long long*>(rng), elem_offset, out, n, static_cast<cudaStream_t>(stream));
@@ -1473,6 +1530,42 @@ int32_t ditto_p_sample_ragged_multistep_rng(ditto_engine_t* e, const float* x, c
   DITTO_TRY(require_multistep(e, hist, "p_sample_ragged_multistep_rng"));
   return p_sample_ragged_rng_impl(e, x, groups, n_groups, t, rng, guided, guidance_scale, eps_scratch, x_out, hist, workspace,
                                   workspace_bytes, advance, stream);
+}
+
+int32_t ditto_p_sample_ragged_known(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
+                                    const float* z, uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out,
+                                    float* hist, const float* known, const uint8_t* known_mask, void* workspace, int64_t workspace_bytes,
+                                    int32_t advance, void* stream) {
+  DITTO_REQUIRE(e && x && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_ragged_known: null argument");
+  DITTO_REQUIRE(e->finalized && !e->blocks_only, DITTO_E_STATE, "p_sample_ragged_known: engine not finalized");
+  DITTO_TRY(require_known(e, z, rng, hist, known, known_mask, advance, "p_sample_ragged_known"));
+  std::vector<SeqGroup> gs;
+  DITTO_TRY(parse_groups(e, groups, n_groups, true, gs));
+  int64_t n_t = 0;
+  for (const SeqGroup& g : gs) {
+    DITTO_REQUIRE(g.n == (guided ? 2 : 1) * g.n_x, DITTO_E_BADARG, "p_sample_ragged_known: n_seq must be n_x (unguided) or 2 n_x (guided)");
+    n_t += g.n;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  DITTO_TRY(forward_impl(e, x, t, gs.data(), static_cast<int>(gs.size()), eps_scratch, workspace, workspace_bytes, st));
+  const int64_t H = e->H;
+  std::unique_lock<std::recursive_mutex> fork_lock(e->fork_mutex, std::defer_lock);
+  if (gs.size() > 1 && e->n_side > 0) fork_lock.lock();
+  Fork fork(e, st);
+  DITTO_TRY(fork.begin(static_cast<int>(gs.size())));
+  for (size_t gi = 0; gi < gs.size(); ++gi) {
+    const SeqGroup& g = gs[gi];
+    const int64_t per = g.T * H;
+    const float* ec = eps_scratch + g.row0 * H;
+    // x, z, hist, known: packed rows from xrow0; the mask: one byte per packed row; noise offset = packed element position
+    DITTO_TRY(launch_update_known(e, ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, z ? z + g.xrow0 * H : nullptr, rng,
+                                  t + g.seq0, g.n, guidance_scale, x_out + g.xrow0 * H, hist ? hist + g.xrow0 * H : nullptr,
+                                  known + g.xrow0 * H, known_mask + g.xrow0, g.n_x, g.T, g.xrow0 * H, false,
+                                  fork.stream(static_cast<int>(gi))));
+  }
+  DITTO_TRY(fork.end());
+  if (advance) DITTO_TRY(launch_step_advance(reinterpret_cast<unsigned long long*>(rng), t, n_t, st));
+  return 0;
 }
 
 // ---- block-level operators (the reference's component signatures, src/components/DiT.py) -----------------------------

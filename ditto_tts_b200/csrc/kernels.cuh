@@ -72,6 +72,13 @@ int launch_cfg_multistep_update(const float* eps_c, const float* eps_u, const fl
 int launch_cfg_multistep_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t,
                                     int64_t n_t, const float* coef, int steps, float w, float* out, float* hist, int64_t B,
                                     int64_t elems_per_seq, int64_t elem_offset, bool advance, cudaStream_t st);
+// replacement conditioning (speech prompt / infilling): frames with mask[frame] != 0 of x_out [B, T, H] become a p + s z with
+// {a, s} = coef_known[t] and p = known; the others take the DDPM-form update (hist == null, coef [steps, 3]) or the multistep
+// one (coef [steps, 6]).  Exactly one of z / rng; rng: in-kernel noise at element elem_offset + i, advance as above
+int launch_cfg_update_known(const float* eps_c, const float* eps_u, const float* x, const float* z, unsigned long long* rng, int64_t* t,
+                            int64_t n_t, const float* coef, const float* coef_known, int steps, float w, float* out, float* hist,
+                            const float* known, const uint8_t* mask, int64_t B, int64_t T, int64_t H, int64_t elem_offset, bool advance,
+                            cudaStream_t st);
 int launch_step_advance(unsigned long long* rng, int64_t* t, int64_t n_t, cudaStream_t st);
 int launch_randn(const unsigned long long* rng, int64_t elem_offset, float* out, int64_t n, cudaStream_t st);
 int launch_rope_angles(const float* t, const float* pos, float* out, int64_t batch, int T, int heads, int d, cudaStream_t st);

@@ -424,6 +424,19 @@ class DiTTO(nn.Module, _EngineHost):
                        "ditto_engine_load_multistep_table")
             torch.cuda.current_stream().synchronize()
 
+    def load_known_table(self, coef: torch.Tensor):
+        """Hand a [diffusion_steps, 2] known-frame table (schedules.known_coef: the re-noising of a speech prompt or of the
+        frames around an infilled span) to the engine."""
+        eng = self.engine()
+        dev = self.proj_in.weight.device
+        if tuple(coef.shape) != (self.diffusion_steps, 2):
+            raise DittoError(f"known table must be [{self.diffusion_steps}, 2]")
+        tab = coef.detach().to(device=dev, dtype=torch.float32).contiguous()
+        with torch.cuda.device(dev):
+            _lib.check(_lib.load().ditto_engine_load_known_table(eng, _ptr(tab), self.diffusion_steps, _stream()),
+                       "ditto_engine_load_known_table")
+            torch.cuda.current_stream().synchronize()
+
     def _ensure_schedule(self):
         """The module's own (reference) schedule: what q_sample reads (DiTTO.py:63-64,106-126)."""
         if not self._schedule_loaded or getattr(self, "_schedule_owner", None) is not None:

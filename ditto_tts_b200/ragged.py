@@ -112,6 +112,17 @@ class RaggedBatch:
             out[self.x_offset[i]:self.x_offset[i] + self.lengths[i]] = x
         return out
 
+    def pack_mask(self, masks: Sequence[torch.Tensor]) -> torch.Tensor:
+        """[T_i] frame mask per utterance -> packed uint8 [sum T] in group order (one byte per packed latent row)."""
+        if len(masks) != self.B:
+            raise DittoError("one mask per utterance expected")
+        out = torch.empty((self.x_rows,), dtype=torch.uint8, device=self.device)
+        for i, q in enumerate(masks):
+            if tuple(q.shape) != (self.lengths[i],):
+                raise DittoError(f"mask[{i}] must be [{self.lengths[i]}]")
+            out[self.x_offset[i]:self.x_offset[i] + self.lengths[i]] = q != 0
+        return out
+
     def unpack(self, packed: torch.Tensor) -> List[torch.Tensor]:
         return [packed[self.x_offset[i]:self.x_offset[i] + self.lengths[i]].clone() for i in range(self.B)]
 
@@ -147,10 +158,18 @@ class RaggedBatch:
                        "ditto_forward_ragged")
         return out
 
-    def p_sample(self, x_packed, t_seq, z_packed, w: float, eps: torch.Tensor, x_out: torch.Tensor, ws=None, hist=None):
-        """One sampler step; ``hist`` (packed like x): the multistep update (ditto_p_sample_ragged_multistep)."""
+    def p_sample(self, x_packed, t_seq, z_packed, w: float, eps: torch.Tensor, x_out: torch.Tensor, ws=None, hist=None,
+                 known=None, mask=None):
+        """One sampler step; ``hist`` (packed like x): the multistep update (ditto_p_sample_ragged_multistep); ``known`` /
+        ``mask`` (packed like x / one byte per packed row): known frames (ditto_p_sample_ragged_known)."""
         ws = self.workspace() if ws is None else ws
         with torch.cuda.device(self.device):
+            if known is not None:
+                _lib.check(_lib.load().ditto_p_sample_ragged_known(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
+                                                                   _ptr(t_seq), _ptr(z_packed), None, 1 if self.guided else 0, float(w),
+                                                                   _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(known), _ptr(mask),
+                                                                   _ptr(ws), ws.numel(), 0, _stream()), "ditto_p_sample_ragged_known")
+                return
             if hist is not None:
                 _lib.check(_lib.load().ditto_p_sample_ragged_multistep(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
                                                                        _ptr(t_seq), _ptr(z_packed), 1 if self.guided else 0, float(w),
@@ -165,13 +184,16 @@ class RaggedBatch:
 
 class RaggedStepGraph:
     """One sampler iteration over a ragged batch as a CUDA graph (noise draw, forward, CFG + update, t decrement).  With
-    ``multistep`` the update is DPM-Solver++(2M)'s and the graph owns its ``hist`` buffer (packed like x)."""
+    ``multistep`` the update is DPM-Solver++(2M)'s and the graph owns its ``hist`` buffer (packed like x).  With ``known``
+    it owns the known latents (packed like x) and the frame mask (one byte per packed row), filled by ``reset``."""
 
-    def __init__(self, batch: RaggedBatch, w: float, draw_noise: bool, multistep: bool = False):
+    def __init__(self, batch: RaggedBatch, w: float, draw_noise: bool, multistep: bool = False, known: bool = False):
         self.batch, self.w, self.draw_noise = batch, w, draw_noise
         dev = batch.device
         self.x = torch.zeros((batch.x_rows, batch.H), dtype=torch.float32, device=dev)
         self.hist = torch.zeros_like(self.x) if multistep else None
+        self.known = torch.zeros_like(self.x) if known else None
+        self.mask = torch.zeros((batch.x_rows,), dtype=torch.uint8, device=dev) if known else None
         self.z = None if draw_noise else torch.zeros_like(self.x)
         self.rng = torch.zeros((4,), dtype=torch.int64, device=dev)
         self._ctx_ptrs = [c.data_ptr() for c in batch._ctx]
@@ -192,6 +214,13 @@ class RaggedStepGraph:
 
     def _step(self):
         b = self.batch
+        if self.known is not None and self.draw_noise:
+            with torch.cuda.device(b.device):
+                _lib.check(_lib.load().ditto_p_sample_ragged_known(
+                    b.model.engine(), _ptr(self.x), b.c_groups, len(b.groups), _ptr(self.t), None, _ptr(self.rng), 1 if b.guided else 0,
+                    float(self.w), _ptr(self.eps), _ptr(self.x), _ptr(self.hist), _ptr(self.known), _ptr(self.mask), _ptr(self.ws),
+                    self.ws.numel(), 1, _stream()), "ditto_p_sample_ragged_known")
+            return
         if self.draw_noise:   # noise drawn inside the per-group update kernels, bookkeeping in a one-block kernel after them
             with torch.cuda.device(b.device):
                 if self.hist is not None:
@@ -205,7 +234,7 @@ class RaggedStepGraph:
                                                                  _ptr(self.x), _ptr(self.ws), self.ws.numel(), 1, _stream()),
                            "ditto_p_sample_ragged_rng")
             return
-        b.p_sample(self.x, self.t, self.z, self.w, self.eps, self.x, ws=self.ws, hist=self.hist)
+        b.p_sample(self.x, self.t, self.z, self.w, self.eps, self.x, ws=self.ws, hist=self.hist, known=self.known, mask=self.mask)
         self.t.sub_(1)
 
     def valid_for(self, batch: "RaggedBatch") -> bool:
@@ -216,11 +245,15 @@ class RaggedStepGraph:
     def rebind(self, batch: "RaggedBatch"):
         self.batch = batch
 
-    def reset(self, x_packed: torch.Tensor, t_start: int, seed: Optional[int] = None):
+    def reset(self, x_packed: torch.Tensor, t_start: int, seed: Optional[int] = None, known: Optional[torch.Tensor] = None,
+              known_mask: Optional[torch.Tensor] = None):
         self.x.copy_(x_packed)
         self.t.fill_(t_start)
         if self.hist is not None:
             self.hist.zero_()
+        if self.known is not None:
+            self.known.copy_(known)
+            self.mask.copy_(known_mask)
         if self.draw_noise:
             if seed is None:
                 seed = int(torch.randint(0, 2 ** 62, (1,)).item())

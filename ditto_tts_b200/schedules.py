@@ -20,7 +20,10 @@ CFG scale 5.0, noise-schedule scale-shift 0.3, PDF p.25 Fig. 6):
   * ``shifted_cosine_betas``  -- the cosine schedule with its SNR multiplied by scale^2 (logSNR shift 2 log scale);
   * ``dpmpp_2m_coef``         -- DPM-Solver++(2M) (Lu et al. 2022, "DPM-Solver++", Alg. 2) and its SDE variant: a second-order
                                  multistep update that also carries the previous step's x0 prediction (a [diffusion_steps, 6]
-                                 table for ``ditto_engine_load_multistep_table``).
+                                 table for ``ditto_engine_load_multistep_table``);
+  * ``known_coef``            -- known frames (speech prompt, infilling): the re-noising rows {sqrt(abar_next),
+                                 sqrt(1 - abar_next)} of replacement conditioning (a [diffusion_steps, 2] table for
+                                 ``ditto_engine_load_known_table``).
 """
 from __future__ import annotations
 
@@ -28,7 +31,7 @@ from typing import Sequence
 
 import torch
 
-__all__ = ["spaced_timesteps", "ddpm_coef", "ddim_coef", "dpmpp_2m_coef", "shifted_cosine_betas", "coef_table"]
+__all__ = ["spaced_timesteps", "ddpm_coef", "ddim_coef", "dpmpp_2m_coef", "known_coef", "shifted_cosine_betas", "coef_table"]
 
 
 def spaced_timesteps(train_steps: int, num_steps: int) -> torch.Tensor:
@@ -124,6 +127,15 @@ def dpmpp_2m_coef(alphas_cumprod: torch.Tensor, taus: Sequence[int], eta: float 
     return out
 
 
+def known_coef(alphas_cumprod: torch.Tensor, taus: Sequence[int]) -> torch.Tensor:
+    """Replacement conditioning (Song et al. 2021, score SDE, "imputation"): the step that starts at tau_i writes a known
+    frame as q(x_{i+1} | p) = sqrt(abar_next) p + sqrt(1 - abar_next) z, abar_next = abar_{tau_{i+1}} of THIS schedule (the
+    sampler's own cumprod, not the model's betas buffer) and 1 after the last visited step, whose row {1, 0} returns p.
+    Returns float64 [len(taus), 2] = {sqrt(abar_next), sqrt(1 - abar_next)}."""
+    _, _, a_p = _acp_pairs(alphas_cumprod, taus)
+    return torch.stack([a_p.sqrt(), (1.0 - a_p).sqrt()], dim=1)
+
+
 def shifted_cosine_betas(timesteps: int, scale: float, s: float = 0.008) -> torch.Tensor:
     """DiTTO.cosine_beta_schedule (DiTTO.py:96-104) with the signal-to-noise ratio of every level multiplied by scale^2
     (abar' = scale^2 abar / (scale^2 abar + 1 - abar)); scale = 1 returns the reference's betas (same clip)."""
@@ -137,10 +149,11 @@ def shifted_cosine_betas(timesteps: int, scale: float, s: float = 0.008) -> torc
 
 
 def coef_table(diffusion_steps: int, taus: Sequence[int], coef: torch.Tensor) -> torch.Tensor:
-    """Scatter per-visited-step rows into the engine's [diffusion_steps, 3] fp32 table, or its [diffusion_steps, 6] multistep
-    table for 6-column rows (unvisited rows: identity, c1 = d1 = 1)."""
-    if coef.dim() != 2 or coef.shape[1] not in (3, 6):
-        raise ValueError("coef_table: rows must have 3 or 6 columns")
+    """Scatter per-visited-step rows into the engine's [diffusion_steps, 3] fp32 table, its [diffusion_steps, 6] multistep
+    table for 6-column rows or its [diffusion_steps, 2] known-frame table for 2-column rows (unvisited rows: identity,
+    c1 = d1 = 1; {1, 0} for known frames)."""
+    if coef.dim() != 2 or coef.shape[1] not in (2, 3, 6):
+        raise ValueError("coef_table: rows must have 2, 3 or 6 columns")
     tab = torch.zeros((diffusion_steps, coef.shape[1]), dtype=torch.float32)
     tab[:, 0] = 1.0
     if coef.shape[1] == 6:

@@ -118,6 +118,12 @@ int32_t ditto_engine_load_update_table(ditto_engine_t* e, const float* coef, int
  * order steps) do not read hist.  Held in its own engine buffer, next to the DDPM-form table, until replaced; the host
  * computes it (schedules.dpmpp_2m_coef).  DITTO_E_STATE without a loaded schedule, DITTO_E_BADARG if steps != diffusion_steps. */
 int32_t ditto_engine_load_multistep_table(ditto_engine_t* e, const float* coef6, int64_t steps, void* stream);
+/* Known frames (speech prompt, infilling; ditto_*_known below).  coef2 [diffusion_steps, 2] fp32 (device), row t =
+ * {sqrt(abar_next), sqrt(1 - abar_next)}: the noise level of the OUTPUT of the step that starts at t, abar taken from the
+ * sampler's own schedule (abar_next = 1 on the last visited step: row {1, 0}).  Held in its own engine buffer until replaced;
+ * the host computes it (schedules.known_coef).  DITTO_E_STATE without a loaded schedule, DITTO_E_BADARG if
+ * steps != diffusion_steps. */
+int32_t ditto_engine_load_known_table(ditto_engine_t* e, const float* coef2, int64_t steps, void* stream);
 /* Pack weights (bf16 copies, interleaved [fc1;gate], permuted QKV), build the per-step modulation table
  * time_mlp(SiLU(time_embed(t_embedding))) [steps, 2H] (DiTTO.py:75-76 + DiT.py:30) and the RoPE cos/sin
  * tables (DiT.py:46-59).  Synchronises the stream. */
@@ -193,6 +199,26 @@ int32_t ditto_p_sample_multistep_rng(ditto_engine_t* e, const float* x, const vo
                                      float* eps_scratch, float* x_out, float* hist, void* workspace,
                                      int64_t workspace_bytes, int32_t advance, void* stream);
 
+/* Known frames: replacement conditioning (the imputation of Song et al. 2021, score SDE) for a speech prompt
+ * (known_mask[b, :P] = 1) or an infilled span.  known [B, T, H] holds the given latents p, known_mask [B, T] uint8 (nonzero =
+ * known).  Frames that are not known take exactly the update of the calls above (bit-identical: the DDPM-form table, or with
+ * hist != NULL the multistep table); a known frame becomes
+ *     x_out = a p + s z,     {a, s} = the row t of ditto_engine_load_known_table's table
+ * where z is the normal the update uses for that element.  Known frames read neither eps, x nor hist and leave hist as it was.
+ * Exactly one of z (supplied noise [B, T, H]) or rng (in-kernel noise, as ditto_p_sample_rng) is non-NULL; advance != 0
+ * needs rng.  DITTO_E_STATE without a known table (or, with hist, without a multistep table).  One launch per step, like the
+ * calls above; x_out may alias x.  t [n_t] (n_t >= B) is read-write when advance != 0. */
+int32_t ditto_cfg_update_known(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
+                               uint64_t* rng, int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist,
+                               const float* known, const uint8_t* known_mask, int64_t B, int64_t T, int32_t advance,
+                               void* stream);
+/* ditto_p_sample / _rng / _multistep(_rng) with known frames: the forward on (guided ? 2B : B) sequences sharing x (the
+ * known frames are seen by both CFG branches), then ditto_cfg_update_known. */
+int32_t ditto_p_sample_known(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, const float* z, uint64_t* rng,
+                             int32_t guided, float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch,
+                             float* x_out, float* hist, const float* known, const uint8_t* known_mask, void* workspace,
+                             int64_t workspace_bytes, int32_t advance, void* stream);
+
 /* DiTTO.q_sample (DiTTO.py:106-126) with the reference's betas-as-alphas_cumprod buffer. */
 int32_t ditto_q_sample(ditto_engine_t* e, const float* x_start, const float* noise, const int64_t* t,
                        float* out, int64_t B, int64_t elems_per_seq, void* stream);
@@ -234,6 +260,14 @@ int32_t ditto_p_sample_ragged_multistep_rng(ditto_engine_t* e, const float* x, c
                                             int64_t* t, uint64_t* rng, int32_t guided, float guidance_scale,
                                             float* eps_scratch, float* x_out, float* hist, void* workspace,
                                             int64_t workspace_bytes, int32_t advance, void* stream);
+/* The ragged calls with known frames (ditto_p_sample_known): known packed like x, known_mask uint8 [sum n_x*T] (one byte per
+ * packed latent row); noise offsets are packed positions, each group's update runs on its fork stream and advance != 0
+ * runs the bookkeeping in a one-block kernel after them. */
+int32_t ditto_p_sample_ragged_known(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
+                                    int64_t* t, const float* z, uint64_t* rng, int32_t guided, float guidance_scale,
+                                    float* eps_scratch, float* x_out, float* hist, const float* known,
+                                    const uint8_t* known_mask, void* workspace, int64_t workspace_bytes, int32_t advance,
+                                    void* stream);
 
 /* ---- block-level operators: the component signatures of src/components/DiT.py ------------------------------- */
 /* DiT.forward(x, text_emb, time_emb, rotary_pos) (DiT.py:100-157) for block `layer` of the engine: x [n_seq, T, H] -> out
