@@ -88,7 +88,16 @@ struct XfDev {
   const float* gamma; const float* beta;      // LayerNorm after the block
   float inv_h;
   const float2* ln_stat; int ln_parts; const float* ln_c;   // deferred LayerNorm of the query operand (nullptr: off)
+  const uint8_t* skip_seq;                    // [n_seq] sequences whose tiles are not processed (nullptr: none)
 };
+
+// first tile at or after `tile` (stepping over the grid) that this launch processes.  Every role walks the same tiles, and
+// the iteration counters that drive the barrier phases count processed tiles only.
+__device__ __forceinline__ int xf_next_tile(const XfDev& p, int tile, int step) {
+  if (p.skip_seq != nullptr)
+    while (tile < p.num_tiles && __ldg(p.skip_seq + tile / p.m_tiles) != 0) tile += step;
+  return tile;
+}
 
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(32 * XF_EPI_WARPS) : "memory"); }
 // the four warps that share a TMEM lane quarter (= the same 32 tile rows): named barriers 2..5
@@ -211,9 +220,11 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
         }
       };
       // same order as the MMA issuer consumes: scores(0), then per tile its P.V boxes followed by scores(next tile)
-      if (first < p.num_tiles) load_scores_operands(first);
-      for (int tile = first; tile < p.num_tiles; tile += step) {
+      const int tile0 = xf_next_tile(p, first, step);
+      if (tile0 < p.num_tiles) load_scores_operands(tile0);
+      for (int tile = tile0; tile < p.num_tiles;) {
         const int seq = tile / p.m_tiles;
+        const int next = xf_next_tile(p, tile + step, step);
         for (int hc = 0; hc < p.num_hc; ++hc, ++vc) {
           const uint32_t vs = vc % XF_VF_RING;
           mbar_wait(&vf_empty[vs], ((vc / XF_VF_RING) & 1u) ^ 1u);  // the MMAs that read this box have retired
@@ -224,7 +235,8 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
           }
           __syncwarp();
         }
-        if (tile + step < p.num_tiles) load_scores_operands(tile + step);
+        if (next < p.num_tiles) load_scores_operands(next);
+        tile = next;
       }
     }
   } else if (warp == 1) {
@@ -261,8 +273,10 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
         __syncwarp();
       };
       uint32_t it = 0, oc = 0, vc = 0;
-      if (first < p.num_tiles) issue_scores(0);
-      for (int tile = first; tile < p.num_tiles; tile += step, ++it) {
+      const int tile0 = xf_next_tile(p, first, step);
+      if (tile0 < p.num_tiles) issue_scores(0);
+      for (int tile = tile0; tile < p.num_tiles; ++it) {
+        const int next = xf_next_tile(p, tile + step, step);
         mbar_wait(p_full, it & 1u);
         for (int hc = 0; hc < p.num_hc; ++hc, ++vc) {
           const uint32_t ob = oc % XF_O_BUFS, vs = vc % XF_VF_RING;
@@ -283,7 +297,8 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
         }
         // the next tile's scores AFTER this tile's P.V (the issuer is sequential: ahead of the P.V they would put their
         // operand stream on the critical path); they still overlap the rest of this tile's epilogue
-        if (tile + step < p.num_tiles) issue_scores(it + 1);
+        if (next < p.num_tiles) issue_scores(it + 1);
+        tile = next;
       }
     }
   } else if (warp == 2 || warp == 3) {
@@ -295,12 +310,22 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
     xf_regs_ctrl();
     {
       const bool leader = elect_one();
-      const int my_tiles = first < p.num_tiles ? (p.num_tiles - 1 - first) / step + 1 : 0;
+      const int tile0 = xf_next_tile(p, first, step);
+      int my_tiles = 0;
+      if (p.skip_seq == nullptr) my_tiles = first < p.num_tiles ? (p.num_tiles - 1 - first) / step + 1 : 0;
+      else for (int t = tile0; t < p.num_tiles; t = xf_next_tile(p, t + step, step)) ++my_tiles;
       const int jobs_per_tile = 2 * p.num_hc;
       const int J = my_tiles * jobs_per_tile;
+      // tile of this CTA's ti-th processed tile: a cursor per caller, every caller asks for non-decreasing ti
+      struct Cursor { int ti, tile; };
+      auto tile_at = [&](Cursor& cur, int ti) {
+        for (; cur.ti < ti; ++cur.ti) cur.tile = xf_next_tile(p, cur.tile + step, step);
+        return cur.tile;
+      };
+      Cursor jc{0, tile0}, pc{0, tile0};
       auto job_coords = [&](int j, int& seq, int& row, int& pass, int& hc) {
         const int ti = j / jobs_per_tile, r = j - ti * jobs_per_tile;
-        const int tile = first + ti * step;
+        const int tile = tile_at(jc, ti);
         seq = tile / p.m_tiles;
         row = (tile - seq * p.m_tiles) * p.rt;
         pass = r / p.num_hc;
@@ -316,7 +341,7 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
           limit = limit < P0 ? limit : P0;
           for (; pf_next < limit; ++pf_next) {
             const int ti = pf_next / p.num_hc, hc = pf_next - ti * p.num_hc;
-            const int tile = first + ti * step, seq = tile / p.m_tiles, row = (tile - seq * p.m_tiles) * p.rt;
+            const int tile = tile_at(pc, ti), seq = tile / p.m_tiles, row = (tile - seq * p.m_tiles) * p.rt;
             if (leader && pf_next >= XF_NB) {   // the first XF_NB loads are issued at once anyway
               tma_prefetch_4d(&tmap_h, hc * XF_HC, row, 0, seq);
               tma_prefetch_4d(&tmap_h, hc * XF_HC + 32, row, 0, seq);
@@ -381,7 +406,7 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
     const int g = lane >> 2, q = lane & 3, q2 = q * 2;
     const bool writer = q == 0;
     uint32_t it = 0, oc = 0, job = 0;
-    for (int tile = first; tile < p.num_tiles; tile += step, ++it) {
+    for (int tile = xf_next_tile(p, first, step); tile < p.num_tiles; tile = xf_next_tile(p, tile + step, step), ++it) {
       const int seq = tile / p.m_tiles;
       const uint32_t sb = it & 1u;
       // ---------------- softmax of the 128 x 64 score tile -> bf16 probabilities in shared memory ----------------
@@ -719,9 +744,10 @@ int launch_cross_fused(const CrossFusedParams& q, cudaStream_t st) {
   // kernel is short of HBM / L2 throughput, not of requests in flight, and the early requests only displace lines that are still needed
   p.pf_dist = g_opt.xf_prefetch > 0 ? std::min(g_opt.xf_prefetch, 2 * p.num_hc) : 0;
   p.ln_stat = q.ln_stat; p.ln_parts = q.ln_parts; p.ln_c = q.ln_c;
+  p.skip_seq = q.skip_seq;
   if (q.ln_stat != nullptr) DITTO_REQUIRE(q.ln_parts > 0 && q.ln_c != nullptr, DITTO_E_BADARG, "cross_fused: deferred LayerNorm arguments");
   // flops: both contractions; bytes: u read, h read + write, u3 write (the HBM stream that bounds the kernel)
-  const double rows = static_cast<double>(q.n_seq) * q.T;
+  const double rows = static_cast<double>(q.n_seq - (q.skip_seq ? profiled_nonzero(q.skip_seq, q.n_seq, st) : 0)) * q.T;
   ProfScope prof(q.tag, st, 4.0 * rows * q.S * q.H, rows * q.H * 12.0);
   const int grid = static_cast<int>(std::min<int64_t>(sms, tiles));
   cross_fused_kernel<<<grid, XF_THREADS, XF_SMEM_BYTES, st>>>(mu, mk, mv, mh, mo, p);

@@ -578,6 +578,36 @@ int launch_fold_bias(const bf16* kv, int64_t ld, const float* bq, float* sb, int
   return 0;
 }
 
+// one block per sequence.  A sequence whose text rows are all equal has equal rows of V Wo^T, so its cross-attention output
+// softmax(scores) (V Wo^T) + bo is the row vfold[0] + bo whatever the scores are.  Bitwise equality of the inputs is what
+// makes the rows of the folded projections equal: the GEMMs that build them treat every row alike.
+__global__ void const_text_kernel(const float* __restrict__ text, int S, int D, const bf16* __restrict__ vfold, int64_t vf_seq,
+                                  bool vf_perm4, const float* __restrict__ bo, uint8_t* __restrict__ flag, float* __restrict__ crow,
+                                  int H) {
+  const int64_t seq = blockIdx.x;
+  if (flag != nullptr) {
+    const uint32_t* t = reinterpret_cast<const uint32_t*>(text) + seq * S * D;
+    int diff = 0;
+    for (int64_t i = D + threadIdx.x; i < static_cast<int64_t>(S) * D; i += blockDim.x) diff |= t[i] != t[i % D];
+    diff = __syncthreads_or(diff);
+    if (threadIdx.x == 0) flag[seq] = diff ? 0 : 1;
+  }
+  const bf16* v = vfold + seq * vf_seq;
+  for (int c = threadIdx.x; c < H; c += blockDim.x) {
+    // perm4 (gemm_resid_ln_weight_row): plain column 64 blk + 16 (kb / 2) + 4 q + 2 (kb % 2) + e sits at 64 blk + 8 kb + 2 q + e
+    const int cp = c & 63, kb = 2 * (cp >> 4) + ((cp & 3) >> 1);
+    const int src = vf_perm4 ? (c - cp) + 8 * kb + 2 * ((cp & 15) >> 2) + (cp & 1) : c;
+    crow[seq * H + c] = __bfloat162float(v[src]) + bo[c];
+  }
+}
+int launch_const_text(const float* text, int64_t n, int S, int D, const bf16* vfold, int64_t vf_seq, bool vf_perm4, const float* bo,
+                      uint8_t* flag, float* crow, int H, cudaStream_t st) {
+  DITTO_REQUIRE(!vf_perm4 || H % 64 == 0, DITTO_E_BADARG, "const_text: perm4 column order needs H % 64 == 0");
+  const_text_kernel<<<static_cast<unsigned>(n), 256, 0, st>>>(text, S, D, vfold, vf_seq, vf_perm4, bo, flag, crow, H);
+  DITTO_LAUNCH_CHECK();
+  return 0;
+}
+
 // V [T, d] slices of qkv (ld) -> Vt [n*heads, d, Tp] (keys contiguous): fallback operand layout for P@V
 __global__ void transpose_v_kernel(const bf16* __restrict__ v, int64_t ld, bf16* __restrict__ vt, int T, int Tp, int heads,
                                    int d) {
@@ -937,9 +967,8 @@ __global__ void __launch_bounds__(256)
   if (RNG && advance) last_block_advances(rng, t, n_t, draw);
 }
 
-// known frames of mask[0, n) for the profiler's byte count; only while profiling (which synchronises anyway and is never
-// captured), so a step graph never sees the copy
-static int64_t profiled_known_frames(const uint8_t* mask, int64_t n, cudaStream_t st) {
+// only while profiling (which synchronises anyway and is never captured), so a step graph never sees the copy
+int64_t profiled_nonzero(const uint8_t* mask, int64_t n, cudaStream_t st) {
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
   if (!g_prof_enabled || cudaStreamIsCapturing(st, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) return 0;
   std::vector<uint8_t> h(static_cast<size_t>(n));
@@ -962,7 +991,7 @@ int launch_cfg_update_known(const float* eps_c, const float* eps_u, const float*
   const int64_t want = ceil_div(total_vec, 256 * 4);
   const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
   // bytes moved: 16 B per float4 of every stream a frame touches, plus one mask byte per frame
-  const int64_t known_vec = profiled_known_frames(mask, B * T, st) * vec_per_frame;
+  const int64_t known_vec = profiled_nonzero(mask, B * T, st) * vec_per_frame;
   const double unknown_streams = (ms ? 5 : 3) + (eps_u ? 1 : 0) + (draw ? 0 : 1), known_streams = 2 + (draw ? 0 : 1);
   ProfScope prof(PC_CFG_UPDATE, st, 0.0,
                  16.0 * (static_cast<double>(total_vec - known_vec) * unknown_streams + static_cast<double>(known_vec) * known_streams) +

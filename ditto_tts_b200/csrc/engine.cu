@@ -101,6 +101,7 @@ struct ditto_engine {
   bool fused_attn = false;  // scores + softmax fused (cluster kernel); falls back per call when a row needs > 16 tiles
   bool fold_cross = false;  // cross-attn q/out projections folded into the per-utterance text K/V (heads == 1 only)
   bool defer_ln = false;    // block LayerNorms folded into the neighbouring GEMM epilogues (no LayerNorm launches)
+  bool const_text = true;   // sequences with constant text rows: constant cross-attention output added by the self-attention kernel
   int pv_transpose = 0;  // debug: use the transposed-V operand instead of the MN-major descriptor
   bool rope_table_in_epilogue = false;  // debug (DITTO_ROPE_TABLE=1): fused RoPE reads the cos/sin tables instead of computing them
   std::map<std::string, int64_t> expected;  // key -> numel
@@ -202,9 +203,13 @@ struct CtxLayout {
   //   vfold [n, heads*Sp, H]   = V_h Wo_h^T         (out = P . vfold + bo), zero rows for s >= S
   //   sbias [n, heads, Sp] f32 = sqrt(1/d) K_h bq_h
   //   cvec  [n, heads, Sp] f32 = row sums of the gamma2-scaled kfold (deferred LayerNorm only), strided like sbias
+  // and, single head only, for sequences whose S text rows are all equal (the unconditional CFG half, S = 1):
+  //   cflag [n] u8             = 1 when they are (cross-attention output = vfold[0] + bo for every query row)
+  //   crow  [n, H] f32         = vfold[seq][0] + bo, plain column order, per layer
   bf16 *kfold0 = nullptr, *vfold0 = nullptr;
-  float *sbias0 = nullptr, *cvec0 = nullptr;
-  size_t kfold_stride = 0, vfold_stride = 0, sbias_stride = 0;  // elements between layers
+  float *sbias0 = nullptr, *cvec0 = nullptr, *crow0 = nullptr;
+  uint8_t* cflag = nullptr;
+  size_t kfold_stride = 0, vfold_stride = 0, sbias_stride = 0, crow_stride = 0;  // elements between layers
   size_t total = 0;
 };
 static bool fold_active(const ditto_engine* e, int64_t S) {
@@ -239,6 +244,11 @@ static CtxLayout ctx_layout(const ditto_engine* e, void* base, int64_t n, int64_
     c.vfold0 = a.take<bf16>(static_cast<int64_t>(c.vfold_stride) * e->L);
     c.sbias0 = a.take<float>(static_cast<int64_t>(c.sbias_stride) * e->L);
     if (e->defer_ln || e->defer_ln2) c.cvec0 = a.take<float>(static_cast<int64_t>(c.sbias_stride) * e->L);
+    if (e->heads == 1) {
+      c.crow_stride = static_cast<size_t>(n * e->H);
+      c.cflag = a.take<uint8_t>(n);
+      c.crow0 = a.take<float>(static_cast<int64_t>(c.crow_stride) * e->L);
+    }
   }
   c.total = a.off + 256;
   return c;
@@ -568,13 +578,24 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
         // norm2 deferred for this group (context built with the gamma2-folded K): whole-model DITTO_F_DEFER_LN, or norm2 only
         const bool dln2 = dln ? dln2_all : fold_ln_active(e, S) && do_self;   // the row statistics come from the self-attention
         float2* lnstat_g = w.lnstat ? w.lnstat + grp.row0 * std::max(w.ln_parts_h, w.ln_parts_attn) : nullptr;
+        const bool self768 = do_self && e->flash768 && !dln2 && flash768_supported(H, e->heads, static_cast<int>(T));
+        // constant-text sequences (all text rows equal: the unconditional CFG half, S = 1): their cross-attention output is one
+        // row per layer, added by the self-attention kernel together with norm3; the cross-attention kernel skips them.  Only
+        // where both sections run here and both kernels know the flags (four-CTA self-attention, folded fused cross-attention)
+        const uint8_t* kflag = e->const_text && c.cflag != nullptr && do_cross && self768 && !dln && flash768_picks_quad(static_cast<int>(T)) &&
+                                       (cross_flash_active(e, S) || fuse_cross_group(grp))
+                                   ? c.cflag : nullptr;
         if (!do_self) {
           // stand-alone cross-attention / MLP section: u already holds that section's LayerNorm of the input
-        } else if (e->flash768 && !dln2 && flash768_supported(H, e->heads, static_cast<int>(T))) {
+        } else if (self768) {
           // scores, softmax, P.V, + residual AND norm2 in one kernel: no S / P in HBM, no LayerNorm launch     DiT.py:117-143
           Flash768Params f;
           f.qkv = q; f.ld = 3 * H; f.n_seq = n; f.T = static_cast<int>(T); f.H = H; f.alpha = inv_sqrt_d; f.h = hg;
           f.gamma = e->LW(i, "norm2.weight"); f.beta = e->LW(i, "norm2.bias"); f.u_out = ug; f.tag = PC_FLASH768;
+          if (kflag) {
+            f.const_flag = kflag; f.const_row = c.crow0 + c.crow_stride * i;
+            f.gamma_c = e->LW(i, "norm3.weight"); f.beta_c = e->LW(i, "norm3.bias");
+          }
           DITTO_TRY(launch_flash768(f, st));
         } else {
           DITTO_TRY(attention_bf16(e, wg, q, 3 * H, T * 3 * H, q + H, 3 * H, T * 3 * H, q + 2 * H, 3 * H, T * 3 * H, n, static_cast<int>(T),
@@ -598,6 +619,7 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
             f.vf_rows = static_cast<int>(Sp); f.Tk = static_cast<int>(S); f.kbias = c.sbias0 + c.sbias_stride * i; f.kb_seq = Sp;
             f.out_bias = e->LW(i, "cross_attn.out_proj.bias");
             f.gamma = e->LW(i, "norm3.weight"); f.beta = e->LW(i, "norm3.bias"); f.u_out = ug; f.tag = PC_CROSS_FLASH;
+            f.const_flag = kflag;
             DITTO_TRY(launch_flash768_quad(f, st));
             continue;
           }
@@ -607,7 +629,7 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
             f.u = ug; f.kfold = c.kfold0 + c.kfold_stride * i; f.kf_seq = S * H; f.vfold = c.vfold0 + c.vfold_stride * i; f.vf_seq = Sp * H;
             f.sbias = c.sbias0 + c.sbias_stride * i; f.sb_seq = Sp; f.out_bias = e->LW(i, "cross_attn.out_proj.bias");
             f.h = hg; f.gamma = e->LW(i, "norm3.weight"); f.beta = e->LW(i, "norm3.bias"); f.u_out = ug;
-            f.n_seq = n; f.T = T; f.S = S; f.Sp = Sp; f.H = H; f.alpha = sqrt_inv_d; f.tag = PC_TC_CROSS_FUSED;
+            f.n_seq = n; f.T = T; f.S = S; f.Sp = Sp; f.H = H; f.alpha = sqrt_inv_d; f.tag = PC_TC_CROSS_FUSED; f.skip_seq = kflag;
             if (dln2) { f.ln_stat = lnstat_g; f.ln_parts = w.ln_parts_attn; f.ln_c = c.cvec0 + c.sbias_stride * i; }
             DITTO_TRY(launch_cross_fused(f, st));
             continue;
@@ -873,6 +895,7 @@ int32_t ditto_engine_create(const ditto_config_t* cfg, ditto_engine_t** out) {
     e->flash_attn = e->fused_attn;
     if (g_opt.no_flash) e->flash_attn = false;
     if (g_opt.no_fused_cross) e->fused_cross = false;
+    e->const_text = !g_opt.no_const_text;
     e->defer_ln2 = !e->defer_ln && e->fused_cross && e->bf16_mode && e->heads == 1 && g_opt.defer_ln2 != 0;
     e->pv_transpose = g_opt.pv_transpose != 0;
     e->rope_table_in_epilogue = g_opt.rope_table != 0;
@@ -1218,6 +1241,9 @@ int32_t ditto_text_context(ditto_engine_t* e, const float* text_emb, int64_t n, 
                                    static_cast<int>(S), static_cast<int>(Sp), heads, d, sqrtf(1.0f / static_cast<float>(d)), st));
         if (fln)
           DITTO_TRY(launch_rowsum_bf16(kf, c.cvec0 + c.sbias_stride * i, n * heads, static_cast<int>(S), static_cast<int>(Sp), H, st));
+        if (c.cflag != nullptr)   // the flags once (layer 0), the constant rows of every layer
+          DITTO_TRY(launch_const_text(text_emb, n, static_cast<int>(S), Xd, vf, Sp * H, cross_flash_active(e, S),
+                                      e->LW(i, "cross_attn.out_proj.bias"), i == 0 ? c.cflag : nullptr, c.crow0 + c.crow_stride * i, H, st));
       }
     } else {
       DITTO_TRY(sgemm_nt(text_emb, Xd, e->LW(i, "cross_attn.in_proj_weight") + static_cast<int64_t>(H) * H, H, static_cast<float*>(kv),
@@ -1665,7 +1691,7 @@ int32_t ditto_debug_option(const char* name, int32_t value) {
       {"pv_transpose", &g_opt.pv_transpose}, {"rope_table", &g_opt.rope_table}, {"rope_generic", &g_opt.rope_generic},
       {"glu_generic", &g_opt.glu_generic}, {"no_rope_fast32", &g_opt.no_rope_fast32}, {"no_pv_perm4", &g_opt.no_pv_perm4},
       {"side_streams", &g_opt.side_streams}, {"no_fused_ln", &g_opt.no_fused_ln}, {"flash768_quad", &g_opt.flash768_quad},
-      {"no_fc2_ln", &g_opt.no_fc2_ln}, {"no_cross_flash", &g_opt.no_cross_flash}, {"dbg_nostore", &g_opt.dbg_nostore}};
+      {"no_fc2_ln", &g_opt.no_fc2_ln}, {"no_cross_flash", &g_opt.no_cross_flash}, {"no_const_text", &g_opt.no_const_text}, {"dbg_nostore", &g_opt.dbg_nostore}};
   if (strcmp(name, "reset") == 0) { g_opt = DebugOptions(); return 0; }
   for (const Opt& o : opts)
     if (strcmp(name, o.n) == 0) { *o.p = value; return 0; }

@@ -704,11 +704,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
 
 bool flash768_supported(int H, int heads, int T) { return heads == 1 && H == F7_D && T >= 1; }
 
+// four-CTA clusters (two cta_group::2 pairs, K / V loaded once per pair) when 256-row query tiles fit the sequence length
+bool flash768_picks_quad(int T) {
+  return g_opt.flash768_quad != 1 && T >= 1 && (g_opt.flash768_quad == 2 || flash768_quad_preferred(T)) && flash768_quad_schedulable();
+}
+
 int launch_flash768(const Flash768Params& q, cudaStream_t st) {
-  // four-CTA clusters (two cta_group::2 pairs, K / V loaded once per pair) when 256-row query tiles fit the sequence length
-  if (g_opt.flash768_quad != 1 && q.T >= 1 && (g_opt.flash768_quad == 2 || flash768_quad_preferred(q.T)) && flash768_quad_schedulable())
-    return launch_flash768_quad(q, st);
+  if (flash768_picks_quad(q.T)) return launch_flash768_quad(q, st);
   DITTO_TRY(tc_gemm_init());
+  DITTO_REQUIRE(q.const_flag == nullptr, DITTO_E_UNSUPPORTED, "flash768: constant-text rows need the four-CTA kernel");
   DITTO_REQUIRE(flash768_supported(q.H, 1, q.T), DITTO_E_UNSUPPORTED, "flash768: single head of 768 only");
   DITTO_REQUIRE(q.qkv && q.h && q.n_seq >= 1 && q.ld % 8 == 0 && q.ld >= 3 * F7_D, DITTO_E_BADARG, "flash768: bad argument");
   DITTO_REQUIRE(q.u_out == nullptr || (q.gamma && q.beta), DITTO_E_BADARG, "flash768: LayerNorm output needs gamma and beta");

@@ -60,7 +60,8 @@ constexpr int Q7_BAR_BYTES = 512;
 constexpr int Q7_OFF_XCH = Q7_OFF_BAR + Q7_BAR_BYTES;
 constexpr int Q7_XCH_HDR = 0, Q7_XCH_L = 2 * Q7_BM * 4, Q7_XCH_STAT = 4 * Q7_BM * 4;
 constexpr int Q7_XCH_BYTES = 4 * Q7_BM * 4 + 2 * Q7_BM * 8;
-constexpr int Q7_SMEM_BYTES = Q7_OFF_XCH + Q7_XCH_BYTES + 1024;
+constexpr int Q7_OFF_CROW = Q7_OFF_XCH + Q7_XCH_BYTES;   // [2][384] fp32: a constant-text item's row, this CTA's column half
+constexpr int Q7_SMEM_BYTES = Q7_OFF_CROW + 2 * Q7_DH * 4 + 1024;
 static_assert(Q7_SMEM_BYTES <= 232448, "exceeds the 227 KiB shared memory of an sm_100 CTA");
 static_assert(Q7_OFF_POWN % 1024 == 0, "operand buffers must be 1024-byte aligned (128-B swizzle atoms)");
 constexpr int Q7_TMEM_COLS = 512;
@@ -92,13 +93,16 @@ struct Q7Dev {
   int Tk;                             // keys per sequence (self-attention: T; cross-attention: text tokens S)
   int m_tiles, k_tiles, num_items;    // m_tiles: 256-row query tiles per utterance
   const float* kbias; long long kb_seq;   // CROSS: additive score bias per key [n_seq, kb_seq] (already scaled; folded k-bias)
-  const float* obias;                 // CROSS: output bias [768] (cross_attn.out_proj.bias)
+  const float* obias;                 // CROSS: output bias [768] (cross_attn.out_proj.bias); KONST: constant rows [n_seq][768]
   float alpha2;
   float* h;
   const float* gamma; const float* beta;
   bf16* u_out;
   int force_rescale;
   int dbg;
+  // constant-text sequences (Flash768Params::const_flag); self-attention: norm3, which replaces norm2 for them.  (Few new
+  // fields, at the end: a larger parameter block costs the plain self-attention kernel spills.)
+  const uint8_t* const_flag; const float* gamma_c; const float* beta_c;
 };
 
 __device__ __forceinline__ void q7_tmem_st_16x64(uint32_t taddr, const uint32_t (&r)[32]) {
@@ -129,12 +133,23 @@ __device__ __forceinline__ void q7_bulk_copy_to_peer(uint32_t remote_dst, uint32
                : "memory");
 }
 __device__ __forceinline__ void q7_prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+// first item at or after `item` (stepping over the grid) that this launch processes: the cross-attention kernel skips the
+// items of constant-text sequences, whose output the self-attention kernel has already added.  Every role walks the same
+// items, so the barrier phases (counted per processed item) agree.
+template <bool CROSS>
+__device__ __forceinline__ int q7_next_item(const Q7Dev& p, int item, int step) {
+  if (CROSS && p.const_flag != nullptr)
+    while (item < p.num_items && __ldg(p.const_flag + item / p.m_tiles) != 0) item += step;
+  return item;
+}
 
 // CROSS = false: self-attention (q, k, v = column thirds of the QKV GEMM output).  CROSS = true: the folded cross-attention
 // of a single-head model with 64 < S <= 256 text tokens (DiT.py:141-151 -> torch MHA math path):
 //   h <- h + softmax(alpha u (K Wq)^T + kbias) (V Wo^T) + bo ;  u <- LayerNorm(h) gamma3 + beta3
 // q = u (norm2 output, overwritten in place with norm3's), k = K-fold [S, 768], v = V-fold [Sp, 768] in the perm4 column order.
-template <bool CROSS>
+// KONST (self-attention only): the launch carries constant-text sequences (Q7Dev::const_flag); a separate instantiation, so
+// that the plain self-attention kernel keeps its registers.
+template <bool CROSS, bool KONST = false>
 __global__ void __launch_bounds__(Q7_THREADS, 1)
     flash_attn768q_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                           const __grid_constant__ CUtensorMap tmap_v, const Q7Dev p) {
@@ -222,7 +237,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
     Q7Tr tr; tr.init(p.trace, rank, 2, first == 0 && leader, t_sync);
     int stage = 0;
     uint32_t phase = 0;
-    for (int item = first; item < p.num_items; item += num_clusters) {
+    for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items; item = q7_next_item<CROSS>(p, item + num_clusters, num_clusters)) {
       const int qt = item % p.m_tiles, seq = item / p.m_tiles;
       const int q_row0 = qt * (2 * Q7_BM) + a * Q7_BM;
       auto load_s = [&](int j) {
@@ -352,7 +367,8 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
         if (own) ++oc; else ++rc;
         ++pvi;
       };
-      for (int item = first; item < p.num_items; item += num_clusters, ++it) {
+      for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items;
+           item = q7_next_item<CROSS>(p, item + num_clusters, num_clusters), ++it) {
         if (c < KT) issue_s();
         for (int j = 0; j < KT; ++j) {
           if ((j & 1) == c && j + 2 < KT) issue_s();
@@ -369,7 +385,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
     const bool leader = elect_one();
     const uint32_t dst = q7_mapa(smem_u32(p_land), peer), src = smem_u32(p_own), bar = q7_mapa(smem_u32(land_full), peer);
     uint32_t oc = 0;
-    for (int item = first; item < p.num_items; item += num_clusters)
+    for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items; item = q7_next_item<CROSS>(p, item + num_clusters, num_clusters))
       for (int j = c; j < KT; j += 2, ++oc) {
         mbar_wait(p_ready, oc & 1u);   // written + fence.proxy.async by this CTA's softmax warps; the peer's landing buffer is
         if (leader) q7_bulk_copy_to_peer(dst, src, Q7_P_BYTES, bar);   // free: p_free (awaited before the tile was written)
@@ -379,7 +395,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
     // =========================== landing relay ===========================
     regs_shrink_ctrl();
     uint32_t rc = 0;
-    for (int item = first; item < p.num_items; item += num_clusters)
+    for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items; item = q7_next_item<CROSS>(p, item + num_clusters, num_clusters))
       for (int j = c ^ 1; j < KT; j += 2, ++rc) {
         if (lane == 0) {
           mbar_expect_tx(land_full, Q7_P_BYTES);   // arm this tile's landing (the copy may already be on its way)
@@ -422,9 +438,22 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
       q7_tmem_st_wait();
       tcgen05_fence_before();
     };
-    for (int item = first; item < p.num_items; item += num_clusters, ++it) {
+    for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items;
+         item = q7_next_item<CROSS>(p, item + num_clusters, num_clusters), ++it) {
       const int qt = item % p.m_tiles, seq = item / p.m_tiles;
       const int row0 = qt * (2 * Q7_BM) + a * Q7_BM;               // first row of this CTA inside the utterance
+      // a constant-text sequence (warp-uniform, per item): sweep 1 adds its constant cross-attention output row the way
+      // CROSS adds the output bias, sweep 2 applies norm3 instead of norm2
+      const bool konst = KONST && __ldg(p.const_flag + seq) != 0;
+      // the row goes to shared memory once per item (two buffers by item parity: a warp fills the next item's only after
+      // every epilogue warp has passed this item's barrier, i.e. finished the previous item's sweep 1)
+      float* crow = reinterpret_cast<float*>(smem + Q7_OFF_CROW) + (it & 1u) * Q7_DH;
+      if (KONST) {
+        if (konst)
+          for (int i = ew * 32 + lane; i < Q7_DH / 4; i += Q7_EPI_WARPS * 32)
+            reinterpret_cast<float4*>(crow)[i] = __ldg(reinterpret_cast<const float4*>(p.obias + seq * Q7_D + col_half) + i);
+        asm volatile("bar.sync 1, %0;" ::"n"(Q7_EPI_WARPS * 32) : "memory");
+      }
       const int lrowA = row0 + rA;
       const bool okA = lrowA < p.T, okB = lrowA + 8 < p.T;
       const long long growA = static_cast<long long>(seq) * p.T + lrowA;
@@ -636,7 +665,8 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
           vB.y = fmaf(iB, __uint_as_float(o[4 * k0 + 3]), f[4 + jj].y);
           vB.z = fmaf(iB, __uint_as_float(o[4 * k1 + 2]), f[4 + jj].z);
           vB.w = fmaf(iB, __uint_as_float(o[4 * k1 + 3]), f[4 + jj].w);
-          if (CROSS) {   // + out_proj bias (the torch MHA output projection, folded into V)
+          if (konst) ob[jj] = *reinterpret_cast<const float4*>(crow + q * 4 + cb * 64 + jj * 16);
+          if (CROSS || konst) {   // + out_proj bias (the torch MHA output projection, folded into V) / constant row
             vA.x += ob[jj].x; vA.y += ob[jj].y; vA.z += ob[jj].z; vA.w += ob[jj].w;
             vB.x += ob[jj].x; vB.y += ob[jj].y; vB.z += ob[jj].z; vB.w += ob[jj].w;
           }
@@ -686,8 +716,8 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
         const float2 aB2 = make_float2(rsB, rsB), cB2 = make_float2(-meanB * rsB, -meanB * rsB);
         bf16* uA = p.u_out + growA * Q7_D + col_half + q * 4;
         bf16* uB = uA + 8 * Q7_D;
-        const float* gp = p.gamma + col_half + q * 4;
-        const float* bp = p.beta + col_half + q * 4;
+        const float* gp = (konst ? p.gamma_c : p.gamma) + col_half + q * 4;
+        const float* bp = (konst ? p.beta_c : p.beta) + col_half + q * 4;
         // the TMEM load of chunk cb + 1 is in flight while chunk cb is normalised and stored (tcgen05.wait::ld waits for every
         // outstanding load, so the next load is issued right after the wait and consumed one iteration later)
         auto sweep2 = [&](int cb, const uint32_t(&o)[32]) {
@@ -762,6 +792,7 @@ static int q7_clusters(DeviceState* ds) {
   if (ds->f768q_clusters == 0) {
     int n = 0;
     if (cudaFuncSetAttribute(flash_attn768q_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q7_SMEM_BYTES) == cudaSuccess &&
+        cudaFuncSetAttribute(flash_attn768q_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q7_SMEM_BYTES) == cudaSuccess &&
         cudaFuncSetAttribute(flash_attn768q_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q7_SMEM_BYTES) == cudaSuccess) {
       cudaLaunchConfig_t cfg = {};
       cudaLaunchAttribute attr[1];
@@ -797,6 +828,9 @@ int launch_flash768_quad(const Flash768Params& q, cudaStream_t st) {
                            q.kf_seq % 8 == 0 && q.vf_seq % 8 == 0 && (reinterpret_cast<uintptr_t>(q.out_bias) & 15) == 0),
                 DITTO_E_BADARG, "flash768 (cross-attention): folded keys / values, score bias and output bias for 1..256 text tokens");
   DITTO_REQUIRE(q.u_out == nullptr || (q.gamma && q.beta), DITTO_E_BADARG, "flash768: LayerNorm output needs gamma and beta");
+  DITTO_REQUIRE(q.const_flag == nullptr || cross ||
+                    (q.u_out && q.const_row && q.gamma_c && q.beta_c && (reinterpret_cast<uintptr_t>(q.const_row) & 15) == 0),
+                DITTO_E_BADARG, "flash768 (constant text): 16-byte aligned constant rows, norm3 and a LayerNorm output");
   DITTO_REQUIRE((reinterpret_cast<uintptr_t>(q.h) & 15) == 0 && (reinterpret_cast<uintptr_t>(q.u_out) & 7) == 0, DITTO_E_BADARG,
                 "flash768: h must be 16-byte, u 8-byte aligned");
   DeviceState* ds = device_state();
@@ -829,7 +863,7 @@ int launch_flash768_quad(const Flash768Params& q, cudaStream_t st) {
   Q7Dev p;
   p.n_seq = static_cast<int>(q.n_seq); p.T = q.T;
   p.Tk = cross ? q.Tk : q.T;
-  p.kbias = q.kbias; p.kb_seq = q.kb_seq; p.obias = q.out_bias;
+  p.kbias = q.kbias; p.kb_seq = q.kb_seq; p.obias = cross ? q.out_bias : q.const_row;
   p.m_tiles = static_cast<int>(ceil_div(q.T, 2 * Q7_BM));
   p.k_tiles = static_cast<int>(ceil_div(p.Tk, Q7_BN));
   const int64_t items = static_cast<int64_t>(p.m_tiles) * q.n_seq;
@@ -837,17 +871,22 @@ int launch_flash768_quad(const Flash768Params& q, cudaStream_t st) {
   p.num_items = static_cast<int>(items);
   p.alpha2 = q.alpha * 1.4426950408889634f;
   p.h = q.h; p.gamma = q.gamma; p.beta = q.beta; p.u_out = q.u_out;
+  p.const_flag = q.const_flag; p.gamma_c = q.gamma_c; p.beta_c = q.beta_c;
   p.force_rescale = q.force_rescale ? 1 : 0;
   p.dbg = q.dbg;
   p.trace = DITTO_F7_TRACE ? tc_gemm_debug_counters() : nullptr;
-  const double rows = static_cast<double>(q.n_seq) * q.T;
-  ProfScope prof(q.tag, st, 4.0 * q.T * static_cast<double>(p.Tk) * Q7_D * q.n_seq,
-                 rows * Q7_D * ((cross ? 2.0 : 6.0) + 8.0 + (q.u_out ? 2.0 : 0.0)) + (cross ? 4.0 * q.n_seq * static_cast<double>(p.Tk) * Q7_D : 0.0));
+  // the cross-attention kernel does no work for the skipped sequences (profiler byte / flop counts over the processed ones)
+  const double n_run = static_cast<double>(q.n_seq - (cross && q.const_flag ? profiled_nonzero(q.const_flag, q.n_seq, st) : 0));
+  const double rows = n_run * q.T;
+  ProfScope prof(q.tag, st, 4.0 * q.T * static_cast<double>(p.Tk) * Q7_D * n_run,
+                 rows * Q7_D * ((cross ? 2.0 : 6.0) + 8.0 + (q.u_out ? 2.0 : 0.0)) + (cross ? 4.0 * n_run * static_cast<double>(p.Tk) * Q7_D : 0.0));
   const int clusters = static_cast<int>(std::min<int64_t>(max_clusters, items));
   cfg.gridDim = dim3(static_cast<unsigned>(4 * clusters), 1, 1);
   void* args[4] = {&mq, &mk, &mv, &p};
-  DITTO_CUDA(cudaLaunchKernelExC(&cfg, cross ? reinterpret_cast<const void*>(flash_attn768q_kernel<true>)
-                                             : reinterpret_cast<const void*>(flash_attn768q_kernel<false>), args));
+  const void* fn = cross ? reinterpret_cast<const void*>(flash_attn768q_kernel<true>)
+                 : q.const_flag ? reinterpret_cast<const void*>(flash_attn768q_kernel<false, true>)
+                                : reinterpret_cast<const void*>(flash_attn768q_kernel<false>);
+  DITTO_CUDA(cudaLaunchKernelExC(&cfg, fn, args));
   count_launch();
   return 0;
 }

@@ -23,6 +23,8 @@ struct DebugOptions {
   int no_fc2_ln = 0;
   // engine.cu: cross-attention with 64 < S <= 256 text tokens as scores+softmax / P.V / LayerNorm launches instead of flash_attn768q<CROSS>
   int no_cross_flash = 0;
+  // engine.cu (read by ditto_engine_create): sequences with constant text rows go through the cross-attention kernel too
+  int no_const_text = 0;
 };
 extern DebugOptions g_opt;
 
@@ -55,6 +57,13 @@ int launch_silu(float* x, int64_t n, cudaStream_t st);
 int launch_mean_silu(const float* text, float* out, int64_t n, int S, int D, cudaStream_t st);
 int launch_fold_bias(const bf16* kv, int64_t ld, const float* bq, float* sb, int64_t n, int S, int Sp, int heads, int d, float scale,
                      cudaStream_t st);
+// constant text (all S rows of a sequence's text_emb [n, S, D] bitwise equal): flag[seq] (written when flag != nullptr) and,
+// for every sequence, crow[seq] = vfold[seq][0] + bo in the plain column order (vf_perm4: vfold columns in the perm4 order)
+int launch_const_text(const float* text, int64_t n, int S, int D, const bf16* vfold, int64_t vf_seq, bool vf_perm4, const float* bo,
+                      uint8_t* flag, float* crow, int H, cudaStream_t st);
+// number of nonzero bytes of flags[0, n) for the profiler's byte counts; 0 without synchronising unless profiling (which
+// synchronises anyway and is never captured)
+int64_t profiled_nonzero(const uint8_t* flags, int64_t n, cudaStream_t st);
 int launch_transpose_v(const bf16* v, int64_t ld, bf16* vt, int64_t n_seq, int T, int Tp, int heads, int d, cudaStream_t st);
 int launch_cfg_ddpm_update(const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
                            const float* coef, int steps, float w, float* out, int64_t B, int64_t elems_per_seq,
@@ -190,6 +199,9 @@ struct CrossFusedParams {
   // deferred norm2: u is the raw bf16 residual stream, kfold carries gamma2, sbias carries the beta2 term; the scores are
   // rstd (u kfold^T) - rstd mean c + sbias with (sum, sum of squares) partials ln_stat[row * ln_parts + part] over H columns
   const float2* ln_stat = nullptr; int ln_parts = 0; const float* ln_c = nullptr;  // ln_c [n_seq, Sp] like sbias
+  // [n_seq]: tiles of sequences with skip_seq[seq] != 0 are not processed (constant text: the self-attention kernel has
+  // already added their constant cross-attention output and written norm3); nullptr: every tile
+  const uint8_t* skip_seq = nullptr;
   int64_t n_seq = 0, T = 0, S = 0, Sp = 0; int H = 0;
   float alpha = 1.f;
   int tag = PC_TC_OTHER;
@@ -224,13 +236,20 @@ struct Flash768Params {
   int Tk = 0;                                                       // text tokens (<= 256)
   const float* kbias = nullptr; int64_t kb_seq = 0;                 // [n_seq][kb_seq] additive score bias (already scaled)
   const float* out_bias = nullptr;                                  // [768]
-  bool force_rescale = false;                  // tests: take the online-softmax rescale path whenever a tile raises the maximum
+  // constant text (four-CTA kernel only).  Self-attention: sequences with const_flag[seq] != 0 get h <- h + attn + const_row[seq]
+  // and u <- LayerNorm(h) gamma_c + beta_c (norm3: their cross-attention output is the constant row, so the cross-attention
+  // section is done here).  Cross-attention: items of flagged sequences are skipped.  nullptr: off
+  const uint8_t* const_flag = nullptr;
+  const float* const_row = nullptr;                                 // [n_seq][768] fp32, plain column order
+  const float* gamma_c = nullptr; const float* beta_c = nullptr;
+  bool force_rescale = false;                 // tests: take the online-softmax rescale path whenever a tile raises the maximum
   int dbg = 0;                                 // timing experiments (wrong results): ditto_attn_self768 flags >> 8
   int tag = PC_TC_OTHER;
 };
 bool flash768_supported(int H, int heads, int T);
 int launch_flash768(const Flash768Params& p, cudaStream_t st);   // picks the two- or the four-CTA kernel
 bool flash768_quad_preferred(int T);
+bool flash768_picks_quad(int T);   // launch_flash768 takes the four-CTA kernel at this length (constant-text rows need it)
 bool flash768_quad_schedulable();   // four-CTA clusters fit the current device (else the two-CTA kernel is used)
 int launch_flash768_quad(const Flash768Params& p, cudaStream_t st);   // flash_attn768q.cu
 
