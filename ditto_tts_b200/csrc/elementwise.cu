@@ -1,5 +1,5 @@
 // HBM-bound kernels of the DiT denoiser hot path: LayerNorm / AdaLN, RoPE, softmax, gated activation,
-// CFG-combine + DDPM update, q_sample, casts and weight packing.  All coalesced + 128-bit vectorised.
+// CFG-combine + sampler update, q_sample, casts and weight packing.  All coalesced + 128-bit vectorised.
 #include <vector>
 
 #include "kernels.cuh"
@@ -635,9 +635,11 @@ int launch_transpose_v(const bf16* v, int64_t ld, bf16* vt, int64_t n_seq, int T
 }
 
 // =====================================================================================================
-// CFG combine + DDPM ancestral update, one pass (SpeechGenerator.py:137-147 + the guidance extension)
-//   coef[t] = { 1/sqrt(alpha_t), (1-alpha_t)/sqrt(1-acp_t), [t>0]*sqrt(beta_t) }
-// 20 B/element with guidance + noise (4 reads, 1 write), 128-bit accesses, grid = multiple of 148.
+// The sampler update, one pass: CFG combine + DDPM-form or multistep update, optionally with the noise drawn in the kernel and
+// with known frames (launch_cfg_update, kernels.cuh).
+//   DDPM form (SpeechGenerator.py:137-147 + the guidance extension):  x_out = c1 (x - c2 eps) + c3 z
+//     coef[t] = { 1/sqrt(alpha_t), (1-alpha_t)/sqrt(1-acp_t), [t>0]*sqrt(beta_t) } for the reference sampler
+// 20 B/element with guidance + supplied noise (4 reads, 1 write), 128-bit accesses, grid = multiple of 148.
 // =====================================================================================================
 // one element: eps = eps_u + w (eps_c - eps_u);  x_out = c1 (x - c2 eps) + c3 z   -- explicit roundings so that the variant
 // with caller-supplied noise and the one that draws it in the kernel agree bit for bit
@@ -645,52 +647,31 @@ __device__ __forceinline__ float cfg_combine(float ec, float eu, float w) { retu
 __device__ __forceinline__ float ddpm_update(float x, float e, float z, float c1, float c2, float c3) {
   return __fmaf_rn(c3, z, __fmul_rn(c1, __fmaf_rn(-c2, e, x)));
 }
-
-__global__ void __launch_bounds__(256)
-    cfg_ddpm_update_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
-                           const float4* __restrict__ z, const int64_t* __restrict__ t, const float* __restrict__ coef,
-                           int steps, float w, float4* __restrict__ out, int64_t vec_per_seq, int64_t total_vec) {
-  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int64_t seq = i / vec_per_seq;
-    int64_t tt = t[seq];
-    tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
-    const float c1 = coef[tt * 3 + 0], c2 = coef[tt * 3 + 1], c3 = coef[tt * 3 + 2];
-    float4 e = eps_c[i];
-    if (eps_u != nullptr) {
-      const float4 u = eps_u[i];
-      e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
-    }
-    const float4 xv = x[i];
-    const float4 zv = z != nullptr ? z[i] : make_float4(0.f, 0.f, 0.f, 0.f);   // + c3 * 0 == the reference's masked noise term
-    out[i] = make_float4(ddpm_update(xv.x, e.x, zv.x, c1, c2, c3), ddpm_update(xv.y, e.y, zv.y, c1, c2, c3),
-                         ddpm_update(xv.z, e.z, zv.z, c1, c2, c3), ddpm_update(xv.w, e.w, zv.w, c1, c2, c3));
-  }
+__device__ __forceinline__ float4 ddpm_update4(float4 xv, float4 e, float4 zv, float c1, float c2, float c3) {
+  return make_float4(ddpm_update(xv.x, e.x, zv.x, c1, c2, c3), ddpm_update(xv.y, e.y, zv.y, c1, c2, c3),
+                     ddpm_update(xv.z, e.z, zv.z, c1, c2, c3), ddpm_update(xv.w, e.w, zv.w, c1, c2, c3));
 }
-
-int launch_cfg_ddpm_update(const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
-                           const float* coef, int steps, float w, float* out, int64_t B, int64_t elems_per_seq,
-                           cudaStream_t st) {
-  DITTO_REQUIRE(elems_per_seq % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_ddpm_update: elems_per_seq % 4");
-  const int64_t total_vec = B * elems_per_seq / 4;
-  if (total_vec == 0) return 0;
-  const int64_t want = ceil_div(total_vec, 256 * 4);  // ~4 vectors per thread
-  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
-  ProfScope prof(PC_CFG_UPDATE, st, 0.0, static_cast<double>(total_vec) * 16 * (3 + (eps_u ? 1 : 0) + (z ? 1 : 0)));
-  cfg_ddpm_update_kernel<<<blocks, 256, 0, st>>>(
-      reinterpret_cast<const float4*>(eps_c), reinterpret_cast<const float4*>(eps_u), reinterpret_cast<const float4*>(x),
-      reinterpret_cast<const float4*>(z), t, coef, steps, w, reinterpret_cast<float4*>(out), elems_per_seq / 4, total_vec);
-  DITTO_LAUNCH_CHECK();
-  return 0;
+__device__ __forceinline__ float4 guided_eps(const float4* eps_c, const float4* eps_u, int64_t i, float w) {
+  float4 e = eps_c[i];
+  if (eps_u != nullptr) {
+    const float4 u = eps_u[i];
+    e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
+  }
+  return e;
+}
+// supplied noise; without known frames a null z means "no noise term" (+ c3 * 0 == the reference's masked noise term)
+template <bool KNOWN>
+__device__ __forceinline__ float4 supplied_noise(const float4* z, int64_t i) {
+  return (KNOWN || z != nullptr) ? z[i] : make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
 // =====================================================================================================
-// The same with the step's noise drawn in the kernel: z = randn_like(x) of SpeechGenerator.py:145 without the separate
-// generator launch and its 8 B / element of HBM round trip.  Philox4x32-10 (Salmon et al., SC'11: the counter-based generator
-// behind curand and torch's CUDA randn) keyed by the 64-bit seed, counter = (vector index, draw counter); four uniforms ->
-// two Box-Muller pairs -> the four normals of one float4.  The draw counter lives in device memory so that a captured CUDA
-// graph draws fresh noise on every replay; with `advance` the LAST block to finish (ticket counter) adds 1 to it and
-// subtracts 1 from every t[i] -- the bookkeeping of `for t_val in reversed(range(steps))` (SpeechGenerator.py:161-162).
+// Noise drawn in the kernel: z = randn_like(x) of SpeechGenerator.py:145 without the separate generator launch and its
+// 8 B / element of HBM round trip.  Philox4x32-10 (Salmon et al., SC'11: the counter-based generator behind curand and torch's
+// CUDA randn) keyed by the 64-bit seed, counter = (vector index, draw counter); four uniforms -> two Box-Muller pairs -> the
+// four normals of one float4.  The draw counter lives in device memory so that a captured CUDA graph draws fresh noise on
+// every replay; with `advance` the LAST block to finish (ticket counter) adds 1 to it and subtracts 1 from every t[i] -- the
+// bookkeeping of `for t_val in reversed(range(steps))` (SpeechGenerator.py:161-162).
 // rng: device uint64[4] = {seed, draw counter, ticket (kept 0 between launches), reserved}.
 // =====================================================================================================
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
@@ -721,7 +702,7 @@ __device__ __forceinline__ float4 philox_normal4(unsigned long long seed, unsign
   return make_float4(m0 * c0, m0 * s0, m1 * c1, m1 * s1);
 }
 
-// `advance` of the in-kernel-noise update kernels: called by every block after its last read of rng / t
+// `advance` of the in-kernel-noise instances: called by every block after its last read of rng / t
 __device__ __forceinline__ void last_block_advances(unsigned long long* rng, int64_t* t, int64_t n_t, unsigned long long draw) {
   // every thread of every block has read rng / t before its block takes a ticket; the block holding the last ticket owns them
   __shared__ int s_last;
@@ -741,61 +722,18 @@ __device__ __forceinline__ void last_block_advances(unsigned long long* rng, int
   }
 }
 
-__global__ void __launch_bounds__(256)
-    cfg_ddpm_update_rng_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
-                               unsigned long long* rng, int64_t* t, int64_t n_t, const float* __restrict__ coef, int steps, float w,
-                               float4* __restrict__ out, int64_t vec_per_seq, int64_t total_vec, int64_t vec_offset, int advance) {
-  const unsigned long long seed = rng[0], draw = rng[1];
-  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const int64_t seq = i / vec_per_seq;
-    int64_t tt = t[seq];
-    tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
-    const float c1 = coef[tt * 3 + 0], c2 = coef[tt * 3 + 1], c3 = coef[tt * 3 + 2];
-    float4 e = eps_c[i];
-    if (eps_u != nullptr) {
-      const float4 u = eps_u[i];
-      e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
-    }
-    const float4 xv = x[i];
-    const float4 zv = philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i));
-    out[i] = make_float4(ddpm_update(xv.x, e.x, zv.x, c1, c2, c3), ddpm_update(xv.y, e.y, zv.y, c1, c2, c3),
-                         ddpm_update(xv.z, e.z, zv.z, c1, c2, c3), ddpm_update(xv.w, e.w, zv.w, c1, c2, c3));
-  }
-  if (advance) last_block_advances(rng, t, n_t, draw);
-}
-
-int launch_cfg_ddpm_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t, int64_t n_t,
-                               const float* coef, int steps, float w, float* out, int64_t B, int64_t elems_per_seq,
-                               int64_t elem_offset, bool advance, cudaStream_t st) {
-  DITTO_REQUIRE(elems_per_seq % 4 == 0 && elem_offset % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_ddpm_update_rng: elems_per_seq % 4");
-  const int64_t total_vec = B * elems_per_seq / 4;
-  if (total_vec == 0) return advance ? launch_step_advance(rng, t, n_t, st) : 0;
-  const int64_t want = ceil_div(total_vec, 256 * 4);
-  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
-  ProfScope prof(PC_CFG_UPDATE, st, 0.0, static_cast<double>(total_vec) * 16 * (3 + (eps_u ? 1 : 0)));
-  cfg_ddpm_update_rng_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(eps_c), reinterpret_cast<const float4*>(eps_u),
-                                                     reinterpret_cast<const float4*>(x), rng, t, n_t, coef, steps, w,
-                                                     reinterpret_cast<float4*>(out), elems_per_seq / 4, total_vec, elem_offset / 4,
-                                                     advance ? 1 : 0);
-  DITTO_LAUNCH_CHECK();
-  return 0;
-}
-
 // =====================================================================================================
-// CFG combine + multistep update (DPM-Solver++(2M), Lu et al. 2022 Alg. 2, and its SDE variant), one pass:
+// Multistep form (DPM-Solver++(2M), Lu et al. 2022 Alg. 2, and its SDE variant):
 //   x_out = c1 (x - c2 eps) + c3 z + c4 hist        hist <- d1 (x - d2 eps)   (the x0 prediction of this step)
 //   coef_ms[t] = {c1, c2, c3, c4, d1, d2}, computed on the host (schedules.dpmpp_2m_coef).
 // The first term is ddpm_update with the same roundings, the history term one more fma; a row with c4 == 0 (first-order
-// steps) neither reads hist nor adds the term, so x_out is bit-identical to cfg_ddpm_update_kernel with (c1, c2, c3) and
-// whatever hist held before the first step (uninitialised, NaN) cannot reach it.  c4 is uniform per sequence (one row per
-// t[seq]), so the branch does not diverge inside a sequence's vectors.  x_out may alias x and hist is updated in place:
-// every thread reads its elements before it writes them.  +8 B / element over the DDPM kernel (hist read + write).
+// steps) neither reads hist nor adds the term, so x_out is bit-identical to the DDPM form with (c1, c2, c3) and whatever hist
+// held before the first step (uninitialised, NaN) cannot reach it.  c4 is uniform per sequence (one row per t[seq]), so the
+// branch does not diverge inside a sequence's vectors.  x_out may alias x and hist is updated in place: every thread reads its
+// elements before it writes them.  +8 B / element over the DDPM form (hist read + write).
 // =====================================================================================================
 __device__ __forceinline__ float x0_pred(float x, float e, float d1, float d2) { return __fmul_rn(d1, __fmaf_rn(-d2, e, x)); }
 
-// one row of the table; the hist read is issued together with the other loads of the element (before the noise is drawn),
-// predicated on c4 so that first-order rows never touch it
 struct MultistepRow {
   float c1, c2, c3, c4, d1, d2;
 };
@@ -805,13 +743,14 @@ __device__ __forceinline__ MultistepRow multistep_row(const float* __restrict__ 
   const float* r = coef + tt * 6;
   return MultistepRow{r[0], r[1], r[2], r[3], r[4], r[5]};
 }
+// issued together with the other loads of the element (before the noise is drawn: loading it after the draw made a C4 step
+// 4x slower), predicated on c4 so that first-order rows never touch it
 __device__ __forceinline__ float4 multistep_hist(const float4* __restrict__ hist, int64_t i, float c4) {
   return c4 != 0.f ? hist[i] : make_float4(0.f, 0.f, 0.f, 0.f);
 }
 __device__ __forceinline__ void multistep_store(const MultistepRow& c, float4 xv, float4 e, float4 zv, float4 h,
                                                 float4* __restrict__ out, float4* __restrict__ hist, int64_t i) {
-  float4 o = make_float4(ddpm_update(xv.x, e.x, zv.x, c.c1, c.c2, c.c3), ddpm_update(xv.y, e.y, zv.y, c.c1, c.c2, c.c3),
-                         ddpm_update(xv.z, e.z, zv.z, c.c1, c.c2, c.c3), ddpm_update(xv.w, e.w, zv.w, c.c1, c.c2, c.c3));
+  float4 o = ddpm_update4(xv, e, zv, c.c1, c.c2, c.c3);
   if (c.c4 != 0.f)
     o = make_float4(__fmaf_rn(c.c4, h.x, o.x), __fmaf_rn(c.c4, h.y, o.y), __fmaf_rn(c.c4, h.z, o.z), __fmaf_rn(c.c4, h.w, o.w));
   hist[i] = make_float4(x0_pred(xv.x, e.x, c.d1, c.d2), x0_pred(xv.y, e.y, c.d1, c.d2), x0_pred(xv.z, e.z, c.d1, c.d2),
@@ -819,116 +758,41 @@ __device__ __forceinline__ void multistep_store(const MultistepRow& c, float4 xv
   out[i] = o;
 }
 
-__global__ void __launch_bounds__(256)
-    cfg_multistep_update_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
-                                const float4* __restrict__ z, const int64_t* __restrict__ t, const float* __restrict__ coef,
-                                int steps, float w, float4* __restrict__ out, float4* __restrict__ hist, int64_t vec_per_seq,
-                                int64_t total_vec) {
-  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const MultistepRow c = multistep_row(coef, t, i / vec_per_seq, steps);
-    float4 e = eps_c[i];
-    if (eps_u != nullptr) {
-      const float4 u = eps_u[i];
-      e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
-    }
-    const float4 xv = x[i];
-    const float4 zv = z != nullptr ? z[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-    const float4 h = multistep_hist(hist, i, c.c4);
-    multistep_store(c, xv, e, zv, h, out, hist, i);
-  }
-}
-
-int launch_cfg_multistep_update(const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
-                                const float* coef, int steps, float w, float* out, float* hist, int64_t B, int64_t elems_per_seq,
-                                cudaStream_t st) {
-  DITTO_REQUIRE(elems_per_seq % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_multistep_update: elems_per_seq % 4");
-  const int64_t total_vec = B * elems_per_seq / 4;
-  if (total_vec == 0) return 0;
-  const int64_t want = ceil_div(total_vec, 256 * 4);
-  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
-  ProfScope prof(PC_CFG_UPDATE, st, 0.0, static_cast<double>(total_vec) * 16 * (5 + (eps_u ? 1 : 0) + (z ? 1 : 0)));
-  cfg_multistep_update_kernel<<<blocks, 256, 0, st>>>(
-      reinterpret_cast<const float4*>(eps_c), reinterpret_cast<const float4*>(eps_u), reinterpret_cast<const float4*>(x),
-      reinterpret_cast<const float4*>(z), t, coef, steps, w, reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(hist),
-      elems_per_seq / 4, total_vec);
-  DITTO_LAUNCH_CHECK();
-  return 0;
-}
-
-// the same with the noise drawn in the kernel: Philox stream, element offsets and `advance` bookkeeping exactly as
-// cfg_ddpm_update_rng_kernel (the normals equal ditto_randn's at the same {seed, draw})
-__global__ void __launch_bounds__(256)
-    cfg_multistep_update_rng_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
-                                    unsigned long long* rng, int64_t* t, int64_t n_t, const float* __restrict__ coef, int steps,
-                                    float w, float4* __restrict__ out, float4* __restrict__ hist, int64_t vec_per_seq,
-                                    int64_t total_vec, int64_t vec_offset, int advance) {
-  const unsigned long long seed = rng[0], draw = rng[1];
-  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
-       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-    const MultistepRow c = multistep_row(coef, t, i / vec_per_seq, steps);
-    float4 e = eps_c[i];
-    if (eps_u != nullptr) {
-      const float4 u = eps_u[i];
-      e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
-    }
-    const float4 xv = x[i];
-    const float4 h = multistep_hist(hist, i, c.c4);
-    const float4 zv = philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i));
-    multistep_store(c, xv, e, zv, h, out, hist, i);
-  }
-  if (advance) last_block_advances(rng, t, n_t, draw);
-}
-
-int launch_cfg_multistep_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t,
-                                    int64_t n_t, const float* coef, int steps, float w, float* out, float* hist, int64_t B,
-                                    int64_t elems_per_seq, int64_t elem_offset, bool advance, cudaStream_t st) {
-  DITTO_REQUIRE(elems_per_seq % 4 == 0 && elem_offset % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_multistep_update_rng: elems_per_seq % 4");
-  const int64_t total_vec = B * elems_per_seq / 4;
-  if (total_vec == 0) return advance ? launch_step_advance(rng, t, n_t, st) : 0;
-  const int64_t want = ceil_div(total_vec, 256 * 4);
-  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
-  ProfScope prof(PC_CFG_UPDATE, st, 0.0, static_cast<double>(total_vec) * 16 * (5 + (eps_u ? 1 : 0)));
-  cfg_multistep_update_rng_kernel<<<blocks, 256, 0, st>>>(
-      reinterpret_cast<const float4*>(eps_c), reinterpret_cast<const float4*>(eps_u), reinterpret_cast<const float4*>(x), rng, t,
-      n_t, coef, steps, w, reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(hist), elems_per_seq / 4, total_vec,
-      elem_offset / 4, advance ? 1 : 0);
-  DITTO_LAUNCH_CHECK();
-  return 0;
-}
-
 // =====================================================================================================
-// CFG combine + update with known frames (replacement conditioning: a speech prompt or an infilled span; the imputation
-// of Song et al. 2021, score SDE, i.e. RePaint without its resampling loop), one pass.  A frame flagged in `mask` is
-// the known latent p re-noised to the level of this step's output,
+// Known frames (replacement conditioning: a speech prompt or an infilled span; the imputation of Song et al. 2021, score SDE,
+// i.e. RePaint without its resampling loop).  A frame flagged in `mask` is the known latent p re-noised to the level of this
+// step's output,
 //     x_out = a p + s z,   coef_known[t] = {a, s} = {sqrt(abar_next), sqrt(1 - abar_next)}   (last visited step: {1, 0} -> p)
-// with z the normal the update draws (or is given) for that element, so the draw counter and its bookkeeping are those of
-// the plain update.  Every other frame takes the DDPM-form (MULTISTEP = false) or multistep update through the same device
-// helpers as cfg_ddpm_update(_rng)_kernel / cfg_multistep_update(_rng)_kernel, so it rounds exactly as they do.  A frame is
-// H/4 consecutive float4s (6 warps at H = 768), so the branch is uniform per warp when H % 128 == 0.  A known frame reads
-// the mask byte, p and (supplied noise) z -- no eps, x or hist -- and leaves hist as it was: 8 B / element with drawn noise
-// (12 with supplied z) against 16-28 B for an unknown one.  All loads are issued before the noise is drawn.
+// with z the normal the update draws (or is given) for that element, so the draw counter and its bookkeeping are those of the
+// plain update.  Every other frame takes the update above unchanged.  A frame is H/4 consecutive float4s (6 warps at H = 768),
+// so the branch is uniform per warp when H % 128 == 0.  A known frame reads the mask byte, p and (supplied noise) z -- no eps,
+// x or hist -- and leaves hist as it was: 8 B / element with drawn noise (12 with supplied z) against 16-28 B for an unknown one.
 // =====================================================================================================
 __device__ __forceinline__ float known_value(float p, float z, float a, float s) { return __fmaf_rn(s, z, __fmul_rn(a, p)); }
 
-template <bool MULTISTEP, bool RNG>
+// One instance per (form, noise source, known frames).  Loads in the order t row, eps_c, eps_u, x, supplied z, hist, then the
+// draw.  t_in == t.  The instances without rng and without known frames read t through t_in, whose __restrict__ keeps that
+// load on the read-only path (LDG.CONSTANT; a pointer the rng instances write loses it); the others read it through t.  The
+// t clamps stay written out in place: moving them into a helper changes how the multistep loop is unrolled.
+template <bool MULTISTEP, bool RNG, bool KNOWN>
 __global__ void __launch_bounds__(256)
-    cfg_update_known_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
-                            const float4* __restrict__ z, unsigned long long* rng, int64_t* t, int64_t n_t,
-                            const float* __restrict__ coef, const float* __restrict__ coef_known, int steps, float w,
-                            float4* __restrict__ out, float4* __restrict__ hist, const float4* __restrict__ known,
-                            const uint8_t* __restrict__ mask, int64_t vec_per_seq, int64_t vec_per_frame, int64_t total_vec,
-                            int64_t vec_offset, int advance) {
+    cfg_update_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
+                      const float4* __restrict__ z, const int64_t* __restrict__ t_in, unsigned long long* rng, int64_t* t, int64_t n_t,
+                      const float* __restrict__ coef, const float* __restrict__ coef_known, int steps, float w,
+                      float4* __restrict__ out, float4* __restrict__ hist, const float4* __restrict__ known,
+                      const uint8_t* __restrict__ mask, int64_t vec_per_seq, int64_t vec_per_frame, int64_t total_vec,
+                      int64_t vec_offset, int advance) {
   unsigned long long seed = 0ull, draw = 0ull;
   if (RNG) {
     seed = rng[0];
     draw = rng[1];
   }
+  const int64_t* ts = (RNG || KNOWN) ? t : t_in;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int64_t seq = i / vec_per_seq;
-    if (mask[i / vec_per_frame] != 0) {
-      int64_t tt = t[seq];
+    if (KNOWN && mask[i / vec_per_frame] != 0) {
+      int64_t tt = ts[seq];
       tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
       const float a = coef_known[tt * 2 + 0], s = coef_known[tt * 2 + 1];
       const float4 pv = known[i];
@@ -938,30 +802,21 @@ __global__ void __launch_bounds__(256)
       continue;
     }
     if (MULTISTEP) {
-      const MultistepRow c = multistep_row(coef, t, seq, steps);
-      float4 e = eps_c[i];
-      if (eps_u != nullptr) {
-        const float4 u = eps_u[i];
-        e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
-      }
+      const MultistepRow c = multistep_row(coef, ts, seq, steps);
+      const float4 e = guided_eps(eps_c, eps_u, i, w);
       const float4 xv = x[i];
-      float4 zv = RNG ? make_float4(0.f, 0.f, 0.f, 0.f) : z[i];
+      float4 zv = RNG ? make_float4(0.f, 0.f, 0.f, 0.f) : supplied_noise<KNOWN>(z, i);
       const float4 h = multistep_hist(hist, i, c.c4);
       if (RNG) zv = philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i));
       multistep_store(c, xv, e, zv, h, out, hist, i);
     } else {
-      int64_t tt = t[seq];
+      int64_t tt = ts[seq];
       tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
       const float c1 = coef[tt * 3 + 0], c2 = coef[tt * 3 + 1], c3 = coef[tt * 3 + 2];
-      float4 e = eps_c[i];
-      if (eps_u != nullptr) {
-        const float4 u = eps_u[i];
-        e = make_float4(cfg_combine(e.x, u.x, w), cfg_combine(e.y, u.y, w), cfg_combine(e.z, u.z, w), cfg_combine(e.w, u.w, w));
-      }
+      const float4 e = guided_eps(eps_c, eps_u, i, w);
       const float4 xv = x[i];
-      const float4 zv = RNG ? philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i)) : z[i];
-      out[i] = make_float4(ddpm_update(xv.x, e.x, zv.x, c1, c2, c3), ddpm_update(xv.y, e.y, zv.y, c1, c2, c3),
-                           ddpm_update(xv.z, e.z, zv.z, c1, c2, c3), ddpm_update(xv.w, e.w, zv.w, c1, c2, c3));
+      const float4 zv = RNG ? philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i)) : supplied_noise<KNOWN>(z, i);
+      out[i] = ddpm_update4(xv, e, zv, c1, c2, c3);
     }
   }
   if (RNG && advance) last_block_advances(rng, t, n_t, draw);
@@ -980,40 +835,32 @@ int64_t profiled_nonzero(const uint8_t* mask, int64_t n, cudaStream_t st) {
   return k;
 }
 
-int launch_cfg_update_known(const float* eps_c, const float* eps_u, const float* x, const float* z, unsigned long long* rng, int64_t* t,
-                            int64_t n_t, const float* coef, const float* coef_known, int steps, float w, float* out, float* hist,
-                            const float* known, const uint8_t* mask, int64_t B, int64_t T, int64_t H, int64_t elem_offset, bool advance,
-                            cudaStream_t st) {
-  DITTO_REQUIRE(H % 4 == 0 && elem_offset % 4 == 0, DITTO_E_UNSUPPORTED, "cfg_update_known: H % 4 and element offset % 4");
-  const bool draw = rng != nullptr, ms = hist != nullptr;
-  const int64_t vec_per_frame = H / 4, total_vec = B * T * vec_per_frame;
-  if (total_vec == 0) return (draw && advance) ? launch_step_advance(rng, t, n_t, st) : 0;
-  const int64_t want = ceil_div(total_vec, 256 * 4);
+int launch_cfg_update(const CfgUpdateParams& p, cudaStream_t st) {
+  const bool ms = p.hist != nullptr, draw = p.rng != nullptr, kn = p.mask != nullptr;
+  DITTO_REQUIRE(p.per % 4 == 0 && p.elem_offset % 4 == 0 && (!kn || (p.frame % 4 == 0 && p.frame > 0 && p.per % p.frame == 0)),
+                DITTO_E_UNSUPPORTED, "cfg_update: elements per sequence, per frame and the element offset must be multiples of 4");
+  const int64_t total_vec = p.B * p.per / 4;
+  if (total_vec == 0) return (draw && p.advance) ? launch_step_advance(p.rng, p.t, p.n_t, st) : 0;
+  const int64_t want = ceil_div(total_vec, 256 * 4);  // ~4 vectors per thread
   const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(want, 148), 148 * 32));
-  // bytes moved: 16 B per float4 of every stream a frame touches, plus one mask byte per frame
-  const int64_t known_vec = profiled_nonzero(mask, B * T, st) * vec_per_frame;
-  const double unknown_streams = (ms ? 5 : 3) + (eps_u ? 1 : 0) + (draw ? 0 : 1), known_streams = 2 + (draw ? 0 : 1);
+  // bytes moved: 16 B per float4 of every stream a vector touches, plus one mask byte per frame
+  const int64_t frames = kn ? p.B * p.per / p.frame : 0, known_vec = kn ? profiled_nonzero(p.mask, frames, st) * (p.frame / 4) : 0;
+  const double unknown_streams = (ms ? 5 : 3) + (p.eps_u ? 1 : 0) + (p.z ? 1 : 0), known_streams = 2 + (p.z ? 1 : 0);
   ProfScope prof(PC_CFG_UPDATE, st, 0.0,
                  16.0 * (static_cast<double>(total_vec - known_vec) * unknown_streams + static_cast<double>(known_vec) * known_streams) +
-                     static_cast<double>(B * T));
-  const float4 *ec = reinterpret_cast<const float4*>(eps_c), *eu = reinterpret_cast<const float4*>(eps_u);
-  const float4 *xv = reinterpret_cast<const float4*>(x), *zv = reinterpret_cast<const float4*>(z);
-  const float4* kv = reinterpret_cast<const float4*>(known);
-  float4 *o = reinterpret_cast<float4*>(out), *h = reinterpret_cast<float4*>(hist);
-  const int64_t vps = T * vec_per_frame, voff = elem_offset / 4;
-  const int adv = advance ? 1 : 0;
-  if (ms && draw)
-    cfg_update_known_kernel<true, true><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv, mask,
-                                                                vps, vec_per_frame, total_vec, voff, adv);
-  else if (ms)
-    cfg_update_known_kernel<true, false><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv, mask,
-                                                                 vps, vec_per_frame, total_vec, voff, adv);
-  else if (draw)
-    cfg_update_known_kernel<false, true><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv, mask,
-                                                                 vps, vec_per_frame, total_vec, voff, adv);
-  else
-    cfg_update_known_kernel<false, false><<<blocks, 256, 0, st>>>(ec, eu, xv, zv, rng, t, n_t, coef, coef_known, steps, w, o, h, kv,
-                                                                  mask, vps, vec_per_frame, total_vec, voff, adv);
+                     static_cast<double>(frames));
+  using Kernel = void (*)(const float4*, const float4*, const float4*, const float4*, const int64_t*, unsigned long long*, int64_t*,
+                          int64_t, const float*, const float*, int, float, float4*, float4*, const float4*, const uint8_t*, int64_t,
+                          int64_t, int64_t, int64_t, int);
+  static const Kernel kernels[8] = {cfg_update_kernel<false, false, false>, cfg_update_kernel<false, false, true>,
+                                    cfg_update_kernel<false, true, false>,  cfg_update_kernel<false, true, true>,
+                                    cfg_update_kernel<true, false, false>,  cfg_update_kernel<true, false, true>,
+                                    cfg_update_kernel<true, true, false>,   cfg_update_kernel<true, true, true>};
+  kernels[(ms ? 4 : 0) + (draw ? 2 : 0) + (kn ? 1 : 0)]<<<blocks, 256, 0, st>>>(
+      reinterpret_cast<const float4*>(p.eps_c), reinterpret_cast<const float4*>(p.eps_u), reinterpret_cast<const float4*>(p.x),
+      reinterpret_cast<const float4*>(p.z), p.t, p.rng, p.t, p.n_t, p.coef, p.coef_known, p.steps, p.w,
+      reinterpret_cast<float4*>(p.out), reinterpret_cast<float4*>(p.hist), reinterpret_cast<const float4*>(p.known), p.mask,
+      p.per / 4, p.frame / 4, total_vec, p.elem_offset / 4, p.advance ? 1 : 0);
   DITTO_LAUNCH_CHECK();
   return 0;
 }

@@ -1262,165 +1262,151 @@ int32_t ditto_forward(ditto_engine_t* e, const float* x, int64_t n_x, const void
   return forward_impl(e, x, n_x, ctx, t, n_seq, T, S, out, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
-int32_t ditto_cfg_ddpm_update(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
-                              const int64_t* t, float guidance_scale, float* x_out, int64_t B, int64_t elems_per_seq, void* stream) {
-  DITTO_REQUIRE(e && eps_c && x && t && x_out, DITTO_E_BADARG, "cfg_ddpm_update: null argument");
-  DITTO_REQUIRE(e->have_schedule, DITTO_E_STATE, "cfg_ddpm_update: schedule not loaded");
-  DITTO_REQUIRE(B >= 0 && elems_per_seq >= 0, DITTO_E_BADARG, "cfg_ddpm_update: negative size");
-  return launch_cfg_ddpm_update(eps_c, eps_u, x, z, t, e->coef, e->steps, guidance_scale, x_out, B, elems_per_seq,
-                                static_cast<cudaStream_t>(stream));
-}
+// ---- sampler updates and steps ---------------------------------------------------------------------------------
+// What one sampler update takes besides eps, x and t.  The extern "C" update and sampler calls differ only in which of these
+// they accept: each forwards to update_call, p_sample_dense or p_sample_ragged with the others fixed.
+struct Update {
+  const float* z = nullptr;        // supplied noise; null with rng (drawn in the kernel) or, where allowed, for no noise term
+  uint64_t* rng = nullptr;         // in-kernel noise {seed, draw counter, ticket, -}
+  float* hist = nullptr;           // the multistep update's x0 history; null: the DDPM-form update
+  const float* known = nullptr;    // latents of the known frames, with one mask byte per frame; both null: no known frame
+  const uint8_t* mask = nullptr;
+  int32_t advance = 0;             // t -= 1 and draw counter += 1 after the update (needs rng)
+  bool multistep = false;          // a multistep call: hist is required
+  bool need_noise = false;         // exactly one of z / rng is required
+};
 
-// the update of one sampler step: the [steps, 3] DDPM-form table, or (hist != null) the [steps, 6] multistep table
-static int launch_update(const ditto_engine* e, const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
-                         float w, float* x_out, float* hist, int64_t B, int64_t per, cudaStream_t st) {
-  if (hist) return launch_cfg_multistep_update(eps_c, eps_u, x, z, t, e->coef_ms, e->steps, w, x_out, hist, B, per, st);
-  return launch_cfg_ddpm_update(eps_c, eps_u, x, z, t, e->coef, e->steps, w, x_out, B, per, st);
-}
-static int launch_update_rng(const ditto_engine* e, const float* eps_c, const float* eps_u, const float* x, uint64_t* rng, int64_t* t,
-                             int64_t n_t, float w, float* x_out, float* hist, int64_t B, int64_t per, int64_t elem_offset, bool advance,
-                             cudaStream_t st) {
-  unsigned long long* r = reinterpret_cast<unsigned long long*>(rng);
-  if (hist)
-    return launch_cfg_multistep_update_rng(eps_c, eps_u, x, r, t, n_t, e->coef_ms, e->steps, w, x_out, hist, B, per, elem_offset, advance, st);
-  return launch_cfg_ddpm_update_rng(eps_c, eps_u, x, r, t, n_t, e->coef, e->steps, w, x_out, B, per, elem_offset, advance, st);
-}
-// what every multistep entry point checks on top of its DDPM-form twin
-static int require_multistep(const ditto_engine* e, const float* hist, const char* what) {
-  DITTO_REQUIRE(e && hist, DITTO_E_BADARG, std::string(what) + ": null argument (hist)");
-  DITTO_REQUIRE(e->coef_ms, DITTO_E_STATE, std::string(what) + ": no multistep table loaded (ditto_engine_load_multistep_table)");
+// the checks on the update's own arguments, after the caller's null-argument and size checks: bad arguments (-1) first, then
+// missing engine state (-4)
+static int check_update(const ditto_engine* e, const std::string& what, const Update& u) {
+  DITTO_REQUIRE(!u.multistep || u.hist, DITTO_E_BADARG, what + ": null argument (hist)");
+  DITTO_REQUIRE((u.known == nullptr) == (u.mask == nullptr), DITTO_E_BADARG, what + ": known and known_mask go together (both or neither)");
+  DITTO_REQUIRE(!(u.z && u.rng) && (u.z || u.rng || !u.need_noise), DITTO_E_BADARG,
+                what + ": exactly one of z / rng (known frames need the step's noise)");
+  DITTO_REQUIRE(!u.advance || u.rng, DITTO_E_BADARG, what + ": advance needs rng (in-kernel noise)");
+  DITTO_REQUIRE(e->have_schedule, DITTO_E_STATE, what + ": schedule not loaded");
+  DITTO_REQUIRE(!u.known || e->coef_known, DITTO_E_STATE, what + ": no known table loaded (ditto_engine_load_known_table)");
+  DITTO_REQUIRE(!u.hist || e->coef_ms, DITTO_E_STATE, what + ": no multistep table loaded (ditto_engine_load_multistep_table)");
   return 0;
 }
 
-static int32_t p_sample_impl(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
-                             float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
-                             void* workspace, int64_t workspace_bytes, void* stream) {
-  DITTO_REQUIRE(e && x && ctx && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample: null argument");
-  DITTO_REQUIRE(e->finalized && e->have_schedule && !e->blocks_only, DITTO_E_STATE, "p_sample: engine not finalized / schedule not loaded");
-  DITTO_REQUIRE(B > 0 && T > 0 && S > 0 && T <= e->maxT, DITTO_E_BADARG, "p_sample: bad sizes");
+// the calls that run the whole model: a blocks-only engine holds no proj_in, t embedding or AdaLN weights
+static int require_model(const ditto_engine* e, const std::string& what) {
+  DITTO_REQUIRE(e->finalized && !e->blocks_only, DITTO_E_STATE, what + ": engine not finalized (or a blocks-only engine)");
+  return 0;
+}
+
+// one update of B sequences of `per` elements (x, z, hist, known packed like x_out; one mask byte per H elements); t [n_t];
+// the in-kernel noise of element i is the normal of element elem_offset + i
+static int update(const ditto_engine* e, const float* eps_c, const float* eps_u, const float* x, int64_t* t, int64_t n_t, float w,
+                  float* x_out, const Update& u, int64_t B, int64_t per, int64_t elem_offset, cudaStream_t st) {
+  CfgUpdateParams p;
+  p.eps_c = eps_c; p.eps_u = eps_u; p.x = x; p.z = u.z; p.rng = reinterpret_cast<unsigned long long*>(u.rng);
+  p.t = t; p.n_t = n_t; p.coef = u.hist ? e->coef_ms : e->coef; p.coef_known = e->coef_known; p.steps = e->steps; p.w = w;
+  p.out = x_out; p.hist = u.hist; p.known = u.known; p.mask = u.mask;
+  p.B = B; p.per = per; p.frame = e->H; p.elem_offset = elem_offset; p.advance = u.advance != 0;
+  return launch_cfg_update(p, st);
+}
+
+// the update on its own (the ditto_cfg_*update* calls)
+static int32_t update_call(ditto_engine_t* e, const char* what, const float* eps_c, const float* eps_u, const float* x, int64_t* t,
+                           int64_t n_t, float w, float* x_out, int64_t B, int64_t per, const Update& u, void* stream) {
+  const std::string s(what);
+  DITTO_REQUIRE(e && eps_c && x && t && x_out, DITTO_E_BADARG, s + ": null argument");
+  DITTO_REQUIRE(B >= 0 && per >= 0 && (!u.rng || n_t >= B), DITTO_E_BADARG, s + ": bad sizes");
+  DITTO_TRY(check_update(e, s, u));
+  return update(e, eps_c, eps_u, x, t, n_t, w, x_out, u, B, per, 0, static_cast<cudaStream_t>(stream));
+}
+
+// one sampler step (SpeechGenerator.__p_sample + CFG): the forward on (guided ? 2B : B) sequences sharing x, then the update,
+// which also does the bookkeeping of advance
+static int32_t p_sample_dense(ditto_engine_t* e, const char* what, const float* x, const void* ctx, int64_t* t, int32_t guided, float w,
+                              int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, const Update& u, void* workspace,
+                              int64_t workspace_bytes, void* stream) {
+  const std::string s(what);
+  DITTO_REQUIRE(e && x && ctx && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, s + ": null argument");
+  DITTO_TRY(require_model(e, s));
+  DITTO_REQUIRE(B > 0 && T > 0 && S > 0 && T <= e->maxT, DITTO_E_BADARG, s + ": bad sizes");
+  DITTO_TRY(check_update(e, s, u));
   const int64_t n = guided ? 2 * B : B;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DITTO_TRY(forward_impl(e, x, B, ctx, t, n, T, S, eps_scratch, workspace, workspace_bytes, st));
   const int64_t per = T * e->H;
-  return launch_update(e, eps_scratch, guided ? eps_scratch + B * per : nullptr, x, z, t, guidance_scale, x_out, hist, B, per, st);
+  return update(e, eps_scratch, guided ? eps_scratch + B * per : nullptr, x, t, n, w, x_out, u, B, per, 0, st);
 }
 
-int32_t ditto_p_sample(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
-                       float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
-                       int64_t workspace_bytes, void* stream) {
-  return p_sample_impl(e, x, ctx, t, z, guided, guidance_scale, B, T, S, eps_scratch, x_out, nullptr, workspace, workspace_bytes, stream);
-}
-
-int32_t ditto_p_sample_multistep(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
-                                 float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
-                                 void* workspace, int64_t workspace_bytes, void* stream) {
-  DITTO_TRY(require_multistep(e, hist, "p_sample_multistep"));
-  return p_sample_impl(e, x, ctx, t, z, guided, guidance_scale, B, T, S, eps_scratch, x_out, hist, workspace, workspace_bytes, stream);
-}
-
-static int32_t p_sample_rng_impl(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
-                                 float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
-                                 void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
-  DITTO_REQUIRE(e && x && ctx && t && rng && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_rng: null argument");
-  DITTO_REQUIRE(e->finalized && e->have_schedule && !e->blocks_only, DITTO_E_STATE, "p_sample_rng: engine not finalized / schedule not loaded");
-  DITTO_REQUIRE(B > 0 && T > 0 && S > 0 && T <= e->maxT, DITTO_E_BADARG, "p_sample_rng: bad sizes");
-  const int64_t n = guided ? 2 * B : B;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  DITTO_TRY(forward_impl(e, x, B, ctx, t, n, T, S, eps_scratch, workspace, workspace_bytes, st));
-  const int64_t per = T * e->H;
-  return launch_update_rng(e, eps_scratch, guided ? eps_scratch + B * per : nullptr, x, rng, t, n, guidance_scale, x_out, hist, B, per, 0,
-                           advance != 0, st);
-}
-
-int32_t ditto_p_sample_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
-                           float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
-                           int64_t workspace_bytes, int32_t advance, void* stream) {
-  return p_sample_rng_impl(e, x, ctx, t, rng, guided, guidance_scale, B, T, S, eps_scratch, x_out, nullptr, workspace, workspace_bytes,
-                           advance, stream);
-}
-
-int32_t ditto_p_sample_multistep_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
-                                     float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
-                                     void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
-  DITTO_TRY(require_multistep(e, hist, "p_sample_multistep_rng"));
-  return p_sample_rng_impl(e, x, ctx, t, rng, guided, guidance_scale, B, T, S, eps_scratch, x_out, hist, workspace, workspace_bytes,
-                           advance, stream);
+// t is written only with advance, which the calls taking a const t do not have
+int32_t ditto_cfg_ddpm_update(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
+                              const int64_t* t, float guidance_scale, float* x_out, int64_t B, int64_t elems_per_seq, void* stream) {
+  return update_call(e, "cfg_ddpm_update", eps_c, eps_u, x, const_cast<int64_t*>(t), B, guidance_scale, x_out, B, elems_per_seq,
+                     Update{.z = z}, stream);
 }
 
 int32_t ditto_cfg_ddpm_update_rng(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, uint64_t* rng, int64_t* t,
                                   int64_t n_t, float guidance_scale, float* x_out, int64_t B, int64_t elems_per_seq, int32_t advance,
                                   void* stream) {
-  DITTO_REQUIRE(e && eps_c && x && t && rng && x_out, DITTO_E_BADARG, "cfg_ddpm_update_rng: null argument");
-  DITTO_REQUIRE(e->have_schedule, DITTO_E_STATE, "cfg_ddpm_update_rng: schedule not loaded");
-  DITTO_REQUIRE(B >= 0 && elems_per_seq >= 0 && n_t >= B, DITTO_E_BADARG, "cfg_ddpm_update_rng: bad sizes");
-  return launch_cfg_ddpm_update_rng(eps_c, eps_u, x, reinterpret_cast<unsigned long long*>(rng), t, n_t, e->coef, e->steps, guidance_scale,
-                                    x_out, B, elems_per_seq, 0, advance != 0, static_cast<cudaStream_t>(stream));
+  return update_call(e, "cfg_ddpm_update_rng", eps_c, eps_u, x, t, n_t, guidance_scale, x_out, B, elems_per_seq,
+                     Update{.rng = rng, .advance = advance, .need_noise = true}, stream);
 }
 
 int32_t ditto_cfg_multistep_update(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
                                    const int64_t* t, float guidance_scale, float* x_out, float* hist, int64_t B, int64_t elems_per_seq,
                                    void* stream) {
-  DITTO_REQUIRE(e && eps_c && x && t && x_out, DITTO_E_BADARG, "cfg_multistep_update: null argument");
-  DITTO_REQUIRE(B >= 0 && elems_per_seq >= 0, DITTO_E_BADARG, "cfg_multistep_update: negative size");
-  DITTO_TRY(require_multistep(e, hist, "cfg_multistep_update"));
-  return launch_update(e, eps_c, eps_u, x, z, t, guidance_scale, x_out, hist, B, elems_per_seq, static_cast<cudaStream_t>(stream));
+  return update_call(e, "cfg_multistep_update", eps_c, eps_u, x, const_cast<int64_t*>(t), B, guidance_scale, x_out, B, elems_per_seq,
+                     Update{.z = z, .hist = hist, .multistep = true}, stream);
 }
 
 int32_t ditto_cfg_multistep_update_rng(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, uint64_t* rng,
                                        int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist, int64_t B,
                                        int64_t elems_per_seq, int32_t advance, void* stream) {
-  DITTO_REQUIRE(e && eps_c && x && t && rng && x_out, DITTO_E_BADARG, "cfg_multistep_update_rng: null argument");
-  DITTO_REQUIRE(B >= 0 && elems_per_seq >= 0 && n_t >= B, DITTO_E_BADARG, "cfg_multistep_update_rng: bad sizes");
-  DITTO_TRY(require_multistep(e, hist, "cfg_multistep_update_rng"));
-  return launch_update_rng(e, eps_c, eps_u, x, rng, t, n_t, guidance_scale, x_out, hist, B, elems_per_seq, 0, advance != 0,
-                           static_cast<cudaStream_t>(stream));
-}
-
-// ---- known frames (speech prompt / infilling) -----------------------------------------------------------
-// what every known-frame entry point checks before it launches anything
-static int require_known(const ditto_engine* e, const float* z, const uint64_t* rng, const float* hist, const float* known,
-                         const uint8_t* known_mask, int32_t advance, const char* what) {
-  const std::string w(what);
-  DITTO_REQUIRE(e && known && known_mask, DITTO_E_BADARG, w + ": null argument (known / known_mask)");
-  DITTO_REQUIRE((z == nullptr) != (rng == nullptr), DITTO_E_BADARG, w + ": exactly one of z / rng (known frames need the step's noise)");
-  DITTO_REQUIRE(!advance || rng, DITTO_E_BADARG, w + ": advance needs rng (in-kernel noise)");
-  DITTO_REQUIRE(e->have_schedule, DITTO_E_STATE, w + ": schedule not loaded");
-  DITTO_REQUIRE(e->coef_known, DITTO_E_STATE, w + ": no known table loaded (ditto_engine_load_known_table)");
-  DITTO_REQUIRE(!hist || e->coef_ms, DITTO_E_STATE, w + ": no multistep table loaded (ditto_engine_load_multistep_table)");
-  return 0;
-}
-// the update of one step with known frames: the DDPM-form table, or (hist != null) the multistep table
-static int launch_update_known(const ditto_engine* e, const float* eps_c, const float* eps_u, const float* x, const float* z, uint64_t* rng,
-                               int64_t* t, int64_t n_t, float w, float* x_out, float* hist, const float* known, const uint8_t* mask,
-                               int64_t B, int64_t T, int64_t elem_offset, bool advance, cudaStream_t st) {
-  return launch_cfg_update_known(eps_c, eps_u, x, z, reinterpret_cast<unsigned long long*>(rng), t, n_t, hist ? e->coef_ms : e->coef,
-                                 e->coef_known, e->steps, w, x_out, hist, known, mask, B, T, e->H, elem_offset, advance, st);
+  return update_call(e, "cfg_multistep_update_rng", eps_c, eps_u, x, t, n_t, guidance_scale, x_out, B, elems_per_seq,
+                     Update{.rng = rng, .hist = hist, .advance = advance, .multistep = true, .need_noise = true}, stream);
 }
 
 int32_t ditto_cfg_update_known(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z, uint64_t* rng,
                                int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist, const float* known,
                                const uint8_t* known_mask, int64_t B, int64_t T, int32_t advance, void* stream) {
-  DITTO_REQUIRE(e && eps_c && x && t && x_out, DITTO_E_BADARG, "cfg_update_known: null argument");
-  DITTO_REQUIRE(B >= 0 && T >= 0 && (!rng || n_t >= B), DITTO_E_BADARG, "cfg_update_known: bad sizes");
-  DITTO_TRY(require_known(e, z, rng, hist, known, known_mask, advance, "cfg_update_known"));
-  return launch_update_known(e, eps_c, eps_u, x, z, rng, t, n_t, guidance_scale, x_out, hist, known, known_mask, B, T, 0, advance != 0,
-                             static_cast<cudaStream_t>(stream));
+  return update_call(e, "cfg_update_known", eps_c, eps_u, x, t, n_t, guidance_scale, x_out, B, e ? T * e->H : 0,
+                     Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true},
+                     stream);
+}
+
+int32_t ditto_p_sample(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
+                       float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
+                       int64_t workspace_bytes, void* stream) {
+  return p_sample_dense(e, "p_sample", x, ctx, const_cast<int64_t*>(t), guided, guidance_scale, B, T, S, eps_scratch, x_out,
+                        Update{.z = z}, workspace, workspace_bytes, stream);
+}
+
+int32_t ditto_p_sample_multistep(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
+                                 float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
+                                 void* workspace, int64_t workspace_bytes, void* stream) {
+  return p_sample_dense(e, "p_sample_multistep", x, ctx, const_cast<int64_t*>(t), guided, guidance_scale, B, T, S, eps_scratch, x_out,
+                        Update{.z = z, .hist = hist, .multistep = true}, workspace, workspace_bytes, stream);
+}
+
+int32_t ditto_p_sample_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
+                           float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, void* workspace,
+                           int64_t workspace_bytes, int32_t advance, void* stream) {
+  return p_sample_dense(e, "p_sample_rng", x, ctx, t, guided, guidance_scale, B, T, S, eps_scratch, x_out,
+                        Update{.rng = rng, .advance = advance, .need_noise = true}, workspace, workspace_bytes, stream);
+}
+
+int32_t ditto_p_sample_multistep_rng(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, uint64_t* rng, int32_t guided,
+                                     float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
+                                     void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
+  return p_sample_dense(e, "p_sample_multistep_rng", x, ctx, t, guided, guidance_scale, B, T, S, eps_scratch, x_out,
+                        Update{.rng = rng, .hist = hist, .advance = advance, .multistep = true, .need_noise = true}, workspace,
+                        workspace_bytes, stream);
 }
 
 int32_t ditto_p_sample_known(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, const float* z, uint64_t* rng, int32_t guided,
                              float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
                              const float* known, const uint8_t* known_mask, void* workspace, int64_t workspace_bytes, int32_t advance,
                              void* stream) {
-  DITTO_REQUIRE(e && x && ctx && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_known: null argument");
-  DITTO_REQUIRE(e->finalized && !e->blocks_only, DITTO_E_STATE, "p_sample_known: engine not finalized");
-  DITTO_REQUIRE(B > 0 && T > 0 && S > 0 && T <= e->maxT, DITTO_E_BADARG, "p_sample_known: bad sizes");
-  DITTO_TRY(require_known(e, z, rng, hist, known, known_mask, advance, "p_sample_known"));
-  const int64_t n = guided ? 2 * B : B;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  DITTO_TRY(forward_impl(e, x, B, ctx, t, n, T, S, eps_scratch, workspace, workspace_bytes, st));
-  const int64_t per = T * e->H;
-  return launch_update_known(e, eps_scratch, guided ? eps_scratch + B * per : nullptr, x, z, rng, t, n, guidance_scale, x_out, hist, known,
-                             known_mask, B, T, 0, advance != 0, st);
+  return p_sample_dense(e, "p_sample_known", x, ctx, t, guided, guidance_scale, B, T, S, eps_scratch, x_out,
+                        Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true},
+                        workspace, workspace_bytes, stream);
 }
 
 int32_t ditto_randn(const uint64_t* rng, int64_t elem_offset, float* out, int64_t n, void* stream) {
@@ -1460,21 +1446,28 @@ int64_t ditto_workspace_bytes_ragged(const ditto_engine_t* e, const ditto_seq_gr
 int32_t ditto_forward_ragged(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, const int64_t* t,
                              float* out, void* workspace, int64_t workspace_bytes, void* stream) {
   DITTO_REQUIRE(e && x && t && out && workspace, DITTO_E_BADARG, "forward_ragged: null argument");
-  DITTO_REQUIRE(e->finalized, DITTO_E_STATE, "forward_ragged: engine not finalized");
+  DITTO_TRY(require_model(e, "forward_ragged"));
   std::vector<SeqGroup> gs;
   DITTO_TRY(parse_groups(e, groups, n_groups, true, gs));
   return forward_impl(e, x, t, gs.data(), static_cast<int>(gs.size()), out, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
-static int32_t p_sample_ragged_impl(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, const int64_t* t,
-                                    const float* z, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, float* hist,
-                                    void* workspace, int64_t workspace_bytes, void* stream) {
-  DITTO_REQUIRE(e && x && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_ragged: null argument");
-  DITTO_REQUIRE(e->finalized && e->have_schedule, DITTO_E_STATE, "p_sample_ragged: engine not finalized / schedule not loaded");
+// one sampler step on a ragged batch: the forward, then one update per group on the fork streams; the bookkeeping of advance
+// runs once after them (the groups' update kernels run concurrently, so none of them can own it)
+static int32_t p_sample_ragged(ditto_engine_t* e, const char* what, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
+                               int64_t* t, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, const Update& u,
+                               void* workspace, int64_t workspace_bytes, void* stream) {
+  const std::string s(what);
+  DITTO_REQUIRE(e && x && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, s + ": null argument");
+  DITTO_TRY(require_model(e, s));
+  DITTO_TRY(check_update(e, s, u));
   std::vector<SeqGroup> gs;
   DITTO_TRY(parse_groups(e, groups, n_groups, true, gs));
-  for (const SeqGroup& g : gs)
-    DITTO_REQUIRE(g.n == (guided ? 2 : 1) * g.n_x, DITTO_E_BADARG, "p_sample_ragged: n_seq must be n_x (unguided) or 2 n_x (guided)");
+  int64_t n_t = 0;
+  for (const SeqGroup& g : gs) {
+    DITTO_REQUIRE(g.n == (guided ? 2 : 1) * g.n_x, DITTO_E_BADARG, s + ": n_seq must be n_x (unguided) or 2 n_x (guided)");
+    n_t += g.n;
+  }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DITTO_TRY(forward_impl(e, x, t, gs.data(), static_cast<int>(gs.size()), eps_scratch, workspace, workspace_bytes, st));
   const int64_t H = e->H;
@@ -1484,114 +1477,60 @@ static int32_t p_sample_ragged_impl(ditto_engine_t* e, const float* x, const dit
   DITTO_TRY(fork.begin(static_cast<int>(gs.size())));
   for (size_t gi = 0; gi < gs.size(); ++gi) {  // offsets were filled in by the layout pass of forward_impl
     const SeqGroup& g = gs[gi];
-    const int64_t per = g.T * H;
+    const int64_t per = g.T * H, row = g.xrow0 * H;
     const float* ec = eps_scratch + g.row0 * H;
-    DITTO_TRY(launch_update(e, ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, z ? z + g.xrow0 * H : nullptr, t + g.seq0,
-                            guidance_scale, x_out + g.xrow0 * H, hist ? hist + g.xrow0 * H : nullptr, g.n_x, per,
-                            fork.stream(static_cast<int>(gi))));
+    // x, z, hist, known: packed rows from xrow0; the mask: one byte per packed row; noise offset = packed element position
+    Update ug = u;
+    ug.z = u.z ? u.z + row : nullptr;
+    ug.hist = u.hist ? u.hist + row : nullptr;
+    ug.known = u.known ? u.known + row : nullptr;
+    ug.mask = u.mask ? u.mask + g.xrow0 : nullptr;
+    ug.advance = 0;
+    DITTO_TRY(update(e, ec, guided ? ec + g.n_x * per : nullptr, x + row, t + g.seq0, g.n, guidance_scale, x_out + row, ug, g.n_x, per,
+                     row, fork.stream(static_cast<int>(gi))));
   }
   DITTO_TRY(fork.end());
+  if (u.advance) DITTO_TRY(launch_step_advance(reinterpret_cast<unsigned long long*>(u.rng), t, n_t, st));
   return 0;
 }
 
 int32_t ditto_p_sample_ragged(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, const int64_t* t,
                               const float* z, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, void* workspace,
                               int64_t workspace_bytes, void* stream) {
-  return p_sample_ragged_impl(e, x, groups, n_groups, t, z, guided, guidance_scale, eps_scratch, x_out, nullptr, workspace,
-                              workspace_bytes, stream);
+  return p_sample_ragged(e, "p_sample_ragged", x, groups, n_groups, const_cast<int64_t*>(t), guided, guidance_scale, eps_scratch, x_out,
+                         Update{.z = z}, workspace, workspace_bytes, stream);
 }
 
 int32_t ditto_p_sample_ragged_multistep(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
                                         const int64_t* t, const float* z, int32_t guided, float guidance_scale, float* eps_scratch,
                                         float* x_out, float* hist, void* workspace, int64_t workspace_bytes, void* stream) {
-  DITTO_TRY(require_multistep(e, hist, "p_sample_ragged_multistep"));
-  return p_sample_ragged_impl(e, x, groups, n_groups, t, z, guided, guidance_scale, eps_scratch, x_out, hist, workspace,
-                              workspace_bytes, stream);
-}
-
-static int32_t p_sample_ragged_rng_impl(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
-                                        uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out,
-                                        float* hist, void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
-  DITTO_REQUIRE(e && x && t && rng && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_ragged_rng: null argument");
-  DITTO_REQUIRE(e->finalized && e->have_schedule && !e->blocks_only, DITTO_E_STATE, "p_sample_ragged_rng: engine not finalized / schedule not loaded");
-  std::vector<SeqGroup> gs;
-  DITTO_TRY(parse_groups(e, groups, n_groups, true, gs));
-  int64_t n_t = 0;
-  for (const SeqGroup& g : gs) {
-    DITTO_REQUIRE(g.n == (guided ? 2 : 1) * g.n_x, DITTO_E_BADARG, "p_sample_ragged_rng: n_seq must be n_x (unguided) or 2 n_x (guided)");
-    n_t += g.n;
-  }
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  DITTO_TRY(forward_impl(e, x, t, gs.data(), static_cast<int>(gs.size()), eps_scratch, workspace, workspace_bytes, st));
-  const int64_t H = e->H;
-  std::unique_lock<std::recursive_mutex> fork_lock(e->fork_mutex, std::defer_lock);
-  if (gs.size() > 1 && e->n_side > 0) fork_lock.lock();
-  Fork fork(e, st);
-  DITTO_TRY(fork.begin(static_cast<int>(gs.size())));
-  for (size_t gi = 0; gi < gs.size(); ++gi) {
-    const SeqGroup& g = gs[gi];
-    const int64_t per = g.T * H;
-    const float* ec = eps_scratch + g.row0 * H;
-    // element offset = position in the packed latent buffer: every element of the batch draws its own normal
-    DITTO_TRY(launch_update_rng(e, ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, rng, t + g.seq0, g.n, guidance_scale,
-                                x_out + g.xrow0 * H, hist ? hist + g.xrow0 * H : nullptr, g.n_x, per, g.xrow0 * H, false,
-                                fork.stream(static_cast<int>(gi))));
-  }
-  DITTO_TRY(fork.end());
-  if (advance) DITTO_TRY(launch_step_advance(reinterpret_cast<unsigned long long*>(rng), t, n_t, st));
-  return 0;
+  return p_sample_ragged(e, "p_sample_ragged_multistep", x, groups, n_groups, const_cast<int64_t*>(t), guided, guidance_scale,
+                         eps_scratch, x_out, Update{.z = z, .hist = hist, .multistep = true}, workspace, workspace_bytes, stream);
 }
 
 int32_t ditto_p_sample_ragged_rng(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
                                   uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out, void* workspace,
                                   int64_t workspace_bytes, int32_t advance, void* stream) {
-  return p_sample_ragged_rng_impl(e, x, groups, n_groups, t, rng, guided, guidance_scale, eps_scratch, x_out, nullptr, workspace,
-                                  workspace_bytes, advance, stream);
+  return p_sample_ragged(e, "p_sample_ragged_rng", x, groups, n_groups, t, guided, guidance_scale, eps_scratch, x_out,
+                         Update{.rng = rng, .advance = advance, .need_noise = true}, workspace, workspace_bytes, stream);
 }
 
 int32_t ditto_p_sample_ragged_multistep_rng(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
                                             int64_t* t, uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch,
                                             float* x_out, float* hist, void* workspace, int64_t workspace_bytes, int32_t advance,
                                             void* stream) {
-  DITTO_TRY(require_multistep(e, hist, "p_sample_ragged_multistep_rng"));
-  return p_sample_ragged_rng_impl(e, x, groups, n_groups, t, rng, guided, guidance_scale, eps_scratch, x_out, hist, workspace,
-                                  workspace_bytes, advance, stream);
+  return p_sample_ragged(e, "p_sample_ragged_multistep_rng", x, groups, n_groups, t, guided, guidance_scale, eps_scratch, x_out,
+                         Update{.rng = rng, .hist = hist, .advance = advance, .multistep = true, .need_noise = true}, workspace,
+                         workspace_bytes, stream);
 }
 
 int32_t ditto_p_sample_ragged_known(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
                                     const float* z, uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out,
                                     float* hist, const float* known, const uint8_t* known_mask, void* workspace, int64_t workspace_bytes,
                                     int32_t advance, void* stream) {
-  DITTO_REQUIRE(e && x && t && eps_scratch && x_out && workspace, DITTO_E_BADARG, "p_sample_ragged_known: null argument");
-  DITTO_REQUIRE(e->finalized && !e->blocks_only, DITTO_E_STATE, "p_sample_ragged_known: engine not finalized");
-  DITTO_TRY(require_known(e, z, rng, hist, known, known_mask, advance, "p_sample_ragged_known"));
-  std::vector<SeqGroup> gs;
-  DITTO_TRY(parse_groups(e, groups, n_groups, true, gs));
-  int64_t n_t = 0;
-  for (const SeqGroup& g : gs) {
-    DITTO_REQUIRE(g.n == (guided ? 2 : 1) * g.n_x, DITTO_E_BADARG, "p_sample_ragged_known: n_seq must be n_x (unguided) or 2 n_x (guided)");
-    n_t += g.n;
-  }
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  DITTO_TRY(forward_impl(e, x, t, gs.data(), static_cast<int>(gs.size()), eps_scratch, workspace, workspace_bytes, st));
-  const int64_t H = e->H;
-  std::unique_lock<std::recursive_mutex> fork_lock(e->fork_mutex, std::defer_lock);
-  if (gs.size() > 1 && e->n_side > 0) fork_lock.lock();
-  Fork fork(e, st);
-  DITTO_TRY(fork.begin(static_cast<int>(gs.size())));
-  for (size_t gi = 0; gi < gs.size(); ++gi) {
-    const SeqGroup& g = gs[gi];
-    const int64_t per = g.T * H;
-    const float* ec = eps_scratch + g.row0 * H;
-    // x, z, hist, known: packed rows from xrow0; the mask: one byte per packed row; noise offset = packed element position
-    DITTO_TRY(launch_update_known(e, ec, guided ? ec + g.n_x * per : nullptr, x + g.xrow0 * H, z ? z + g.xrow0 * H : nullptr, rng,
-                                  t + g.seq0, g.n, guidance_scale, x_out + g.xrow0 * H, hist ? hist + g.xrow0 * H : nullptr,
-                                  known + g.xrow0 * H, known_mask + g.xrow0, g.n_x, g.T, g.xrow0 * H, false,
-                                  fork.stream(static_cast<int>(gi))));
-  }
-  DITTO_TRY(fork.end());
-  if (advance) DITTO_TRY(launch_step_advance(reinterpret_cast<unsigned long long*>(rng), t, n_t, st));
-  return 0;
+  return p_sample_ragged(e, "p_sample_ragged_known", x, groups, n_groups, t, guided, guidance_scale, eps_scratch, x_out,
+                         Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true},
+                         workspace, workspace_bytes, stream);
 }
 
 // ---- block-level operators (the reference's component signatures, src/components/DiT.py) -----------------------------

@@ -65,29 +65,26 @@ int launch_const_text(const float* text, int64_t n, int S, int D, const bf16* vf
 // synchronises anyway and is never captured)
 int64_t profiled_nonzero(const uint8_t* flags, int64_t n, cudaStream_t st);
 int launch_transpose_v(const bf16* v, int64_t ld, bf16* vt, int64_t n_seq, int T, int Tp, int heads, int d, cudaStream_t st);
-int launch_cfg_ddpm_update(const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
-                           const float* coef, int steps, float w, float* out, int64_t B, int64_t elems_per_seq,
-                           cudaStream_t st);
-// noise drawn in the kernel (Philox4x32-10 + Box-Muller from rng = {seed, draw counter, ticket, -}); advance: the last block
-// to finish adds 1 to the counter and subtracts 1 from t[0 .. n_t)
-int launch_cfg_ddpm_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t, int64_t n_t,
-                               const float* coef, int steps, float w, float* out, int64_t B, int64_t elems_per_seq,
-                               int64_t elem_offset, bool advance, cudaStream_t st);
-// multistep (DPM-Solver++(2M)) form: coef [steps, 6] = {c1, c2, c3, c4, d1, d2}; x_out = c1 (x - c2 eps) + c3 z + c4 hist,
-// then hist <- d1 (x - d2 eps); hist [B, elems_per_seq] is read only on rows with c4 != 0
-int launch_cfg_multistep_update(const float* eps_c, const float* eps_u, const float* x, const float* z, const int64_t* t,
-                                const float* coef, int steps, float w, float* out, float* hist, int64_t B, int64_t elems_per_seq,
-                                cudaStream_t st);
-int launch_cfg_multistep_update_rng(const float* eps_c, const float* eps_u, const float* x, unsigned long long* rng, int64_t* t,
-                                    int64_t n_t, const float* coef, int steps, float w, float* out, float* hist, int64_t B,
-                                    int64_t elems_per_seq, int64_t elem_offset, bool advance, cudaStream_t st);
-// replacement conditioning (speech prompt / infilling): frames with mask[frame] != 0 of x_out [B, T, H] become a p + s z with
-// {a, s} = coef_known[t] and p = known; the others take the DDPM-form update (hist == null, coef [steps, 3]) or the multistep
-// one (coef [steps, 6]).  Exactly one of z / rng; rng: in-kernel noise at element elem_offset + i, advance as above
-int launch_cfg_update_known(const float* eps_c, const float* eps_u, const float* x, const float* z, unsigned long long* rng, int64_t* t,
-                            int64_t n_t, const float* coef, const float* coef_known, int steps, float w, float* out, float* hist,
-                            const float* known, const uint8_t* mask, int64_t B, int64_t T, int64_t H, int64_t elem_offset, bool advance,
-                            cudaStream_t st);
+// One sampler update over B sequences of `per` elements: eps = eps_u + w (eps_c - eps_u) (eps_u == null: eps = eps_c), then
+//   DDPM form (hist == null, coef [steps, 3] = {c1, c2, c3}):  x_out = c1 (x - c2 eps) + c3 z
+//   multistep (hist != null, coef [steps, 6] = {c1, c2, c3, c4, d1, d2}, DPM-Solver++(2M)): the same + c4 hist, then
+//     hist <- d1 (x - d2 eps); hist is read only on rows with c4 != 0
+// with the row t[seq] of the table.  Noise: supplied z, or (rng != null) drawn in the kernel (Philox4x32-10 + Box-Muller from
+// rng = {seed, draw counter, ticket, -}) at element elem_offset + i; neither: no noise term.  advance (needs rng): the last
+// block to finish adds 1 to the draw counter and subtracts 1 from t[0 .. n_t).  Known frames (replacement conditioning, speech
+// prompt / infilling; mask != null): every `frame` elements share one mask byte, and a frame with mask != 0 becomes a p + s z
+// with {a, s} = coef_known[t] and p = known.
+struct CfgUpdateParams {
+  const float* eps_c = nullptr; const float* eps_u = nullptr; const float* x = nullptr;
+  const float* z = nullptr; unsigned long long* rng = nullptr;
+  int64_t* t = nullptr; int64_t n_t = 0;   // t is written only with advance
+  const float* coef = nullptr; const float* coef_known = nullptr; int steps = 0; float w = 0.f;
+  float* out = nullptr; float* hist = nullptr;
+  const float* known = nullptr; const uint8_t* mask = nullptr;
+  int64_t B = 0, per = 0, frame = 0, elem_offset = 0;
+  bool advance = false;
+};
+int launch_cfg_update(const CfgUpdateParams& p, cudaStream_t st);
 int launch_step_advance(unsigned long long* rng, int64_t* t, int64_t n_t, cudaStream_t st);
 int launch_randn(const unsigned long long* rng, int64_t elem_offset, float* out, int64_t n, cudaStream_t st);
 int launch_rope_angles(const float* t, const float* pos, float* out, int64_t batch, int T, int heads, int d, cudaStream_t st);

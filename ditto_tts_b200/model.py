@@ -402,39 +402,27 @@ class DiTTO(nn.Module, _EngineHost):
 
     def load_update_table(self, coef: torch.Tensor):
         """Replace the per-timestep update coefficients [diffusion_steps, 3] (sampler variants, schedules.py)."""
-        eng = self.engine()
-        dev = self.proj_in.weight.device
-        if tuple(coef.shape) != (self.diffusion_steps, 3):
-            raise DittoError(f"update table must be [{self.diffusion_steps}, 3]")
-        tab = coef.detach().to(device=dev, dtype=torch.float32).contiguous()
-        with torch.cuda.device(dev):
-            _lib.check(_lib.load().ditto_engine_load_update_table(eng, _ptr(tab), self.diffusion_steps, _stream()),
-                       "ditto_engine_load_update_table")
-            torch.cuda.current_stream().synchronize()
+        self._load_table("update", coef, 3)
 
     def load_multistep_table(self, coef: torch.Tensor):
         """Hand a [diffusion_steps, 6] multistep update table (schedules.dpmpp_2m_coef) to the engine."""
-        eng = self.engine()
-        dev = self.proj_in.weight.device
-        if tuple(coef.shape) != (self.diffusion_steps, 6):
-            raise DittoError(f"multistep table must be [{self.diffusion_steps}, 6]")
-        tab = coef.detach().to(device=dev, dtype=torch.float32).contiguous()
-        with torch.cuda.device(dev):
-            _lib.check(_lib.load().ditto_engine_load_multistep_table(eng, _ptr(tab), self.diffusion_steps, _stream()),
-                       "ditto_engine_load_multistep_table")
-            torch.cuda.current_stream().synchronize()
+        self._load_table("multistep", coef, 6)
 
     def load_known_table(self, coef: torch.Tensor):
         """Hand a [diffusion_steps, 2] known-frame table (schedules.known_coef: the re-noising of a speech prompt or of the
         frames around an infilled span) to the engine."""
+        self._load_table("known", coef, 2)
+
+    def _load_table(self, kind: str, coef: torch.Tensor, cols: int):
+        """ditto_engine_load_<kind>_table with a checked [diffusion_steps, cols] fp32 copy of ``coef`` on the engine's device."""
         eng = self.engine()
         dev = self.proj_in.weight.device
-        if tuple(coef.shape) != (self.diffusion_steps, 2):
-            raise DittoError(f"known table must be [{self.diffusion_steps}, 2]")
+        if tuple(coef.shape) != (self.diffusion_steps, cols):
+            raise DittoError(f"{kind} table must be [{self.diffusion_steps}, {cols}]")
         tab = coef.detach().to(device=dev, dtype=torch.float32).contiguous()
+        name = f"ditto_engine_load_{kind}_table"
         with torch.cuda.device(dev):
-            _lib.check(_lib.load().ditto_engine_load_known_table(eng, _ptr(tab), self.diffusion_steps, _stream()),
-                       "ditto_engine_load_known_table")
+            _lib.check(getattr(_lib.load(), name)(eng, _ptr(tab), self.diffusion_steps, _stream()), name)
             torch.cuda.current_stream().synchronize()
 
     def _ensure_schedule(self):

@@ -4,7 +4,7 @@ The reference has no padding masks -- ``DiT.forward`` attends over every frame i
 and ``SpeechGenerator.__sample_latents`` (src/model/SpeechGenerator.py:150-164) draws ``[1, L_pred, 768]`` per utterance --
 so utterances of different length only match it when they run UNPADDED.  A ``RaggedBatch`` sorts the utterances into
 groups of equal (frames, text tokens), packs their rows back to back and hands the group list to
-``ditto_forward_ragged`` / ``ditto_p_sample_ragged`` (include/ditto_b200.h): the row-wise work (LayerNorms, QKV / GLU /
+``ditto_forward_ragged`` / ``ditto_p_sample_ragged_known`` (include/ditto_b200.h): the row-wise work (LayerNorms, QKV / GLU /
 fc2 / projection GEMMs) is ONE launch over all packed rows, only AdaLN modulation, RoPE positions and the two
 attentions run per group.  Nothing is padded, so no flop is spent on frames that do not exist.
 """
@@ -18,6 +18,7 @@ import torch
 from . import _lib
 from ._lib import DittoError
 from .model import DiTTO, _need_cuda_f32, _ptr, _stream
+from .sampler import _CapturedStep
 
 __all__ = ["RaggedBatch", "RaggedStepGraph"]
 
@@ -159,83 +160,36 @@ class RaggedBatch:
         return out
 
     def p_sample(self, x_packed, t_seq, z_packed, w: float, eps: torch.Tensor, x_out: torch.Tensor, ws=None, hist=None,
-                 known=None, mask=None):
-        """One sampler step; ``hist`` (packed like x): the multistep update (ditto_p_sample_ragged_multistep); ``known`` /
-        ``mask`` (packed like x / one byte per packed row): known frames (ditto_p_sample_ragged_known)."""
+                 known=None, mask=None, rng=None):
+        """One sampler step (ditto_p_sample_ragged_known); ``hist`` (packed like x): the multistep update; ``known`` /
+        ``mask`` (packed like x / one byte per packed row): known frames; ``rng``: noise drawn in the per-group update kernels
+        instead of ``z_packed``, and the "t -= 1" bookkeeping in a one-block kernel after them."""
         ws = self.workspace() if ws is None else ws
         with torch.cuda.device(self.device):
-            if known is not None:
-                _lib.check(_lib.load().ditto_p_sample_ragged_known(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
-                                                                   _ptr(t_seq), _ptr(z_packed), None, 1 if self.guided else 0, float(w),
-                                                                   _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(known), _ptr(mask),
-                                                                   _ptr(ws), ws.numel(), 0, _stream()), "ditto_p_sample_ragged_known")
-                return
-            if hist is not None:
-                _lib.check(_lib.load().ditto_p_sample_ragged_multistep(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
-                                                                       _ptr(t_seq), _ptr(z_packed), 1 if self.guided else 0, float(w),
-                                                                       _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(ws), ws.numel(),
-                                                                       _stream()), "ditto_p_sample_ragged_multistep")
-                return
-            _lib.check(_lib.load().ditto_p_sample_ragged(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
-                                                         _ptr(t_seq), _ptr(z_packed), 1 if self.guided else 0, float(w),
-                                                         _ptr(eps), _ptr(x_out), _ptr(ws), ws.numel(), _stream()),
-                       "ditto_p_sample_ragged")
+            _lib.check(_lib.load().ditto_p_sample_ragged_known(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
+                                                               _ptr(t_seq), _ptr(z_packed), _ptr(rng), 1 if self.guided else 0, float(w),
+                                                               _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(known), _ptr(mask), _ptr(ws),
+                                                               ws.numel(), 0 if rng is None else 1, _stream()),
+                       "ditto_p_sample_ragged_known")
 
 
-class RaggedStepGraph:
+class RaggedStepGraph(_CapturedStep):
     """One sampler iteration over a ragged batch as a CUDA graph (noise draw, forward, CFG + update, t decrement).  With
     ``multistep`` the update is DPM-Solver++(2M)'s and the graph owns its ``hist`` buffer (packed like x).  With ``known``
     it owns the known latents (packed like x) and the frame mask (one byte per packed row), filled by ``reset``."""
 
     def __init__(self, batch: RaggedBatch, w: float, draw_noise: bool, multistep: bool = False, known: bool = False):
-        self.batch, self.w, self.draw_noise = batch, w, draw_noise
+        self.batch, self.w = batch, w
         dev = batch.device
-        self.x = torch.zeros((batch.x_rows, batch.H), dtype=torch.float32, device=dev)
-        self.hist = torch.zeros_like(self.x) if multistep else None
-        self.known = torch.zeros_like(self.x) if known else None
-        self.mask = torch.zeros((batch.x_rows,), dtype=torch.uint8, device=dev) if known else None
-        self.z = None if draw_noise else torch.zeros_like(self.x)
-        self.rng = torch.zeros((4,), dtype=torch.int64, device=dev)
+        self._buffers((batch.x_rows, batch.H), batch.n_seq, draw_noise, multistep, known, dev)
         self._ctx_ptrs = [c.data_ptr() for c in batch._ctx]
         self.eps = torch.empty((batch.seq_rows, batch.H), dtype=torch.float32, device=dev)
-        self.t = torch.zeros((batch.n_seq,), dtype=torch.int64, device=dev)
         self.ws = batch.workspace()
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):
-            self._step()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        torch.cuda.synchronize(dev)
-        self.graph = torch.cuda.CUDAGraph()
-        n0 = _lib.launch_count()
-        with torch.cuda.graph(self.graph):
-            self._step()
-        self.launches_per_step = _lib.launch_count() - n0
+        self._capture(dev)
 
-    def _step(self):
-        b = self.batch
-        if self.known is not None and self.draw_noise:
-            with torch.cuda.device(b.device):
-                _lib.check(_lib.load().ditto_p_sample_ragged_known(
-                    b.model.engine(), _ptr(self.x), b.c_groups, len(b.groups), _ptr(self.t), None, _ptr(self.rng), 1 if b.guided else 0,
-                    float(self.w), _ptr(self.eps), _ptr(self.x), _ptr(self.hist), _ptr(self.known), _ptr(self.mask), _ptr(self.ws),
-                    self.ws.numel(), 1, _stream()), "ditto_p_sample_ragged_known")
-            return
-        if self.draw_noise:   # noise drawn inside the per-group update kernels, bookkeeping in a one-block kernel after them
-            with torch.cuda.device(b.device):
-                if self.hist is not None:
-                    _lib.check(_lib.load().ditto_p_sample_ragged_multistep_rng(
-                        b.model.engine(), _ptr(self.x), b.c_groups, len(b.groups), _ptr(self.t), _ptr(self.rng), 1 if b.guided else 0,
-                        float(self.w), _ptr(self.eps), _ptr(self.x), _ptr(self.hist), _ptr(self.ws), self.ws.numel(), 1, _stream()),
-                        "ditto_p_sample_ragged_multistep_rng")
-                    return
-                _lib.check(_lib.load().ditto_p_sample_ragged_rng(b.model.engine(), _ptr(self.x), b.c_groups, len(b.groups), _ptr(self.t),
-                                                                 _ptr(self.rng), 1 if b.guided else 0, float(self.w), _ptr(self.eps),
-                                                                 _ptr(self.x), _ptr(self.ws), self.ws.numel(), 1, _stream()),
-                           "ditto_p_sample_ragged_rng")
-            return
-        b.p_sample(self.x, self.t, self.z, self.w, self.eps, self.x, ws=self.ws, hist=self.hist, known=self.known, mask=self.mask)
-        self.t.sub_(1)
+    def _p_sample(self, rng):
+        self.batch.p_sample(self.x, self.t, self.z, self.w, self.eps, self.x, ws=self.ws, hist=self.hist, known=self.known,
+                            mask=self.mask, rng=rng)
 
     def valid_for(self, batch: "RaggedBatch") -> bool:
         """The captured kernels read the context buffers and the workspace by address."""
@@ -244,20 +198,3 @@ class RaggedStepGraph:
 
     def rebind(self, batch: "RaggedBatch"):
         self.batch = batch
-
-    def reset(self, x_packed: torch.Tensor, t_start: int, seed: Optional[int] = None, known: Optional[torch.Tensor] = None,
-              known_mask: Optional[torch.Tensor] = None):
-        self.x.copy_(x_packed)
-        self.t.fill_(t_start)
-        if self.hist is not None:
-            self.hist.zero_()
-        if self.known is not None:
-            self.known.copy_(known)
-            self.mask.copy_(known_mask)
-        if self.draw_noise:
-            if seed is None:
-                seed = int(torch.randint(0, 2 ** 62, (1,)).item())
-            self.rng.copy_(torch.tensor([seed, 0, 0, 0], dtype=torch.int64))
-
-    def replay(self):
-        self.graph.replay()

@@ -4,12 +4,13 @@ Mirrors the sampling part of the reference's ``SpeechGenerator`` (src/model/Spee
 schedule tables :70-72, ``__p_sample`` :131-147, ``__sample_latents`` :150-164 -- same arithmetic, same
 argument meaning -- plus the classifier-free-guidance extension BASELINE.json asks for
 (eps = eps_u + w (eps_c - eps_u), unconditional branch = zero text embedding unless supplied).
-One sampler iteration is a single C-ABI call (ditto_p_sample): the 2B-sequence forward and the fused
-CFG-combine + update kernel; the text K/V and modulation vectors are built once per utterance batch.
+One sampler iteration is a single C-ABI call (ditto_p_sample_known, which without known frames is ditto_p_sample): the
+2B-sequence forward and the fused CFG-combine + update kernel; the text K/V and modulation vectors are built once per
+utterance batch.
 ``method="dpmpp_2m"`` (DPM-Solver++(2M), schedules.dpmpp_2m_coef) also carries the previous step's x0 prediction in a
-device buffer ``hist`` that the update kernel reads and rewrites (ditto_p_sample_multistep).
+device buffer ``hist`` that the update kernel reads and rewrites.
 ``sample_latents(..., known=p, known_mask=m)`` continues a speech prompt or fills a span: frames with m True are given
-(replacement conditioning, schedules.known_coef; the update kernel re-noises them, ditto_p_sample_known).
+(replacement conditioning, schedules.known_coef; the update kernel re-noises them).
 """
 from __future__ import annotations
 
@@ -27,83 +28,42 @@ from .model import DiTTO, _check_t_range, _need_cuda_f32, _ptr, _stream
 __all__ = ["DiTTOSampler", "StepGraph"]
 
 
-class StepGraph:
-    """One sampler iteration captured as a CUDA graph and replayed once per step.
+class _CapturedStep:
+    """What StepGraph and RaggedStepGraph share: the buffers a captured sampler step reads and writes (owned here, so that
+    the captured pointers stay valid), the capture, the per-job reset and the replay loop.  A subclass allocates eps and the
+    workspace and makes the step's one C call in ``_p_sample(rng)``."""
 
-    The graph holds the 2B-sequence forward and the fused CFG + DDPM update (in place on ``x``); when the noise is not
-    supplied by the caller that same kernel draws it (Philox, ``ditto_p_sample_rng``) and, as its last act, decrements
-    the device-resident step index ``t`` and bumps the draw counter -- so the host issues ONE launch per denoising step
-    instead of ~70 and the graph contains kernels of libditto_b200 only.  All buffers the graph touches are owned here
-    (or pinned by reference) so that the captured pointers stay valid.  A multistep sampler's graph also owns ``hist``, the
-    x0 prediction one step carries to the next (zero-filled by ``reset``).  A graph for known frames (speech prompt,
-    infilling) owns the known latents and the frame mask, filled by ``reset``; it launches as many kernels per step."""
-
-    def __init__(self, sampler: "DiTTOSampler", B: int, T: int, S: int, guided: bool, w: float, ctx: torch.Tensor,
-                 draw_noise: bool, device, known: bool = False):
-        m = sampler.model
-        H = m.hidden_dim
-        n = 2 * B if guided else B
-        self.B, self.T, self.S, self.guided, self.w, self.draw_noise = B, T, S, guided, w, draw_noise
-        self.x = torch.zeros((B, T, H), dtype=torch.float32, device=device)
+    def _buffers(self, shape, n_seq: int, draw_noise: bool, multistep: bool, known: bool, device):
+        self.draw_noise = draw_noise
+        self.x = torch.zeros(shape, dtype=torch.float32, device=device)
         # caller-supplied noise lands here; drawn noise never touches HBM
-        self.z = None if draw_noise else torch.zeros((B, T, H), dtype=torch.float32, device=device)
+        self.z = None if draw_noise else torch.zeros_like(self.x)
         self.rng = torch.zeros((4,), dtype=torch.int64, device=device)   # {seed, draw counter, ticket, -} of ditto_p_sample_rng
-        self.hist = torch.zeros((B, T, H), dtype=torch.float32, device=device) if sampler.multistep else None
-        self.known = torch.zeros((B, T, H), dtype=torch.float32, device=device) if known else None
-        self.mask = torch.zeros((B, T), dtype=torch.uint8, device=device) if known else None
-        self.eps = torch.empty((n, T, H), dtype=torch.float32, device=device)
-        self.t = torch.zeros((n,), dtype=torch.int64, device=device)
-        self.ctx = ctx
-        self.ws = m.workspace(n, T, S)
-        self.launches_per_step = 0
-        self._sampler_model = m
+        self.hist = torch.zeros_like(self.x) if multistep else None       # the x0 prediction one multistep step carries
+        self.known = torch.zeros_like(self.x) if known else None          # known frames and their mask, filled by reset
+        self.mask = torch.zeros(tuple(shape[:-1]), dtype=torch.uint8, device=device) if known else None
+        self.t = torch.zeros((n_seq,), dtype=torch.int64, device=device)
+
+    def _capture(self, device):
         # eager warm-up (engine set-up, lazy initialisation) on a side stream, then capture
         side = torch.cuda.Stream(device=device)
         side.wait_stream(torch.cuda.current_stream(device))
         with torch.cuda.stream(side):
-            self._step(sampler)
+            self._step()
         torch.cuda.current_stream(device).wait_stream(side)
         torch.cuda.synchronize(device)
         self.graph = torch.cuda.CUDAGraph()
         n0 = _lib.launch_count()
         with torch.cuda.graph(self.graph):
-            self._step(sampler)
+            self._step()
         self.launches_per_step = _lib.launch_count() - n0
-        self._keys = (self.ctx.data_ptr(), self.ws.data_ptr())
 
-    def _step(self, sampler):
-        if self.known is not None:
-            m = self._sampler_model
-            with torch.cuda.device(self.x.device):
-                _lib.check(_lib.load().ditto_p_sample_known(
-                    m.engine(), _ptr(self.x), _ptr(self.ctx), _ptr(self.t), _ptr(self.z), _ptr(self.rng) if self.draw_noise else None,
-                    1 if self.guided else 0, float(self.w), self.B, self.T, self.S, _ptr(self.eps), _ptr(self.x), _ptr(self.hist),
-                    _ptr(self.known), _ptr(self.mask), _ptr(self.ws), self.ws.numel(), 1 if self.draw_noise else 0, _stream()),
-                    "ditto_p_sample_known")
-            if not self.draw_noise:
-                self.t.sub_(1)
-            return
-        if self.draw_noise:   # drawn every step incl. t = 0, like the reference's randn_like (SpeechGenerator.py:145)
-            m = self._sampler_model
-            lib = _lib.load()
-            with torch.cuda.device(self.x.device):
-                if self.hist is not None:
-                    _lib.check(lib.ditto_p_sample_multistep_rng(m.engine(), _ptr(self.x), _ptr(self.ctx), _ptr(self.t), _ptr(self.rng),
-                                                                1 if self.guided else 0, float(self.w), self.B, self.T, self.S,
-                                                                _ptr(self.eps), _ptr(self.x), _ptr(self.hist), _ptr(self.ws),
-                                                                self.ws.numel(), 1, _stream()), "ditto_p_sample_multistep_rng")
-                    return
-                _lib.check(lib.ditto_p_sample_rng(m.engine(), _ptr(self.x), _ptr(self.ctx), _ptr(self.t), _ptr(self.rng),
-                                                  1 if self.guided else 0, float(self.w), self.B, self.T, self.S,
-                                                  _ptr(self.eps), _ptr(self.x), _ptr(self.ws), self.ws.numel(), 1, _stream()),
-                           "ditto_p_sample_rng")
-            return
-        sampler._p_sample_raw(self.x, self.ctx, self.t, self.z, self.guided, self.w, self.S, self.eps, self.x, ws=self.ws,
-                              hist=self.hist)
-        self.t.sub_(1)
-
-    def valid_for(self, ctx: torch.Tensor, ws: torch.Tensor) -> bool:
-        return self._keys == (ctx.data_ptr(), ws.data_ptr())
+    def _step(self):
+        # drawn noise: drawn every step incl. t = 0, like the reference's randn_like (SpeechGenerator.py:145), and the update
+        # kernel does the "t -= 1" and draw-counter bookkeeping
+        self._p_sample(self.rng if self.draw_noise else None)
+        if not self.draw_noise:
+            self.t.sub_(1)
 
     def reset(self, x_init: torch.Tensor, t_start: int, seed: Optional[int] = None, known: Optional[torch.Tensor] = None,
               known_mask: Optional[torch.Tensor] = None):
@@ -121,6 +81,47 @@ class StepGraph:
 
     def replay(self):
         self.graph.replay()
+
+    def run(self, x_init: torch.Tensor, taus: List[int], consecutive: bool, noise=None, known=None, known_mask=None):
+        """One sampling job: reset, then one replay per visited timestep (``noise`` indexed by timestep, as ``x``)."""
+        self.reset(x_init, taus[0], known=known, known_mask=known_mask)
+        for t_val in taus:
+            if noise is not None:
+                self.z.copy_(noise[t_val], non_blocking=True)
+            if not consecutive:
+                self.t.fill_(t_val)      # the graph's own "t -= 1" only covers the reference's consecutive timesteps
+            self.replay()
+
+
+class StepGraph(_CapturedStep):
+    """One sampler iteration captured as a CUDA graph and replayed once per step.
+
+    The graph holds the 2B-sequence forward and the fused CFG + DDPM update (in place on ``x``); when the noise is not
+    supplied by the caller that same kernel draws it (Philox, ``ditto_p_sample_rng``) and, as its last act, decrements
+    the device-resident step index ``t`` and bumps the draw counter -- so the host issues ONE launch per denoising step
+    instead of ~70 and the graph contains kernels of libditto_b200 only.  A multistep sampler's graph also owns ``hist``,
+    the x0 prediction one step carries to the next (zero-filled by ``reset``).  A graph for known frames (speech prompt,
+    infilling) owns the known latents and the frame mask, filled by ``reset``; it launches as many kernels per step."""
+
+    def __init__(self, sampler: "DiTTOSampler", B: int, T: int, S: int, guided: bool, w: float, ctx: torch.Tensor,
+                 draw_noise: bool, device, known: bool = False):
+        m = sampler.model
+        n = 2 * B if guided else B
+        self.B, self.T, self.S, self.guided, self.w = B, T, S, guided, w
+        self._buffers((B, T, m.hidden_dim), n, draw_noise, sampler.multistep, known, device)
+        self.eps = torch.empty((n, T, m.hidden_dim), dtype=torch.float32, device=device)
+        self.ctx = ctx
+        self.ws = m.workspace(n, T, S)
+        self._sampler = sampler
+        self._capture(device)
+        self._keys = (self.ctx.data_ptr(), self.ws.data_ptr())
+
+    def _p_sample(self, rng):
+        self._sampler._p_sample_raw(self.x, self.ctx, self.t, self.z, self.guided, self.w, self.S, self.eps, self.x, ws=self.ws,
+                                    hist=self.hist, known=self.known, mask=self.mask, rng=rng)
+
+    def valid_for(self, ctx: torch.Tensor, ws: torch.Tensor) -> bool:
+        return self._keys == (ctx.data_ptr(), ws.data_ptr())
 
 
 class DiTTOSampler:
@@ -206,26 +207,18 @@ class DiTTOSampler:
             text_emb = torch.cat([text_emb, null], dim=0)  # [cond(B); uncond(B)]
         return self.model.text_context(text_emb, name="sampler_ctx", T_hint=T)
 
-    def _p_sample_raw(self, x, ctx, t_n, z, guided, w, S, eps, x_out, ws=None, hist=None, known=None, mask=None):
+    def _p_sample_raw(self, x, ctx, t_n, z, guided, w, S, eps, x_out, ws=None, hist=None, known=None, mask=None, rng=None):
+        """One step: ``hist`` the multistep update, ``known`` / ``mask`` known frames, ``rng`` the noise drawn in the update
+        kernel (which then also does the "t -= 1" bookkeeping) instead of ``z``."""
         m = self.model
         B, T, H = x.shape
         n = 2 * B if guided else B
         with torch.cuda.device(x.device):
             if ws is None:
                 ws = m.workspace(n, T, S)
-            if known is not None:
-                _lib.check(_lib.load().ditto_p_sample_known(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), None, 1 if guided else 0,
-                                                            float(w), B, T, S, _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(known),
-                                                            _ptr(mask), _ptr(ws), ws.numel(), 0, _stream()), "ditto_p_sample_known")
-                return
-            if hist is not None:
-                _lib.check(_lib.load().ditto_p_sample_multistep(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), 1 if guided else 0,
-                                                                float(w), B, T, S, _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(ws),
-                                                                ws.numel(), _stream()), "ditto_p_sample_multistep")
-                return
-            _lib.check(_lib.load().ditto_p_sample(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), 1 if guided else 0,
-                                                  float(w), B, T, S, _ptr(eps), _ptr(x_out), _ptr(ws), ws.numel(),
-                                                  _stream()), "ditto_p_sample")
+            _lib.check(_lib.load().ditto_p_sample_known(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), _ptr(rng), 1 if guided else 0,
+                                                        float(w), B, T, S, _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(known), _ptr(mask),
+                                                        _ptr(ws), ws.numel(), 0 if rng is None else 1, _stream()), "ditto_p_sample_known")
 
     # ------------------------------------------------------------------------------------------
     @torch.no_grad()
@@ -326,13 +319,7 @@ class DiTTOSampler:
         if use_graph and record is None and generator is None:
             # one CUDA-graph replay per denoising step (noise drawn inside the graph unless supplied)
             g = self.step_graph(B, T, S, guided, w if guided else 0.0, ctx, noise is None, dev, known=has_known)
-            g.reset(x, taus[0], known=known, known_mask=known_mask)
-            for t_val in taus:
-                if noise is not None:
-                    g.z.copy_(noise[t_val], non_blocking=True)
-                if not consecutive:
-                    g.t.fill_(t_val)      # the graph's own "t -= 1" only covers the reference's consecutive timesteps
-                g.replay()
+            g.run(x, taus, consecutive, noise=noise, known=known, known_mask=known_mask)
             return g.x.clone()
         # t for every step, all sequences share it (SpeechGenerator.py:162)
         t_all = self._taus(dev).unsqueeze(1).repeat(1, n).contiguous()
@@ -413,13 +400,7 @@ class DiTTOSampler:
             else:
                 g.rebind(rb)
             self._ragged_graphs.move_to_end(sig)
-            g.reset(x, taus[0], known=kp, known_mask=km)
-            for t_val in taus:
-                if zs is not None:
-                    g.z.copy_(zs[t_val], non_blocking=True)
-                if not consecutive:
-                    g.t.fill_(t_val)
-                g.replay()
+            g.run(x, taus, consecutive, noise=zs, known=kp, known_mask=km)
             return rb.unpack(g.x)
         eps = torch.empty((rb.seq_rows, H), dtype=torch.float32, device=dev)
         x_next = torch.empty_like(x)

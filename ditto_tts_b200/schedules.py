@@ -7,7 +7,7 @@ src/model/DiTTO.py:96-104).  Its update has the form
     x_prev = c1 (x - c2 eps) + c3 z                                     (SpeechGenerator.py:143-145)
 
 and so do DDIM(eta) and DDPM over a sub-sequence of the timesteps, only with other (c1, c2, c3).  The device kernel
-(``cfg_ddpm_update_kernel``) reads the three numbers from a ``[diffusion_steps, 3]`` table indexed by the model timestep;
+(``cfg_update_kernel``) reads the three numbers from a ``[diffusion_steps, 3]`` table indexed by the model timestep;
 this module builds such tables on the host in float64 (they are a few hundred scalars) and
 ``ditto_engine_load_update_table`` hands them to the engine.  Nothing here touches the hot path.
 

@@ -50,7 +50,8 @@ enum {
   DITTO_F_FOLD_CROSS = 1 << 1, /* fold cross-attn q/out projections into the per-utterance text K/V */
   DITTO_F_FUSED_ATTN = 1 << 2, /* scores + softmax in one cluster kernel (fp32 scores never leave TMEM)   */
   DITTO_F_BLOCKS_ONLY = 1 << 4, /* the engine holds DiT blocks only (keys "blocks.i.*"): a stand-alone components/DiT.py module;
-                                   ditto_dit_block / ditto_text_context work, ditto_forward / ditto_p_sample do not        */
+                                   ditto_dit_block / ditto_text_context work; ditto_forward(_ragged) and every
+                                   ditto_p_sample* call return DITTO_E_STATE                                               */
   DITTO_F_DEFER_LN = 1 << 3    /* block LayerNorms (DiT.py:105,143,151) folded into the neighbouring GEMMs: the producer
                                   epilogue emits bf16(h) + per-row partial (sum, sum of squares), gamma/beta live in the
                                   consumer's weights/bias and its epilogue applies rstd / mean (needs DITTO_F_FUSED_ROPE)  */
@@ -207,7 +208,9 @@ int32_t ditto_p_sample_multistep_rng(ditto_engine_t* e, const float* x, const vo
  * where z is the normal the update uses for that element.  Known frames read neither eps, x nor hist and leave hist as it was.
  * Exactly one of z (supplied noise [B, T, H]) or rng (in-kernel noise, as ditto_p_sample_rng) is non-NULL; advance != 0
  * needs rng.  DITTO_E_STATE without a known table (or, with hist, without a multistep table).  One launch per step, like the
- * calls above; x_out may alias x.  t [n_t] (n_t >= B) is read-write when advance != 0. */
+ * calls above; x_out may alias x.  t [n_t] (n_t >= B) is read-write when advance != 0.  known == known_mask == NULL means no
+ * known frame: the call is then exactly the plain one with the same z / rng / hist (same kernel, same result, no known table
+ * needed); one of the two without the other is DITTO_E_BADARG. */
 int32_t ditto_cfg_update_known(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
                                uint64_t* rng, int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist,
                                const float* known, const uint8_t* known_mask, int64_t B, int64_t T, int32_t advance,

@@ -113,6 +113,31 @@ def test_standalone_dit_block_and_adaln_vs_oracle(dev, hidden, heads, T, S):
     assert rel(blk(x.to(dev), text.to(dev)), O.dit_block(sd, 0, x, text, O.rotary_angles(T, hidden // heads), heads)) <= BAR["bf16"]
 
 
+def test_blocks_only_engine_refuses_the_whole_model_calls(dev):
+    """A stand-alone block's engine (DITTO_F_BLOCKS_ONLY) holds no proj_in, t embedding or AdaLN weights: even with a schedule
+    loaded, the ragged forward and sampler calls return DITTO_E_STATE and launch nothing."""
+    torch.manual_seed(9)
+    blk = D.DiT(256, 4, 64, 256).to(dev)
+    x, text = torch.randn(1, 8, 256, device=dev), torch.randn(1, 3, 256, device=dev)
+    blk(x, text)                                                    # builds the block's engine
+    lib, eng = _lib.load(), blk._own.engine()
+    half = torch.full((1,), 0.5, device=dev)                        # betas, alphas, alphas_cumprod of its one step
+    assert lib.ditto_engine_load_schedule(eng, P(half), P(half), P(half), 1, ST()) == 0
+    torch.cuda.synchronize()
+    buf = torch.zeros(1 << 20, device=dev)                           # stands in for every buffer: nothing may touch it
+    t = torch.zeros(1, dtype=torch.int64, device=dev)
+    grp = (_lib.SeqGroup * 1)(_lib.SeqGroup(n_seq=1, n_x=1, T=8, S=3, ctx=buf.data_ptr()))
+    n0 = _lib.launch_count()
+    assert lib.ditto_forward_ragged(eng, P(x), grp, 1, P(t), P(buf), P(buf), buf.numel() * 4, ST()) == -4
+    assert lib.ditto_p_sample_ragged(eng, P(x), grp, 1, P(t), P(buf), 0, 0.0, P(buf), P(buf), P(buf), buf.numel() * 4, ST()) == -4
+    assert lib.ditto_p_sample_ragged_multistep(eng, P(x), grp, 1, P(t), P(buf), 0, 0.0, P(buf), P(buf), P(buf), P(buf),
+                                               buf.numel() * 4, ST()) == -4
+    assert b"blocks-only" in lib.ditto_last_error()
+    assert _lib.launch_count() == n0
+    torch.cuda.synchronize()
+    assert not bool(buf.any())
+
+
 @pytest.mark.parametrize("b,T,h,d", [(2, 24, 2, 32), (1, 750, 1, 768), (3, 5, 12, 64)])
 def test_apply_rope_vs_oracle(dev, b, T, h, d):
     g = torch.Generator().manual_seed(3)

@@ -355,3 +355,76 @@ def test_argument_checks(dev, setup):
             s.sample_latents(td, x_init=xd, **bad)
     with pytest.raises(D.DittoError):
         s.sample_latents_ragged([td[0]], [40], known=[kd[0]])
+
+
+@pytest.mark.parametrize("draw", [False, True], ids=["supplied", "drawn"])
+@pytest.mark.parametrize("multistep", [False, True], ids=["ddpm", "2m"])
+def test_known_calls_without_known_frames_are_the_plain_calls(dev, setup, multistep, draw):
+    """known == known_mask == NULL means no known frame: ditto_cfg_update_known, ditto_p_sample_known and
+    ditto_p_sample_ragged_known then are the plain update / dense / ragged call with the same noise and hist, bit for bit
+    (x_out, hist, t, the draw counter), with as many launches, and need no known table."""
+    cfg, sd, x, text, *_ = setup
+    m = model(cfg, sd, "fp32", dev)
+    s = D.DiTTOSampler(m, guidance_scale=3.0, method="dpmpp_2m" if multistep else "ddim", num_steps=10, eta=1.0)
+    lib, eng = _lib.load(), m.engine()
+    B, T, S, H = 2, 40, text.shape[1], cfg.hidden_dim
+    n = 2 * B
+    g = torch.Generator().manual_seed(21)
+    xs, z, hist0 = (torch.randn(B, T, H, generator=g).to(dev) for _ in range(3))
+    eps_in = torch.randn(n, T, H, generator=g).to(dev)
+    ctx = m.text_context(torch.cat([text[:B], torch.zeros_like(text[:B])]).to(dev))
+    grp = (_lib.SeqGroup * 1)(_lib.SeqGroup(n_seq=n, n_x=B, T=T, S=S, ctx=ctx.data_ptr()))
+    ws = torch.empty(max(lib.ditto_workspace_bytes(eng, n, T, S), lib.ditto_workspace_bytes_ragged(eng, grp, 1)), dtype=torch.uint8,
+                     device=dev)
+    t_val = int(s.timesteps[3])              # a second-order row of the 2M table
+    zp = None if draw else P(z)
+    adv = 1 if draw else 0
+    w = 3.0
+
+    def run(call):
+        t = torch.full((n,), t_val, dtype=torch.int64, device=dev)
+        rng = torch.tensor([77, 3, 0, 0], dtype=torch.int64, device=dev)
+        hist = hist0.clone() if multistep else None
+        out, eps = torch.empty_like(xs), torch.empty(n, T, H, device=dev)
+        rp, hp = (P(rng) if draw else None), (P(hist) if multistep else None)
+        n0 = _lib.launch_count()
+        _lib.check(call(P(t), rp, hp, P(out), P(eps)), "call")
+        launches = _lib.launch_count() - n0
+        torch.cuda.synchronize()
+        return out, hist, t, rng, launches
+
+    ec, eu = P(eps_in[:B]), P(eps_in[B:])
+    if multistep and draw:
+        plain = [lambda t, r, h, o, e: lib.ditto_cfg_multistep_update_rng(eng, ec, eu, P(xs), r, t, n, w, o, h, B, T * H, 1, ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample_multistep_rng(eng, P(xs), P(ctx), t, r, 1, w, B, T, S, e, o, h, P(ws),
+                                                                        ws.numel(), 1, ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample_ragged_multistep_rng(eng, P(xs), grp, 1, t, r, 1, w, e, o, h, P(ws),
+                                                                               ws.numel(), 1, ST())]
+    elif multistep:
+        plain = [lambda t, r, h, o, e: lib.ditto_cfg_multistep_update(eng, ec, eu, P(xs), zp, t, w, o, h, B, T * H, ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample_multistep(eng, P(xs), P(ctx), t, zp, 1, w, B, T, S, e, o, h, P(ws),
+                                                                    ws.numel(), ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample_ragged_multistep(eng, P(xs), grp, 1, t, zp, 1, w, e, o, h, P(ws), ws.numel(),
+                                                                           ST())]
+    elif draw:
+        plain = [lambda t, r, h, o, e: lib.ditto_cfg_ddpm_update_rng(eng, ec, eu, P(xs), r, t, n, w, o, B, T * H, 1, ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample_rng(eng, P(xs), P(ctx), t, r, 1, w, B, T, S, e, o, P(ws), ws.numel(), 1, ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample_ragged_rng(eng, P(xs), grp, 1, t, r, 1, w, e, o, P(ws), ws.numel(), 1, ST())]
+    else:
+        plain = [lambda t, r, h, o, e: lib.ditto_cfg_ddpm_update(eng, ec, eu, P(xs), zp, t, w, o, B, T * H, ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample(eng, P(xs), P(ctx), t, zp, 1, w, B, T, S, e, o, P(ws), ws.numel(), ST()),
+                 lambda t, r, h, o, e: lib.ditto_p_sample_ragged(eng, P(xs), grp, 1, t, zp, 1, w, e, o, P(ws), ws.numel(), ST())]
+    known = [lambda t, r, h, o, e: lib.ditto_cfg_update_known(eng, ec, eu, P(xs), zp, r, t, n, w, o, h, None, None, B, T, adv, ST()),
+             lambda t, r, h, o, e: lib.ditto_p_sample_known(eng, P(xs), P(ctx), t, zp, r, 1, w, B, T, S, e, o, h, None, None, P(ws),
+                                                            ws.numel(), adv, ST()),
+             lambda t, r, h, o, e: lib.ditto_p_sample_ragged_known(eng, P(xs), grp, 1, t, zp, r, 1, w, e, o, h, None, None, P(ws),
+                                                                   ws.numel(), adv, ST())]
+    for want_call, got_call in zip(plain, known):
+        want, got = run(want_call), run(got_call)
+        assert torch.equal(want[0], got[0]) and bool(torch.isfinite(got[0]).all())
+        if multistep:
+            assert torch.equal(want[1], got[1]) and not torch.equal(got[1], hist0)
+        assert torch.equal(want[2], got[2]) and torch.equal(want[3], got[3])
+        assert want[4] == got[4] > 0
+    if draw:      # the bookkeeping ran
+        assert got[2].tolist() == [t_val - 1] * n and got[3].tolist() == [77, 4, 0, 0]

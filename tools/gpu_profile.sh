@@ -8,7 +8,7 @@ timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 700 --c
     python bench.py --steps 3 --warmup 3 > $O/${TAG}_ncu_bench.log 2>&1
 tail -1 $O/${TAG}_ncu_bench.log | cut -c1-200
 # one forward's kernels of the eager warm-up step inside step_profile (skip the text-context / finalize launches)
-timeout 900 ncu --set full --clock-control none --import-source on -k regex:'tc_gemm|tc_scores|layernorm|adaln|cfg_ddpm|softmax' -s ${2:-20} -c ${3:-14} -f -o /tmp/${TAG}_full \
+timeout 900 ncu --set full --clock-control none --import-source on -k regex:'tc_gemm|tc_scores|layernorm|adaln|cfg_update_kernel|softmax' -s ${2:-20} -c ${3:-14} -f -o /tmp/${TAG}_full \
     python tools/step_profile.py --steps 3 > $O/${TAG}_ncu_full.log 2>&1
 tail -2 $O/${TAG}_ncu_full.log
 ncu -i /tmp/${TAG}_full.ncu-rep --page raw --csv > $O/${TAG}_full_raw.csv 2>/dev/null

@@ -8,7 +8,7 @@ timeout 1200 ncu --metrics gpu__time_duration.sum --clock-control none -c 900 --
 tail -1 $O/${TAG}_ncu_bench.log | cut -c1-200
 # kernels of one eager step (skip the text-context / finalize launches and the first steps)
 timeout 1200 ncu --set full --clock-control none --import-source on \
-    -k regex:'tc_gemm|flash_attn768|cross_fused|layernorm|adaln|cfg_ddpm' -s ${2:-40} -c ${3:-14} -f -o /tmp/${TAG}_full \
+    -k regex:'tc_gemm|flash_attn768|cross_fused|layernorm|adaln|cfg_update_kernel' -s ${2:-40} -c ${3:-14} -f -o /tmp/${TAG}_full \
     python tools/step_profile.py --steps 3 > $O/${TAG}_ncu_full.log 2>&1
 tail -2 $O/${TAG}_ncu_full.log
 ncu -i /tmp/${TAG}_full.ncu-rep --page raw --csv > $O/${TAG}_full_raw.csv 2>/dev/null

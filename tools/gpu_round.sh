@@ -20,7 +20,7 @@ tail -2 $O/${TAG}_ncu_bench.log
 echo "##### ncu full"
 # one forward's kernels of the eager warm-up step (one DiT block and a half); the report stays in /tmp unless it is small:
 # gpurun copies back at most 64 MiB
-timeout 900 ncu --set full --clock-control none --import-source on -k regex:'tc_gemm|tc_scores|cross_fused|softmax|adaln|layernorm|cfg_ddpm' -s 20 -c 12 \
+timeout 900 ncu --set full --clock-control none --import-source on -k regex:'tc_gemm|tc_scores|cross_fused|softmax|adaln|layernorm|cfg_update_kernel' -s 20 -c 12 \
     -o /tmp/${TAG}_prof -f python tools/step_profile.py --steps 3 > $O/${TAG}_ncu_full.log 2>&1
 tail -2 $O/${TAG}_ncu_full.log
 ncu -i /tmp/${TAG}_prof.ncu-rep --page raw --csv > $O/${TAG}_full_raw.csv 2>/dev/null
