@@ -295,6 +295,25 @@ __device__ __forceinline__ float quad_sum(float v) {
   v += __shfl_xor_sync(0xffffffffu, v, 1);
   return v + __shfl_xor_sync(0xffffffffu, v, 2);
 }
+// LayerNorm row statistics of the fused epilogues, free of the cancellation of E[v^2] - mean^2 (which loses the variance
+// once |mean| / spread ~ 1e3).  A partial is (mean, M2 = sum (v - mean)^2) of n values.  A thread accumulates d = v - K and
+// d^2 against its own first value K of the row, which keeps both sums at the scale of the row's spread, and turns them into
+// a partial; partials of equal counts merge by Chan's pairwise formula.  ln_merge is symmetric in a and b, so every lane of
+// a shuffle and both CTAs of an exchange get the same bits.
+__device__ __forceinline__ float2 ln_partial(float K, float sd, float sdd, float inv_n) {
+  const float m = sd * inv_n;
+  return make_float2(K + m, fmaf(-sd, m, sdd));
+}
+// a, b: partials of n values each
+__device__ __forceinline__ float2 ln_merge(float2 a, float2 b, float n) {
+  const float d = b.x - a.x;
+  return make_float2(0.5f * (a.x + b.x), (a.y + b.y) + d * d * (0.5f * n));
+}
+// merge of the four partials (n values each) of a lane quad; every lane gets the quad's partial of 4 n values
+__device__ __forceinline__ float2 ln_quad_merge(float2 s, float n) {
+  s = ln_merge(s, make_float2(__shfl_xor_sync(0xffffffffu, s.x, 1), __shfl_xor_sync(0xffffffffu, s.y, 1)), n);
+  return ln_merge(s, make_float2(__shfl_xor_sync(0xffffffffu, s.x, 2), __shfl_xor_sync(0xffffffffu, s.y, 2)), 2.f * n);
+}
 __device__ __forceinline__ float ex2_approx(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));

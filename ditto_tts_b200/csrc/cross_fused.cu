@@ -506,9 +506,10 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
       // fp32 slab (32 columns) in shared memory, TMA 128-B swizzle: row r at r * 128 B, 16-B chunk j at position j ^ (r & 7).
       const int lrow0 = quarter * 32;
       const int slab_sel = sub >> 1, jbase = (sub & 1) * 4 + (q >> 1);   // 32-column slab, first 16-B chunk of this thread
-      float2 sm2[4], sq2[4];                                  // [hh][A|B] packed (sum, sum) / (sumsq, sumsq) accumulators
+      // [hh][A|B] packed sums of v - K and (v - K)^2, K = this thread's first value of the row (nk = -K; common.cuh)
+      float2 sm2[4], sq2[4], nk[4];
 #pragma unroll
-      for (int j = 0; j < 4; ++j) sm2[j] = sq2[j] = make_float2(0.f, 0.f);
+      for (int j = 0; j < 4; ++j) sm2[j] = sq2[j] = nk[j] = make_float2(0.f, 0.f);
       uint32_t ob = 0;
       float2 b2N[2];
 #pragma unroll
@@ -555,10 +556,12 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
                                          rsA[hh][kbl]);
             const float2 vB = __fadd2_rn(__fadd2_rn(make_float2(__uint_as_float(r[hh][4 * kbl + 2]), __uint_as_float(r[hh][4 * kbl + 3])), b2[kbl]),
                                          rsB[hh][kbl]);
-            sm2[2 * hh] = __fadd2_rn(sm2[2 * hh], vA);
-            sq2[2 * hh] = __ffma2_rn(vA, vA, sq2[2 * hh]);
-            sm2[2 * hh + 1] = __fadd2_rn(sm2[2 * hh + 1], vB);
-            sq2[2 * hh + 1] = __ffma2_rn(vB, vB, sq2[2 * hh + 1]);
+            if (hc == 0 && kbl == 0) { nk[2 * hh] = make_float2(-vA.x, -vA.x); nk[2 * hh + 1] = make_float2(-vB.x, -vB.x); }
+            const float2 dA = __fadd2_rn(vA, nk[2 * hh]), dB = __fadd2_rn(vB, nk[2 * hh + 1]);
+            sm2[2 * hh] = __fadd2_rn(sm2[2 * hh], dA);
+            sq2[2 * hh] = __ffma2_rn(dA, dA, sq2[2 * hh]);
+            sm2[2 * hh + 1] = __fadd2_rn(sm2[2 * hh + 1], dB);
+            sq2[2 * hh + 1] = __ffma2_rn(dB, dB, sq2[2 * hh + 1]);
             *reinterpret_cast<float2*>(slab + rA * 128 + ((j ^ (rA & 7)) << 4)) = vA;   // in place: one owner per element
             *reinterpret_cast<float2*>(slab + rB * 128 + ((j ^ (rB & 7)) << 4)) = vB;
           }
@@ -573,11 +576,13 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
         if (hc & 1) ++oc;
       }
       // ---------------- row statistics: the four column quarters of a row live in four warps ----------------
+      // partials (mean, M2): a thread has 4 num_hc values of a row, a quad 16 num_hc, a warp's quarter H / 4
       float2* sp = stat + (it & 1u) * (XF_BM * 4);
+      const float n_t = static_cast<float>(4 * p.num_hc);
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        const float s1 = quad_sum(sm2[j].x + sm2[j].y), s2 = quad_sum(sq2[j].x + sq2[j].y);
-        if (writer) sp[(lrow0 + (j >> 1) * 16 + g + (j & 1) * 8) * 4 + sub] = make_float2(s1, s2);
+        const float2 st = ln_quad_merge(ln_partial(-nk[j].x, sm2[j].x + sm2[j].y, sq2[j].x + sq2[j].y, 1.0f / n_t), n_t);
+        if (writer) sp[(lrow0 + (j >> 1) * 16 + g + (j & 1) * 8) * 4 + sub] = st;
       }
       epi_bar_sync();
       float mean[4], rstd[4];
@@ -585,10 +590,10 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
       for (int j = 0; j < 4; ++j) {
         const int lr = lrow0 + (j >> 1) * 16 + g + (j & 1) * 8;
         const float4 a = *reinterpret_cast<const float4*>(sp + lr * 4), c = *reinterpret_cast<const float4*>(sp + lr * 4 + 2);
-        const float m = (a.x + a.z + c.x + c.z) * p.inv_h;
-        const float var = fmaxf(fmaf(-m, m, (a.y + a.w + c.y + c.w) * p.inv_h), 0.f);
-        mean[j] = m;
-        rstd[j] = rsqrtf(var + 1e-5f);
+        const float2 st = ln_merge(ln_merge(make_float2(a.x, a.y), make_float2(a.z, a.w), 4.f * n_t),
+                                   ln_merge(make_float2(c.x, c.y), make_float2(c.z, c.w), 4.f * n_t), 8.f * n_t);
+        mean[j] = st.x;
+        rstd[j] = rsqrtf(fmaxf(st.y, 0.f) * p.inv_h + 1e-5f);
       }
       // ---------------- pass 1: LayerNorm of the updated rows -> bf16, written over the staging buffer ----------------
       // bf16 box in shared memory: row r at r * 128 B (64 columns), 16-B chunk j (8 columns) at position j ^ (r & 7)

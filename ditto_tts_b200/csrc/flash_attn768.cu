@@ -589,7 +589,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
       mbar_wait(o_full, it & 1u);
       tcgen05_fence_after();
       tr.ev(16, it);
-      float smA = 0.f, sqA = 0.f, smB = 0.f, sqB = 0.f;
+      // row statistics of this thread's 96 values of rows A and B: sums of v - K and (v - K)^2, K = its first value (common.cuh)
+      float smA = 0.f, sqA = 0.f, smB = 0.f, sqB = 0.f, kA = 0.f, kB = 0.f;
       auto sweep1 = [&](int cb, const float4(&f)[8]) {
         uint32_t o[32];
         tmem_ld_16x64(t_lane + cb * 64, o);
@@ -608,10 +609,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
           vB.w = fmaf(iB, __uint_as_float(o[4 * k1 + 3]), f[4 + jj].w);
           if (okA && !(p.dbg & 4)) *reinterpret_cast<float4*>(hA + cb * 64 + jj * 16) = vA;
           if (okB && !(p.dbg & 4)) *reinterpret_cast<float4*>(hB + cb * 64 + jj * 16) = vB;
-          smA += (vA.x + vA.y) + (vA.z + vA.w);
-          sqA = fmaf(vA.x, vA.x, fmaf(vA.y, vA.y, fmaf(vA.z, vA.z, fmaf(vA.w, vA.w, sqA))));
-          smB += (vB.x + vB.y) + (vB.z + vB.w);
-          sqB = fmaf(vB.x, vB.x, fmaf(vB.y, vB.y, fmaf(vB.z, vB.z, fmaf(vB.w, vB.w, sqB))));
+          if (cb == 0 && jj == 0) { kA = vA.x; kB = vB.x; }
+          const float4 dA = make_float4(vA.x - kA, vA.y - kA, vA.z - kA, vA.w - kA);
+          const float4 dB = make_float4(vB.x - kB, vB.y - kB, vB.z - kB, vB.w - kB);
+          smA += (dA.x + dA.y) + (dA.z + dA.w);
+          sqA = fmaf(dA.x, dA.x, fmaf(dA.y, dA.y, fmaf(dA.z, dA.z, fmaf(dA.w, dA.w, sqA))));
+          smB += (dB.x + dB.y) + (dB.z + dB.w);
+          sqB = fmaf(dB.x, dB.x, fmaf(dB.y, dB.y, fmaf(dB.z, dB.z, fmaf(dB.w, dB.w, sqB))));
           o[4 * k0] = __float_as_uint(vA.x); o[4 * k0 + 1] = __float_as_uint(vA.y);
           o[4 * k1] = __float_as_uint(vA.z); o[4 * k1 + 1] = __float_as_uint(vA.w);
           o[4 * k0 + 2] = __float_as_uint(vB.x); o[4 * k0 + 3] = __float_as_uint(vB.y);
@@ -630,24 +634,27 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
       if (p.u_out != nullptr) {
         tmem_st_wait();
         // ---------------- LayerNorm statistics: this CTA has 384 of the 768 columns; the peer has the rest ----------------
-        smA = quad_sum(smA); sqA = quad_sum(sqA); smB = quad_sum(smB); sqB = quad_sum(sqB);
+        // partials (mean, M2) of this CTA's 384 columns; the peer's are merged in below
+        const float2 pA = ln_quad_merge(ln_partial(kA, smA, sqA, 1.0f / (F7_DH / 4)), F7_DH / 4);
+        const float2 pB = ln_quad_merge(ln_partial(kB, smB, sqB, 1.0f / (F7_DH / 4)), F7_DH / 4);
         if (ew == 0 && lane == 0) mbar_expect_tx(&stat_bar[par], F7_BM * 8);
         if (writer) {
           const uint32_t slot = f7_mapa(smem_u32(stat_x + (par * F7_BM + rA) * 2), peer);
           const uint32_t bar = f7_mapa(smem_u32(&stat_bar[par]), peer);
-          f7_st_async(slot, smA, bar);
-          f7_st_async(slot + 4, sqA, bar);
-          f7_st_async(slot + 8 * 8, smB, bar);
-          f7_st_async(slot + 8 * 8 + 4, sqB, bar);
+          f7_st_async(slot, pA.x, bar);
+          f7_st_async(slot + 4, pA.y, bar);
+          f7_st_async(slot + 8 * 8, pB.x, bar);
+          f7_st_async(slot + 8 * 8 + 4, pB.y, bar);
         }
         mbar_wait(&stat_bar[par], (it >> 1) & 1u);
         tr.ev(18, it);
         const float2 xA = *reinterpret_cast<const float2*>(stat_x + (par * F7_BM + rA) * 2);
         const float2 xB = *reinterpret_cast<const float2*>(stat_x + (par * F7_BM + rB) * 2);
         const float inv_h = 1.0f / static_cast<float>(F7_D);
-        const float meanA = (smA + xA.x) * inv_h, meanB = (smB + xB.x) * inv_h;
-        const float rsA = rsqrtf(fmaxf(fmaf(-meanA, meanA, (sqA + xA.y) * inv_h), 0.f) + 1e-5f);
-        const float rsB = rsqrtf(fmaxf(fmaf(-meanB, meanB, (sqB + xB.y) * inv_h), 0.f) + 1e-5f);
+        const float2 stA = ln_merge(pA, xA, F7_DH), stB = ln_merge(pB, xB, F7_DH);
+        const float meanA = stA.x, meanB = stB.x;
+        const float rsA = rsqrtf(fmaxf(stA.y, 0.f) * inv_h + 1e-5f);
+        const float rsB = rsqrtf(fmaxf(stB.y, 0.f) * inv_h + 1e-5f);
         // ---------------- sweep 2: u = LayerNorm(h) gamma + beta, bf16, 8-byte stores ----------------
         bf16* uA = p.u_out + growA * F7_D + col_half + q * 4;
         bf16* uB = uA + 8 * F7_D;

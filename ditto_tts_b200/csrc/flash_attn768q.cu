@@ -642,7 +642,8 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
       mbar_wait(o_full, it & 1u);
       tcgen05_fence_after();
       tr.ev(16, it);
-      float smA = 0.f, sqA = 0.f, smB = 0.f, sqB = 0.f;
+      // row statistics of this thread's 96 values of rows A and B: sums of v - K and (v - K)^2, K = its first value (common.cuh)
+      float smA = 0.f, sqA = 0.f, smB = 0.f, sqB = 0.f, kA = 0.f, kB = 0.f;
       auto sweep1 = [&](int cb, const float4(&f)[8]) {
         uint32_t o[32];
         tmem_ld_16x64(t_lane + cb * 64, o);
@@ -672,10 +673,13 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
           }
           if (okA && !(p.dbg & 4)) *reinterpret_cast<float4*>(hA + cb * 64 + jj * 16) = vA;
           if (okB && !(p.dbg & 4)) *reinterpret_cast<float4*>(hB + cb * 64 + jj * 16) = vB;
-          smA += (vA.x + vA.y) + (vA.z + vA.w);
-          sqA = fmaf(vA.x, vA.x, fmaf(vA.y, vA.y, fmaf(vA.z, vA.z, fmaf(vA.w, vA.w, sqA))));
-          smB += (vB.x + vB.y) + (vB.z + vB.w);
-          sqB = fmaf(vB.x, vB.x, fmaf(vB.y, vB.y, fmaf(vB.z, vB.z, fmaf(vB.w, vB.w, sqB))));
+          if (cb == 0 && jj == 0) { kA = vA.x; kB = vB.x; }
+          const float4 dA = make_float4(vA.x - kA, vA.y - kA, vA.z - kA, vA.w - kA);
+          const float4 dB = make_float4(vB.x - kB, vB.y - kB, vB.z - kB, vB.w - kB);
+          smA += (dA.x + dA.y) + (dA.z + dA.w);
+          sqA = fmaf(dA.x, dA.x, fmaf(dA.y, dA.y, fmaf(dA.z, dA.z, fmaf(dA.w, dA.w, sqA))));
+          smB += (dB.x + dB.y) + (dB.z + dB.w);
+          sqB = fmaf(dB.x, dB.x, fmaf(dB.y, dB.y, fmaf(dB.z, dB.z, fmaf(dB.w, dB.w, sqB))));
           o[4 * k0] = __float_as_uint(vA.x); o[4 * k0 + 1] = __float_as_uint(vA.y);
           o[4 * k1] = __float_as_uint(vA.z); o[4 * k1 + 1] = __float_as_uint(vA.w);
           o[4 * k0 + 2] = __float_as_uint(vB.x); o[4 * k0 + 3] = __float_as_uint(vB.y);
@@ -694,24 +698,27 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
       tr.ev(17, it);
       if (p.u_out != nullptr) {
         q7_tmem_st_wait();
-        smA = quad_sum(smA); sqA = quad_sum(sqA); smB = quad_sum(smB); sqB = quad_sum(sqB);
+        // partials (mean, M2) of this CTA's 384 columns; the peer's are merged in below
+        const float2 pA = ln_quad_merge(ln_partial(kA, smA, sqA, 1.0f / (Q7_DH / 4)), Q7_DH / 4);
+        const float2 pB = ln_quad_merge(ln_partial(kB, smB, sqB, 1.0f / (Q7_DH / 4)), Q7_DH / 4);
         if (ew == 0 && lane == 0) mbar_expect_tx(&stat_bar[par], Q7_BM * 8);
         if (writer) {
           const uint32_t slot = q7_mapa(smem_u32(stat_x + (par * Q7_BM + rA) * 2), peer);
           const uint32_t bar = q7_mapa(smem_u32(&stat_bar[par]), peer);
-          q7_st_async(slot, smA, bar);
-          q7_st_async(slot + 4, sqA, bar);
-          q7_st_async(slot + 8 * 8, smB, bar);
-          q7_st_async(slot + 8 * 8 + 4, sqB, bar);
+          q7_st_async(slot, pA.x, bar);
+          q7_st_async(slot + 4, pA.y, bar);
+          q7_st_async(slot + 8 * 8, pB.x, bar);
+          q7_st_async(slot + 8 * 8 + 4, pB.y, bar);
         }
         mbar_wait(&stat_bar[par], (it >> 1) & 1u);
         tr.ev(18, it);
         const float2 xA = *reinterpret_cast<const float2*>(stat_x + (par * Q7_BM + rA) * 2);
         const float2 xB = *reinterpret_cast<const float2*>(stat_x + (par * Q7_BM + rB) * 2);
         const float inv_h = 1.0f / static_cast<float>(Q7_D);
-        const float meanA = (smA + xA.x) * inv_h, meanB = (smB + xB.x) * inv_h;
-        const float rsA = rsqrtf(fmaxf(fmaf(-meanA, meanA, (sqA + xA.y) * inv_h), 0.f) + 1e-5f);
-        const float rsB = rsqrtf(fmaxf(fmaf(-meanB, meanB, (sqB + xB.y) * inv_h), 0.f) + 1e-5f);
+        const float2 stA = ln_merge(pA, xA, Q7_DH), stB = ln_merge(pB, xB, Q7_DH);
+        const float meanA = stA.x, meanB = stB.x;
+        const float rsA = rsqrtf(fmaxf(stA.y, 0.f) * inv_h + 1e-5f);
+        const float rsB = rsqrtf(fmaxf(stB.y, 0.f) * inv_h + 1e-5f);
         const float2 aA2 = make_float2(rsA, rsA), cA2 = make_float2(-meanA * rsA, -meanA * rsA);
         const float2 aB2 = make_float2(rsB, rsB), cB2 = make_float2(-meanB * rsB, -meanB * rsB);
         bf16* uA = p.u_out + growA * Q7_D + col_half + q * 4;

@@ -227,7 +227,8 @@ __global__ void __launch_bounds__(RL_THREADS, 1)
       if (norm && ew == 0 && lane == 0) mbar_expect_tx(&stat_bar[par], static_cast<uint32_t>(parts * RL_BM * 8));
       mbar_wait(&tmem_full[as], aphase);
       tcgen05_fence_after();
-      float sm[4] = {0.f, 0.f, 0.f, 0.f}, sq[4] = {0.f, 0.f, 0.f, 0.f};
+      // row statistics of this thread's 32 values of each row: sums of v - K and (v - K)^2, K = its first value (common.cuh)
+      float sm[4] = {0.f, 0.f, 0.f, 0.f}, sq[4] = {0.f, 0.f, 0.f, 0.f}, kk[4];
       auto sweep1 = [&](int hh, int cb, const float4(&f)[8]) {
         uint32_t o[32];
         tmem_ld_16x64(t_lane + (static_cast<uint32_t>(16 * hh) << 16) + cb * 64, o);
@@ -253,10 +254,13 @@ __global__ void __launch_bounds__(RL_THREADS, 1)
           if (okA) *reinterpret_cast<float4*>(oa + jj * 16) = vA;
           if (okB) *reinterpret_cast<float4*>(ob + jj * 16) = vB;
           if (norm) {
-            sm[2 * hh] += (vA.x + vA.y) + (vA.z + vA.w);
-            sq[2 * hh] = fmaf(vA.x, vA.x, fmaf(vA.y, vA.y, fmaf(vA.z, vA.z, fmaf(vA.w, vA.w, sq[2 * hh]))));
-            sm[2 * hh + 1] += (vB.x + vB.y) + (vB.z + vB.w);
-            sq[2 * hh + 1] = fmaf(vB.x, vB.x, fmaf(vB.y, vB.y, fmaf(vB.z, vB.z, fmaf(vB.w, vB.w, sq[2 * hh + 1]))));
+            if (cb == 0 && jj == 0) { kk[2 * hh] = vA.x; kk[2 * hh + 1] = vB.x; }
+            const float4 dA = make_float4(vA.x - kk[2 * hh], vA.y - kk[2 * hh], vA.z - kk[2 * hh], vA.w - kk[2 * hh]);
+            const float4 dB = make_float4(vB.x - kk[2 * hh + 1], vB.y - kk[2 * hh + 1], vB.z - kk[2 * hh + 1], vB.w - kk[2 * hh + 1]);
+            sm[2 * hh] += (dA.x + dA.y) + (dA.z + dA.w);
+            sq[2 * hh] = fmaf(dA.x, dA.x, fmaf(dA.y, dA.y, fmaf(dA.z, dA.z, fmaf(dA.w, dA.w, sq[2 * hh]))));
+            sm[2 * hh + 1] += (dB.x + dB.y) + (dB.z + dB.w);
+            sq[2 * hh + 1] = fmaf(dB.x, dB.x, fmaf(dB.y, dB.y, fmaf(dB.z, dB.z, fmaf(dB.w, dB.w, sq[2 * hh + 1]))));
             o[4 * k0] = __float_as_uint(vA.x); o[4 * k0 + 1] = __float_as_uint(vA.y);
             o[4 * k1] = __float_as_uint(vA.z); o[4 * k1 + 1] = __float_as_uint(vA.w);
             o[4 * k0 + 2] = __float_as_uint(vB.x); o[4 * k0 + 3] = __float_as_uint(vB.y);
@@ -275,9 +279,12 @@ __global__ void __launch_bounds__(RL_THREADS, 1)
       sweep1(1, 1, f1);
       if (norm) {
         rl_tmem_st_wait();
-        // this warp's slab statistics of its 32 rows -> every CTA that holds columns of these rows (same a, every pair)
+        // this warp's slab partials (mean, M2) of its 32 rows -> every CTA that holds columns of these rows (same a, every pair)
 #pragma unroll
-        for (int i = 0; i < 4; ++i) { sm[i] = quad_sum(sm[i]); sq[i] = quad_sum(sq[i]); }
+        for (int i = 0; i < 4; ++i) {
+          const float2 st = ln_quad_merge(ln_partial(kk[i], sm[i], sq[i], 1.0f / 32.f), 32.f);
+          sm[i] = st.x; sq[i] = st.y;
+        }
         if (writer) {
           const uint32_t slot = smem_u32(stat_x + (par * parts + part) * RL_BM + quarter * 32 + g);
           const uint32_t bar = smem_u32(&stat_bar[par]);
@@ -291,14 +298,19 @@ __global__ void __launch_bounds__(RL_THREADS, 1)
         mbar_wait(&stat_bar[par], (it >> 1) & 1u);
         float mean[4], rstd[4];
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          float s = 0.f, qq = 0.f;
+        for (int i = 0; i < 4; ++i) {   // parts of 128 values each: mean of the means, then M2 = sum M2_c + 128 sum (mean_c - mean)^2
+          const float2* sx = stat_x + par * parts * RL_BM + quarter * 32 + g + 8 * i;
+          float s = 0.f;
+          for (int c = 0; c < parts; ++c) s += sx[c * RL_BM].x;
+          const float m = s * (128.f * p.inv_n);
+          float m2 = 0.f, dd = 0.f;
           for (int c = 0; c < parts; ++c) {
-            const float2 v = stat_x[(par * parts + c) * RL_BM + quarter * 32 + g + 8 * i];
-            s += v.x; qq += v.y;
+            const float2 v = sx[c * RL_BM];
+            m2 += v.y;
+            dd = fmaf(v.x - m, v.x - m, dd);
           }
-          mean[i] = s * p.inv_n;
-          rstd[i] = rsqrtf(fmaxf(fmaf(-mean[i], mean[i], qq * p.inv_n), 0.f) + 1e-5f);
+          mean[i] = m;
+          rstd[i] = rsqrtf(fmaxf(fmaf(128.f, dd, m2), 0.f) * p.inv_n + 1e-5f);
         }
         // ---------------- sweep 2: u = LayerNorm(h) gamma + beta, bf16, 8-byte stores ----------------
 #pragma unroll

@@ -7,8 +7,11 @@ The tests therefore compare the increment ``out - x`` with the fp64 increment of
 This module holds what tests/test_gpu_section_increments.py (the CUDA kernels, -m gpu) and tests/test_section_sensitivity.py
 (the CPU guard of the bars) share, so that the two cannot drift apart:
 
-  * CASES, the bars and the seeded inputs of every case (per-row offsets that stress the LayerNorm statistics,
-    optionally q / k projections sharpened so that softmax is peaked, optionally loud text tokens);
+  * CASES, the bars and the seeded inputs of every case (optionally q / k projections sharpened so that softmax is peaked,
+    optionally loud text tokens);
+  * OFFSET_CASES: whole blocks whose rows carry a constant offset of ~1e3 times their spread.  LayerNorm is shift-invariant
+    and every sublayer reads only LayerNorm outputs, so the offset leaves the reference increment unchanged; row statistics
+    that cancel (fp32 E[v^2] - mean^2) do not;
   * the fp64 reference increments (the oracle's own functions, minus x);
   * a restatement of each section with the bf16 kernels' rounding points (bf16 operands u, W, q / k / v, the
     probabilities P, the attention output), which gives the error floor a correct kernel can reach;
@@ -52,6 +55,8 @@ class Case:
     loud_text: bool = False      # text tokens 128.. with 4x the norm: the second key tile raises the row maxima
     sections: Tuple[str, ...] = SECTIONS
     fp32: bool = False           # also run the fp32 engine
+    offset: float = 0.0          # |row offset| in [offset / 2, offset], sign mixed per row (0: none)
+    const_text: bool = False     # every text row of a sequence equal (the constant-text path of the four-CTA kernel)
 
 
 def _c(name, hidden, heads, n, T, S, **kw):
@@ -90,6 +95,21 @@ CASES = (
 )
 CASE = {c.name: c for c in CASES}
 assert len(CASE) == len(CASES)
+
+# whole blocks under a row offset, one per fused-LayerNorm site (tests/test_gpu_section_increments.py names the kernel each
+# must reach).  bf16: |offset| <= 2048 keeps the fp32 rounding of h (ulp 2.4e-4) far below the bars.  fp32: the rounding of
+# x + increment near the offset is itself ~1e-4 x offset / 1000 of the increment, so its offset is ~100.
+OFFSET_CASES = (
+    _c("off_t750", 768, 1, 2, 750, 40, sections=("block",), offset=2048.0),           # norm2: flash_attn768 / 768q
+    _c("off_s64", 768, 1, 2, 300, 64, sections=("block",), offset=2048.0),            # norm3: cross_fused
+    _c("off_s129", 768, 1, 2, 300, 129, sections=("block",), offset=2048.0),          # norm3: flash_attn768q<CROSS>
+    _c("off_const", 768, 1, 2, 750, 40, sections=("block",), offset=2048.0, const_text=True),   # norm3: constant text
+    _c("off_h12_s100", 768, 12, 2, 257, 100, sections=("block",), offset=2048.0),     # norm3: gemm_resid_ln after out_proj
+    _c("off_s129_fp32", 768, 1, 2, 257, 129, sections=("block",), offset=128.0, fp32=True),
+)
+CASE.update({c.name: c for c in OFFSET_CASES})
+assert len(CASE) == len(CASES) + len(OFFSET_CASES)
+OFFSET_GUARD_CASES = ("off_t750", "off_h12_s100")
 
 # the cases the CPU guard re-derives the bars on, each with its "_sharp" twin: every attention path of the table
 GUARD_CASES = ("s64", "s129", "s257", "s512", "s200_loud", "h12_t257_s100", "h256_t300")
@@ -131,8 +151,9 @@ def sharpen(sd: Dict[str, Tensor], layer: int, factor: float) -> Dict[str, Tenso
 
 
 def case_inputs(case: Case):
-    """(cfg, fp32 state dict, x, text) of a case.  x has a N(0, 4^2) offset per row (LayerNorm statistics under a large
-    mean); loud_text scales text tokens 128.. by 4."""
+    """(cfg, fp32 state dict, x, text) of a case.  x is N(0, 1) around a N(0, 4^2) mean per row, so |mean| / spread stays
+    below ~12: too small to expose cancelling row statistics, which is what OFFSET_CASES add (see row_offsets).  loud_text
+    scales text tokens 128.. by 4; const_text repeats each sequence's first text row."""
     cfg = O.OracleConfig(case.hidden, 2, case.heads, 64, case.hidden, 50)
     sd = O.make_state_dict(cfg, WEIGHT_SEED)
     if case.sharp:
@@ -142,7 +163,22 @@ def case_inputs(case: Case):
     text = torch.randn(case.n, case.S, case.hidden, generator=g)
     if case.loud_text:
         text[:, 128:] *= 4.0
+    if case.const_text:
+        text = text[:, :1].expand_as(text).contiguous()
+    if case.offset:
+        x = (x.double() + row_offsets(case)).float()
     return cfg, sd, x, text
+
+
+def row_offsets(case: Case) -> Tensor:
+    """fp64 [n, T, 1] offsets added to x (fp32) by case_inputs: integers of either sign, |c| in [offset / 2, offset] (zeros
+    without an offset).  ``x.double() - row_offsets(case)`` is exact, so the reference sees the input that was fed, unshifted."""
+    if not case.offset:
+        return torch.zeros(case.n, case.T, 1, dtype=torch.float64)
+    g = torch.Generator().manual_seed(INPUT_SEED + 1)
+    mag = torch.round(case.offset * (1 + torch.rand(case.n, case.T, 1, generator=g, dtype=torch.float64)) / 2)
+    sign = torch.where(torch.rand(case.n, case.T, 1, generator=g) < 0.5, -1.0, 1.0).double()
+    return sign * mag
 
 
 def _f64(sd, x, text):
@@ -150,8 +186,11 @@ def _f64(sd, x, text):
 
 
 def increments(case: Case, sd, x, text) -> Dict[str, Tensor]:
-    """fp64 increments ``section(x) - x`` of the oracle for the case's sections ("block": the whole DiT block)."""
+    """fp64 increments ``section(x) - x`` of the oracle for the case's sections ("block": the whole DiT block).  The row
+    offsets of the case are taken off x first: the sections are shift-invariant, so this is the increment of x itself,
+    computed without the offset's cancellation."""
     sd, x, text = _f64(sd, x, text)
+    x = x - row_offsets(case)
     rot = O.rotary_angles(case.T, case.hidden // case.heads, torch.float64)
     p = f"blocks.{LAYER}."
     f = {"self": lambda: O.self_attention(sd, p, x, rot, case.heads),
@@ -179,10 +218,39 @@ DEFECTS = {
 }
 # kept to record what bf16 cannot see: its effect (~2e-4) is below the rounding of an increment, it is not a checked defect
 INVISIBLE = {("mlp", "gelu_tanh")}
+# norm2 and norm3 with one-pass fp32 statistics (_ln_one_pass_fp32), planted in a whole block: only a row offset makes it
+# visible (at the |mean| / spread <= ~12 of CASES it moves an increment by ~1e-5), so only OFFSET_CASES are checked for it
+OFFSET_DEFECT = ("block", "layernorm_one_pass_fp32")
 
 
 def _bf(z: Tensor) -> Tensor:
     return z.to(torch.bfloat16).to(z.dtype)
+
+
+def _ln_one_pass_fp32(x, w, b):
+    """LayerNorm with fp32 one-pass statistics var = E[v^2] - mean^2 in the partial-sum order of gemm_resid_ln's epilogue:
+    column parts of 128, each 4 threads x 32 serial (fused) multiply-adds, then the 4-thread sums and the parts in turn.
+    Wrong by ~eps (mean / spread)^2 in the variance: the defect a cancelling row-statistics kernel makes."""
+    H = x.shape[-1]
+    assert H % 128 == 0
+    v = x.float().reshape(*x.shape[:-1], H // 128, 4, 32)
+    s = torch.zeros(v.shape[:-1], dtype=torch.float32)
+    q = torch.zeros_like(s)
+    for k in range(32):                       # fp32 sum; fma: exact product (fp64) + one rounding to fp32
+        s = s + v[..., k]
+        q = (v[..., k].double() ** 2 + q.double()).float()
+    s, q = s.sum(-1), q.sum(-1)               # 4-thread (quad) sums in fp32
+    S, Q = s[..., 0], q[..., 0]
+    for c in range(1, H // 128):
+        S, Q = S + s[..., c], Q + q[..., c]
+    inv_n = torch.tensor(1.0 / H, dtype=torch.float32)
+    mean = S * inv_n
+    rstd = torch.rsqrt(torch.clamp_min(Q * inv_n - mean * mean, 0.0) + 1e-5)
+    return (x - mean.double()[..., None]) * rstd.double()[..., None] * w + b
+
+
+def _ln(x, w, b, one_pass):
+    return _ln_one_pass_fp32(x, w, b) if one_pass else F.layer_norm(x, (x.shape[-1],), w, b, 1e-5)
 
 
 def _self(sd, p, x, heads, rot, r, defect):
@@ -215,10 +283,10 @@ def _self(sd, p, x, heads, rot, r, defect):
     return o
 
 
-def _cross(sd, p, x, text, heads, r, defect):
+def _cross(sd, p, x, text, heads, r, defect, ln_one_pass=False):
     n, T, H = x.shape
     S, d = text.shape[1], H // heads
-    u = r(F.layer_norm(x, (H,), sd[p + "norm2.weight"], sd[p + "norm2.bias"], 1e-5))
+    u = r(_ln(x, sd[p + "norm2.weight"], sd[p + "norm2.bias"], ln_one_pass))
     w, b = sd[p + "cross_attn.in_proj_weight"], sd[p + "cross_attn.in_proj_bias"]
     bq = torch.zeros_like(b[:H]) if defect == "score_bias_dropped" else b[:H]   # folded: the score bias sqrt(1/d) bq.k_j
     q = F.linear(u, r(w[:H]), bq).reshape(n, T, heads, d).permute(0, 2, 1, 3)
@@ -234,9 +302,9 @@ def _cross(sd, p, x, text, heads, r, defect):
     return F.linear(r(o), r(sd[p + "cross_attn.out_proj.weight"]), sd[p + "cross_attn.out_proj.bias"])
 
 
-def _mlp(sd, p, x, r, defect):
+def _mlp(sd, p, x, r, defect, ln_one_pass=False):
     H = x.shape[-1]
-    u = r(F.layer_norm(x, (H,), sd[p + "norm3.weight"], sd[p + "norm3.bias"], 1e-5))
+    u = r(_ln(x, sd[p + "norm3.weight"], sd[p + "norm3.bias"], ln_one_pass))
     a = F.linear(u, r(sd[p + "mlp_fc1.weight"]), sd[p + "mlp_fc1.bias"])
     gate = F.linear(u, r(sd[p + "gate.weight"]), sd[p + "gate.bias"])
     g = F.gelu(a, approximate="tanh" if defect == "gelu_tanh" else "none") * torch.sigmoid(gate)
@@ -247,18 +315,23 @@ def _mlp(sd, p, x, r, defect):
 
 def restated(case: Case, sd, x, text, section: str, bf16: bool = False, defect: Optional[Tuple[str, str]] = None) -> Tensor:
     """fp64 increment of ``section`` from the restatement above: with the kernels' bf16 rounding points (bf16=True) and / or
-    one planted defect (section, name).  "block" chains the three sections, the defect landing in its own section."""
+    one planted defect (section, name).  "block" chains the three sections, the defect landing in its own section (a "block"
+    defect in norm2 and norm3), and with bf16=True keeps the residual stream in fp32 as the kernels do.  x is what was fed,
+    row offsets included."""
     sd, x, text = _f64(sd, x, text)
     rot = O.rotary_angles(case.T, case.hidden // case.heads, torch.float64)
     p = f"blocks.{LAYER}."
     r = _bf if bf16 else (lambda z: z)
     dd = lambda s: defect[1] if defect is not None and defect[0] == s else None  # noqa: E731
+    one_pass = defect == OFFSET_DEFECT
     f = {"self": lambda h: _self(sd, p, h, case.heads, rot, r, dd("self")),
-         "cross": lambda h: _cross(sd, p, h, text, case.heads, r, dd("cross")),
-         "mlp": lambda h: _mlp(sd, p, h, r, dd("mlp"))}
+         "cross": lambda h: _cross(sd, p, h, text, case.heads, r, dd("cross"), one_pass),
+         "mlp": lambda h: _mlp(sd, p, h, r, dd("mlp"), one_pass)}
     if section != "block":
         return f[section](x)
     h = x
     for s in ("self", "cross", "mlp"):
         h = h + f[s](h)
+        if bf16:
+            h = h.float().double()
     return h - x

@@ -6,7 +6,10 @@ the mean of V pass; the increment does not.  The cases cover the kernels each se
 RoPE and GEGLU epilogues, flash_attn768 / flash_attn768q, flash_attn_d64, cross_fused, flash_attn768q<CROSS> (including its
 online-softmax rescale), the cluster scores + softmax kernel with row_lsum -- with default and sharpened (peaked softmax)
 weights, and again under the developer switches that select another kernel for the same section.  Each run also checks that
-the kernel class it was meant to exercise actually ran.  tests/test_section_sensitivity.py guards the bars on the CPU."""
+the kernel class it was meant to exercise actually ran.  Whole blocks with a row offset of ~1e3 x the row spread
+(R.OFFSET_CASES) reach every LayerNorm fused into a kernel epilogue, and the developer switches that move those LayerNorms
+to the two-pass kernel must agree with the default under that offset.  tests/test_section_sensitivity.py guards the bars on
+the CPU."""
 import functools
 
 import pytest
@@ -20,6 +23,7 @@ pytestmark = pytest.mark.gpu
 
 F768, SELF_PV, FLASH64 = "tc_gemm.flash768_ln", "tc_gemm.self_pv", "tc_gemm.flash_attn"
 XFUSED, XFLASH, XPV = "tc_gemm.cross_fused_ln", "tc_gemm.cross_flash_ln", "tc_gemm.cross_pv"
+XOUT = "tc_gemm.cross_out"
 
 
 @pytest.fixture(scope="module")
@@ -60,7 +64,12 @@ def expected_kernels(case, opts):
         cross_k = ((XFLASH,), ())
     else:
         cross_k = ((XPV,), (XFUSED, XFLASH))
-    return {"self": self_k, "cross": cross_k}
+    if not folded and not on("no_fc2_ln"):   # multi-head out-projection + residual + norm3 in gemm_resid_ln
+        cross_k = (cross_k[0] + (XOUT,), cross_k[1])
+    out = {"self": self_k, "cross": cross_k}
+    if case.offset:   # whole block: both sections' kernels (a constant-text block skips the cross kernel's work)
+        out["block"] = (self_k[0] + (() if case.const_text else cross_k[0]), self_k[1] + cross_k[1])
+    return out
 
 
 def run_and_check(case, precision, dev, opts=None):
@@ -104,9 +113,55 @@ def test_section_increments_bf16(dev, name):
     run_and_check(R.CASE[name], "bf16", dev)
 
 
-@pytest.mark.parametrize("name", [c.name for c in R.CASES if c.fp32])
+@pytest.mark.parametrize("name", [c.name for c in R.CASES + R.OFFSET_CASES if c.fp32])
 def test_section_increments_fp32(dev, name):
     run_and_check(R.CASE[name], "fp32", dev)
+
+
+# every fused-LayerNorm site under a row offset: (options, case)
+OFFSET_RUNS = [
+    ({"flash768_quad": 1}, "off_t750"),       # norm2 in flash_attn768 (two-CTA)
+    ({"flash768_quad": 2}, "off_t750"),       # norm2 in flash_attn768q (four-CTA); norm3 in cross_fused
+    ({}, "off_s64"),                          # norm3 in cross_fused
+    ({}, "off_s129"),                         # norm3 in flash_attn768q<CROSS>
+    ({"flash768_quad": 2}, "off_const"),      # norm3 of constant-text sequences in flash_attn768q
+    ({}, "off_h12_s100"),                     # norm3 in gemm_resid_ln after the multi-head out-projection
+]
+OFFSET_IDS = [f"{'+'.join(f'{k}={v}' for k, v in o.items()) or 'default'}-{n}" for o, n in OFFSET_RUNS]
+
+
+@pytest.mark.parametrize("opts,name", OFFSET_RUNS, ids=OFFSET_IDS)
+def test_block_increment_under_row_offset(dev, opts, name):
+    run_and_check(R.CASE[name], "bf16", dev, opts)
+
+
+def block_increment(case, dev, opts):
+    cfg, sd, x, text, _ = reference(case.name)
+    for k, v in opts.items():
+        _lib.debug_option(k, v)
+    try:
+        m = build_model(cfg, sd, "bf16", dev)
+        out = m.blocks[R.LAYER](x.to(dev), text.to(dev))
+        return out.double().cpu() - x.double()
+    finally:
+        _lib.debug_option("reset", 0)
+
+
+# DESIGN §9: these switches move a LayerNorm out of a fused epilogue into the two-pass layernorm kernel (or move the
+# constant-text sequences back to the cross-attention kernel) and change results by bf16 rounding only, offset or not
+OFFSET_SWITCHES = [("no_fc2_ln", "off_h12_s100"), ("no_fc2_ln", "off_s129"), ("no_flash768", "off_t750"),
+                   ("no_fused_cross", "off_s64"), ("no_const_text", "off_const")]
+
+
+@pytest.mark.parametrize("switch,name", OFFSET_SWITCHES, ids=[f"{s}-{n}" for s, n in OFFSET_SWITCHES])
+def test_switches_agree_under_row_offset(dev, switch, name):
+    case = R.CASE[name]
+    base = {"flash768_quad": 2} if case.const_text else {}
+    default = block_increment(case, dev, base)
+    switched = block_increment(case, dev, {**base, switch: 1})
+    e, row = R.errors(switched, default)
+    print(f"[offset-switch] {name} {switch}: {e:.2e}/{row:.2e}")
+    assert e <= R.bar(case, "bf16", "block") and row <= R.row_bar(case, "bf16", "block"), (name, switch, e, row)
 
 
 ONE_HEAD_T = ("t1", "t129", "t257", "t750_sharp", "t2250")

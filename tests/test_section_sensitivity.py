@@ -4,6 +4,8 @@ For the guard cases of oracle/section_ref.py (every attention path of the case t
 asserts that the bars can still tell a correct kernel from a wrong one:
   (a) the bf16-emulated error floor of every section is at most half its bar (the per-row floor at most half the row bar);
   (b) every planted defect moves the checked error by at least 2.5x its bar, in the default case or in its sharpened twin.
+For the row-offset cases (whole blocks at |mean| / spread ~ 1e3) it asserts the same of the one-pass LayerNorm statistics,
+with the fp32 rounding of the offset residual stream in the floor.
 A change that loosens a bar, the sharpening or the inputs until a defect could pass fails here."""
 import pytest
 import torch
@@ -72,3 +74,42 @@ def test_every_planted_defect_clears_the_bar_by_a_margin(evaluated, name):
             assert m < 1.0, (name, key, m)          # recorded: below what bf16 rounding lets a test see
         else:
             assert m >= R.DEFECT_MARGIN, (name, key, m)
+
+
+@pytest.fixture(scope="module")
+def offset_evaluated():
+    """case name -> (case, reference increment, emulated increment, one-pass LayerNorm increment) of the block."""
+    torch.set_num_threads(max(1, min(8, torch.get_num_threads())))
+    out = {}
+    for name in R.OFFSET_GUARD_CASES:
+        c = R.CASE[name]
+        _, sd, x, text = R.case_inputs(c)
+        want = R.increments(c, sd, x, text)["block"]
+        emul = R.restated(c, sd, x, text, "block", bf16=True)
+        bad = R.restated(c, sd, x, text, "block", bf16=True, defect=R.OFFSET_DEFECT)
+        out[name] = (c, x, want, emul, bad)
+    return out
+
+
+@pytest.mark.parametrize("name", R.OFFSET_GUARD_CASES)
+def test_offset_case_shape(offset_evaluated, name):
+    """The offsets are what the cases claim: |mean| / spread ~ 1e3 per row, both signs, and an exact fp64 reference input."""
+    c, x, _, _, _ = offset_evaluated[name]
+    off = R.row_offsets(c)
+    ratio = (x.double().mean(-1) / x.double().std(-1)).abs()
+    assert float(ratio.min()) >= 300 and bool((off > 0).any()) and bool((off < 0).any())
+    assert bool(((x.double() - off) + off == x.double()).all())
+
+
+@pytest.mark.parametrize("name", R.OFFSET_GUARD_CASES)
+def test_offset_floor_is_at_most_half_the_bar(offset_evaluated, name):
+    c, _, want, emul, _ = offset_evaluated[name]
+    e, row = R.errors(emul, want)
+    assert e <= R.FLOOR_MARGIN * R.bar(c, "bf16", "block"), (name, e)
+    assert row <= R.FLOOR_MARGIN * R.row_bar(c, "bf16", "block"), (name, row)
+
+
+@pytest.mark.parametrize("name", R.OFFSET_GUARD_CASES)
+def test_offset_cases_catch_one_pass_layernorm(offset_evaluated, name):
+    c, _, want, _, bad = offset_evaluated[name]
+    assert margin(c, "block", bad, want) >= R.DEFECT_MARGIN, (name, R.errors(bad, want))
