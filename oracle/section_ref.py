@@ -74,6 +74,12 @@ CASES = (
     _c("t750", 768, 1, 2, 750, 40),
     _c("t750_sharp", 768, 1, 2, 750, 40, sharp=True),
     _c("t2250", 768, 1, 1, 2250, 40),
+    # max_seq_len: RoPE angles up to 4095 rad (inv_freq = 1), 32 key tiles, attention flatter than at any shorter length
+    _c("t4096", 768, 1, 1, 4096, 40),
+    # two of C5's own kernel combinations (parallel.c5_lengths): the two-CTA kernel with a partial 119-row query tile and
+    # cross_fused; the four-CTA kernel over six query tiles and <CROSS> with exactly one full key tile
+    _c("c5_t375_s32", 768, 1, 2, 375, 32),
+    _c("c5_t1500_s128", 768, 1, 2, 1500, 128),
     # several work items per cluster / CTA: hand-over between consecutive items
     _c("load", 768, 1, 40, 750, 40, sections=("self", "cross")),
     # text lengths: cross_fused (S <= 64), flash_attn768q<CROSS> (64 < S <= 256), scores + softmax + P.V on the folded
@@ -113,6 +119,9 @@ OFFSET_GUARD_CASES = ("off_t750", "off_h12_s100")
 
 # the cases the CPU guard re-derives the bars on, each with its "_sharp" twin: every attention path of the table
 GUARD_CASES = ("s64", "s129", "s257", "s512", "s200_loud", "h12_t257_s100", "h256_t300")
+# cases whose floor the guard checks without planted defects: their paths are guard cases above, but not their lengths
+# (the score-bias defect at S = 128, one key tile, moves the increment by only 2.05 bars: a guard case would need a twin)
+FLOOR_CASES = ("t4096", "c5_t375_s32", "c5_t1500_s128")
 
 
 def _peaked(case: Case, section: str) -> bool:

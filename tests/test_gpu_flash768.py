@@ -75,7 +75,8 @@ def run(dev, n, T, flags=0, key_scale=None, seed=0, with_ln=True):
         (O.rel_l2(u.float().view(n, T, H).cpu(), want_u.cpu()) if with_ln else 0.0), bool(torch.isfinite(hh).all())
 
 
-@pytest.mark.parametrize("n,T", [(2, 750), (3, 1), (1, 100), (2, 128), (1, 129), (1, 257), (1, 2250), (5, 40)])
+@pytest.mark.parametrize("n,T", [(2, 750), (3, 1), (1, 100), (2, 128), (1, 129), (1, 257), (1, 375), (1, 2250), (1, 4096),
+                                 (5, 40)])
 def test_flash768_vs_torch(dev, n, T):
     eo, eh, eu, finite = run(dev, n, T)
     assert finite and eo <= 1e-2 and eh <= 3e-3 and eu <= 6e-3, (eo, eh, eu)

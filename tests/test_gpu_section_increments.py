@@ -166,8 +166,8 @@ def test_switches_agree_under_row_offset(dev, switch, name):
 
 ONE_HEAD_T = ("t1", "t129", "t257", "t750_sharp", "t2250")
 SWITCH_RUNS = [
-    ({"flash768_quad": 1}, ONE_HEAD_T + ("load",)),            # two-CTA flash_attn768 at every length
-    ({"flash768_quad": 2}, ONE_HEAD_T + ("load",)),            # four-CTA flash_attn768q at every length
+    ({"flash768_quad": 1}, ONE_HEAD_T + ("load", "t4096")),   # two-CTA flash_attn768 at every length
+    ({"flash768_quad": 2}, ONE_HEAD_T + ("load", "t4096")),   # four-CTA flash_attn768q at every length
     ({"no_flash768": 1}, ONE_HEAD_T),
     ({"no_flash": 1}, ("h12_t130_s9", "h12_t257_s100_sharp", "h12_t750_s100", "h256_t300", "h128_t77")),
     ({"no_fused_cross": 1}, ("s1", "s64", "s64_sharp", "s65", "s129_sharp", "s256", "s200_loud_sharp")),

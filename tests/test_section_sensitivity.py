@@ -56,6 +56,19 @@ def test_bf16_floor_is_at_most_half_the_bar(evaluated, name):
             assert rb is None or row <= R.FLOOR_MARGIN * rb, (c.name, s, row)
 
 
+@pytest.mark.parametrize("name", R.FLOOR_CASES)
+def test_bf16_floor_is_at_most_half_the_bar_at_long_and_c5_lengths(name):
+    """The same floor check at max_seq_len (flatter attention: nothing else bounds its floor) and at C5's kernel combinations."""
+    torch.set_num_threads(max(1, min(8, torch.get_num_threads())))
+    c = R.CASE[name]
+    _, sd, x, text = R.case_inputs(c)
+    want = R.increments(c, sd, x, text)
+    for s in c.sections:
+        e, row = R.errors(R.restated(c, sd, x, text, s, bf16=True), want[s])
+        assert e <= R.FLOOR_MARGIN * R.bar(c, "bf16", s), (name, s, e)
+        assert row <= R.FLOOR_MARGIN * R.row_bar(c, "bf16", s), (name, s, row)
+
+
 def margin(c, section, got, want):
     """How many bars the checked error of an increment is away from passing (the larger of the global and the row check)."""
     e, row = R.errors(got, want)
