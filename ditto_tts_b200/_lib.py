@@ -66,6 +66,10 @@ SIGNATURES = {
     "ditto_p_sample_multistep_rng": (_I32, [_P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _I32, _P]),
     "ditto_cfg_update_known": (_I32, [_P, _P, _P, _P, _P, _P, _P, _I64, _F, _P, _P, _P, _P, _I64, _I64, _I32, _P]),
     "ditto_p_sample_known": (_I32, [_P, _P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _P, _P, _P, _I64, _I32, _P]),
+    "ditto_p_sample_per_utt": (_I32, [_P, _P, _P, _P, _P, _P, _P, _I32, _F, _P, _I64, _I64, _I64, _P, _P, _P, _P, _P, _P, _I64, _I32,
+                                      _P]),
+    "ditto_cfg_update_per_utt": (_I32, [_P, _P, _P, _P, _P, _P, _P, _P, _I64, _F, _P, _P, _P, _P, _P, _I64, _I64, _I32, _P]),
+    "ditto_randn_latents": (_I32, [_P, _P, _I64, _I64, _P, _P]),
     "ditto_q_sample": (_I32, [_P, _P, _P, _P, _P, _I64, _I64, _P]),
     "ditto_workspace_bytes_ragged": (_I64, [_P, C.POINTER(SeqGroup), _I64]),
     "ditto_forward_ragged": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _P, _I64, _P]),
@@ -76,6 +80,8 @@ SIGNATURES = {
                                                    _P]),
     "ditto_p_sample_ragged_known": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _P, _I32, _F, _P, _P, _P, _P, _P, _P, _I64,
                                            _I32, _P]),
+    "ditto_p_sample_ragged_per_utt": (_I32, [_P, _P, C.POINTER(SeqGroup), _I64, _P, _P, _P, _P, _I32, _F, _P, _P, _P, _P, _P, _P,
+                                             _P, _I64, _I32, _P]),
     "ditto_dit_block": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),
     "ditto_attn_self": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),
     "ditto_attn_cross": (_I32, [_P, _I32, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),

@@ -770,18 +770,34 @@ __device__ __forceinline__ void multistep_store(const MultistepRow& c, float4 xv
 // =====================================================================================================
 __device__ __forceinline__ float known_value(float p, float z, float a, float s) { return __fmaf_rn(s, z, __fmul_rn(a, p)); }
 
-// One instance per (form, noise source, known frames).  Loads in the order t row, eps_c, eps_u, x, supplied z, hist, then the
-// draw.  t_in == t.  The instances without rng and without known frames read t through t_in, whose __restrict__ keeps that
-// load on the read-only path (LDG.CONSTANT; a pointer the rng instances write loses it); the others read it through t.  The
-// t clamps stay written out in place: moving them into a helper changes how the multistep loop is unrolled.
-template <bool MULTISTEP, bool RNG, bool KNOWN>
+// the normal4 of vector i (sequence seq) of the current draw: keyed by seeds[seq] and counted from the sequence's first vector
+// (per-utterance seeds), else keyed by rng[0] and counted from vec_offset
+template <bool PER_UTT>
+__device__ __forceinline__ float4 drawn_noise(unsigned long long seed, unsigned long long draw, const unsigned long long* seeds, int64_t seq,
+                                              int64_t i, int64_t vec_per_seq, int64_t vec_offset) {
+  if (PER_UTT && seeds != nullptr) return philox_normal4(seeds[seq], draw, static_cast<unsigned long long>(i - seq * vec_per_seq));
+  return philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i));
+}
+
+// One instance per (form, noise source, known frames, per-utterance parameters).  Loads in the order t row, eps_c, eps_u, x,
+// supplied z, hist, then the draw.  t_in == t.  The instances without rng and without known frames read t through t_in, whose
+// __restrict__ keeps that load on the read-only path (LDG.CONSTANT; a pointer the rng instances write loses it); the others
+// read it through t.  The t clamps stay written out in place: moving them into a helper changes how the multistep loop is
+// unrolled.
+// PER_UTT (seeds and / or w_seq may be non-null; the noise contract is in include/ditto_b200.h, ditto_p_sample_per_utt): the
+// scale is w_seq[seq] and, with seeds, the Philox key is seeds[seq] and the counter's vector index is counted from the
+// sequence's own first element.  It is a template parameter, not a runtime branch, so that the other instances keep their
+// code and time: the per-vector row loads, the division remainder and two more live registers stay out of them.  Its two
+// pointers are the last kernel parameters so that the other instances also keep their parameter offsets.
+template <bool MULTISTEP, bool RNG, bool KNOWN, bool PER_UTT>
 __global__ void __launch_bounds__(256)
     cfg_update_kernel(const float4* __restrict__ eps_c, const float4* __restrict__ eps_u, const float4* __restrict__ x,
                       const float4* __restrict__ z, const int64_t* __restrict__ t_in, unsigned long long* rng, int64_t* t, int64_t n_t,
-                      const float* __restrict__ coef, const float* __restrict__ coef_known, int steps, float w,
+                      const float* __restrict__ coef, const float* __restrict__ coef_known, int steps, float w_all,
                       float4* __restrict__ out, float4* __restrict__ hist, const float4* __restrict__ known,
                       const uint8_t* __restrict__ mask, int64_t vec_per_seq, int64_t vec_per_frame, int64_t total_vec,
-                      int64_t vec_offset, int advance) {
+                      int64_t vec_offset, int advance, const unsigned long long* __restrict__ seeds,
+                      const float* __restrict__ w_seq) {
   unsigned long long seed = 0ull, draw = 0ull;
   if (RNG) {
     seed = rng[0];
@@ -791,12 +807,13 @@ __global__ void __launch_bounds__(256)
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < total_vec;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int64_t seq = i / vec_per_seq;
+    const float w = (PER_UTT && w_seq != nullptr) ? w_seq[seq] : w_all;
     if (KNOWN && mask[i / vec_per_frame] != 0) {
       int64_t tt = ts[seq];
       tt = tt < 0 ? 0 : (tt >= steps ? steps - 1 : tt);
       const float a = coef_known[tt * 2 + 0], s = coef_known[tt * 2 + 1];
       const float4 pv = known[i];
-      const float4 zv = RNG ? philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i)) : z[i];
+      const float4 zv = RNG ? drawn_noise<PER_UTT>(seed, draw, seeds, seq, i, vec_per_seq, vec_offset) : z[i];
       out[i] = make_float4(known_value(pv.x, zv.x, a, s), known_value(pv.y, zv.y, a, s), known_value(pv.z, zv.z, a, s),
                            known_value(pv.w, zv.w, a, s));
       continue;
@@ -807,7 +824,7 @@ __global__ void __launch_bounds__(256)
       const float4 xv = x[i];
       float4 zv = RNG ? make_float4(0.f, 0.f, 0.f, 0.f) : supplied_noise<KNOWN>(z, i);
       const float4 h = multistep_hist(hist, i, c.c4);
-      if (RNG) zv = philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i));
+      if (RNG) zv = drawn_noise<PER_UTT>(seed, draw, seeds, seq, i, vec_per_seq, vec_offset);
       multistep_store(c, xv, e, zv, h, out, hist, i);
     } else {
       int64_t tt = ts[seq];
@@ -815,7 +832,7 @@ __global__ void __launch_bounds__(256)
       const float c1 = coef[tt * 3 + 0], c2 = coef[tt * 3 + 1], c3 = coef[tt * 3 + 2];
       const float4 e = guided_eps(eps_c, eps_u, i, w);
       const float4 xv = x[i];
-      const float4 zv = RNG ? philox_normal4(seed, draw, static_cast<unsigned long long>(vec_offset + i)) : supplied_noise<KNOWN>(z, i);
+      const float4 zv = RNG ? drawn_noise<PER_UTT>(seed, draw, seeds, seq, i, vec_per_seq, vec_offset) : supplied_noise<KNOWN>(z, i);
       out[i] = ddpm_update4(xv, e, zv, c1, c2, c3);
     }
   }
@@ -851,16 +868,19 @@ int launch_cfg_update(const CfgUpdateParams& p, cudaStream_t st) {
                      static_cast<double>(frames));
   using Kernel = void (*)(const float4*, const float4*, const float4*, const float4*, const int64_t*, unsigned long long*, int64_t*,
                           int64_t, const float*, const float*, int, float, float4*, float4*, const float4*, const uint8_t*, int64_t,
-                          int64_t, int64_t, int64_t, int);
-  static const Kernel kernels[8] = {cfg_update_kernel<false, false, false>, cfg_update_kernel<false, false, true>,
-                                    cfg_update_kernel<false, true, false>,  cfg_update_kernel<false, true, true>,
-                                    cfg_update_kernel<true, false, false>,  cfg_update_kernel<true, false, true>,
-                                    cfg_update_kernel<true, true, false>,   cfg_update_kernel<true, true, true>};
-  kernels[(ms ? 4 : 0) + (draw ? 2 : 0) + (kn ? 1 : 0)]<<<blocks, 256, 0, st>>>(
+                          int64_t, int64_t, int64_t, int, const unsigned long long*, const float*);
+#define DITTO_CFG_UPDATE_INSTANCES(PU)                                                                                      \
+  cfg_update_kernel<false, false, false, PU>, cfg_update_kernel<false, false, true, PU>, cfg_update_kernel<false, true, false, PU>, \
+      cfg_update_kernel<false, true, true, PU>, cfg_update_kernel<true, false, false, PU>, cfg_update_kernel<true, false, true, PU>, \
+      cfg_update_kernel<true, true, false, PU>, cfg_update_kernel<true, true, true, PU>
+  static const Kernel kernels[16] = {DITTO_CFG_UPDATE_INSTANCES(false), DITTO_CFG_UPDATE_INSTANCES(true)};
+#undef DITTO_CFG_UPDATE_INSTANCES
+  const bool per_utt = p.seeds != nullptr || p.w_seq != nullptr;
+  kernels[(per_utt ? 8 : 0) + (ms ? 4 : 0) + (draw ? 2 : 0) + (kn ? 1 : 0)]<<<blocks, 256, 0, st>>>(
       reinterpret_cast<const float4*>(p.eps_c), reinterpret_cast<const float4*>(p.eps_u), reinterpret_cast<const float4*>(p.x),
       reinterpret_cast<const float4*>(p.z), p.t, p.rng, p.t, p.n_t, p.coef, p.coef_known, p.steps, p.w,
       reinterpret_cast<float4*>(p.out), reinterpret_cast<float4*>(p.hist), reinterpret_cast<const float4*>(p.known), p.mask,
-      p.per / 4, p.frame / 4, total_vec, p.elem_offset / 4, p.advance ? 1 : 0);
+      p.per / 4, p.frame / 4, total_vec, p.elem_offset / 4, p.advance ? 1 : 0, p.seeds, p.w_seq);
   DITTO_LAUNCH_CHECK();
   return 0;
 }
@@ -896,6 +916,28 @@ int launch_randn(const unsigned long long* rng, int64_t elem_offset, float* out,
   if (n <= 0) return 0;
   const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(round_up(ceil_div(n, 1024), 148), 148 * 32));
   randn_kernel<<<blocks, 256, 0, st>>>(rng, elem_offset / 4, out, n);
+  DITTO_LAUNCH_CHECK();
+  return 0;
+}
+
+// x_T of every utterance of a job in one launch: utterance b owns rows row0[b] .. row0[b + 1] - 1 of out [rows, H] and gets the
+// normals of draw 2^64 - 1 under its own seed, counted from its own first element (the x_T rule of the noise contract,
+// include/ditto_b200.h).  blockIdx.y = utterance; its blocks stride over its vectors.
+__global__ void randn_latents_kernel(const unsigned long long* __restrict__ seeds, const int64_t* __restrict__ row0, int64_t vec_per_row,
+                                     float4* __restrict__ out) {
+  const int64_t b = blockIdx.y;
+  const unsigned long long seed = seeds[b];
+  const int64_t first = row0[b] * vec_per_row, nv = (row0[b + 1] - row0[b]) * vec_per_row;
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < nv; i += static_cast<int64_t>(gridDim.x) * blockDim.x)
+    out[first + i] = philox_normal4(seed, ~0ull, static_cast<unsigned long long>(i));
+}
+int launch_randn_latents(const unsigned long long* seeds, const int64_t* row0, int64_t B, int64_t H, float* out, cudaStream_t st) {
+  DITTO_REQUIRE(H % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && B <= 65535, DITTO_E_BADARG,
+                "randn_latents: H % 4, 16-B aligned output and B <= 65535");
+  if (B <= 0) return 0;
+  // about 8 blocks per SM over the job whatever its utterance count (the lengths stay on the device)
+  const unsigned per_utt = static_cast<unsigned>(std::max<int64_t>(1, ceil_div(148 * 8, B)));
+  randn_latents_kernel<<<dim3(per_utt, static_cast<unsigned>(B)), 256, 0, st>>>(seeds, row0, H / 4, reinterpret_cast<float4*>(out));
   DITTO_LAUNCH_CHECK();
   return 0;
 }

@@ -1274,6 +1274,8 @@ struct Update {
   int32_t advance = 0;             // t -= 1 and draw counter += 1 after the update (needs rng)
   bool multistep = false;          // a multistep call: hist is required
   bool need_noise = false;         // exactly one of z / rng is required
+  const uint64_t* seeds = nullptr; // per-utterance noise keys (need rng, exclude z); null: the key rng[0], packed positions
+  const float* w = nullptr;        // per-utterance guidance scales; null: the scalar scale
 };
 
 // the checks on the update's own arguments, after the caller's null-argument and size checks: bad arguments (-1) first, then
@@ -1281,6 +1283,8 @@ struct Update {
 static int check_update(const ditto_engine* e, const std::string& what, const Update& u) {
   DITTO_REQUIRE(!u.multistep || u.hist, DITTO_E_BADARG, what + ": null argument (hist)");
   DITTO_REQUIRE((u.known == nullptr) == (u.mask == nullptr), DITTO_E_BADARG, what + ": known and known_mask go together (both or neither)");
+  DITTO_REQUIRE(!(u.seeds && u.z), DITTO_E_BADARG, what + ": seeds and z exclude each other (seeds key the noise drawn in the kernel)");
+  DITTO_REQUIRE(!u.seeds || u.rng, DITTO_E_BADARG, what + ": seeds need rng (its draw counter and ticket)");
   DITTO_REQUIRE(!(u.z && u.rng) && (u.z || u.rng || !u.need_noise), DITTO_E_BADARG,
                 what + ": exactly one of z / rng (known frames need the step's noise)");
   DITTO_REQUIRE(!u.advance || u.rng, DITTO_E_BADARG, what + ": advance needs rng (in-kernel noise)");
@@ -1305,6 +1309,7 @@ static int update(const ditto_engine* e, const float* eps_c, const float* eps_u,
   p.t = t; p.n_t = n_t; p.coef = u.hist ? e->coef_ms : e->coef; p.coef_known = e->coef_known; p.steps = e->steps; p.w = w;
   p.out = x_out; p.hist = u.hist; p.known = u.known; p.mask = u.mask;
   p.B = B; p.per = per; p.frame = e->H; p.elem_offset = elem_offset; p.advance = u.advance != 0;
+  p.seeds = reinterpret_cast<const unsigned long long*>(u.seeds); p.w_seq = u.w;
   return launch_cfg_update(p, st);
 }
 
@@ -1363,12 +1368,21 @@ int32_t ditto_cfg_multistep_update_rng(ditto_engine_t* e, const float* eps_c, co
                      Update{.rng = rng, .hist = hist, .advance = advance, .multistep = true, .need_noise = true}, stream);
 }
 
+int32_t ditto_cfg_update_per_utt(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
+                                 uint64_t* rng, const uint64_t* seeds, int64_t* t, int64_t n_t, float guidance_scale, const float* w,
+                                 float* x_out, float* hist, const float* known, const uint8_t* known_mask, int64_t B, int64_t T,
+                                 int32_t advance, void* stream) {
+  return update_call(e, "cfg_update_per_utt", eps_c, eps_u, x, t, n_t, guidance_scale, x_out, B, e ? T * e->H : 0,
+                     Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true,
+                            .seeds = seeds, .w = w},
+                     stream);
+}
+
 int32_t ditto_cfg_update_known(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z, uint64_t* rng,
                                int64_t* t, int64_t n_t, float guidance_scale, float* x_out, float* hist, const float* known,
                                const uint8_t* known_mask, int64_t B, int64_t T, int32_t advance, void* stream) {
-  return update_call(e, "cfg_update_known", eps_c, eps_u, x, t, n_t, guidance_scale, x_out, B, e ? T * e->H : 0,
-                     Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true},
-                     stream);
+  return ditto_cfg_update_per_utt(e, eps_c, eps_u, x, z, rng, nullptr, t, n_t, guidance_scale, nullptr, x_out, hist, known, known_mask, B,
+                                  T, advance, stream);
 }
 
 int32_t ditto_p_sample(ditto_engine_t* e, const float* x, const void* ctx, const int64_t* t, const float* z, int32_t guided,
@@ -1400,18 +1414,32 @@ int32_t ditto_p_sample_multistep_rng(ditto_engine_t* e, const float* x, const vo
                         workspace_bytes, stream);
 }
 
+int32_t ditto_p_sample_per_utt(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, const float* z, uint64_t* rng,
+                               const uint64_t* seeds, int32_t guided, float guidance_scale, const float* w, int64_t B, int64_t T, int64_t S,
+                               float* eps_scratch, float* x_out, float* hist, const float* known, const uint8_t* known_mask,
+                               void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
+  return p_sample_dense(e, "p_sample_per_utt", x, ctx, t, guided, guidance_scale, B, T, S, eps_scratch, x_out,
+                        Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true,
+                               .seeds = seeds, .w = w},
+                        workspace, workspace_bytes, stream);
+}
+
 int32_t ditto_p_sample_known(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, const float* z, uint64_t* rng, int32_t guided,
                              float guidance_scale, int64_t B, int64_t T, int64_t S, float* eps_scratch, float* x_out, float* hist,
                              const float* known, const uint8_t* known_mask, void* workspace, int64_t workspace_bytes, int32_t advance,
                              void* stream) {
-  return p_sample_dense(e, "p_sample_known", x, ctx, t, guided, guidance_scale, B, T, S, eps_scratch, x_out,
-                        Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true},
-                        workspace, workspace_bytes, stream);
+  return ditto_p_sample_per_utt(e, x, ctx, t, z, rng, nullptr, guided, guidance_scale, nullptr, B, T, S, eps_scratch, x_out, hist, known,
+                                known_mask, workspace, workspace_bytes, advance, stream);
 }
 
 int32_t ditto_randn(const uint64_t* rng, int64_t elem_offset, float* out, int64_t n, void* stream) {
   DITTO_REQUIRE(rng && out && n >= 0 && elem_offset >= 0, DITTO_E_BADARG, "randn: bad argument");
   return launch_randn(reinterpret_cast<const unsigned long long*>(rng), elem_offset, out, n, static_cast<cudaStream_t>(stream));
+}
+
+int32_t ditto_randn_latents(const uint64_t* seeds, const int64_t* row0, int64_t B, int64_t H, float* out, void* stream) {
+  DITTO_REQUIRE(seeds && row0 && out && B >= 0 && H > 0, DITTO_E_BADARG, "randn_latents: bad argument");
+  return launch_randn_latents(reinterpret_cast<const unsigned long long*>(seeds), row0, B, H, out, static_cast<cudaStream_t>(stream));
 }
 
 int32_t ditto_q_sample(ditto_engine_t* e, const float* x_start, const float* noise, const int64_t* t, float* out, int64_t B,
@@ -1475,6 +1503,7 @@ static int32_t p_sample_ragged(ditto_engine_t* e, const char* what, const float*
   if (gs.size() > 1 && e->n_side > 0) fork_lock.lock();
   Fork fork(e, st);
   DITTO_TRY(fork.begin(static_cast<int>(gs.size())));
+  int64_t utt0 = 0;                             // the group's first utterance: seeds / w are in packed-group order
   for (size_t gi = 0; gi < gs.size(); ++gi) {  // offsets were filled in by the layout pass of forward_impl
     const SeqGroup& g = gs[gi];
     const int64_t per = g.T * H, row = g.xrow0 * H;
@@ -1485,9 +1514,12 @@ static int32_t p_sample_ragged(ditto_engine_t* e, const char* what, const float*
     ug.hist = u.hist ? u.hist + row : nullptr;
     ug.known = u.known ? u.known + row : nullptr;
     ug.mask = u.mask ? u.mask + g.xrow0 : nullptr;
+    ug.seeds = u.seeds ? u.seeds + utt0 : nullptr;
+    ug.w = u.w ? u.w + utt0 : nullptr;
     ug.advance = 0;
     DITTO_TRY(update(e, ec, guided ? ec + g.n_x * per : nullptr, x + row, t + g.seq0, g.n, guidance_scale, x_out + row, ug, g.n_x, per,
                      row, fork.stream(static_cast<int>(gi))));
+    utt0 += g.n_x;
   }
   DITTO_TRY(fork.end());
   if (u.advance) DITTO_TRY(launch_step_advance(reinterpret_cast<unsigned long long*>(u.rng), t, n_t, st));
@@ -1524,13 +1556,22 @@ int32_t ditto_p_sample_ragged_multistep_rng(ditto_engine_t* e, const float* x, c
                          workspace_bytes, stream);
 }
 
+int32_t ditto_p_sample_ragged_per_utt(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
+                                      const float* z, uint64_t* rng, const uint64_t* seeds, int32_t guided, float guidance_scale,
+                                      const float* w, float* eps_scratch, float* x_out, float* hist, const float* known,
+                                      const uint8_t* known_mask, void* workspace, int64_t workspace_bytes, int32_t advance, void* stream) {
+  return p_sample_ragged(e, "p_sample_ragged_per_utt", x, groups, n_groups, t, guided, guidance_scale, eps_scratch, x_out,
+                         Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true,
+                                .seeds = seeds, .w = w},
+                         workspace, workspace_bytes, stream);
+}
+
 int32_t ditto_p_sample_ragged_known(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups, int64_t* t,
                                     const float* z, uint64_t* rng, int32_t guided, float guidance_scale, float* eps_scratch, float* x_out,
                                     float* hist, const float* known, const uint8_t* known_mask, void* workspace, int64_t workspace_bytes,
                                     int32_t advance, void* stream) {
-  return p_sample_ragged(e, "p_sample_ragged_known", x, groups, n_groups, t, guided, guidance_scale, eps_scratch, x_out,
-                         Update{.z = z, .rng = rng, .hist = hist, .known = known, .mask = known_mask, .advance = advance, .need_noise = true},
-                         workspace, workspace_bytes, stream);
+  return ditto_p_sample_ragged_per_utt(e, x, groups, n_groups, t, z, rng, nullptr, guided, guidance_scale, nullptr, eps_scratch, x_out,
+                                       hist, known, known_mask, workspace, workspace_bytes, advance, stream);
 }
 
 // ---- block-level operators (the reference's component signatures, src/components/DiT.py) -----------------------------

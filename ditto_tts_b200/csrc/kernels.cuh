@@ -73,7 +73,9 @@ int launch_transpose_v(const bf16* v, int64_t ld, bf16* vt, int64_t n_seq, int T
 // rng = {seed, draw counter, ticket, -}) at element elem_offset + i; neither: no noise term.  advance (needs rng): the last
 // block to finish adds 1 to the draw counter and subtracts 1 from t[0 .. n_t).  Known frames (replacement conditioning, speech
 // prompt / infilling; mask != null): every `frame` elements share one mask byte, and a frame with mask != 0 becomes a p + s z
-// with {a, s} = coef_known[t] and p = known.
+// with {a, s} = coef_known[t] and p = known.  Per sequence (w_seq / seeds non-null): the scale w_seq[seq] instead of w, and
+// (with rng) the key seeds[seq] instead of rng[0], the element counted from the sequence's first element instead of
+// elem_offset + i.
 struct CfgUpdateParams {
   const float* eps_c = nullptr; const float* eps_u = nullptr; const float* x = nullptr;
   const float* z = nullptr; unsigned long long* rng = nullptr;
@@ -83,10 +85,13 @@ struct CfgUpdateParams {
   const float* known = nullptr; const uint8_t* mask = nullptr;
   int64_t B = 0, per = 0, frame = 0, elem_offset = 0;
   bool advance = false;
+  const unsigned long long* seeds = nullptr; const float* w_seq = nullptr;
 };
 int launch_cfg_update(const CfgUpdateParams& p, cudaStream_t st);
 int launch_step_advance(unsigned long long* rng, int64_t* t, int64_t n_t, cudaStream_t st);
 int launch_randn(const unsigned long long* rng, int64_t elem_offset, float* out, int64_t n, cudaStream_t st);
+// x_T of B utterances: rows row0[b] .. row0[b + 1] - 1 of out [rows, H] get draw 2^64 - 1 under seeds[b] (row0 [B + 1], device)
+int launch_randn_latents(const unsigned long long* seeds, const int64_t* row0, int64_t B, int64_t H, float* out, cudaStream_t st);
 int launch_rope_angles(const float* t, const float* pos, float* out, int64_t batch, int T, int heads, int d, cudaStream_t st);
 int launch_schedule_coef(const float* betas, const float* alphas, const float* acp, float* coef, int steps, cudaStream_t st);
 int launch_q_sample(const float* x0, const float* noise, const int64_t* t, const float* buf, int steps, float* out, int64_t B,

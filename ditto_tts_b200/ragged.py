@@ -124,6 +124,20 @@ class RaggedBatch:
             out[self.x_offset[i]:self.x_offset[i] + self.lengths[i]] = q != 0
         return out
 
+    def pack_seeds(self, seeds: Sequence[int]) -> torch.Tensor:
+        """One seed per utterance (checked ints in [0, 2^64)) -> int64 [B] bit patterns in group order, the order of the
+        groups' latents (ditto_p_sample_ragged_per_utt)."""
+        from .sampler import _seed_tensor
+        return _seed_tensor([seeds[i] for i in self.order], self.device)
+
+    def pack_w(self, w: Sequence[float]) -> torch.Tensor:
+        """One guidance scale per utterance -> fp32 [B] in group order."""
+        return torch.tensor([float(w[i]) for i in self.order], dtype=torch.float32).to(self.device)
+
+    def row0(self) -> torch.Tensor:
+        """First packed latent row of every utterance in group order, then x_rows: the row table of ditto_randn_latents."""
+        return torch.tensor([self.x_offset[i] for i in self.order] + [self.x_rows], dtype=torch.int64).to(self.device)
+
     def unpack(self, packed: torch.Tensor) -> List[torch.Tensor]:
         return [packed[self.x_offset[i]:self.x_offset[i] + self.lengths[i]].clone() for i in range(self.B)]
 
@@ -136,15 +150,17 @@ class RaggedBatch:
             parts.append(torch.cat([tg, tg]) if self.guided else tg)
         return torch.cat(parts).contiguous()
 
-    def unpack_eps(self, eps: torch.Tensor, w: Optional[float]) -> List[torch.Tensor]:
-        """packed sequence-layout output -> per-utterance eps_hat (guided: the CFG combine, as ditto_cfg_ddpm_update)."""
+    def unpack_eps(self, eps: torch.Tensor, w) -> List[torch.Tensor]:
+        """packed sequence-layout output -> per-utterance eps_hat (guided: the CFG combine, as ditto_cfg_ddpm_update; ``w`` a
+        scalar or one scale per utterance)."""
         out = [None] * self.B
         row = 0
         for T, _, idx in self.groups:
             n = len(idx)
             blk = eps[row:row + (2 if self.guided else 1) * n * T].view(-1, T, self.H)
             for j, i in enumerate(idx):
-                out[i] = (blk[n + j] + w * (blk[j] - blk[n + j])) if self.guided else blk[j].clone()
+                wi = w[i] if isinstance(w, (list, tuple)) else w
+                out[i] = (blk[n + j] + wi * (blk[j] - blk[n + j])) if self.guided else blk[j].clone()
             row += blk.shape[0] * T
         return out
 
@@ -160,36 +176,44 @@ class RaggedBatch:
         return out
 
     def p_sample(self, x_packed, t_seq, z_packed, w: float, eps: torch.Tensor, x_out: torch.Tensor, ws=None, hist=None,
-                 known=None, mask=None, rng=None):
-        """One sampler step (ditto_p_sample_ragged_known); ``hist`` (packed like x): the multistep update; ``known`` /
+                 known=None, mask=None, rng=None, seeds=None, w_dev=None, advance=None):
+        """One sampler step (ditto_p_sample_ragged_per_utt); ``hist`` (packed like x): the multistep update; ``known`` /
         ``mask`` (packed like x / one byte per packed row): known frames; ``rng``: noise drawn in the per-group update kernels
-        instead of ``z_packed``, and the "t -= 1" bookkeeping in a one-block kernel after them."""
+        instead of ``z_packed``, and (unless ``advance`` is False) the "t -= 1" bookkeeping in a one-block kernel after them.
+        ``seeds`` / ``w_dev`` [B] in group order (pack_seeds / pack_w): per-utterance noise keys (with rng) and scales."""
         ws = self.workspace() if ws is None else ws
+        if advance is None:
+            advance = rng is not None
         with torch.cuda.device(self.device):
-            _lib.check(_lib.load().ditto_p_sample_ragged_known(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
-                                                               _ptr(t_seq), _ptr(z_packed), _ptr(rng), 1 if self.guided else 0, float(w),
-                                                               _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(known), _ptr(mask), _ptr(ws),
-                                                               ws.numel(), 0 if rng is None else 1, _stream()),
-                       "ditto_p_sample_ragged_known")
+            _lib.check(_lib.load().ditto_p_sample_ragged_per_utt(self.model.engine(), _ptr(x_packed), self.c_groups, len(self.groups),
+                                                                 _ptr(t_seq), _ptr(z_packed), _ptr(rng), _ptr(seeds),
+                                                                 1 if self.guided else 0, float(w), _ptr(w_dev), _ptr(eps), _ptr(x_out),
+                                                                 _ptr(hist), _ptr(known), _ptr(mask), _ptr(ws), ws.numel(),
+                                                                 1 if advance else 0, _stream()),
+                       "ditto_p_sample_ragged_per_utt")
 
 
 class RaggedStepGraph(_CapturedStep):
     """One sampler iteration over a ragged batch as a CUDA graph (noise draw, forward, CFG + update, t decrement).  With
     ``multistep`` the update is DPM-Solver++(2M)'s and the graph owns its ``hist`` buffer (packed like x).  With ``known``
-    it owns the known latents (packed like x) and the frame mask (one byte per packed row), filled by ``reset``."""
+    it owns the known latents (packed like x) and the frame mask (one byte per packed row), filled by ``reset``.  A guided
+    graph reads one guidance scale per utterance (group order) from ``w_dev`` (``set_scale``); a ``seeded`` one keys each
+    utterance's noise by its entry of ``seeds`` (group order, filled by ``reset``)."""
 
-    def __init__(self, batch: RaggedBatch, w: float, draw_noise: bool, multistep: bool = False, known: bool = False):
-        self.batch, self.w = batch, w
+    def __init__(self, batch: RaggedBatch, w, draw_noise: bool, multistep: bool = False, known: bool = False,
+                 seeded: bool = False):
+        self.batch = batch
         dev = batch.device
-        self._buffers((batch.x_rows, batch.H), batch.n_seq, draw_noise, multistep, known, dev)
+        self._buffers((batch.x_rows, batch.H), batch.n_seq, draw_noise, multistep, known, dev, batch.B, batch.guided, seeded)
+        self.set_scale(w)
         self._ctx_ptrs = [c.data_ptr() for c in batch._ctx]
         self.eps = torch.empty((batch.seq_rows, batch.H), dtype=torch.float32, device=dev)
         self.ws = batch.workspace()
         self._capture(dev)
 
     def _p_sample(self, rng):
-        self.batch.p_sample(self.x, self.t, self.z, self.w, self.eps, self.x, ws=self.ws, hist=self.hist, known=self.known,
-                            mask=self.mask, rng=rng)
+        self.batch.p_sample(self.x, self.t, self.z, 0.0, self.eps, self.x, ws=self.ws, hist=self.hist, known=self.known,
+                            mask=self.mask, rng=rng, seeds=self.seeds, w_dev=self.w_dev)
 
     def valid_for(self, batch: "RaggedBatch") -> bool:
         """The captured kernels read the context buffers and the workspace by address."""

@@ -11,13 +11,18 @@ utterance batch.
 device buffer ``hist`` that the update kernel reads and rewrites.
 ``sample_latents(..., known=p, known_mask=m)`` continues a speech prompt or fills a span: frames with m True are given
 (replacement conditioning, schedules.known_coef; the update kernel re-noises them).
+``sample_latents(..., seeds=[s_0, ...], guidance_scale=[w_0, ...])`` gives every utterance its own noise stream (x_T and every
+step's noise depend on its seed alone, not on its batch-mates: include/ditto_b200.h, ditto_p_sample_per_utt) and its own
+guidance scale; one captured step graph serves every scale.
 """
 from __future__ import annotations
 
 import ctypes as C
 import math
+import numbers
+import operator
 from collections import OrderedDict
-from typing import List, Optional
+from typing import List, Optional, Union
 
 import torch
 
@@ -25,7 +30,76 @@ from . import _lib, schedules
 from ._lib import DittoError
 from .model import DiTTO, _check_t_range, _need_cuda_f32, _ptr, _stream
 
-__all__ = ["DiTTOSampler", "StepGraph"]
+__all__ = ["DiTTOSampler", "StepGraph", "randn_latents"]
+
+
+def _check_seeds(seeds, B: int, noise=None, generator=None) -> Optional[List[int]]:
+    """None, or B integer seeds in [0, 2^64) (one per utterance); refused together with ``noise`` / ``generator``, which
+    are the other two sources of the job's noise."""
+    if seeds is None:
+        return None
+    if noise is not None or generator is not None:
+        raise DittoError("seeds excludes noise= and generator=: each is a different source of the job's noise")
+    try:
+        vals = seeds.tolist() if hasattr(seeds, "tolist") else list(seeds)
+    except TypeError:
+        vals = None
+    if isinstance(seeds, (str, bytes)) or not isinstance(vals, list):
+        raise DittoError("seeds must be a sequence of one integer per utterance")
+    out = []
+    for i, v in enumerate(vals):
+        if isinstance(v, bool):
+            raise DittoError(f"seeds[{i}] must be an integer, got a bool")
+        try:
+            v = operator.index(v)
+        except TypeError:
+            raise DittoError(f"seeds[{i}] must be an integer, got {type(v).__name__}") from None
+        if not 0 <= v < 1 << 64:
+            raise DittoError(f"seeds[{i}] = {v} is outside [0, 2^64)")
+        out.append(v)
+    if len(out) != B:
+        raise DittoError(f"seeds must hold one seed per utterance: {B} expected, got {len(out)}")
+    return out
+
+
+def _check_scale(w, B: int) -> Union[None, float, List[float]]:
+    """The guidance scale of a job: None (unguided), a scalar for every utterance, or a sequence of B finite scales.
+    A scalar is whatever ``float(w)`` took before per-utterance scales existed: a real number (numpy scalars too) or a
+    one-element tensor / array, whatever B is.  It is passed on as before, without a finiteness check, so a scalar job
+    behaves exactly as it did; only per-utterance lists are checked to be finite."""
+    if w is None:
+        return None
+    if isinstance(w, numbers.Real):
+        return float(w)
+    size = w.numel() if isinstance(w, torch.Tensor) else getattr(w, "size", None)
+    if size == 1 and (isinstance(w, torch.Tensor) or hasattr(w, "__array__")):
+        return float(w.item())
+    try:
+        vals = w.tolist() if hasattr(w, "tolist") else list(w)
+    except TypeError:
+        raise DittoError("guidance_scale must be a number or a sequence of one number per utterance") from None
+    if len(vals) != B:
+        raise DittoError(f"guidance_scale must be a scalar or hold one scale per utterance: {B} expected, got {len(vals)}")
+    out = [float(v) for v in vals]
+    if not all(math.isfinite(v) for v in out):
+        raise DittoError("guidance_scale: every per-utterance scale must be finite")
+    return out
+
+
+def _seed_tensor(seeds: List[int], dev) -> torch.Tensor:
+    """uint64 seeds as the int64 bit patterns the device reads as uint64."""
+    return torch.tensor([v - (1 << 64) if v >= 1 << 63 else v for v in seeds], dtype=torch.int64).to(dev)
+
+
+def randn_latents(seeds: torch.Tensor, row0: torch.Tensor, rows: int, H: int) -> torch.Tensor:
+    """x_T of a seeded job in one launch (ditto_randn_latents): utterance b owns rows row0[b] .. row0[b + 1] - 1 of the
+    [rows, H] result and gets the normals of its own seed's reserved draw.  seeds int64 [B] (uint64 bit patterns), row0
+    int64 [B + 1], both on the device."""
+    out = torch.empty((rows, H), dtype=torch.float32, device=seeds.device)
+    with torch.cuda.device(seeds.device):
+        _lib.check(_lib.load().ditto_randn_latents(_ptr(seeds), _ptr(row0), seeds.numel(), H, _ptr(out), _stream()),
+                   "ditto_randn_latents")
+    return out
 
 
 class _CapturedStep:
@@ -33,7 +107,8 @@ class _CapturedStep:
     the captured pointers stay valid), the capture, the per-job reset and the replay loop.  A subclass allocates eps and the
     workspace and makes the step's one C call in ``_p_sample(rng)``."""
 
-    def _buffers(self, shape, n_seq: int, draw_noise: bool, multistep: bool, known: bool, device):
+    def _buffers(self, shape, n_seq: int, draw_noise: bool, multistep: bool, known: bool, device, n_utt: int = 0,
+                 guided: bool = False, seeded: bool = False):
         self.draw_noise = draw_noise
         self.x = torch.zeros(shape, dtype=torch.float32, device=device)
         # caller-supplied noise lands here; drawn noise never touches HBM
@@ -43,6 +118,17 @@ class _CapturedStep:
         self.known = torch.zeros_like(self.x) if known else None          # known frames and their mask, filled by reset
         self.mask = torch.zeros(tuple(shape[:-1]), dtype=torch.uint8, device=device) if known else None
         self.t = torch.zeros((n_seq,), dtype=torch.int64, device=device)
+        # per-utterance guidance scales (a scalar scale is broadcast into it, so one capture serves every scale) and seeds
+        self.w_dev = torch.zeros((n_utt,), dtype=torch.float32, device=device) if guided else None
+        self.seeds = torch.zeros((n_utt,), dtype=torch.int64, device=device) if seeded else None
+
+    def set_scale(self, w):
+        """The guidance scale the next replays use: a scalar for every utterance or a [n_utt] tensor (graph order)."""
+        if self.w_dev is not None:
+            if isinstance(w, torch.Tensor):
+                self.w_dev.copy_(w)
+            else:
+                self.w_dev.fill_(float(w))
 
     def _capture(self, device):
         # eager warm-up (engine set-up, lazy initialisation) on a side stream, then capture
@@ -66,7 +152,7 @@ class _CapturedStep:
             self.t.sub_(1)
 
     def reset(self, x_init: torch.Tensor, t_start: int, seed: Optional[int] = None, known: Optional[torch.Tensor] = None,
-              known_mask: Optional[torch.Tensor] = None):
+              known_mask: Optional[torch.Tensor] = None, seeds: Optional[torch.Tensor] = None):
         self.x.copy_(x_init)
         self.t.fill_(t_start)
         if self.hist is not None:
@@ -74,7 +160,10 @@ class _CapturedStep:
         if self.known is not None:
             self.known.copy_(known)
             self.mask.copy_(known_mask)
-        if self.draw_noise:   # fresh seed per sampling job (from torch's CPU generator: torch.manual_seed makes runs repeatable)
+        if self.seeds is not None:   # per-utterance seeds (graph order) key the noise; the draw counter starts at 0
+            self.seeds.copy_(seeds)
+            self.rng.zero_()
+        elif self.draw_noise:   # fresh seed per sampling job (from torch's CPU generator: torch.manual_seed makes runs repeatable)
             if seed is None:
                 seed = int(torch.randint(0, 2 ** 62, (1,)).item())
             self.rng.copy_(torch.tensor([seed, 0, 0, 0], dtype=torch.int64), non_blocking=False)
@@ -82,9 +171,9 @@ class _CapturedStep:
     def replay(self):
         self.graph.replay()
 
-    def run(self, x_init: torch.Tensor, taus: List[int], consecutive: bool, noise=None, known=None, known_mask=None):
+    def run(self, x_init: torch.Tensor, taus: List[int], consecutive: bool, noise=None, known=None, known_mask=None, seeds=None):
         """One sampling job: reset, then one replay per visited timestep (``noise`` indexed by timestep, as ``x``)."""
-        self.reset(x_init, taus[0], known=known, known_mask=known_mask)
+        self.reset(x_init, taus[0], known=known, known_mask=known_mask, seeds=seeds)
         for t_val in taus:
             if noise is not None:
                 self.z.copy_(noise[t_val], non_blocking=True)
@@ -101,14 +190,17 @@ class StepGraph(_CapturedStep):
     the device-resident step index ``t`` and bumps the draw counter -- so the host issues ONE launch per denoising step
     instead of ~70 and the graph contains kernels of libditto_b200 only.  A multistep sampler's graph also owns ``hist``,
     the x0 prediction one step carries to the next (zero-filled by ``reset``).  A graph for known frames (speech prompt,
-    infilling) owns the known latents and the frame mask, filled by ``reset``; it launches as many kernels per step."""
+    infilling) owns the known latents and the frame mask, filled by ``reset``; it launches as many kernels per step.  A guided
+    graph reads its guidance scales from ``w_dev`` (one per utterance, ``set_scale``); a ``seeded`` graph keys every
+    utterance's noise by its entry of ``seeds`` (filled by ``reset``)."""
 
-    def __init__(self, sampler: "DiTTOSampler", B: int, T: int, S: int, guided: bool, w: float, ctx: torch.Tensor,
-                 draw_noise: bool, device, known: bool = False):
+    def __init__(self, sampler: "DiTTOSampler", B: int, T: int, S: int, guided: bool, w, ctx: torch.Tensor,
+                 draw_noise: bool, device, known: bool = False, seeded: bool = False):
         m = sampler.model
         n = 2 * B if guided else B
-        self.B, self.T, self.S, self.guided, self.w = B, T, S, guided, w
-        self._buffers((B, T, m.hidden_dim), n, draw_noise, sampler.multistep, known, device)
+        self.B, self.T, self.S, self.guided = B, T, S, guided
+        self._buffers((B, T, m.hidden_dim), n, draw_noise, sampler.multistep, known, device, B, guided, seeded)
+        self.set_scale(w)
         self.eps = torch.empty((n, T, m.hidden_dim), dtype=torch.float32, device=device)
         self.ctx = ctx
         self.ws = m.workspace(n, T, S)
@@ -117,8 +209,8 @@ class StepGraph(_CapturedStep):
         self._keys = (self.ctx.data_ptr(), self.ws.data_ptr())
 
     def _p_sample(self, rng):
-        self._sampler._p_sample_raw(self.x, self.ctx, self.t, self.z, self.guided, self.w, self.S, self.eps, self.x, ws=self.ws,
-                                    hist=self.hist, known=self.known, mask=self.mask, rng=rng)
+        self._sampler._p_sample_raw(self.x, self.ctx, self.t, self.z, self.guided, 0.0, self.S, self.eps, self.x, ws=self.ws,
+                                    hist=self.hist, known=self.known, mask=self.mask, rng=rng, seeds=self.seeds, w_dev=self.w_dev)
 
     def valid_for(self, ctx: torch.Tensor, ws: torch.Tensor) -> bool:
         return self._keys == (ctx.data_ptr(), ws.data_ptr())
@@ -207,18 +299,23 @@ class DiTTOSampler:
             text_emb = torch.cat([text_emb, null], dim=0)  # [cond(B); uncond(B)]
         return self.model.text_context(text_emb, name="sampler_ctx", T_hint=T)
 
-    def _p_sample_raw(self, x, ctx, t_n, z, guided, w, S, eps, x_out, ws=None, hist=None, known=None, mask=None, rng=None):
+    def _p_sample_raw(self, x, ctx, t_n, z, guided, w, S, eps, x_out, ws=None, hist=None, known=None, mask=None, rng=None,
+                      seeds=None, w_dev=None, advance=None):
         """One step: ``hist`` the multistep update, ``known`` / ``mask`` known frames, ``rng`` the noise drawn in the update
-        kernel (which then also does the "t -= 1" bookkeeping) instead of ``z``."""
+        kernel (which then also does the "t -= 1" bookkeeping unless ``advance`` is False) instead of ``z``; ``seeds`` [B]
+        keys utterance b's noise (with rng), ``w_dev`` [B] its guidance scale (instead of ``w``)."""
+        if advance is None:
+            advance = rng is not None
         m = self.model
         B, T, H = x.shape
         n = 2 * B if guided else B
         with torch.cuda.device(x.device):
             if ws is None:
                 ws = m.workspace(n, T, S)
-            _lib.check(_lib.load().ditto_p_sample_known(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), _ptr(rng), 1 if guided else 0,
-                                                        float(w), B, T, S, _ptr(eps), _ptr(x_out), _ptr(hist), _ptr(known), _ptr(mask),
-                                                        _ptr(ws), ws.numel(), 0 if rng is None else 1, _stream()), "ditto_p_sample_known")
+            _lib.check(_lib.load().ditto_p_sample_per_utt(m.engine(), _ptr(x), _ptr(ctx), _ptr(t_n), _ptr(z), _ptr(rng), _ptr(seeds),
+                                                          1 if guided else 0, float(w), _ptr(w_dev), B, T, S, _ptr(eps), _ptr(x_out),
+                                                          _ptr(hist), _ptr(known), _ptr(mask), _ptr(ws), ws.numel(), 1 if advance else 0,
+                                                          _stream()), "ditto_p_sample_per_utt")
 
     # ------------------------------------------------------------------------------------------
     @torch.no_grad()
@@ -259,27 +356,30 @@ class DiTTOSampler:
         self._p_sample_raw(x, ctx, t_n, z, guided, w if guided else 0.0, text_emb.shape[1], eps, out)
         return out
 
-    def step_graph(self, B: int, T: int, S: int, guided: bool, w: float, ctx: torch.Tensor, draw_noise: bool, device,
-                   known: bool = False):
-        """Cached CUDA graph of one sampler iteration for this shape (re-captured if the buffers moved)."""
-        key = (B, T, S, guided, float(w), draw_noise, str(device), bool(known))
+    def step_graph(self, B: int, T: int, S: int, guided: bool, w, ctx: torch.Tensor, draw_noise: bool, device,
+                   known: bool = False, seeded: bool = False):
+        """Cached CUDA graph of one sampler iteration for this shape (re-captured if the buffers moved), set to the guidance
+        scale ``w`` (a scalar, or a [B] tensor of per-utterance scales).  The scale is not part of the key: the graph reads
+        it from its own buffer."""
+        key = (B, T, S, guided, draw_noise, str(device), bool(known), bool(seeded))
         g = self._graphs.get(key)
         n = 2 * B if guided else B
         if g is None or not g.valid_for(ctx, self.model.workspace(n, T, S)):
             self._graphs.pop(key, None)
             while len(self._graphs) >= self.max_cached_graphs:
                 self._graphs.popitem(last=False)          # least recently used; its buffers and graph pool are released
-            g = StepGraph(self, B, T, S, guided, float(w), ctx, draw_noise, device, known=known)
+            g = StepGraph(self, B, T, S, guided, w, ctx, draw_noise, device, known=known, seeded=seeded)
             self._graphs[key] = g
         else:
             self._graphs.move_to_end(key)
+            g.set_scale(w)
         return g
 
     @torch.no_grad()
     def sample_latents(self, text_emb, audio_emb=None, *, x_init=None, noise=None, guidance_scale=None,
                        null_text_emb=None, cond_by_audio=False, record: Optional[List[torch.Tensor]] = None,
                        generator: Optional[torch.Generator] = None, use_graph: bool = True,
-                       known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None):
+                       known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None, seeds=None):
         """All reverse steps (reference: __sample_latents, SpeechGenerator.py:150-164).
 
         text_emb [B,S,text_dim]; ``audio_emb`` [B,T,H] gives the latent shape (and the start point when
@@ -291,20 +391,36 @@ class DiTTOSampler:
         (``known_mask[:, :P] = True``, ``known[:, :P]`` = the prompt's codec latents) to continue, or the context of a span
         to fill.  Replacement conditioning (Song et al. 2021, score SDE): each step writes the known frames as p re-noised
         to the level of its output, with the noise the step draws, so the result holds them exactly.  Both CFG branches see
-        them."""
+        them.
+
+        ``seeds`` (B integers in [0, 2^64)) gives utterance b a noise stream of its own: x_T (unless ``x_init`` /
+        ``cond_by_audio`` supplies it) and every step's noise are functions of seeds[b] alone (include/ditto_b200.h), so an
+        utterance samples the same whatever else is in the batch.  Not together with ``noise`` or ``generator``.
+        ``guidance_scale`` may hold one scale per utterance."""
         m = self.model
         w = self.guidance_scale if guidance_scale is None else guidance_scale
         guided = w is not None
         text_emb = _need_cuda_f32("text_emb", text_emb)
         dev = text_emb.device
+        x = None
         if x_init is not None:
             x = _need_cuda_f32("x_init", x_init).clone()
         elif audio_emb is not None:
             audio_emb = _need_cuda_f32("audio_emb", audio_emb)
-            x = audio_emb.clone() if cond_by_audio else torch.randn(audio_emb.shape, device=dev, generator=generator)
+            if cond_by_audio:
+                x = audio_emb.clone()
+            elif seeds is None:
+                x = torch.randn(audio_emb.shape, device=dev, generator=generator)
         else:
             raise DittoError("sample_latents needs audio_emb (shape donor) or x_init")
-        B, T, H = x.shape
+        B, T, H = x.shape if x is not None else audio_emb.shape
+        seeds = _check_seeds(seeds, B, noise, generator)
+        w = _check_scale(w, B)
+        seeds_dev = None if seeds is None else _seed_tensor(seeds, dev)
+        if x is None:   # x_T from the seeds
+            x = randn_latents(seeds_dev, torch.arange(0, (B + 1) * T, T, dtype=torch.int64, device=dev), B * T, H).view(B, T, H)
+        # per-utterance scales on the device; a scalar stays a kernel argument outside the graphs
+        w_dev = torch.tensor(w, dtype=torch.float32, device=dev) if isinstance(w, list) else None
         S = text_emb.shape[1]
         has_known = known is not None or known_mask is not None
         if has_known:
@@ -318,27 +434,35 @@ class DiTTOSampler:
             x = self._known_start(x, known, known_mask)
         if use_graph and record is None and generator is None:
             # one CUDA-graph replay per denoising step (noise drawn inside the graph unless supplied)
-            g = self.step_graph(B, T, S, guided, w if guided else 0.0, ctx, noise is None, dev, known=has_known)
-            g.run(x, taus, consecutive, noise=noise, known=known, known_mask=known_mask)
+            g = self.step_graph(B, T, S, guided, (w if w_dev is None else w_dev) if guided else 0.0, ctx, noise is None, dev,
+                                known=has_known, seeded=seeds is not None)
+            g.run(x, taus, consecutive, noise=noise, known=known, known_mask=known_mask, seeds=seeds_dev)
             return g.x.clone()
         # t for every step, all sequences share it (SpeechGenerator.py:162)
         t_all = self._taus(dev).unsqueeze(1).repeat(1, n).contiguous()
         eps = torch.empty((n, T, H), dtype=torch.float32, device=dev)
         x_next = torch.empty_like(x)
-        z_buf = None if noise is not None else torch.empty_like(x)
+        z_buf = None if noise is not None or seeds is not None else torch.empty_like(x)
+        # seeded: the update kernel draws step i's noise as draw i of every utterance's seed (rng[1] = i, no bookkeeping)
+        rng = torch.zeros((4,), dtype=torch.int64, device=dev) if seeds is not None else None
         hist = torch.empty_like(x) if self.multistep else None   # first step is first order: never read before written
+        w_rec = w_dev.view(B, 1, 1) if w_dev is not None else w
         for i, t_val in enumerate(taus):
+            z = None
             if noise is not None:
                 z = noise[t_val]
                 if not z.is_cuda:
                     raise DittoError("noise must live on the GPU")
                 z = z.contiguous()
+            elif rng is not None:
+                rng[1] = i
             else:
                 z = z_buf.normal_(generator=generator)  # drawn every step incl. t = 0, as the reference does
-            self._p_sample_raw(x, ctx, t_all[i], z, guided, w if guided else 0.0, S, eps, x_next, hist=hist, known=known,
-                               mask=known_mask)
+            self._p_sample_raw(x, ctx, t_all[i], z, guided, w if guided and w_dev is None else 0.0, S, eps, x_next, hist=hist,
+                               known=known, mask=known_mask, rng=rng, seeds=seeds_dev, w_dev=w_dev if guided else None,
+                               advance=False)
             if record is not None:
-                record.append((eps[B:] + w * (eps[:B] - eps[B:])).clone() if guided else eps.clone())
+                record.append((eps[B:] + w_rec * (eps[:B] - eps[B:])).clone() if guided else eps.clone())
             x, x_next = x_next, x
         return x
 
@@ -346,17 +470,20 @@ class DiTTOSampler:
     @torch.no_grad()
     def sample_latents_ragged(self, texts, lengths, *, x_init=None, noise=None, guidance_scale=None, null_texts=None,
                               record: Optional[List[List[torch.Tensor]]] = None, use_graph: bool = True,
-                              known=None, known_mask=None):
+                              known=None, known_mask=None, seeds=None):
         """``__sample_latents`` (SpeechGenerator.py:150-164) for a mixed-length batch: utterance i has ``lengths[i]`` latent
         frames (what the speech-length predictor returns x 75 fps, SpeechGenerator.py:157-158) and text ``texts[i]``
         [S_i, text_dim].  Every utterance is sampled at its own length, unpadded (see ragged.py).  ``x_init`` /
         ``noise`` are per-utterance lists ([T_i,H] / [steps,T_i,H]) for parity runs.  ``known`` / ``known_mask`` are
-        per-utterance lists ([T_i,H] fp32 / [T_i] bool) of frames to keep, as in ``sample_latents``.  Returns a list of
-        [T_i,H]."""
+        per-utterance lists ([T_i,H] fp32 / [T_i] bool) of frames to keep, as in ``sample_latents``.  ``seeds`` and a
+        per-utterance ``guidance_scale`` (utterance order) as in ``sample_latents``: an utterance's result does not depend on
+        which utterances share its batch, beyond the forward's batch-dependent rounding.  Returns a list of [T_i,H]."""
         from .ragged import RaggedBatch, RaggedStepGraph
         m = self.model
         w = self.guidance_scale if guidance_scale is None else guidance_scale
         guided = w is not None
+        seeds = _check_seeds(seeds, len(texts), noise)
+        w = _check_scale(w, len(texts))
         # graphs (and the text-context buffers their kernels read) are cached per batch signature: a new batch with the same
         # (frames, tokens, count) groups re-fills the cached context buffers instead of capturing again
         sig = RaggedBatch.signature(texts, lengths, guided)
@@ -364,6 +491,8 @@ class DiTTOSampler:
         rb = RaggedBatch(m, texts, lengths, guided=guided, null_texts=null_texts,
                          ctx_storage=cached[0] if cached is not None else None)
         dev, H, steps = rb.device, m.hidden_dim, m.diffusion_steps
+        seeds_dev = None if seeds is None else rb.pack_seeds(seeds)
+        w_dev = rb.pack_w(w) if isinstance(w, list) else None
         has_known = known is not None or known_mask is not None
         kp = km = None
         if has_known:
@@ -376,6 +505,8 @@ class DiTTOSampler:
         consecutive = self.num_steps == steps
         if x_init is not None:
             x = rb.pack(x_init)
+        elif seeds_dev is not None:
+            x = randn_latents(seeds_dev, rb.row0(), rb.x_rows, H)
         else:
             x = torch.randn((rb.x_rows, H), dtype=torch.float32, device=dev)
         if has_known:
@@ -387,29 +518,37 @@ class DiTTOSampler:
                 z = _need_cuda_f32(f"noise[{i}]", z)
                 zs[:, rb.x_offset[i]:rb.x_offset[i] + rb.lengths[i]] = z
         if use_graph and record is None:
-            wv, draw = (w if guided else 0.0), zs is None
-            g = cached[1].get((float(wv), draw, has_known)) if cached is not None else None
+            # the scale is not part of the key: the graph reads it from its own buffer
+            wv, draw, key = ((w if w_dev is None else w_dev) if guided else 0.0), zs is None, (zs is None, has_known, seeds is not None)
+            g = cached[1].get(key) if cached is not None else None
             if g is None or not g.valid_for(rb):
-                g = RaggedStepGraph(rb, wv, draw, multistep=self.multistep, known=has_known)
+                g = RaggedStepGraph(rb, wv, draw, multistep=self.multistep, known=has_known, seeded=seeds is not None)
                 if cached is None:
                     while len(self._ragged_graphs) >= self.max_cached_graphs:
                         self._ragged_graphs.popitem(last=False)
                     cached = (rb._ctx, {})
                     self._ragged_graphs[sig] = cached
-                cached[1][(float(wv), draw, has_known)] = g
+                cached[1][key] = g
             else:
                 g.rebind(rb)
+                g.set_scale(wv)
             self._ragged_graphs.move_to_end(sig)
-            g.run(x, taus, consecutive, noise=zs, known=kp, known_mask=km)
+            g.run(x, taus, consecutive, noise=zs, known=kp, known_mask=km, seeds=seeds_dev)
             return rb.unpack(g.x)
         eps = torch.empty((rb.seq_rows, H), dtype=torch.float32, device=dev)
         x_next = torch.empty_like(x)
-        z_buf = torch.empty_like(x)
+        z_buf = torch.empty_like(x) if zs is None and seeds is None else None
+        rng = torch.zeros((4,), dtype=torch.int64, device=dev) if seeds is not None else None   # as in sample_latents
         hist = torch.empty_like(x) if self.multistep else None
-        for t_val in taus:
+        for i, t_val in enumerate(taus):
             t_seq = torch.full((rb.n_seq,), t_val, dtype=torch.int64, device=dev)
-            z = zs[t_val] if zs is not None else z_buf.normal_()
-            rb.p_sample(x, t_seq, z, w if guided else 0.0, eps, x_next, hist=hist, known=kp, mask=km)
+            z = None
+            if rng is not None:
+                rng[1] = i
+            else:
+                z = zs[t_val] if zs is not None else z_buf.normal_()
+            rb.p_sample(x, t_seq, z, w if guided and w_dev is None else 0.0, eps, x_next, hist=hist, known=kp, mask=km, rng=rng,
+                        seeds=seeds_dev, w_dev=w_dev if guided else None, advance=False)
             if record is not None:
                 record.append(rb.unpack_eps(eps, w))
             x, x_next = x_next, x

@@ -222,6 +222,38 @@ int32_t ditto_p_sample_known(ditto_engine_t* e, const float* x, const void* ctx,
                              float* x_out, float* hist, const float* known, const uint8_t* known_mask, void* workspace,
                              int64_t workspace_bytes, int32_t advance, void* stream);
 
+/* ---- per-utterance seeds and guidance scales -----------------------------------------------------------------------------
+ * Noise stream of an utterance with seed s (any uint64), T frames, hidden size H -- nothing else enters it (not its position in
+ * the batch, the batch size, the uniform or ragged layout, nor the rank that runs it):
+ *   step draw k (k = 0, 1, ... in the order the steps run; the draw counter rng[1]): element j = f H + c (frame f, channel c)
+ *     is component j % 4 of philox_normal4(key = s, counter = (j / 4, k)), where
+ *       philox_normal4: r = Philox4x32-10(counter words {lo32(j/4), hi32(j/4), lo32(k), hi32(k)}, key words {lo32(s), hi32(s)});
+ *       u_i = (r_i >> 8) 2^-24 + 2^-25 for i = x, z; a_i = (r_i >> 8) 2^-24 2 pi for i = y, w;
+ *       normals {m0 cos a_y, m0 sin a_y, m1 cos a_w, m1 sin a_w} with m0 = sqrt(-2 ln u_x), m1 = sqrt(-2 ln u_z), evaluated
+ *       with the fast __log2f / __sincosf (oracle/ditto_oracle.py: philox_normal restates it in numpy to 2e-5)
+ *     (the normals ditto_randn gives: draw k of utterance b == ditto_randn(rng = {s_b, k}, elem_offset = 0, n = T H));
+ *   x_T: the same with the reserved draw index k = 2^64 - 1, which the step counter never reaches.
+ * Per-utterance scales: eps = eps_u + w[b] (eps_c - eps_u) for every element of utterance b.
+ *
+ * ditto_p_sample_known with two more arguments:
+ *   seeds  uint64 [B] (device): key of utterance b (ragged: packed-group order, the order of the groups' latents); needs rng, whose
+ *          draw counter and ticket are used and whose rng[0] is ignored; excludes z.  NULL: the noise of ditto_p_sample_known.
+ *   w      fp32 [B] (device), same order: utterance b's guidance scale (guided calls); NULL: guidance_scale for every utterance.
+ * With seeds == w == NULL the call IS ditto_p_sample_known (which forwards to it).  Seeds without rng, seeds with z: DITTO_E_BADARG. */
+int32_t ditto_p_sample_per_utt(ditto_engine_t* e, const float* x, const void* ctx, int64_t* t, const float* z, uint64_t* rng,
+                               const uint64_t* seeds, int32_t guided, float guidance_scale, const float* w, int64_t B, int64_t T,
+                               int64_t S, float* eps_scratch, float* x_out, float* hist, const float* known,
+                               const uint8_t* known_mask, void* workspace, int64_t workspace_bytes, int32_t advance, void* stream);
+/* ditto_cfg_update_known with seeds / w as above (the update on its own; ditto_cfg_update_known forwards to it). */
+int32_t ditto_cfg_update_per_utt(ditto_engine_t* e, const float* eps_c, const float* eps_u, const float* x, const float* z,
+                                 uint64_t* rng, const uint64_t* seeds, int64_t* t, int64_t n_t, float guidance_scale,
+                                 const float* w, float* x_out, float* hist, const float* known, const uint8_t* known_mask,
+                                 int64_t B, int64_t T, int32_t advance, void* stream);
+/* x_T of B utterances in one launch: utterance b owns rows row0[b] .. row0[b + 1] - 1 of out [rows, H] (row0 int64 [B + 1],
+ * device, nondecreasing; uniform [B, T, H]: row0[b] = b T) and gets the x_T normals of its seeds[b] (draw 2^64 - 1).  H % 4 == 0,
+ * out 16-B aligned, B <= 65535; a NULL seeds / row0 / out is DITTO_E_BADARG. */
+int32_t ditto_randn_latents(const uint64_t* seeds, const int64_t* row0, int64_t B, int64_t H, float* out, void* stream);
+
 /* DiTTO.q_sample (DiTTO.py:106-126) with the reference's betas-as-alphas_cumprod buffer. */
 int32_t ditto_q_sample(ditto_engine_t* e, const float* x_start, const float* noise, const int64_t* t,
                        float* out, int64_t B, int64_t elems_per_seq, void* stream);
@@ -271,6 +303,13 @@ int32_t ditto_p_sample_ragged_known(ditto_engine_t* e, const float* x, const dit
                                     float* eps_scratch, float* x_out, float* hist, const float* known,
                                     const uint8_t* known_mask, void* workspace, int64_t workspace_bytes, int32_t advance,
                                     void* stream);
+/* ditto_p_sample_ragged_known with per-utterance seeds / w (ditto_p_sample_per_utt), both [sum n_x] in packed-group order; each
+ * group's update reads them from its first utterance on.  ditto_p_sample_ragged_known forwards to it with both NULL. */
+int32_t ditto_p_sample_ragged_per_utt(ditto_engine_t* e, const float* x, const ditto_seq_group_t* groups, int64_t n_groups,
+                                      int64_t* t, const float* z, uint64_t* rng, const uint64_t* seeds, int32_t guided,
+                                      float guidance_scale, const float* w, float* eps_scratch, float* x_out, float* hist,
+                                      const float* known, const uint8_t* known_mask, void* workspace, int64_t workspace_bytes,
+                                      int32_t advance, void* stream);
 
 /* ---- block-level operators: the component signatures of src/components/DiT.py ------------------------------- */
 /* DiT.forward(x, text_emb, time_emb, rotary_pos) (DiT.py:100-157) for block `layer` of the engine: x [n_seq, T, H] -> out
