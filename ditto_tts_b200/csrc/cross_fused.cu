@@ -81,7 +81,6 @@ struct XfDev {
   int n_seq, T, S, H;
   int rt;                                     // rows per tile (<= 128, multiple of 8): the TMA boxes carry rt rows, the MMA computes 128
   int m_tiles, num_tiles, num_kb, num_ch, num_hc;
-  int pf_dist;                                // L2 prefetch distance of the residual stream, in pass-0 jobs (0: off)
   float alpha2;                               // alpha * log2(e)
   const float* sbias; long long sb_seq;       // [n_seq, sb_seq] additive score bias
   const float* out_bias;                      // [H]
@@ -114,12 +113,6 @@ __device__ __forceinline__ void tmem_ld_16x16(uint32_t taddr, uint32_t (&r)[8]) 
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, const void* smem, int c0, int c1, int c2, int c3) {
   asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(reinterpret_cast<uint64_t>(m)),
                "r"(smem_u32(smem)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
-// tile of a tensor map -> L2 only (no shared-memory destination, no completion to wait for)
-__device__ __forceinline__ void tma_prefetch_4d(const CUtensorMap* m, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];" ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0),
-               "r"(c1), "r"(c2), "r"(c3)
                : "memory");
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
@@ -322,7 +315,7 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
         for (; cur.ti < ti; ++cur.ti) cur.tile = xf_next_tile(p, cur.tile + step, step);
         return cur.tile;
       };
-      Cursor jc{0, tile0}, pc{0, tile0};
+      Cursor jc{0, tile0};
       auto job_coords = [&](int j, int& seq, int& row, int& pass, int& hc) {
         const int ti = j / jobs_per_tile, r = j - ti * jobs_per_tile;
         const int tile = tile_at(jc, ti);
@@ -332,29 +325,10 @@ __global__ void __launch_bounds__(XF_THREADS, 1)
         hc = r - pass * p.num_hc;
       };
       if (warp == 2) {
-        // Experiment (xf_prefetch = n, off by default): every pass-0 half-chunk requested into L2 n pass-0 jobs ahead, so
-        // that the staging load sees the L2 latency instead of HBM's.  No shared memory, nothing to wait for.
-        const int P0 = my_tiles * p.num_hc;   // pass-0 jobs of this CTA
-        int pf_next = 0;                      // first pass-0 job not requested yet
-        auto prefetch_upto = [&](int limit) {
-          if (p.pf_dist <= 0) return;
-          limit = limit < P0 ? limit : P0;
-          for (; pf_next < limit; ++pf_next) {
-            const int ti = pf_next / p.num_hc, hc = pf_next - ti * p.num_hc;
-            const int tile = tile_at(pc, ti), seq = tile / p.m_tiles, row = (tile - seq * p.m_tiles) * p.rt;
-            if (leader && pf_next >= XF_NB) {   // the first XF_NB loads are issued at once anyway
-              tma_prefetch_4d(&tmap_h, hc * XF_HC, row, 0, seq);
-              tma_prefetch_4d(&tmap_h, hc * XF_HC + 32, row, 0, seq);
-            }
-          }
-        };
         for (int j = 0; j < J; ++j) {
           int seq, row, pass, hc;
           job_coords(j, seq, row, pass, hc);
           const int b = j % XF_NB;
-          // pass-0 index this job corresponds to: own index in pass 0; during pass 1 the next tile's first half + hc / 2
-          const int ti = j / jobs_per_tile;
-          prefetch_upto(pass == 0 ? ti * p.num_hc + hc + p.pf_dist + 1 : (ti + 1) * p.num_hc + p.pf_dist + (hc + 1) / 2 + 1);
           mbar_wait(&hfree[b], ((j / XF_NB) & 1u) ^ 1u);   // the store that last used this buffer has read it
           if (leader) {
             uint8_t* buf = hbuf + b * XF_HBUF_BYTES;
@@ -745,9 +719,6 @@ int launch_cross_fused(const CrossFusedParams& q, cudaStream_t st) {
   p.out_bias = q.out_bias;
   p.gamma = q.gamma; p.beta = q.beta;
   p.inv_h = 1.0f / static_cast<float>(q.H);
-  // off by default: measured 77 -> 73 us at C2 but 433 -> 472 us at 128 utterances (profiles/README.md) -- at the sizes that matter the
-  // kernel is short of HBM / L2 throughput, not of requests in flight, and the early requests only displace lines that are still needed
-  p.pf_dist = g_opt.xf_prefetch > 0 ? std::min(g_opt.xf_prefetch, 2 * p.num_hc) : 0;
   p.ln_stat = q.ln_stat; p.ln_parts = q.ln_parts; p.ln_c = q.ln_c;
   p.skip_seq = q.skip_seq;
   if (q.ln_stat != nullptr) DITTO_REQUIRE(q.ln_parts > 0 && q.ln_c != nullptr, DITTO_E_BADARG, "cross_fused: deferred LayerNorm arguments");

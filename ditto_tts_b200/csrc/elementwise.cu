@@ -608,32 +608,6 @@ int launch_const_text(const float* text, int64_t n, int S, int D, const bf16* vf
   return 0;
 }
 
-// V [T, d] slices of qkv (ld) -> Vt [n*heads, d, Tp] (keys contiguous): fallback operand layout for P@V
-__global__ void transpose_v_kernel(const bf16* __restrict__ v, int64_t ld, bf16* __restrict__ vt, int T, int Tp, int heads,
-                                   int d) {
-  __shared__ bf16 tile[32][33];
-  const int b = blockIdx.z;  // seq * heads + head
-  const int seq = b / heads, head = b % heads;
-  const bf16* src = v + (static_cast<int64_t>(seq) * T) * ld + head * d;
-  bf16* dst = vt + static_cast<int64_t>(b) * d * Tp;
-  const int t0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int tt = t0 + i, c = c0 + threadIdx.x;
-    tile[i][threadIdx.x] = (tt < T && c < d) ? src[static_cast<int64_t>(tt) * ld + c] : __float2bfloat16(0.f);
-  }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int c = c0 + i, tt = t0 + threadIdx.x;
-    if (c < d && tt < Tp) dst[static_cast<int64_t>(c) * Tp + tt] = tile[threadIdx.x][i];
-  }
-}
-int launch_transpose_v(const bf16* v, int64_t ld, bf16* vt, int64_t n_seq, int T, int Tp, int heads, int d, cudaStream_t st) {
-  dim3 grid(static_cast<unsigned>(ceil_div(Tp, 32)), static_cast<unsigned>(ceil_div(d, 32)), static_cast<unsigned>(n_seq * heads));
-  transpose_v_kernel<<<grid, dim3(32, 8), 0, st>>>(v, ld, vt, T, Tp, heads, d);
-  DITTO_LAUNCH_CHECK();
-  return 0;
-}
-
 // =====================================================================================================
 // The sampler update, one pass: CFG combine + DDPM-form or multistep update, optionally with the noise drawn in the kernel and
 // with known frames (launch_cfg_update, kernels.cuh).

@@ -95,15 +95,13 @@ struct ditto_engine {
   bool cross_flash = false; // folded cross-attention with 64 < S <= 256 text tokens through flash_attn768q<CROSS> (+ residual + norm3)
   bool fc2_ln = false;      // fc2 + residual + the next block's norm1 in one cluster kernel (gemm_resid_ln.cu); w_fc2 rows in perm4 order
   bool flash768 = false;    // one head of 768 (repo default): self-attention + residual + norm2 in one cluster kernel (flash_attn768.cu)
-  bool flash_attn = true;   // head_dim 64: self-attention without materialised scores (flash_attn.cu); DITTO_NO_FLASH=1 disables
+  bool flash_attn = true;   // head_dim 64: self-attention without materialised scores (flash_attn.cu)
   bool defer_ln2 = false;   // norm2 only: row statistics from the self-attention P.V epilogue, LayerNorm folded into cross_fused's scores
-  bool fused_cross = true;  // folded cross-attention + residual + norm3 in one kernel (cross_fused.cu); DITTO_NO_FUSED_CROSS=1 disables
+  bool fused_cross = true;  // folded cross-attention + residual + norm3 in one kernel (cross_fused.cu)
   bool fused_attn = false;  // scores + softmax fused (cluster kernel); falls back per call when a row needs > 16 tiles
   bool fold_cross = false;  // cross-attn q/out projections folded into the per-utterance text K/V (heads == 1 only)
   bool defer_ln = false;    // block LayerNorms folded into the neighbouring GEMM epilogues (no LayerNorm launches)
   bool const_text = true;   // sequences with constant text rows: constant cross-attention output added by the self-attention kernel
-  int pv_transpose = 0;  // debug: use the transposed-V operand instead of the MN-major descriptor
-  bool rope_table_in_epilogue = false;  // debug (DITTO_ROPE_TABLE=1): fused RoPE reads the cos/sin tables instead of computing them
   std::map<std::string, int64_t> expected;  // key -> numel
   std::map<std::string, float*> w;          // device fp32 copies (owned)
   std::vector<void*> owned;                 // everything else cudaMalloc'ed by the engine
@@ -263,14 +261,12 @@ struct SeqGroup {
   int64_t seq0 = 0;    // index of the group's first sequence (t, per-sequence tables)
   int64_t p_off = 0;   // element offset of the group's score / P scratch
   int64_t l_off = 0;   // element offset of the group's partial-denominator scratch
-  int64_t vt_off = 0;  // element offset of the transposed-V scratch (debug fallback)
 };
 
 struct Workspace {
   float *h = nullptr, *xskip = nullptr, *scores = nullptr;
   void *u = nullptr, *qkv = nullptr, *P = nullptr, *qc = nullptr, *oc = nullptr, *hid = nullptr, *xb16 = nullptr;
   float *fc1 = nullptr, *gate = nullptr;  // fp32 path only
-  bf16* vt = nullptr;                     // transposed-V fallback
   float* lpart = nullptr;                 // [n*heads, T, ceil(Tp/256)] partial softmax denominators (fused attention)
   float2* lnstat = nullptr;               // [M, ln_parts] per-row partial (sum, sum of squares) of h (deferred LayerNorm)
   int ln_parts_h = 0, ln_parts_attn = 0;  // parts written by an N = H producer / by the per-head P.V producer
@@ -287,15 +283,14 @@ static Workspace ws_layout(const ditto_engine* e, void* base, SeqGroup* gs, int 
   Workspace w;
   const int64_t H = e->H;
   const int es = e->bf16_mode ? 2 : 4;
-  int64_t M = 0, Mx = 0, seqs = 0, p_el = 0, l_el = 0, vt_el = 0, n_tot = 0, text_el = 0;
+  int64_t M = 0, Mx = 0, seqs = 0, p_el = 0, l_el = 0, n_tot = 0, text_el = 0;
   for (int i = 0; i < ng; ++i) {
     SeqGroup& g = gs[i];
     const int64_t ldp = std::max(round_up(g.T, 8), round_up(g.S, 8));
-    g.row0 = M; g.xrow0 = Mx; g.seq0 = seqs; g.p_off = p_el; g.l_off = l_el; g.vt_off = vt_el;
+    g.row0 = M; g.xrow0 = Mx; g.seq0 = seqs; g.p_off = p_el; g.l_off = l_el;
     M += g.n * g.T; Mx += g.n_x * g.T; seqs += g.n;
     p_el += round_up(g.n * e->heads * g.T * ldp, 128);
     l_el += round_up(g.n * e->heads * g.T * ceil_div(ldp, 256), 64);
-    vt_el += round_up(g.n * e->heads * e->d * ldp, 128);
     n_tot = std::max(n_tot, g.n);
     text_el = std::max(text_el, g.n * g.S);
   }
@@ -313,8 +308,6 @@ static Workspace ws_layout(const ditto_engine* e, void* base, SeqGroup* gs, int 
   if (!e->bf16_mode) {
     w.fc1 = a.take<float>(M * 4 * H);
     w.gate = a.take<float>(M * 4 * H);
-  } else if (e->pv_transpose) {
-    w.vt = a.take<bf16>(vt_el);
   }
   if (e->bf16_mode) w.lpart = a.take<float>(l_el);
   w.ln_parts_h = static_cast<int>(ceil_div(H, 128));
@@ -383,15 +376,8 @@ static int attention_bf16(ditto_engine* e, const Workspace& w, const bf16* q, in
   TcGemmParams o;
   o.A.ptr = static_cast<const bf16*>(w.P); o.A.rows = Tq; o.A.cols = Tk; o.A.ld = ldp; o.A.s_inner = static_cast<int64_t>(Tq) * ldp;
   o.A.s_outer = static_cast<int64_t>(heads) * Tq * ldp;
-  if (e->pv_transpose && w.vt) {  // fallback operand: V^T [d, Tp] per (seq, head), keys contiguous
-    DITTO_TRY(launch_transpose_v(v, ldv, w.vt, n, Tk, static_cast<int>(ldp), heads, d, st));
-    o.B.ptr = w.vt; o.B.rows = d; o.B.cols = Tk; o.B.ld = ldp; o.B.s_inner = static_cast<int64_t>(d) * ldp;
-    o.B.s_outer = static_cast<int64_t>(heads) * d * ldp;
-    o.b_kn = false;
-  } else {
-    o.B.ptr = v; o.B.rows = Tk; o.B.cols = d; o.B.ld = ldv; o.B.s_inner = d; o.B.s_outer = v_seq_stride;
-    o.b_kn = true;
-  }
+  o.B.ptr = v; o.B.rows = Tk; o.B.cols = d; o.B.ld = ldv; o.B.s_inner = d; o.B.s_outer = v_seq_stride;
+  o.b_kn = true;
   o.M = Tq; o.N = d; o.K = Tk; o.batch_inner = heads; o.batch_outer = static_cast<int>(n);
   o.out = out; o.out_bf16 = out_bf16; o.ldo = ldo; o.so_inner = d; o.so_outer = o_seq_stride;
   o.resid = resid; o.ldr = ldo; o.sr_inner = d; o.sr_outer = o_seq_stride;
@@ -435,7 +421,6 @@ static Workspace group_view(const ditto_engine* e, const Workspace& w, const Seq
   v.scores = w.scores ? w.scores + g.p_off : nullptr;
   v.P = e->bf16_mode ? static_cast<void*>(static_cast<bf16*>(w.P) + g.p_off) : static_cast<void*>(v.scores);
   v.lpart = w.lpart ? w.lpart + g.l_off : nullptr;
-  v.vt = w.vt ? w.vt + g.vt_off : nullptr;
   return v;
 }
 
@@ -551,8 +536,7 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
         g.M = static_cast<int>(M); g.N = 3 * H; g.K = H; g.bias = lp.b_qkv; g.out = qkv; g.out_bf16 = true; g.ldo = 3 * H;
         g.tag = PC_TC_QKV;
         if (e->fused_rope) {
-          g.epilogue = TC_EPI_QKV_ROPE; g.rope_cos = e->rope_cos; g.rope_sin = e->rope_sin; g.rope_half = e->half;
-          g.rope_freq = e->rope_table_in_epilogue ? nullptr : e->rope_freq;
+          g.epilogue = TC_EPI_QKV_ROPE; g.rope_half = e->half; g.rope_freq = e->rope_freq;
           g.rope_pd = e->rope_pd; g.seq_T = static_cast<int>(g0.T); g.hidden = H;
           g.rope_pos = ragged ? w.row_pos : nullptr;
           g.rope_perm16 = e->qkv_perm16;
@@ -890,20 +874,16 @@ int32_t ditto_engine_create(const ditto_config_t* cfg, ditto_engine_t** out) {
     e->fused_attn = (cfg->flags & DITTO_F_FUSED_ATTN) != 0;
     e->defer_ln = (cfg->flags & DITTO_F_DEFER_LN) != 0 && e->fused_rope && e->fused_attn;
     if (g_opt.no_defer_ln) e->defer_ln = false;
-    if (g_opt.no_fused_attn) e->fused_attn = false;
     e->fused_cross = e->fused_attn;
     e->flash_attn = e->fused_attn;
     if (g_opt.no_flash) e->flash_attn = false;
     if (g_opt.no_fused_cross) e->fused_cross = false;
     e->const_text = !g_opt.no_const_text;
     e->defer_ln2 = !e->defer_ln && e->fused_cross && e->bf16_mode && e->heads == 1 && g_opt.defer_ln2 != 0;
-    e->pv_transpose = g_opt.pv_transpose != 0;
-    e->rope_table_in_epilogue = g_opt.rope_table != 0;
     e->glu_perm16 = !e->defer_ln && e->H % 32 == 0 && !g_opt.glu_generic;
-    // no_rope_fast32: pair distance 32 (head_dim 64) through the generic epilogue
-    const bool pd_ok = e->rope_pd == 128 || (e->rope_pd == 32 && !g_opt.no_rope_fast32);
-    e->qkv_perm16 = e->fused_rope && pd_ok && !e->defer_ln && !e->rope_table_in_epilogue && e->H % 256 == 0 && !g_opt.rope_generic;
-    e->pv_perm4 = e->qkv_perm16 && !e->pv_transpose && !e->defer_ln2 && e->d % 128 == 0 && !g_opt.no_pv_perm4;
+    const bool pd_ok = e->rope_pd == 128 || e->rope_pd == 32;
+    e->qkv_perm16 = e->fused_rope && pd_ok && !e->defer_ln && e->H % 256 == 0 && !g_opt.rope_generic;
+    e->pv_perm4 = e->qkv_perm16 && !e->defer_ln2 && e->d % 128 == 0 && !g_opt.no_pv_perm4;
     // needs the v columns in the 16-byte store order (pv_perm4) and the fused softmax machinery
     e->flash768 = e->fused_attn && e->pv_perm4 && !e->defer_ln && flash768_supported(e->H, e->heads, 1) && !g_opt.no_flash768;
     e->fc2_ln = !e->defer_ln && gemm_resid_ln_supported(e->H, 4 * e->H) && !g_opt.no_fc2_ln && gemm_resid_ln_schedulable(e->H);
@@ -1653,9 +1633,10 @@ int32_t ditto_rope(const float* t, const float* pos, float* out, int64_t batch, 
 int32_t ditto_attn_self768(const void* qkv, int64_t ld, int64_t n_seq, int64_t T, float alpha, float* h, const float* gamma,
                            const float* beta, void* u_out, int32_t flags, void* stream) {
   DITTO_REQUIRE(qkv && h && n_seq > 0 && T > 0 && T < (1ll << 30), DITTO_E_BADARG, "attn_self768: bad argument");
+  DITTO_REQUIRE((flags & ~1) == 0, DITTO_E_BADARG, "attn_self768: unknown flag bits (only bit 0 is defined)");
   Flash768Params f;
   f.qkv = static_cast<const bf16*>(qkv); f.ld = ld; f.n_seq = n_seq; f.T = static_cast<int>(T); f.H = 768; f.alpha = alpha; f.h = h;
-  f.gamma = gamma; f.beta = beta; f.u_out = static_cast<bf16*>(u_out); f.force_rescale = (flags & 1) != 0; f.dbg = flags >> 8; f.tag = PC_FLASH768;
+  f.gamma = gamma; f.beta = beta; f.u_out = static_cast<bf16*>(u_out); f.force_rescale = (flags & 1) != 0; f.tag = PC_FLASH768;
   return launch_flash768(f, static_cast<cudaStream_t>(stream));
 }
 
@@ -1664,14 +1645,11 @@ int32_t ditto_debug_option(const char* name, int32_t value) {
   DITTO_REQUIRE(name != nullptr, DITTO_E_BADARG, "debug_option: null name");
   struct Opt { const char* n; int* p; };
   const Opt opts[] = {
-      {"no_pair", &g_opt.no_pair}, {"cluster_m", &g_opt.cluster_m}, {"cluster_n", &g_opt.cluster_n}, {"generic_epi", &g_opt.generic_epi},
-      {"stages_1cta", &g_opt.stages_1cta}, {"stages_pair", &g_opt.stages_pair}, {"no_mcast", &g_opt.no_mcast}, {"xf_rows", &g_opt.xf_rows}, {"xf_prefetch", &g_opt.xf_prefetch},
-      {"no_defer_ln", &g_opt.no_defer_ln}, {"no_fused_attn", &g_opt.no_fused_attn}, {"no_flash", &g_opt.no_flash},
+      {"xf_rows", &g_opt.xf_rows}, {"no_defer_ln", &g_opt.no_defer_ln}, {"no_flash", &g_opt.no_flash},
       {"no_flash768", &g_opt.no_flash768}, {"no_fused_cross", &g_opt.no_fused_cross}, {"defer_ln2", &g_opt.defer_ln2},
-      {"pv_transpose", &g_opt.pv_transpose}, {"rope_table", &g_opt.rope_table}, {"rope_generic", &g_opt.rope_generic},
-      {"glu_generic", &g_opt.glu_generic}, {"no_rope_fast32", &g_opt.no_rope_fast32}, {"no_pv_perm4", &g_opt.no_pv_perm4},
-      {"side_streams", &g_opt.side_streams}, {"no_fused_ln", &g_opt.no_fused_ln}, {"flash768_quad", &g_opt.flash768_quad},
-      {"no_fc2_ln", &g_opt.no_fc2_ln}, {"no_cross_flash", &g_opt.no_cross_flash}, {"no_const_text", &g_opt.no_const_text}, {"dbg_nostore", &g_opt.dbg_nostore}};
+      {"rope_generic", &g_opt.rope_generic}, {"glu_generic", &g_opt.glu_generic}, {"no_pv_perm4", &g_opt.no_pv_perm4},
+      {"side_streams", &g_opt.side_streams}, {"flash768_quad", &g_opt.flash768_quad}, {"no_fc2_ln", &g_opt.no_fc2_ln},
+      {"no_cross_flash", &g_opt.no_cross_flash}, {"no_const_text", &g_opt.no_const_text}};
   if (strcmp(name, "reset") == 0) { g_opt = DebugOptions(); return 0; }
   for (const Opt& o : opts)
     if (strcmp(name, o.n) == 0) { *o.p = value; return 0; }

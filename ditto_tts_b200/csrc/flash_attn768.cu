@@ -107,7 +107,6 @@ struct F7Dev {
   const float* gamma; const float* beta;
   bf16* u_out;                        // [n_seq * T, 768] LayerNorm(h) (nullptr: no LayerNorm stage)
   int force_rescale;                  // tests: move the reference whenever a tile raises a row maximum
-  int dbg;                            // timing experiments only (WRONG results): bit 0 no reference chain, bit 1 no residual loads, bit 2 no residual stores, bit 3 no LayerNorm-output stores
 };
 
 __device__ __forceinline__ void tmem_st_16x64(uint32_t taddr, const uint32_t (&r)[32]) {  // inverse of tmem_ld_16x64
@@ -217,10 +216,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
   f7_cluster_sync();   // the peer's barriers exist before the first st.async / bulk copy / commit reaches them
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
-  if ((p.dbg >> 8) != 0 && (first & 1)) {   // timing experiment: odd clusters start late (units of 2048 clocks)
-    const long long t_go = clock64() + (static_cast<long long>(p.dbg >> 8) << 11);
-    while (clock64() < t_go) {}
-  }
   const long long t_sync = DITTO_F7_TRACE ? clock64() : 0;   // the cluster barrier released both CTAs at (about) the same moment
 
   if (warp == 0) {
@@ -433,7 +428,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
       float* hA = p.h + growA * F7_D + col_half + q * 4;         // this thread's first output column of a 64-column chunk
       float* hB = hA + 8 * F7_D;
       // residual rows of this warp -> L2 while the tile computes (16 rows x 384 columns = 192 lines of 128 B)
-      if (!(p.dbg & 16))
       for (int i = lane; i < 16 * (F7_DH * 4 / 128); i += 32) {
         const int r = i / (F7_DH * 4 / 128), l = i - r * (F7_DH * 4 / 128);
         if (qt * F7_BM + trow + r < p.T)
@@ -467,7 +461,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
           if (j + 1 < KT && !have_s) load_scores();
           const uint32_t slot = rc & 1u;
           if (ew == 0 && lane == 0) mbar_expect_tx(&hdr_bar[slot], F7_BM * 4);
-          if (!(p.dbg & 1)) mbar_wait(&hdr_bar[slot], (rc >> 1) & 1u);
+          mbar_wait(&hdr_bar[slot], (rc >> 1) & 1u);
           tr.ev(11, j);
           const float nA = hdr_x[slot * F7_BM + rA], nB = hdr_x[slot * F7_BM + rB];
           if (j > 0) {
@@ -575,8 +569,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
       auto load_res = [&](int cb, float4(&f)[8]) {
 #pragma unroll
         for (int jj = 0; jj < 4; ++jj) {
-          f[jj] = (okA && !(p.dbg & 2)) ? *reinterpret_cast<const float4*>(hA + cb * 64 + jj * 16) : make_float4(0.f, 0.f, 0.f, 0.f);
-          f[4 + jj] = (okB && !(p.dbg & 2)) ? *reinterpret_cast<const float4*>(hB + cb * 64 + jj * 16) : make_float4(0.f, 0.f, 0.f, 0.f);
+          f[jj] = okA ? *reinterpret_cast<const float4*>(hA + cb * 64 + jj * 16) : make_float4(0.f, 0.f, 0.f, 0.f);
+          f[4 + jj] = okB ? *reinterpret_cast<const float4*>(hB + cb * 64 + jj * 16) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
       };
       load_res(0, f0);       // both requested before the waits below: their L2 latency hides behind the exchange / the last P.V
@@ -607,8 +601,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
           vB.y = fmaf(iB, __uint_as_float(o[4 * k0 + 3]), f[4 + jj].y);
           vB.z = fmaf(iB, __uint_as_float(o[4 * k1 + 2]), f[4 + jj].z);
           vB.w = fmaf(iB, __uint_as_float(o[4 * k1 + 3]), f[4 + jj].w);
-          if (okA && !(p.dbg & 4)) *reinterpret_cast<float4*>(hA + cb * 64 + jj * 16) = vA;
-          if (okB && !(p.dbg & 4)) *reinterpret_cast<float4*>(hB + cb * 64 + jj * 16) = vB;
+          if (okA) *reinterpret_cast<float4*>(hA + cb * 64 + jj * 16) = vA;
+          if (okB) *reinterpret_cast<float4*>(hB + cb * 64 + jj * 16) = vB;
           if (cb == 0 && jj == 0) { kA = vA.x; kB = vB.x; }
           const float4 dA = make_float4(vA.x - kA, vA.y - kA, vA.z - kA, vA.w - kA);
           const float4 dB = make_float4(vB.x - kB, vB.y - kB, vB.z - kB, vB.w - kB);
@@ -683,8 +677,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
                                fmaf((__uint_as_float(o[4 * k0 + 3]) - meanB) * rsB, gm[jj].y, bt[jj].y));
             wB.y = pack_bf16x2(fmaf((__uint_as_float(o[4 * k1 + 2]) - meanB) * rsB, gm[jj].z, bt[jj].z),
                                fmaf((__uint_as_float(o[4 * k1 + 3]) - meanB) * rsB, gm[jj].w, bt[jj].w));
-            if (okA && !(p.dbg & 8)) *reinterpret_cast<uint2*>(uA + cb * 64 + jj * 16) = wA;
-            if (okB && !(p.dbg & 8)) *reinterpret_cast<uint2*>(uB + cb * 64 + jj * 16) = wB;
+            if (okA) *reinterpret_cast<uint2*>(uA + cb * 64 + jj * 16) = wA;
+            if (okB) *reinterpret_cast<uint2*>(uB + cb * 64 + jj * 16) = wB;
           }
         }
       }
@@ -750,7 +744,6 @@ int launch_flash768(const Flash768Params& q, cudaStream_t st) {
   p.alpha2 = q.alpha * 1.4426950408889634f;
   p.h = q.h; p.gamma = q.gamma; p.beta = q.beta; p.u_out = q.u_out;
   p.force_rescale = q.force_rescale ? 1 : 0;
-  p.dbg = q.dbg;
   p.trace = DITTO_F7_TRACE ? tc_gemm_debug_counters() : nullptr;
   // algorithmic flops: 4 T^2 d per utterance (the second Q K^T of the cluster is not counted); bytes: q, k, v read once, h
   // read + written, u written

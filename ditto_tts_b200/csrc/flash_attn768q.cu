@@ -99,7 +99,7 @@ struct Q7Dev {
   const float* gamma; const float* beta;
   bf16* u_out;
   int force_rescale;
-  int dbg;
+  int dbg;   // always 0: kept only because removing its tests below makes ptxas spill more in the epilogue (slower)
   // constant-text sequences (Flash768Params::const_flag); self-attention: norm3, which replaces norm2 for them.  (Few new
   // fields, at the end: a larger parameter block costs the plain self-attention kernel spills.)
   const uint8_t* const_flag; const float* gamma_c; const float* beta_c;
@@ -880,7 +880,7 @@ int launch_flash768_quad(const Flash768Params& q, cudaStream_t st) {
   p.h = q.h; p.gamma = q.gamma; p.beta = q.beta; p.u_out = q.u_out;
   p.const_flag = q.const_flag; p.gamma_c = q.gamma_c; p.beta_c = q.beta_c;
   p.force_rescale = q.force_rescale ? 1 : 0;
-  p.dbg = q.dbg;
+  p.dbg = 0;
   p.trace = DITTO_F7_TRACE ? tc_gemm_debug_counters() : nullptr;
   // the cross-attention kernel does no work for the skipped sequences (profiler byte / flop counts over the processed ones)
   const double n_run = static_cast<double>(q.n_seq - (cross && q.const_flag ? profiled_nonzero(q.const_flag, q.n_seq, st) : 0));

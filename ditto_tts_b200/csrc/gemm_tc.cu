@@ -69,15 +69,12 @@ struct DevParams {
   const float* resid;
   long long ldr, sr_inner, sr_outer, resid_row_mod;
   bf16* out2; long long ldo2;
-  const float* rope_cos; const float* rope_sin; const float* rope_freq;
+  const float* rope_freq;
   int rope_half, rope_pd, seq_T, hidden;
   const int* rope_pos;  // optional [M] row -> position table (ragged batches); nullptr: position = row % seq_T
   int rope_fast;        // weights packed for the lean pd = 128 epilogue (TcGemmParams::rope_perm16)
   int glu_fast;         // [fc1; gate] rows packed for the lean GEGLU epilogue (TcGemmParams::glu_perm16)
   int out_perm4;        // fp32 + residual result in the 16-byte column order (TcGemmParams::out_perm4)
-  int dbg_nostore;      // timing experiment (wrong results): the lean QKV+RoPE / GEGLU epilogues skip their global stores
-  int stages;  // smem ring depth actually used (<= STAGES / P_STAGES)
-  int cm, cn;  // 1-CTA kernels: cluster shape in tiles (cm x cn CTAs share operands by TMA multicast); 1 x 1 = no cluster
   const float* row_lsum; int row_lparts; long long sl_inner, sl_outer;  // optional per-row 1/sum scale (fast STORE paths)
   // Deferred LayerNorm (DiT.py:105,143,151 without a LayerNorm pass over HBM).
   //  producer (STORE_F32_RESID): besides the fp32 result and its bf16 copy (out2), every epilogue warp writes the
@@ -639,29 +636,14 @@ __device__ __forceinline__ void rope_epilogue_fast128(const DevParams& p, int la
       }
     }
     // one 32-byte store per thread and block: a thread fills whole 32-byte sectors, a quad a whole 128-byte line (two
-    // 16-byte stores wrote half sectors each)
-    if (p.dbg_nostore == 2) {   // A/B: the two 16-byte stores per block of the first version
-      if (okA) {
-        reinterpret_cast<uint4*>(oA)[0] = make_uint4(w1A[0], w1A[1], w1A[2], w1A[3]);
-        reinterpret_cast<uint4*>(oA)[1] = make_uint4(w1A[4], w1A[5], w1A[6], w1A[7]);
-        reinterpret_cast<uint4*>(oA + off2)[0] = make_uint4(w2A[0], w2A[1], w2A[2], w2A[3]);
-        reinterpret_cast<uint4*>(oA + off2)[1] = make_uint4(w2A[4], w2A[5], w2A[6], w2A[7]);
-      }
-      if (okB) {
-        reinterpret_cast<uint4*>(oB)[0] = make_uint4(w1B[0], w1B[1], w1B[2], w1B[3]);
-        reinterpret_cast<uint4*>(oB)[1] = make_uint4(w1B[4], w1B[5], w1B[6], w1B[7]);
-        reinterpret_cast<uint4*>(oB + off2)[0] = make_uint4(w2B[0], w2B[1], w2B[2], w2B[3]);
-        reinterpret_cast<uint4*>(oB + off2)[1] = make_uint4(w2B[4], w2B[5], w2B[6], w2B[7]);
-      }
-    } else {
-    if (okA && !p.dbg_nostore) {
+    // 16-byte stores would write half sectors each)
+    if (okA) {
       st_global_v8(oA, w1A);
       st_global_v8(oA + off2, w2A);
     }
-    if (okB && !p.dbg_nostore) {
+    if (okB) {
       st_global_v8(oB, w1B);
       st_global_v8(oB + off2, w2B);
-    }
     }
   }
 }
@@ -965,7 +947,6 @@ __device__ __forceinline__ void epilogue_tile(const DevParams& p, int lane, int 
     // feeding the operand ring, a dependent load after the wait costs ~1 us and made this epilogue the bottleneck (ncu).
     const int pd = p.rope_pd;
     const int units = pd == 32 ? 2 : 1;
-    const bool on_the_fly = p.rope_freq != nullptr;  // warp-uniform
     const bool dln = p.ln_stat != nullptr;           // deferred LayerNorm: x = rstd acc + (nm c + b') before the rotation
     float lnA0, lnN0, lnA1, lnN1, lnA2, lnN2, lnA3, lnN3;  // rows row0 + g + {0, 8, 16, 24}
     ln_row_coef(p.ln_stat, p.ln_parts, row0 + g, row0 + g < p.M, p.ln_inv_h, lnA0, lnN0);
@@ -1011,7 +992,7 @@ __device__ __forceinline__ void epilogue_tile(const DevParams& p, int lane, int 
             if (dln) cx2[kb] = __ldg(reinterpret_cast<const float2*>(p.ln_c + pc1 + pd + q2 + kb * 8));
           }
         } else if (kb < nkb) {
-          if (on_the_fly) fr[kb] = __ldg(reinterpret_cast<const float2*>(p.rope_freq + jbase + q2 + kb * 8));
+          fr[kb] = __ldg(reinterpret_cast<const float2*>(p.rope_freq + jbase + q2 + kb * 8));
           bx1[kb] = __ldg(reinterpret_cast<const float2*>(bias + pc1 + q2 + kb * 8));
           bx2[kb] = __ldg(reinterpret_cast<const float2*>(bias + pc1 + pd + q2 + kb * 8));
           if (dln) {
@@ -1045,10 +1026,6 @@ __device__ __forceinline__ void epilogue_tile(const DevParams& p, int lane, int 
         }
         const unsigned posA = hh ? pos4[2] : pos4[0], posB = hh ? pos4[3] : pos4[1];
         const float fposA = static_cast<float>(posA), fposB = static_cast<float>(posB);
-        const float* cosA = p.rope_cos + static_cast<long long>(posA) * p.rope_half + jbase + q2;
-        const float* sinA = p.rope_sin + static_cast<long long>(posA) * p.rope_half + jbase + q2;
-        const float* cosB = p.rope_cos + static_cast<long long>(posB) * p.rope_half + jbase + q2;
-        const float* sinB = p.rope_sin + static_cast<long long>(posB) * p.rope_half + jbase + q2;
         bf16* outp = static_cast<bf16*>(p.out) + out_off + rowA * p.ldo + dbase + q2;
         tmem_ld_wait();
 #pragma unroll
@@ -1057,15 +1034,10 @@ __device__ __forceinline__ void epilogue_tile(const DevParams& p, int lane, int 
           const int k2 = (kb + 4) & 7;  // partner block inside r1 when PD == 32
 #pragma unroll
           for (int rr = 0; rr < 2; ++rr) {
-            float2 c2, s2;
-            if (on_the_fly) {  // angle = float(pos) * inv_freq[j] exactly as the reference forms it
-              const float fp = rr == 0 ? fposA : fposB;
-              sincos_reduced(fp * fr[kb].x, s2.x, c2.x);
-              sincos_reduced(fp * fr[kb].y, s2.y, c2.y);
-            } else {
-              c2 = __ldg(reinterpret_cast<const float2*>((rr == 0 ? cosA : cosB) + kb * 8));
-              s2 = __ldg(reinterpret_cast<const float2*>((rr == 0 ? sinA : sinB) + kb * 8));
-            }
+            float2 c2, s2;   // angle = float(pos) * inv_freq[j] exactly as the reference forms it
+            const float fp = rr == 0 ? fposA : fposB;
+            sincos_reduced(fp * fr[kb].x, s2.x, c2.x);
+            sincos_reduced(fp * fr[kb].y, s2.y, c2.y);
             const float ar = rr == 0 ? aA : aB, nr = rr == 0 ? nA : nB;
             const float x1a = fmaf(ar, __uint_as_float(r1[4 * kb + 2 * rr]), fmaf(nr, cx1[kb].x, bx1[kb].x));
             const float x1b = fmaf(ar, __uint_as_float(r1[4 * kb + 2 * rr + 1]), fmaf(nr, cx1[kb].y, bx1[kb].y));
@@ -1092,13 +1064,8 @@ __device__ __forceinline__ void epilogue_tile(const DevParams& p, int lane, int 
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Cluster multicast (1-CTA kernels).  The L2 -> SM operand feed, not the tensor pipe, bounds these GEMMs (ncu: a
-// 128 x 256 tile pulls 48 KiB per k-block, ~2.5x what the L2 can deliver at full MMA rate), so a cluster of cm x cn CTAs
-// computing adjacent tiles shares its operands: the A k-block of a tile row is loaded ONCE and multicast to the cn CTAs
-// of that row, the B k-block once for the cm CTAs of a tile column.  The loader rotates with the k-block index
-// (kb % cn, kb % cm), so every CTA issues an equal share and no tensor-map box has to be split.
-// A shared-memory slot may only be overwritten once every CTA that receives the multicast has consumed it: the MMA
-// issuer's commit is multicast to the empty barriers of its whole row and column group (cm + cn - 1 arrivals per phase).
+// Cluster multicast (scores kernel): a TMA load written into the shared memory of every CTA in `mask`, and an MMA commit
+// that arrives on the barrier at the same offset in every CTA in `mask`.
 // ---------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void tma_load_4d_mc(const CUtensorMap* m, uint64_t* bar, void* smem, int c0, int c1, int c2, int c3,
                                                uint16_t mask) {
@@ -1112,23 +1079,6 @@ __device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
                "h"(mask)
                : "memory");
-}
-
-struct ClusterPos {
-  int csize, rm, rn;          // cluster size, this CTA's tile-row / tile-column inside the cluster
-  uint16_t row_mask, col_mask;  // CTAs sharing this CTA's A block / B block (both include the CTA itself)
-};
-__device__ __forceinline__ ClusterPos cluster_pos(int cm, int cn) {
-  ClusterPos c;
-  c.csize = cm * cn;
-  const int rank = c.csize > 1 ? static_cast<int>(cluster_ctarank()) : 0;
-  c.rm = rank / cn;
-  c.rn = rank - c.rm * cn;
-  c.row_mask = static_cast<uint16_t>(((1u << cn) - 1u) << (c.rm * cn));
-  uint32_t cmask = 0;
-  for (int j = 0; j < cm; ++j) cmask |= 1u << (j * cn + c.rn);
-  c.col_mask = static_cast<uint16_t>(cmask);
-  return c;
 }
 
 // Register re-distribution between the warp roles (setmaxnreg, one instruction per warpgroup): warps 0-3 (TMA producer,
@@ -1149,12 +1099,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
 
   const int warp = warp_id_uniform();   // control warps run on warp-uniform values (see common.cuh: elect_one)
   const int lane = threadIdx.x & 31;
-  const ClusterPos cp = cluster_pos(p.cm, p.cn);
-  const int num_clusters = gridDim.x / cp.csize;
-  const int cluster_id = blockIdx.x / cp.csize;
-  // super tile st = (batch item, sm, sn), sn fastest; this CTA's tile: (sm * cm + rm, sn * cn + rn)
-  const int n_super = (p.n_tiles + p.cn - 1) / p.cn, m_super = (p.m_tiles + p.cm - 1) / p.cm;
-  const int num_super = n_super * m_super * p.batch_inner * p.batch_outer;
+  // tile = (batch item, m_blk, n_blk), n_blk fastest
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_a);
@@ -1163,7 +1108,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], static_cast<uint32_t>(p.cm + p.cn - 1));
+      mbar_init(&empty_bar[s], 1);
     }
     for (int s = 0; s < 2; ++s) {
       mbar_init(&tmem_full[s], 1);
@@ -1174,7 +1119,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
   if (warp == 2) tmem_alloc<TMEM_COLS>(tmem_ptr);
   tcgen05_fence_before();
   __syncthreads();
-  if (cp.csize > 1) cluster_sync_all();  // peers' barriers exist before the first multicast load / commit reaches them
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
 
@@ -1184,12 +1128,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
     const bool leader = elect_one();
     int stage = 0;
     uint32_t phase = 0;
-    for (int st = cluster_id; st < num_super; st += num_clusters) {
-      const int sn = st % n_super;
-      const int rest = st / n_super;
-      const int smi = rest % m_super;
-      const int b = rest / m_super;
-      const int m_blk = smi * p.cm + cp.rm, n_blk = sn * p.cn + cp.rn;  // may lie past the edge: TMA zero-fills
+    for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
+      const int n_blk = tile % p.n_tiles;
+      const int rest = tile / p.n_tiles;
+      const int m_blk = rest % p.m_tiles;
+      const int b = rest / p.m_tiles;
       const int bo = b / p.batch_inner, bi = b - bo * p.batch_inner;
       const int abi = p.a_bi ? bi : 0, abo = p.a_bo ? bo : 0;
       const int bbi = p.b_bi ? bi : 0, bbo = p.b_bo ? bo : 0;
@@ -1199,32 +1142,17 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
           uint8_t* sa = smem + stage * STAGE_BYTES;
           uint8_t* sb = sa + A_STAGE_BYTES;
           mbar_expect_tx(&full_bar[stage], STAGE_BYTES);
-          if (cp.csize == 1) {
-            tma_load_4d(&tmap_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M, abi, abo);
-            if (!B_KN) {
-              tma_load_4d(&tmap_b, &full_bar[stage], sb, kb * BLOCK_K, n_blk * BLOCK_N, bbi, bbo);
-            } else {
-#pragma unroll
-              for (int j = 0; j < BLOCK_N / 64; ++j)  // [64 k-rows x 64 n] boxes, N-contiguous (MN-major operand)
-                tma_load_4d(&tmap_b, &full_bar[stage], sb + j * (BLOCK_K * 128), n_blk * BLOCK_N + j * 64, kb * BLOCK_K, bbi, bbo);
-            }
+          tma_load_4d(&tmap_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M, abi, abo);
+          if (!B_KN) {
+            tma_load_4d(&tmap_b, &full_bar[stage], sb, kb * BLOCK_K, n_blk * BLOCK_N, bbi, bbo);
           } else {
-            if (kb % p.cn == cp.rn)  // this CTA fetches the A block for its whole tile row
-              tma_load_4d_mc(&tmap_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M, abi, abo, cp.row_mask);
-            if (kb % p.cm == cp.rm) {  // ... and the B block for its whole tile column
-              if (!B_KN) {
-                tma_load_4d_mc(&tmap_b, &full_bar[stage], sb, kb * BLOCK_K, n_blk * BLOCK_N, bbi, bbo, cp.col_mask);
-              } else {
 #pragma unroll
-                for (int j = 0; j < BLOCK_N / 64; ++j)
-                  tma_load_4d_mc(&tmap_b, &full_bar[stage], sb + j * (BLOCK_K * 128), n_blk * BLOCK_N + j * 64, kb * BLOCK_K, bbi, bbo,
-                                 cp.col_mask);
-              }
-            }
+            for (int j = 0; j < BLOCK_N / 64; ++j)  // [64 k-rows x 64 n] boxes, N-contiguous (MN-major operand)
+              tma_load_4d(&tmap_b, &full_bar[stage], sb + j * (BLOCK_K * 128), n_blk * BLOCK_N + j * 64, kb * BLOCK_K, bbi, bbo);
           }
         }
         __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1u; }
+        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
       }
     }
   } else if (warp == 1) {
@@ -1232,7 +1160,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
     regs_shrink_ctrl();
     const bool leader = elect_one();
     constexpr uint32_t idesc = umma_idesc_bf16(BLOCK_M, BLOCK_N, false, B_KN);
-    const uint16_t commit_mask = static_cast<uint16_t>(cp.row_mask | cp.col_mask);
     // operand descriptors of ring slot 0; a slot / k-step only adds to the 14-bit address field (16-byte units, no carry:
     // shared memory ends below 256 KiB)
     const uint64_t da0 = umma_smem_desc(smem_u32(smem), 16, 1024);
@@ -1242,7 +1169,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
     uint32_t phase = 0;
     int as = 0;
     uint32_t aphase = 0;
-    for (int st = cluster_id; st < num_super; st += num_clusters) {
+    for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
       mbar_wait(&tmem_empty[as], aphase ^ 1u);  // epilogue has drained this accumulator stage
       tcgen05_fence_after();
       const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(as * BLOCK_N);
@@ -1255,12 +1182,10 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
           for (int k = 0; k < BLOCK_K / UMMA_K; ++k)
             umma_bf16(d_tmem, da + ((k * (UMMA_K * 2)) >> 4), db + ((B_KN ? k * (UMMA_K * 128) : k * (UMMA_K * 2)) >> 4), idesc,
                       (kb | k) != 0 ? 1u : 0u);
-          // smem slot reusable once these MMAs retire -- announced to every CTA that may multicast into this slot
-          if (cp.csize == 1) umma_commit(&empty_bar[stage]);
-          else umma_commit_mc(&empty_bar[stage], commit_mask);
+          umma_commit(&empty_bar[stage]);  // smem slot reusable once these MMAs retire
         }
         __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1u; }
+        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
       }
       if (leader) umma_commit(&tmem_full[as]);  // accumulator complete -> epilogue
       __syncwarp();
@@ -1274,25 +1199,20 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
     const int half_sel = ew >> 2;  // which 4 of the 8 column chunks
     int as = 0;
     uint32_t aphase = 0;
-    for (int st = cluster_id; st < num_super; st += num_clusters) {
-      const int sn = st % n_super;
-      const int rest = st / n_super;
-      const int smi = rest % m_super;
-      const int b = rest / m_super;
-      const int m_blk = smi * p.cm + cp.rm, n_blk = sn * p.cn + cp.rn;
+    for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
+      const int n_blk = tile % p.n_tiles;
+      const int rest = tile / p.n_tiles;
+      const int m_blk = rest % p.m_tiles;
+      const int b = rest / p.m_tiles;
       const int bo = b / p.batch_inner, bi = b - bo * p.batch_inner;
       const long long out_off = bo * p.so_outer + bi * p.so_inner;
       const long long res_off = bo * p.sr_outer + bi * p.sr_inner;
       const long long bias_off = bo * p.sb_outer + bi * p.sb_inner;
-      // a tile past the matrix edge (cluster padding) is computed on zero-filled operands and stores nothing:
-      // row0 >= M and column >= N make every store predicate false
-      const long long row0 = (m_blk < p.m_tiles && n_blk < p.n_tiles) ? static_cast<long long>(m_blk) * BLOCK_M + quarter * 32
-                                                                    : static_cast<long long>(p.M);
+      const long long row0 = static_cast<long long>(m_blk) * BLOCK_M + quarter * 32;
       const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(as * BLOCK_N);
       const long long ls_off = bo * p.sl_outer + bi * p.sl_inner;
       const long long st_off = (bo * p.stat_rows_outer) * p.stat_parts + static_cast<long long>(bi) * p.stat_parts_item;
-      epilogue_tile<EPI>(p, lane, half_sel, t_row, row0, n_blk < p.n_tiles ? n_blk : 0, out_off, res_off, bias_off, ls_off, st_off,
-                         &tmem_full[as], aphase);
+      epilogue_tile<EPI>(p, lane, half_sel, t_row, row0, n_blk, out_off, res_off, bias_off, ls_off, st_off, &tmem_full[as], aphase);
       tcgen05_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[as]);
@@ -1305,7 +1225,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
   __syncwarp();
   tcgen05_fence_before();
   __syncthreads();
-  if (cp.csize > 1) cluster_sync_all();  // nobody leaves while a peer may still multicast into it / signal its barriers
   if (warp == 2) {
     tcgen05_fence_after();
     tmem_dealloc<TMEM_COLS>(tmem_base);
@@ -1399,7 +1318,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
           tma_load_4d_2sm(&tmap_b, &full_bar[stage], sb, kb * BLOCK_K, n0, 0, 0);
         }
         __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1u; }
+        if (++stage == P_STAGES) { stage = 0; phase ^= 1u; }
       }
     }
     if (kDbgCounters && p.dbg && rank == 0 && leader) {
@@ -1446,7 +1365,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
             umma_commit_2sm(&empty_bar[stage]);
           }
           __syncwarp();
-          if (++stage == p.stages) { stage = 0; phase ^= 1u; }
+          if (++stage == P_STAGES) { stage = 0; phase ^= 1u; }
         }
         if (leader) umma_commit_2sm(&tmem_full[as]);
         __syncwarp();
@@ -1514,7 +1433,7 @@ struct SmDev {
   bf16* P; long long ldp, sp_inner, sp_outer;
   int npad;
   float* lpart; long long sl_inner, sl_outer;
-  int csize, cm, stages;  // csize key tiles per row (cluster columns), cm query blocks per cluster (cluster rows)
+  int csize;   // key tiles per row = CTAs per cluster
   // deferred LayerNorm of the query operand (HAS_BIAS variant): s = alpha (rstd acc - rstd mean c[col]) + bias[col];
   // statistics row = outer batch index * M + query row; c has the layout / strides of bias
   const float2* ln_stat; int ln_parts; float ln_inv_h; const float* ln_c;
@@ -1554,15 +1473,13 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
 
   const int warp = warp_id_uniform();
   const int lane = threadIdx.x & 31;
-  // cluster = cm tile rows x csize tile columns: CTA (rm, rank) computes query block mg * cm + rm against key tile `rank`;
-  // Q blocks are multicast along a row, K blocks along a column, row maxima are exchanged along a row
+  // CTA `rank` of the cluster computes the work item's query block against key tile `rank`; the Q block is multicast to
+  // the whole cluster, the row maxima are exchanged across it
   const int csize = p.csize;
-  const ClusterPos cp = cluster_pos(p.cm, csize);
-  const int rank = cp.rn;
-  const int num_clusters = gridDim.x / cp.csize;
-  const int cluster_id = blockIdx.x / cp.csize;
-  const int m_groups = (p.m_tiles + p.cm - 1) / p.cm;
-  const int num_items = m_groups * p.batch_inner * p.batch_outer;
+  const int rank = csize > 1 ? static_cast<int>(cluster_ctarank()) : 0;
+  const uint16_t cluster_mask = static_cast<uint16_t>((1u << csize) - 1u);
+  const int num_clusters = gridDim.x / csize;
+  const int cluster_id = blockIdx.x / csize;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_a);
@@ -1571,7 +1488,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], static_cast<uint32_t>(p.cm + csize - 1));
+      mbar_init(&empty_bar[s], static_cast<uint32_t>(csize));   // a slot is free once every CTA's MMAs have read its Q block
     }
     for (int s = 0; s < 2; ++s) {
       mbar_init(&tmem_full[s], 1);
@@ -1583,7 +1500,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
   if (warp == 2) tmem_alloc<TMEM_COLS>(tmem_ptr);
   tcgen05_fence_before();
   __syncthreads();
-  if (cp.csize > 1) cluster_sync_all();  // every peer's barriers are initialised before the first remote arrive / multicast
+  if (csize > 1) cluster_sync_all();  // every peer's barriers are initialised before the first remote arrive / multicast
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
 
@@ -1593,9 +1510,9 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
     const bool leader = elect_one();
     int stage = 0;
     uint32_t phase = 0;
-    for (int item = cluster_id; item < num_items; item += num_clusters) {
-      const int m_blk = (item % m_groups) * p.cm + cp.rm;  // may lie past the last block (cluster padding): zero-filled
-      const int b = item / m_groups;
+    for (int item = cluster_id; item < p.num_items; item += num_clusters) {
+      const int m_blk = item % p.m_tiles;
+      const int b = item / p.m_tiles;
       const int bo = b / p.batch_inner, bi = b - bo * p.batch_inner;
       const int abi = p.a_bi ? bi : 0, abo = p.a_bo ? bo : 0;
       const int bbi = p.b_bi ? bi : 0, bbo = p.b_bo ? bo : 0;
@@ -1605,18 +1522,14 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
           uint8_t* sa = smem + stage * STAGE_BYTES;
           uint8_t* sb = sa + A_STAGE_BYTES;
           mbar_expect_tx(&full_bar[stage], STAGE_BYTES);
-          if (cp.csize == 1) {
+          if (csize == 1)
             tma_load_4d(&tmap_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M, abi, abo);
-            tma_load_4d(&tmap_b, &full_bar[stage], sb, kb * BLOCK_K, rank * BLOCK_N, bbi, bbo);
-          } else {
-            if (kb % csize == rank)
-              tma_load_4d_mc(&tmap_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M, abi, abo, cp.row_mask);
-            if (kb % p.cm == cp.rm)
-              tma_load_4d_mc(&tmap_b, &full_bar[stage], sb, kb * BLOCK_K, rank * BLOCK_N, bbi, bbo, cp.col_mask);
-          }
+          else if (kb % csize == rank)   // the CTAs take turns fetching the Q block for the whole cluster
+            tma_load_4d_mc(&tmap_a, &full_bar[stage], sa, kb * BLOCK_K, m_blk * BLOCK_M, abi, abo, cluster_mask);
+          tma_load_4d(&tmap_b, &full_bar[stage], sb, kb * BLOCK_K, rank * BLOCK_N, bbi, bbo);
         }
         __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1u; }
+        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
       }
     }
   } else if (warp == 1) {
@@ -1630,8 +1543,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
     uint32_t phase = 0;
     int as = 0;
     uint32_t aphase = 0;
-    const uint16_t commit_mask = static_cast<uint16_t>(cp.row_mask | cp.col_mask);
-    for (int item = cluster_id; item < num_items; item += num_clusters) {
+    for (int item = cluster_id; item < p.num_items; item += num_clusters) {
       mbar_wait(&tmem_empty[as], aphase ^ 1u);
       tcgen05_fence_after();
       const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(as * BLOCK_N);
@@ -1643,11 +1555,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
 #pragma unroll
           for (int k = 0; k < BLOCK_K / UMMA_K; ++k)
             umma_bf16(d_tmem, da + ((k * (UMMA_K * 2)) >> 4), db + ((k * (UMMA_K * 2)) >> 4), idesc, (kb | k) != 0 ? 1u : 0u);
-          if (cp.csize == 1) umma_commit(&empty_bar[stage]);
-          else umma_commit_mc(&empty_bar[stage], commit_mask);
+          if (csize == 1) umma_commit(&empty_bar[stage]);
+          else umma_commit_mc(&empty_bar[stage], cluster_mask);   // every CTA's slot may hold a Q block this CTA multicast
         }
         __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1u; }
+        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
       }
       if (leader) umma_commit(&tmem_full[as]);
       __syncwarp();
@@ -1665,11 +1577,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
     const bool writer = (lane & 3) == 0;
     int as = 0;
     uint32_t aphase = 0;
-    for (int item = cluster_id; item < num_items; item += num_clusters) {
-      const int m_blk = (item % m_groups) * p.cm + cp.rm;
-      const int b = item / m_groups;
+    for (int item = cluster_id; item < p.num_items; item += num_clusters) {
+      const int m_blk = item % p.m_tiles;
+      const int b = item / p.m_tiles;
       const int bo = b / p.batch_inner, bi = b - bo * p.batch_inner;
-      // second row: rowA + 8; a padding block (m_blk >= m_tiles) has every row >= M and stores nothing
+      // second row: rowA + 8
       const long long rowA = static_cast<long long>(m_blk) * BLOCK_M + trow + g;
       const bool okA = rowA < p.M, okB = rowA + 8 < p.M;
       const float* bias = HAS_BIAS ? p.bias + bo * p.sb_outer + bi * p.sb_inner : nullptr;
@@ -1747,9 +1659,9 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
         if (writer) {
           const uint32_t slotA = smem_u32(stat + (as * SM_MAX_CLUSTER + rank) * BLOCK_M + trow + g);
           const uint32_t barl = smem_u32(&stat_bar[as]);
-          for (int c = 0; c < csize; ++c) {  // the CTAs of this tile row: cluster ranks rm * csize + c
-            const uint32_t ra = mapa_shared(slotA, static_cast<uint32_t>(cp.rm * csize + c));
-            const uint32_t rb = mapa_shared(barl, static_cast<uint32_t>(cp.rm * csize + c));
+          for (int c = 0; c < csize; ++c) {
+            const uint32_t ra = mapa_shared(slotA, static_cast<uint32_t>(c));
+            const uint32_t rb = mapa_shared(barl, static_cast<uint32_t>(c));
             st_async_f32(ra, mA, rb);
             st_async_f32(ra + 8 * 4, mB, rb);
           }
@@ -1885,7 +1797,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
   __syncwarp();
   tcgen05_fence_before();
   __syncthreads();
-  if (cp.csize > 1) cluster_sync_all();  // nobody leaves while a peer may still write into this CTA / signal its barriers
+  if (csize > 1) cluster_sync_all();  // nobody leaves while a peer may still write into this CTA / signal its barriers
   if (warp == 2) {
     tcgen05_fence_after();
     tmem_dealloc<TMEM_COLS>(tmem_base);
@@ -2092,7 +2004,7 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
   if (q.epilogue == TC_EPI_GEGLU)
     DITTO_REQUIRE(q.N % 32 == 0 && q.bias && q.out_bf16 && !q.b_kn, DITTO_E_UNSUPPORTED, "tc_gemm: GEGLU epilogue constraints");
   if (q.epilogue == TC_EPI_QKV_ROPE)
-    DITTO_REQUIRE(q.bias && q.out_bf16 && !q.b_kn && q.rope_cos && q.rope_sin && q.N == 3 * q.hidden &&
+    DITTO_REQUIRE(q.bias && q.out_bf16 && !q.b_kn && q.rope_freq && q.N == 3 * q.hidden &&
                       (q.rope_pd == 32 || q.rope_pd == 64 || q.rope_pd == 128) && q.rope_half % q.rope_pd == 0 &&
                       q.hidden % (2 * q.rope_pd) == 0 && q.seq_T > 0 && q.alpha == 1.f && !q.resid && !q.out2,
                   DITTO_E_UNSUPPORTED, "tc_gemm: QKV_ROPE epilogue constraints");
@@ -2101,8 +2013,7 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
   TcOperand A = q.A, B = q.B;
   // paired (cta_group::2) kernel for the large un-batched weight GEMMs
   const int g_num_sms = tc_num_sms();
-  const bool g_force_generic = g_opt.generic_epi != 0;
-  const bool pair = !g_opt.no_pair && !q.b_kn && q.batch_inner == 1 && q.batch_outer == 1 && q.M >= 2 * BLOCK_M && (g_num_sms % 2 == 0);
+  const bool pair = !q.b_kn && q.batch_inner == 1 && q.batch_outer == 1 && q.M >= 2 * BLOCK_M && (g_num_sms % 2 == 0);
   DITTO_TRY(make_map(&ma, A, q.batch_inner, q.batch_outer, BLOCK_K, BLOCK_M));
   if (pair)
     DITTO_TRY(make_map(&mb, B, 1, 1, BLOCK_K, BLOCK_N / 2));
@@ -2127,16 +2038,15 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
   p.ldo = q.ldo; p.so_inner = q.so_inner; p.so_outer = q.so_outer;
   p.resid = q.resid; p.ldr = q.ldr; p.sr_inner = q.sr_inner; p.sr_outer = q.sr_outer; p.resid_row_mod = q.resid_row_mod;
   p.out2 = q.out2; p.ldo2 = q.ldo2;
-  p.rope_cos = q.rope_cos; p.rope_sin = q.rope_sin; p.rope_freq = q.rope_freq;
+  p.rope_freq = q.rope_freq;
   p.rope_half = q.rope_half; p.rope_pd = q.rope_pd; p.seq_T = q.seq_T; p.hidden = q.hidden; p.rope_pos = q.rope_pos; p.rope_fast = q.rope_perm16 ? 1 : 0; p.glu_fast = q.glu_perm16 ? 1 : 0; p.out_perm4 = q.out_perm4 ? 1 : 0;
   p.row_lsum = q.row_lsum; p.row_lparts = q.row_lparts; p.sl_inner = q.sl_inner; p.sl_outer = q.sl_outer;
   p.stat_out = q.stat_out; p.stat_parts = q.stat_parts; p.stat_rows_outer = q.stat_rows_outer;
   p.stat_parts_item = static_cast<int>(ceil_div(q.N, 128));
   p.ln_stat = q.ln_stat; p.ln_parts = q.ln_parts; p.ln_inv_h = q.ln_width > 0 ? 1.0f / static_cast<float>(q.ln_width) : 0.f;
   p.ln_c = q.ln_c;
-  p.dbg_nostore = g_opt.dbg_nostore;
   if (q.stat_out != nullptr)
-    DITTO_REQUIRE(q.epilogue == TC_EPI_STORE && q.resid && !q.out_bf16 && q.N % 2 == 0 && !g_force_generic &&
+    DITTO_REQUIRE(q.epilogue == TC_EPI_STORE && q.resid && !q.out_bf16 && q.N % 2 == 0 &&
                       q.stat_parts == q.batch_inner * p.stat_parts_item && (q.batch_outer == 1 || q.stat_rows_outer >= q.M),
                   DITTO_E_UNSUPPORTED, "tc_gemm: row statistics need the fp32 + residual STORE epilogue and matching stat_parts");
   if (q.ln_stat != nullptr)
@@ -2147,9 +2057,6 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
 
   unsigned grid = static_cast<unsigned>(std::min<int64_t>(tiles, g_num_sms));
   ProfScope prof(q.tag, st, 2.0 * q.M * q.N * q.K * q.batch_inner * q.batch_outer, 0.0);
-  p.stages = pair ? (g_opt.stages_pair >= 2 ? std::min(P_STAGES, g_opt.stages_pair) : P_STAGES)
-                  : (g_opt.stages_1cta >= 2 ? std::min(STAGES, g_opt.stages_1cta) : STAGES);
-  p.cm = 1; p.cn = 1;
   if (q.out_perm4)
     DITTO_REQUIRE(q.epilogue == TC_EPI_STORE && !q.out_bf16 && q.resid != nullptr && q.bias == nullptr && q.out2 == nullptr &&
                       q.stat_out == nullptr && q.resid_row_mod == 0 && q.N % 128 == 0 && q.ldo % 4 == 0 && q.ldr % 4 == 0 &&
@@ -2159,10 +2066,10 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
     DITTO_REQUIRE(q.epilogue == TC_EPI_GEGLU && q.ln_stat == nullptr && q.N % BLOCK_N == 0 && q.out_bf16 && q.ldo % 8 == 0 && q.bias != nullptr,
                   DITTO_E_BADARG, "tc_gemm: glu_perm16 needs the GEGLU epilogue, no deferred LayerNorm, a bias and N % 256 == 0");
   if (q.rope_perm16)
-    DITTO_REQUIRE(q.epilogue == TC_EPI_QKV_ROPE && (q.rope_pd == 128 || q.rope_pd == 32) && q.rope_freq != nullptr && q.ln_stat == nullptr &&
+    DITTO_REQUIRE(q.epilogue == TC_EPI_QKV_ROPE && (q.rope_pd == 128 || q.rope_pd == 32) && q.ln_stat == nullptr &&
                       q.N % BLOCK_N == 0 && q.hidden % BLOCK_N == 0 && q.out_bf16 && q.ldo % 16 == 0 &&
                       (reinterpret_cast<uintptr_t>(q.out) & 31) == 0 && (q.batch_inner * q.batch_outer == 1 || (q.so_inner % 16 == 0 && q.so_outer % 16 == 0)),
-                  DITTO_E_BADARG, "tc_gemm: rope_perm16 needs pd = 128 or 32, on-the-fly frequencies, no deferred LayerNorm, N and hidden % 256 == 0, "
+                  DITTO_E_BADARG, "tc_gemm: rope_perm16 needs pd = 128 or 32, no deferred LayerNorm, N and hidden % 256 == 0, "
                                   "a 32-byte aligned output with a row stride of a multiple of 16 (32-byte stores)");
   // kernel variant: the lean compile-time epilogues cover the hot cases, anything else takes the generic one
   int ke;
@@ -2174,7 +2081,6 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
   } else if (q.N % 2 != 0) ke = K_STORE_GENERIC;
   else if (!q.out_bf16) ke = q.resid ? K_STORE_F32_RESID : (q.out2 ? K_STORE_GENERIC : K_STORE_F32);
   else ke = (q.resid || q.out2) ? K_STORE_GENERIC : K_STORE_BF16;
-  if (g_force_generic && q.epilogue == TC_EPI_STORE) ke = K_STORE_GENERIC;
   if (q.row_lsum != nullptr)
     DITTO_REQUIRE(ke == K_STORE_F32 || ke == K_STORE_F32_RESID || ke == K_STORE_BF16, DITTO_E_UNSUPPORTED,
                   "tc_gemm: row_lsum needs a fast STORE epilogue (even N)");
@@ -2212,20 +2118,9 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
       default: func = DITTO_FUNC_1CTA(K_QKV_ROPE, false); break;
     }
   }
-  {
-    // cluster shape: explicit > DITTO_CLUSTER > 1 x 1.  Measured on B200 (profiles/README.md): for the epilogue-heavy
-    // batched attention GEMMs the lock-step coupling of a multicast cluster costs more than the saved L2 traffic, so
-    // multicast stays opt-in here; the fused scores kernel always shares the Q block across its key-tile cluster.
-    int cm = q.cluster_m > 0 ? q.cluster_m : g_opt.cluster_m, cn = q.cluster_n > 0 ? q.cluster_n : g_opt.cluster_n;
-    if (cm <= 0 || cn <= 0) cm = cn = 1;
-    cm = std::min(cm, p.m_tiles);
-    cn = std::min(cn, p.n_tiles);
-    p.cm = cm; p.cn = cn;
-    const int csize = cm * cn;
-    const int64_t num_super = ceil_div(p.m_tiles, cm) * ceil_div(p.n_tiles, cn) * q.batch_inner * q.batch_outer;
-    DITTO_TRY(launch_clustered(func, csize, SMEM_BYTES, num_super, ma, mb, p, st));
-  }
-  return 0;
+  // no cluster: TMA multicast of the operands across CTAs of adjacent tiles was measured on B200 (profiles/README.md) and
+  // lost -- for these epilogue-heavy batched attention GEMMs the lock-step coupling costs more than the saved L2 traffic
+  return launch_clustered(func, 1, SMEM_BYTES, tiles, ma, mb, p, st);
 }
 #undef DITTO_LAUNCH_PAIR
 #undef DITTO_FUNC_1CTA
@@ -2267,20 +2162,16 @@ int launch_tc_scores_softmax(const TcScoresSoftmaxParams& q, cudaStream_t st) {
   p.P = q.P; p.ldp = q.ldp; p.sp_inner = q.sp_inner; p.sp_outer = q.sp_outer;
   p.npad = q.npad;
   p.lpart = q.lpart; p.sl_inner = q.sl_inner; p.sl_outer = q.sl_outer;
-  p.csize = csize; p.stages = g_opt.stages_1cta >= 2 ? std::min(STAGES, g_opt.stages_1cta) : STAGES;
+  p.csize = csize;
   p.ln_stat = q.ln_stat; p.ln_parts = q.ln_parts; p.ln_inv_h = q.ln_width > 0 ? 1.0f / static_cast<float>(q.ln_width) : 0.f;
   p.ln_c = q.ln_c;
   if (q.ln_stat != nullptr)
     DITTO_REQUIRE(q.bias && q.ln_c && q.ln_parts > 0 && q.ln_width > 0, DITTO_E_BADARG, "tc_scores_softmax: deferred LayerNorm arguments");
-  int cm = q.cluster_m > 0 ? q.cluster_m : (g_opt.cluster_m > 0 ? g_opt.cluster_m : 1);
-  cm = std::max(1, std::min(cm, std::min(p.m_tiles, SM_MAX_CLUSTER / csize)));
-  p.cm = cm;
   // flops: the contraction; bytes: nothing (the fused softmax saves 12 B per score of HBM round trips)
   ProfScope prof(q.tag, st, 2.0 * q.M * q.N * q.K * q.batch_inner * q.batch_outer, 0.0);
-  const int64_t work = ceil_div(p.m_tiles, cm) * q.batch_inner * q.batch_outer;
   const void* func = q.bias != nullptr ? reinterpret_cast<const void*>(&tc_scores_softmax_kernel<true>)
                                        : reinterpret_cast<const void*>(&tc_scores_softmax_kernel<false>);
-  return launch_clustered(func, csize * cm, SM_SMEM_BYTES, work, ma, mb, p, st);
+  return launch_clustered(func, csize, SM_SMEM_BYTES, items, ma, mb, p, st);
 }
 
 }  // namespace ditto

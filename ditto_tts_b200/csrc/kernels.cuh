@@ -9,14 +9,11 @@ namespace ditto {
 // ---- developer options (ditto_debug_option): A/B switches of the kernels, all 0 = the product path.  The library never
 // reads the environment; tools / tests set these through the C-ABI before creating an engine.
 struct DebugOptions {
-  // gemm_tc.cu (read at launch time)
-  int no_pair = 0, cluster_m = 0, cluster_n = 0, generic_epi = 0, stages_1cta = 0, stages_pair = 0, no_mcast = 0, dbg_nostore = 0;
   // cross_fused.cu
   int xf_rows = 0;
-  int xf_prefetch = 0;   // > 0: L2 prefetch of the residual stream, n half-chunk jobs ahead (experiment; off by default)
   // engine.cu (read by ditto_engine_create)
-  int no_defer_ln = 0, no_fused_attn = 0, no_flash = 0, no_flash768 = 0, no_fused_cross = 0, defer_ln2 = 0, pv_transpose = 0,
-      rope_table = 0, rope_generic = 0, glu_generic = 0, no_rope_fast32 = 0, no_pv_perm4 = 0, side_streams = -1, no_fused_ln = 0;
+  int no_defer_ln = 0, no_flash = 0, no_flash768 = 0, no_fused_cross = 0, defer_ln2 = 0, rope_generic = 0, glu_generic = 0,
+      no_pv_perm4 = 0, side_streams = -1;
   // flash_attn768.cu (read at launch time): 1 = always the two-CTA kernel, 2 = the four-CTA kernel whenever it is supported
   int flash768_quad = 0;
   // engine.cu: fc2 + residual + next block's norm1 as separate launches (GEMM, LayerNorm) instead of gemm_resid_ln.cu
@@ -64,7 +61,6 @@ int launch_const_text(const float* text, int64_t n, int S, int D, const bf16* vf
 // number of nonzero bytes of flags[0, n) for the profiler's byte counts; 0 without synchronising unless profiling (which
 // synchronises anyway and is never captured)
 int64_t profiled_nonzero(const uint8_t* flags, int64_t n, cudaStream_t st);
-int launch_transpose_v(const bf16* v, int64_t ld, bf16* vt, int64_t n_seq, int T, int Tp, int heads, int d, cudaStream_t st);
 // One sampler update over B sequences of `per` elements: eps = eps_u + w (eps_c - eps_u) (eps_u == null: eps = eps_c), then
 //   DDPM form (hist == null, coef [steps, 3] = {c1, c2, c3}):  x_out = c1 (x - c2 eps) + c3 z
 //   multistep (hist != null, coef [steps, 6] = {c1, c2, c3, c4, d1, d2}, DPM-Solver++(2M)): the same + c4 hist, then
@@ -139,8 +135,7 @@ struct TcGemmParams {
   int64_t resid_row_mod = 0;                   // >0: residual row = row % resid_row_mod (x_skip shared by CFG branches)
   bf16* out2 = nullptr; int64_t ldo2 = 0;      // optional bf16 copy of the (fp32) result, batch strides as `out`
   // TC_EPI_QKV_ROPE
-  const float* rope_cos = nullptr; const float* rope_sin = nullptr;
-  const float* rope_freq = nullptr;            // [d/2] inv_freq: when set, cos/sin are computed in the epilogue (no table reads)
+  const float* rope_freq = nullptr;            // [d/2] inv_freq (required): cos/sin are computed in the epilogue
   int rope_half = 0, rope_pd = 0, seq_T = 0, hidden = 0;
   const int* rope_pos = nullptr;               // optional [M] row -> position table (ragged batches) instead of row % seq_T
   // weight rows additionally permuted inside every 64-row block (GEMM column kb*8 + 2q + e = output column q*16 + kb*2 + e):
@@ -154,8 +149,6 @@ struct TcGemmParams {
   // optional per-row scale 1 / sum_c row_lsum[row*row_lparts + c] applied to the accumulator (softmax normalisation of an
   // unnormalised P operand, see launch_tc_scores_softmax); batch strides in elements
   const float* row_lsum = nullptr; int row_lparts = 0; int64_t sl_inner = 0, sl_outer = 0;
-  // cluster shape in tiles for the 1-CTA kernel (operands shared by TMA multicast); 0 = library default
-  int cluster_m = 0, cluster_n = 0;
   // Deferred LayerNorm (see DevParams in gemm_tc.cu).
   //  producer (STORE with fp32 residual, even N): stat_out[(outer * stat_rows_outer + row) * stat_parts + inner *
   //    ceil(N / 128) + slab] = (sum, sum of squares) of the 128-column slab of the stored row; stat_parts must equal
@@ -181,7 +174,6 @@ struct TcScoresSoftmaxParams {
   bf16* P = nullptr; int64_t ldp = 0, sp_inner = 0, sp_outer = 0;
   int npad = 0;                                 // zero-fill bound (multiple of 2, >= N)
   float* lpart = nullptr; int64_t sl_inner = 0, sl_outer = 0;  // [M, csize] per batch item; required when csize > 1
-  int cluster_m = 0;                            // query-row tiles per cluster (K blocks multicast across them); 0 = default
   // deferred LayerNorm of Q (needs bias): statistics row = outer batch index * M + query row; ln_c strided like bias
   const float2* ln_stat = nullptr; int ln_parts = 0; int ln_width = 0; const float* ln_c = nullptr;
   int tag = PC_TC_OTHER;
@@ -245,7 +237,6 @@ struct Flash768Params {
   const float* const_row = nullptr;                                 // [n_seq][768] fp32, plain column order
   const float* gamma_c = nullptr; const float* beta_c = nullptr;
   bool force_rescale = false;                 // tests: take the online-softmax rescale path whenever a tile raises the maximum
-  int dbg = 0;                                 // timing experiments (wrong results): ditto_attn_self768 flags >> 8
   int tag = PC_TC_OTHER;
 };
 bool flash768_supported(int H, int heads, int T);

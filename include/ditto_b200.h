@@ -347,7 +347,8 @@ int32_t ditto_rope(const float* t, const float* pos, float* out, int64_t batch, 
  * qkv [n_seq * T, ld] bf16: q at column 0 and k at column 768 (both already rotated), v at column 1536 with its columns in
  * the order the fused QKV epilogue stores them: position 64 b + 8 kb + 2 q + e (kb < 8, q < 4, e < 2) holds column
  * 64 b + 16 (kb / 2) + 4 q + 2 (kb % 2) + e.  h [n_seq * T, 768] fp32 in/out; u_out bf16 = LayerNorm(h) gamma + beta, or NULL.
- * flags bit 0: take the online-softmax rescale path whenever a key tile raises a row maximum (tests). */
+ * flags bit 0: take the online-softmax rescale path whenever a key tile raises a row maximum (tests).  Any other flag bit
+ * set: DITTO_E_BADARG, nothing launched. */
 int32_t ditto_attn_self768(const void* qkv, int64_t ld, int64_t n_seq, int64_t T, float alpha, float* h, const float* gamma,
                            const float* beta, void* u_out, int32_t flags, void* stream);
 

@@ -312,8 +312,32 @@ def test_out_of_range_timesteps_raise(dev):
             D.DiTTOSampler(m).p_sample(x.to(dev), torch.tensor([bad]).to(dev), text.to(dev))
 
 
+REMOVED_OPTIONS = ["no_mcast", "no_fused_ln", "dbg_nostore", "cluster_m", "cluster_n", "stages_1cta", "stages_pair", "xf_prefetch",
+                   "pv_transpose", "rope_table", "no_rope_fast32", "no_pair", "generic_epi", "no_fused_attn"]
+KEPT_OPTIONS = ["no_flash", "no_flash768", "no_fused_cross", "no_cross_flash", "no_const_text", "no_fc2_ln", "flash768_quad",
+                "rope_generic", "glu_generic", "no_pv_perm4", "xf_rows", "side_streams", "defer_ln2", "no_defer_ln"]
+
+
 def test_debug_options_are_explicit(dev):
     lib = _lib.load()
     assert lib.ditto_debug_option(b"no_such_option", 1) == -1
-    _lib.debug_option("no_flash", 1)
-    _lib.debug_option("reset", 0)
+    try:
+        for name in REMOVED_OPTIONS:
+            assert lib.ditto_debug_option(name.encode(), 1) == -1, name
+        for name in KEPT_OPTIONS:
+            assert lib.ditto_debug_option(name.encode(), 0) == 0, name
+    finally:
+        _lib.debug_option("reset", 0)
+    # ditto_attn_self768 defines flag bit 0 only: any other bit is refused before a kernel is launched
+    n, T, H = 1, 64, 768
+    qkv = torch.zeros(n * T, 3 * H, dtype=torch.bfloat16, device=dev)
+    hh = torch.zeros(n * T, H, device=dev)
+    u = torch.zeros(n * T, H, dtype=torch.bfloat16, device=dev)
+    gamma, beta = torch.ones(H, device=dev), torch.zeros(H, device=dev)
+    args = (P(qkv), 3 * H, n, T, 0.125, P(hh), P(gamma), P(beta), P(u))
+    before = lib.ditto_kernel_launch_count()
+    assert lib.ditto_attn_self768(*args, 1 << 16, ST()) == -1
+    assert lib.ditto_kernel_launch_count() == before
+    _lib.check(lib.ditto_attn_self768(*args, 1, ST()), "ditto_attn_self768")   # the same buffers with a defined flag run
+    torch.cuda.synchronize()
+    assert lib.ditto_kernel_launch_count() > before

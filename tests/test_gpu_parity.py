@@ -366,7 +366,7 @@ def test_fused_blocks_under_load_match_their_compositions(dev, B, T, S, switch, 
 
 
 @pytest.mark.parametrize("env", [{"xf_rows": 88}, {"defer_ln2": 1}, {"rope_generic": 1, "glu_generic": 1}, {"no_pv_perm4": 1},
-                                 {"no_flash768": 1}, {"no_fused_ln": 1}, {"no_fc2_ln": 1}, {"flash768_quad": 1}, {"no_cross_flash": 1}],
+                                 {"no_flash768": 1}, {"no_fc2_ln": 1}, {"flash768_quad": 1}, {"no_cross_flash": 1}],
                          ids=lambda e: "+".join(f"{k}={v}" for k, v in e.items()))
 def test_kernel_variants_behind_switches(dev, env):
     """Every developer switch of DESIGN.md section 9 selects a different kernel / weight packing for the same arithmetic: each

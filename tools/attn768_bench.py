@@ -18,7 +18,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--n", type=int, default=32)
 ap.add_argument("--T", type=int, default=750)
 ap.add_argument("--iters", type=int, default=20)
-ap.add_argument("--flags", type=int, default=0)
+ap.add_argument("--flags", type=int, default=0, help="ditto_attn_self768 flags: bit 0 = always take the online-softmax rescale path")
 ap.add_argument("--noln", type=int, default=0)
 a = ap.parse_args()
 dev = torch.device("cuda:0")
