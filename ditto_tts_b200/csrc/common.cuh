@@ -14,6 +14,10 @@
 #error "libditto_b200 must be compiled for sm_100a (-gencode arch=compute_100a,code=sm_100a)"
 #endif
 
+#ifndef DITTO_F7_TRACE   // developer timeline of the flash768 kernels (F7Tr below), off by default
+#define DITTO_F7_TRACE 0
+#endif
+
 namespace ditto {
 
 typedef __nv_bfloat16 bf16;
@@ -190,6 +194,12 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
 }
+// ... on the barrier at this offset in every CTA of `mask` (cluster ranks)
+__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
+               "h"(mask)
+               : "memory");
+}
 
 // ---- cta_group::2 (one SM pair = CTAs 2k, 2k+1 of a cluster; the even CTA issues) -------------------
 constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;  // shared::cluster address of the same offset in the even CTA of the pair
@@ -201,6 +211,31 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
 }
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// shared::cluster address of the same shared-memory offset in the CTA of cluster rank `rank`
+__device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
+  return r;
+}
+// remote shared-memory store that signals the destination CTA's mbarrier with complete_tx (4 or 8 bytes): data and
+// notification travel together through the async proxy, so the sender needs no release fence (a release-scoped arrive
+// would first have to drain this thread's outstanding global stores).
+__device__ __forceinline__ void st_async_f32(uint32_t remote_addr, float v, uint32_t remote_bar) {
+  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(remote_addr),
+               "r"(__float_as_uint(v)), "r"(remote_bar)
+               : "memory");
+}
+__device__ __forceinline__ void st_async_f32x2(uint32_t remote_addr, float a, float b, uint32_t remote_bar) {
+  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v2.b32 [%0], {%1, %2}, [%3];" ::"r"(remote_addr),
+               "r"(__float_as_uint(a)), "r"(__float_as_uint(b)), "r"(remote_bar)
+               : "memory");
+}
+// shared::cta -> peer's shared memory, completion (complete_tx) on the peer's mbarrier
+__device__ __forceinline__ void bulk_copy_to_peer(uint32_t remote_dst, uint32_t local_src, uint32_t bytes, uint32_t remote_bar) {
+  asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(remote_dst),
+               "r"(local_src), "r"(bytes), "r"(remote_bar)
+               : "memory");
 }
 // TMA load into this CTA's shared memory; the bytes are counted on the PAIR LEADER's copy of `bar`
 __device__ __forceinline__ void tma_load_4d_2sm(const CUtensorMap* m, uint64_t* bar, void* smem, int c0, int c1, int c2, int c3) {
@@ -339,6 +374,19 @@ __device__ __forceinline__ void tmem_ld_16x64(uint32_t taddr, uint32_t (&r)[32])
       : "r"(taddr)
       : "memory");
 }
+__device__ __forceinline__ void tmem_st_16x64(uint32_t taddr, const uint32_t (&r)[32]) {  // inverse of tmem_ld_16x64
+  asm volatile(
+      "tcgen05.st.sync.aligned.16x256b.x8.b32 [%0], "
+      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
+      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
+        "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]), "r"(r[19]),
+        "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]), "r"(r[28]), "r"(r[29]),
+        "r"(r[30]), "r"(r[31])
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 // Register re-distribution between the warp roles of the 384-thread tcgen05 kernels (setmaxnreg): warps 0-3 shrink, the two
 // epilogue warpgroups grow.
@@ -346,6 +394,26 @@ constexpr int REGS_CTRL = 56, REGS_EPI = 224;
 static_assert(128 * REGS_CTRL + 256 * REGS_EPI <= 65536, "register re-distribution exceeds the register file");
 __device__ __forceinline__ void regs_shrink_ctrl() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_CTRL)); }
 __device__ __forceinline__ void regs_grow_epi() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_EPI)); }
+
+// Developer timeline of the two flash768 kernels (build with -DDITTO_F7_TRACE=1 through DITTO_NVCC_EXTRA;
+// tools/f7_trace.py): cluster 0 records (tag, item-relative SM clock) pairs of its MMA issuer, TMA producer and first
+// softmax warp into the buffer handed to ditto_debug_set_counters.  Compiled out by default.
+constexpr int F7_TR_MAX = 512;   // events per (CTA, role)
+constexpr int F7_TR_ROLES = 3;   // 0 MMA issuer, 1 softmax warp 0, 2 TMA producer
+struct F7Tr {
+  unsigned long long* b; int n; long long t0;
+  __device__ __forceinline__ void init(unsigned long long* buf, int rank, int role, bool on, long long t_sync) {
+    b = (DITTO_F7_TRACE && buf != nullptr && on) ? buf + (rank * F7_TR_ROLES + role) * F7_TR_MAX : nullptr; n = 0; t0 = t_sync;
+  }
+  __device__ __forceinline__ void ev(int kind, int j) {
+    if (DITTO_F7_TRACE && b != nullptr && n < F7_TR_MAX)
+      b[n++] = (static_cast<unsigned long long>(kind * 256 + (j & 255)) << 40) | (static_cast<unsigned long long>(clock64() - t0) & 0xFFFFFFFFFFull);
+  }
+  __device__ __forceinline__ void val(int kind, int j, long long v) {
+    if (DITTO_F7_TRACE && b != nullptr && n < F7_TR_MAX)
+      b[n++] = (static_cast<unsigned long long>(kind * 256 + (j & 255)) << 40) | (static_cast<unsigned long long>(v) & 0xFFFFFFFFFFull);
+  }
+};
 
 
 #endif  // __CUDACC__

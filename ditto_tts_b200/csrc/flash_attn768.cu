@@ -75,29 +75,6 @@ constexpr int F7_TMEM_COLS = 512;
 constexpr int F7_S_COL = F7_DH;       // 384
 constexpr float F7_TAU = 8.0f;        // lazy-rescale threshold, log2 units
 
-// Developer timeline (build with -DDITTO_F7_TRACE=1 through DITTO_NVCC_EXTRA; tools/f7_trace.py): cluster 0 records
-// (tag, item-relative SM clock) pairs of its MMA issuer, TMA producer and first softmax warp into the buffer handed to
-// ditto_debug_set_counters.  Compiled out by default.
-#ifndef DITTO_F7_TRACE
-#define DITTO_F7_TRACE 0
-#endif
-constexpr int F7_TR_MAX = 512;   // events per (CTA, role)
-constexpr int F7_TR_ROLES = 3;   // 0 MMA issuer, 1 softmax warp 0, 2 TMA producer
-struct F7Tr {
-  unsigned long long* b; int n; long long t0;
-  __device__ __forceinline__ void init(unsigned long long* buf, int rank, int role, bool on, long long t_sync) {
-    b = (DITTO_F7_TRACE && buf != nullptr && on) ? buf + (rank * F7_TR_ROLES + role) * F7_TR_MAX : nullptr; n = 0; t0 = t_sync;
-  }
-  __device__ __forceinline__ void ev(int kind, int j) {
-    if (DITTO_F7_TRACE && b != nullptr && n < F7_TR_MAX)
-      b[n++] = (static_cast<unsigned long long>(kind * 256 + (j & 255)) << 40) | (static_cast<unsigned long long>(clock64() - t0) & 0xFFFFFFFFFFull);
-  }
-  __device__ __forceinline__ void val(int kind, int j, long long v) {
-    if (DITTO_F7_TRACE && b != nullptr && n < F7_TR_MAX)
-      b[n++] = (static_cast<unsigned long long>(kind * 256 + (j & 255)) << 40) | (static_cast<unsigned long long>(v) & 0xFFFFFFFFFFull);
-  }
-};
-
 struct F7Dev {
   unsigned long long* trace;
   int n_seq, T;
@@ -108,50 +85,6 @@ struct F7Dev {
   bf16* u_out;                        // [n_seq * T, 768] LayerNorm(h) (nullptr: no LayerNorm stage)
   int force_rescale;                  // tests: move the reference whenever a tile raises a row maximum
 };
-
-__device__ __forceinline__ void tmem_st_16x64(uint32_t taddr, const uint32_t (&r)[32]) {  // inverse of tmem_ld_16x64
-  asm volatile(
-      "tcgen05.st.sync.aligned.16x256b.x8.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-        "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]), "r"(r[19]),
-        "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]), "r"(r[28]), "r"(r[29]),
-        "r"(r[30]), "r"(r[31])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ uint32_t f7_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void f7_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t f7_mapa(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void f7_st_async(uint32_t remote_addr, float v, uint32_t remote_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(remote_addr),
-               "r"(__float_as_uint(v)), "r"(remote_bar)
-               : "memory");
-}
-// shared::cta -> peer's shared memory, completion (complete_tx) on the peer's mbarrier
-__device__ __forceinline__ void f7_bulk_copy_to_peer(uint32_t remote_dst, uint32_t local_src, uint32_t bytes, uint32_t remote_bar) {
-  asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(remote_dst),
-               "r"(local_src), "r"(bytes), "r"(remote_bar)
-               : "memory");
-}
-// arrive (once the issued MMAs retire) on the barrier at this offset in the CTAs of `mask`
-__device__ __forceinline__ void f7_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void f7_prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
     flash_attn768_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
@@ -183,7 +116,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
 
   const int warp = warp_id_uniform();
   const int lane = threadIdx.x & 31;
-  const uint32_t rank = __shfl_sync(0xffffffffu, f7_ctarank(), 0);   // which half of the output columns / which key tiles
+  const uint32_t rank = __shfl_sync(0xffffffffu, cluster_ctarank(), 0);   // which half of the output columns / which key tiles
   const uint32_t peer = rank ^ 1u;
   const int num_clusters = gridDim.x >> 1;
   const int first = blockIdx.x >> 1;
@@ -213,7 +146,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
   if (warp == 2) tmem_alloc<F7_TMEM_COLS>(tmem_ptr);
   tcgen05_fence_before();
   __syncthreads();
-  f7_cluster_sync();   // the peer's barriers exist before the first st.async / bulk copy / commit reaches them
+  cluster_sync_all();   // the peer's barriers exist before the first st.async / bulk copy / commit reaches them
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   const long long t_sync = DITTO_F7_TRACE ? clock64() : 0;   // the cluster barrier released both CTAs at (about) the same moment
@@ -354,7 +287,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
         umma_commit(&pv_done[pvi & 3u]);
         // the tile's buffer in its OWNER is reusable once both CTAs' P.V have retired
         if (own) umma_commit(p_free);
-        else f7_commit_mc(p_free, peer_mask);
+        else umma_commit_mc(p_free, peer_mask);
       }
       __syncwarp();
       tr.ev(4, j);
@@ -376,12 +309,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
     // =========================== probability courier ===========================
     regs_shrink_ctrl();
     const bool leader = elect_one();
-    const uint32_t dst = f7_mapa(smem_u32(p_land), peer), src = smem_u32(p_own), bar = f7_mapa(smem_u32(land_full), peer);
+    const uint32_t dst = mapa_shared(smem_u32(p_land), peer), src = smem_u32(p_own), bar = mapa_shared(smem_u32(land_full), peer);
     uint32_t oc = 0;
     for (int item = first; item < p.num_items; item += num_clusters)
       for (int j = c; j < KT; j += 2, ++oc) {
         mbar_wait(p_full, oc & 1u);     // written + fence.proxy.async by the softmax warps; the peer's landing buffer is free:
-        if (leader) f7_bulk_copy_to_peer(dst, src, F7_P_BYTES, bar);   // p_free (awaited before the tile was written) includes the peer's P.V
+        if (leader) bulk_copy_to_peer(dst, src, F7_P_BYTES, bar);   // p_free (awaited before the tile was written) includes the peer's P.V
         __syncwarp();
       }
   } else if (warp >= F7_EPI_WARP0) {
@@ -431,7 +364,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
       for (int i = lane; i < 16 * (F7_DH * 4 / 128); i += 32) {
         const int r = i / (F7_DH * 4 / 128), l = i - r * (F7_DH * 4 / 128);
         if (qt * F7_BM + trow + r < p.T)
-          f7_prefetch_l2(p.h + (static_cast<long long>(seq) * p.T + qt * F7_BM + trow + r) * F7_D + col_half + l * 32);
+          prefetch_l2(p.h + (static_cast<long long>(seq) * p.T + qt * F7_BM + trow + r) * F7_D + col_half + l * 32);
       }
       float refA = 0.f, refB = 0.f;                              // softmax references (log2 domain) shared by both CTAs
       float2 lA2 = make_float2(0.f, 0.f), lB2 = make_float2(0.f, 0.f);   // row sums of the OWN tiles relative to the references
@@ -511,10 +444,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
         const float nA = (j == 0 || upA) ? mA : refA, nB = (j == 0 || upB) ? mB : refB;
         if (writer) {   // tell the peer first: its own next tile (and its accumulator) waits for this decision
           const uint32_t slot = oc & 1u;
-          const uint32_t dsta = f7_mapa(smem_u32(hdr_x + slot * F7_BM + rA), peer);
-          const uint32_t barr = f7_mapa(smem_u32(&hdr_bar[slot]), peer);
-          f7_st_async(dsta, nA, barr);
-          f7_st_async(dsta + 8 * 4, nB, barr);
+          const uint32_t dsta = mapa_shared(smem_u32(hdr_x + slot * F7_BM + rA), peer);
+          const uint32_t barr = mapa_shared(smem_u32(&hdr_bar[slot]), peer);
+          st_async_f32(dsta, nA, barr);
+          st_async_f32(dsta + 8 * 4, nB, barr);
         }
         tr.ev(12, j);
         if (__any_sync(0xffffffffu, upA || upB)) {
@@ -559,10 +492,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
       const uint32_t par = it & 1u;
       if (ew == 0 && lane == 0) mbar_expect_tx(&l_bar[par], F7_BM * 4);
       if (writer) {
-        const uint32_t dsta = f7_mapa(smem_u32(l_x + par * F7_BM + rA), peer);
-        const uint32_t barr = f7_mapa(smem_u32(&l_bar[par]), peer);
-        f7_st_async(dsta, lA, barr);
-        f7_st_async(dsta + 8 * 4, lB, barr);
+        const uint32_t dsta = mapa_shared(smem_u32(l_x + par * F7_BM + rA), peer);
+        const uint32_t barr = mapa_shared(smem_u32(&l_bar[par]), peer);
+        st_async_f32(dsta, lA, barr);
+        st_async_f32(dsta + 8 * 4, lB, barr);
       }
       // ---------------- epilogue sweep 1: h <- O / l + h (fp32, in place), row statistics, h kept in TMEM ----------------
       float4 f0[8], f1[8];   // residual of two 64-column chunks in flight (rows A: [0, 4), rows B: [4, 8))
@@ -633,12 +566,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
         const float2 pB = ln_quad_merge(ln_partial(kB, smB, sqB, 1.0f / (F7_DH / 4)), F7_DH / 4);
         if (ew == 0 && lane == 0) mbar_expect_tx(&stat_bar[par], F7_BM * 8);
         if (writer) {
-          const uint32_t slot = f7_mapa(smem_u32(stat_x + (par * F7_BM + rA) * 2), peer);
-          const uint32_t bar = f7_mapa(smem_u32(&stat_bar[par]), peer);
-          f7_st_async(slot, pA.x, bar);
-          f7_st_async(slot + 4, pA.y, bar);
-          f7_st_async(slot + 8 * 8, pB.x, bar);
-          f7_st_async(slot + 8 * 8 + 4, pB.y, bar);
+          const uint32_t slot = mapa_shared(smem_u32(stat_x + (par * F7_BM + rA) * 2), peer);
+          const uint32_t bar = mapa_shared(smem_u32(&stat_bar[par]), peer);
+          st_async_f32(slot, pA.x, bar);
+          st_async_f32(slot + 4, pA.y, bar);
+          st_async_f32(slot + 8 * 8, pB.x, bar);
+          st_async_f32(slot + 8 * 8 + 4, pB.y, bar);
         }
         mbar_wait(&stat_bar[par], (it >> 1) & 1u);
         tr.ev(18, it);
@@ -694,7 +627,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F7_THREADS, 1)
   __syncwarp();
   tcgen05_fence_before();
   __syncthreads();
-  f7_cluster_sync();   // nobody leaves while the peer may still write into this CTA / signal its barriers
+  cluster_sync_all();   // nobody leaves while the peer may still write into this CTA / signal its barriers
   if (warp == 2) {
     tcgen05_fence_after();
     tmem_dealloc<F7_TMEM_COLS>(tmem_base);

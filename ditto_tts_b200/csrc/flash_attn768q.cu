@@ -27,9 +27,6 @@
 //   warp 3   landing relay: the peer's tile has landed in THIS CTA -> arrive on the leader's land_ready
 //   warps 4-11  softmax / reference chain / epilogue, exactly as in flash_attn768.cu
 // TMEM per CTA: [0, 384) O (own 128 rows x the pair's 384 columns), [384, 512) S (own 128 rows x 128 keys).
-#include <algorithm>
-#include <mutex>
-
 #include "common.cuh"
 #include "kernels.cuh"
 
@@ -68,25 +65,6 @@ constexpr int Q7_TMEM_COLS = 512;
 constexpr int Q7_S_COL = Q7_DH;       // 384
 constexpr float Q7_TAU = 8.0f;
 
-#ifndef DITTO_F7_TRACE
-#define DITTO_F7_TRACE 0
-#endif
-constexpr int Q7_TR_MAX = 512, Q7_TR_ROLES = 3;   // developer timeline, see flash_attn768.cu (F7Tr) / tools/f7_trace.py
-struct Q7Tr {
-  unsigned long long* b; int n; long long t0;
-  __device__ __forceinline__ void init(unsigned long long* buf, int rank, int role, bool on, long long t_sync) {
-    b = (DITTO_F7_TRACE && buf != nullptr && on) ? buf + (rank * Q7_TR_ROLES + role) * Q7_TR_MAX : nullptr; n = 0; t0 = t_sync;
-  }
-  __device__ __forceinline__ void ev(int kind, int j) {
-    if (DITTO_F7_TRACE && b != nullptr && n < Q7_TR_MAX)
-      b[n++] = (static_cast<unsigned long long>(kind * 256 + (j & 255)) << 40) | (static_cast<unsigned long long>(clock64() - t0) & 0xFFFFFFFFFFull);
-  }
-  __device__ __forceinline__ void val(int kind, int j, long long v) {
-    if (DITTO_F7_TRACE && b != nullptr && n < Q7_TR_MAX)
-      b[n++] = (static_cast<unsigned long long>(kind * 256 + (j & 255)) << 40) | (static_cast<unsigned long long>(v) & 0xFFFFFFFFFFull);
-  }
-};
-
 struct Q7Dev {
   unsigned long long* trace;
   int n_seq, T;
@@ -105,34 +83,6 @@ struct Q7Dev {
   const uint8_t* const_flag; const float* gamma_c; const float* beta_c;
 };
 
-__device__ __forceinline__ void q7_tmem_st_16x64(uint32_t taddr, const uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.16x256b.x8.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-        "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]), "r"(r[19]),
-        "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]), "r"(r[28]), "r"(r[29]),
-        "r"(r[30]), "r"(r[31])
-      : "memory");
-}
-__device__ __forceinline__ void q7_tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ uint32_t q7_mapa(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void q7_st_async(uint32_t remote_addr, float v, uint32_t remote_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(remote_addr),
-               "r"(__float_as_uint(v)), "r"(remote_bar)
-               : "memory");
-}
-__device__ __forceinline__ void q7_bulk_copy_to_peer(uint32_t remote_dst, uint32_t local_src, uint32_t bytes, uint32_t remote_bar) {
-  asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(remote_dst),
-               "r"(local_src), "r"(bytes), "r"(remote_bar)
-               : "memory");
-}
-__device__ __forceinline__ void q7_prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 // first item at or after `item` (stepping over the grid) that this launch processes: the cross-attention kernel skips the
 // items of constant-text sequences, whose output the self-attention kernel has already added.  Every role walks the same
 // items, so the barrier phases (counted per processed item) agree.
@@ -234,7 +184,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
     // =========================== TMA producer ===========================
     regs_shrink_ctrl();
     const bool leader = elect_one();
-    Q7Tr tr; tr.init(p.trace, rank, 2, first == 0 && leader, t_sync);
+    F7Tr tr; tr.init(p.trace, rank, 2, first == 0 && leader, t_sync);
     int stage = 0;
     uint32_t phase = 0;
     for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items; item = q7_next_item<CROSS>(p, item + num_clusters, num_clusters)) {
@@ -294,7 +244,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
       int stage = 0;
       uint32_t phase = 0;
       uint32_t it = 0, sc = 0, oc = 0, rc = 0, pvi = 0;
-      Q7Tr tr; tr.init(p.trace, rank, 0, first == 0 && leader, t_sync);
+      F7Tr tr; tr.init(p.trace, rank, 0, first == 0 && leader, t_sync);
       auto issue_s = [&]() {
         mbar_wait(s_empty, (sc & 1u) ^ 1u);
         tcgen05_fence_after();
@@ -383,12 +333,12 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
     // =========================== probability courier ===========================
     regs_shrink_ctrl();
     const bool leader = elect_one();
-    const uint32_t dst = q7_mapa(smem_u32(p_land), peer), src = smem_u32(p_own), bar = q7_mapa(smem_u32(land_full), peer);
+    const uint32_t dst = mapa_shared(smem_u32(p_land), peer), src = smem_u32(p_own), bar = mapa_shared(smem_u32(land_full), peer);
     uint32_t oc = 0;
     for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items; item = q7_next_item<CROSS>(p, item + num_clusters, num_clusters))
       for (int j = c; j < KT; j += 2, ++oc) {
         mbar_wait(p_ready, oc & 1u);   // written + fence.proxy.async by this CTA's softmax warps; the peer's landing buffer is
-        if (leader) q7_bulk_copy_to_peer(dst, src, Q7_P_BYTES, bar);   // free: p_free (awaited before the tile was written)
+        if (leader) bulk_copy_to_peer(dst, src, Q7_P_BYTES, bar);   // free: p_free (awaited before the tile was written)
         __syncwarp();                                                  // includes the peer pair's P.V of the previous tile
       }
   } else if (warp == 3) {
@@ -416,7 +366,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
     const bool writer = q == 0;
     const int col_half = c * Q7_DH;
     uint32_t it = 0, sc = 0, oc = 0, rc = 0, pvc = 0;
-    Q7Tr tr; tr.init(p.trace, rank, 1, first == 0 && ew == 0 && lane == 0, t_sync);
+    F7Tr tr; tr.init(p.trace, rank, 1, first == 0 && ew == 0 && lane == 0, t_sync);
     auto rescale_o = [&](float fA, float fB) {
       tr.ev(25, static_cast<int>(pvc));
       mbar_wait(&pv_done[(pvc - 1) & 3u], ((pvc - 1) >> 2) & 1u);
@@ -433,9 +383,9 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
           o[4 * kb + 2] = __float_as_uint(__uint_as_float(o[4 * kb + 2]) * fB);
           o[4 * kb + 3] = __float_as_uint(__uint_as_float(o[4 * kb + 3]) * fB);
         }
-        q7_tmem_st_16x64(t_lane + cb * 64, o);
+        tmem_st_16x64(t_lane + cb * 64, o);
       }
-      q7_tmem_st_wait();
+      tmem_st_wait();
       tcgen05_fence_before();
     };
     for (int item = q7_next_item<CROSS>(p, first, num_clusters); item < p.num_items;
@@ -466,7 +416,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
         for (int i = lane; i < 16 * (Q7_DH * 4 / 128); i += 32) {
           const int r = i / (Q7_DH * 4 / 128), l = i - r * (Q7_DH * 4 / 128);
           if (row0 + trow + r < p.T)
-            q7_prefetch_l2(p.h + (static_cast<long long>(seq) * p.T + row0 + trow + r) * Q7_D + col_half + l * 32);
+            prefetch_l2(p.h + (static_cast<long long>(seq) * p.T + row0 + trow + r) * Q7_D + col_half + l * 32);
         }
       };
       if (c >= KT) prefetch_residual();
@@ -564,10 +514,10 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
         const float nA = (j == 0 || upA) ? mA : refA, nB = (j == 0 || upB) ? mB : refB;
         if (writer) {
           const uint32_t slot = oc & 1u;
-          const uint32_t dsta = q7_mapa(smem_u32(hdr_x + slot * Q7_BM + rA), peer);
-          const uint32_t barr = q7_mapa(smem_u32(&hdr_bar[slot]), peer);
-          q7_st_async(dsta, nA, barr);
-          q7_st_async(dsta + 8 * 4, nB, barr);
+          const uint32_t dsta = mapa_shared(smem_u32(hdr_x + slot * Q7_BM + rA), peer);
+          const uint32_t barr = mapa_shared(smem_u32(&hdr_bar[slot]), peer);
+          st_async_f32(dsta, nA, barr);
+          st_async_f32(dsta + 8 * 4, nB, barr);
         }
         tr.ev(12, j);
         if (__any_sync(0xffffffffu, upA || upB)) {
@@ -615,10 +565,10 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
       const uint32_t par = it & 1u;
       if (ew == 0 && lane == 0) mbar_expect_tx(&l_bar[par], Q7_BM * 4);
       if (writer) {
-        const uint32_t dsta = q7_mapa(smem_u32(l_x + par * Q7_BM + rA), peer);
-        const uint32_t barr = q7_mapa(smem_u32(&l_bar[par]), peer);
-        q7_st_async(dsta, lA, barr);
-        q7_st_async(dsta + 8 * 4, lB, barr);
+        const uint32_t dsta = mapa_shared(smem_u32(l_x + par * Q7_BM + rA), peer);
+        const uint32_t barr = mapa_shared(smem_u32(&l_bar[par]), peer);
+        st_async_f32(dsta, lA, barr);
+        st_async_f32(dsta + 8 * 4, lB, barr);
       }
       // ---------------- epilogue sweep 1: h <- O / l + h, row statistics, h kept in TMEM ----------------
       float4 f0[8], f1[8], f2[8];   // residual of three 64-column chunks in flight (rows A: [0, 4), rows B: [4, 8))
@@ -685,7 +635,7 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
           o[4 * k0 + 2] = __float_as_uint(vB.x); o[4 * k0 + 3] = __float_as_uint(vB.y);
           o[4 * k1 + 2] = __float_as_uint(vB.z); o[4 * k1 + 3] = __float_as_uint(vB.w);
         }
-        if (p.u_out != nullptr) q7_tmem_st_16x64(t_lane + cb * 64, o);
+        if (p.u_out != nullptr) tmem_st_16x64(t_lane + cb * 64, o);
         tr.ev(22, cb);
       };
       static_assert(Q7_DH / 64 == 6, "two rounds of three chunks");
@@ -697,18 +647,18 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
       sweep1(5, f2);
       tr.ev(17, it);
       if (p.u_out != nullptr) {
-        q7_tmem_st_wait();
+        tmem_st_wait();
         // partials (mean, M2) of this CTA's 384 columns; the peer's are merged in below
         const float2 pA = ln_quad_merge(ln_partial(kA, smA, sqA, 1.0f / (Q7_DH / 4)), Q7_DH / 4);
         const float2 pB = ln_quad_merge(ln_partial(kB, smB, sqB, 1.0f / (Q7_DH / 4)), Q7_DH / 4);
         if (ew == 0 && lane == 0) mbar_expect_tx(&stat_bar[par], Q7_BM * 8);
         if (writer) {
-          const uint32_t slot = q7_mapa(smem_u32(stat_x + (par * Q7_BM + rA) * 2), peer);
-          const uint32_t bar = q7_mapa(smem_u32(&stat_bar[par]), peer);
-          q7_st_async(slot, pA.x, bar);
-          q7_st_async(slot + 4, pA.y, bar);
-          q7_st_async(slot + 8 * 8, pB.x, bar);
-          q7_st_async(slot + 8 * 8 + 4, pB.y, bar);
+          const uint32_t slot = mapa_shared(smem_u32(stat_x + (par * Q7_BM + rA) * 2), peer);
+          const uint32_t bar = mapa_shared(smem_u32(&stat_bar[par]), peer);
+          st_async_f32(slot, pA.x, bar);
+          st_async_f32(slot + 4, pA.y, bar);
+          st_async_f32(slot + 8 * 8, pB.x, bar);
+          st_async_f32(slot + 8 * 8 + 4, pB.y, bar);
         }
         mbar_wait(&stat_bar[par], (it >> 1) & 1u);
         tr.ev(18, it);
@@ -786,44 +736,14 @@ __global__ void __launch_bounds__(Q7_THREADS, 1)
   }
 }
 
-std::mutex g_q7_mutex;
-
 }  // namespace
 
 // The four-CTA kernel pays when 256-row query tiles do not pad much more than 128-row tiles would (T = 750: 768 = 768).
 bool flash768_quad_preferred(int T) { return round_up(T, 2 * Q7_BM) * 100 <= round_up(T, Q7_BM) * 120; }
 
-// co-resident four-CTA clusters on the current device (queried once per device); <= 0: cannot be scheduled
-static int q7_clusters(DeviceState* ds) {
-  std::lock_guard<std::mutex> lock(g_q7_mutex);
-  if (ds->f768q_clusters == 0) {
-    int n = 0;
-    if (cudaFuncSetAttribute(flash_attn768q_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q7_SMEM_BYTES) == cudaSuccess &&
-        cudaFuncSetAttribute(flash_attn768q_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q7_SMEM_BYTES) == cudaSuccess &&
-        cudaFuncSetAttribute(flash_attn768q_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Q7_SMEM_BYTES) == cudaSuccess) {
-      cudaLaunchConfig_t cfg = {};
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = 4;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.blockDim = dim3(Q7_THREADS, 1, 1);
-      cfg.dynamicSmemBytes = Q7_SMEM_BYTES;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      cfg.gridDim = dim3(static_cast<unsigned>(4 * std::max(ds->num_sms, 4)), 1, 1);
-      if (cudaOccupancyMaxActiveClusters(&n, flash_attn768q_kernel<false>, &cfg) != cudaSuccess) n = 0;
-    }
-    (void)cudaGetLastError();
-    ds->f768q_clusters = n > 0 ? n : -1;
-  }
-  return ds->f768q_clusters;
-}
-
 bool flash768_quad_schedulable() {
   if (tc_gemm_init() != 0) return false;
-  DeviceState* ds = device_state();
-  return ds != nullptr && q7_clusters(ds) > 0;
+  return max_active_clusters(reinterpret_cast<const void*>(flash_attn768q_kernel<false>), 4, Q7_THREADS, Q7_SMEM_BYTES) > 0;
 }
 
 int launch_flash768_quad(const Flash768Params& q, cudaStream_t st) {
@@ -840,21 +760,11 @@ int launch_flash768_quad(const Flash768Params& q, cudaStream_t st) {
                 DITTO_E_BADARG, "flash768 (constant text): 16-byte aligned constant rows, norm3 and a LayerNorm output");
   DITTO_REQUIRE((reinterpret_cast<uintptr_t>(q.h) & 15) == 0 && (reinterpret_cast<uintptr_t>(q.u_out) & 7) == 0, DITTO_E_BADARG,
                 "flash768: h must be 16-byte, u 8-byte aligned");
-  DeviceState* ds = device_state();
-  if (ds == nullptr) return DITTO_E_CUDA;
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 4;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.blockDim = dim3(Q7_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = Q7_SMEM_BYTES;
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  const int max_clusters = q7_clusters(ds);
-  DITTO_REQUIRE(max_clusters > 0, DITTO_E_UNSUPPORTED, "flash768: four-CTA clusters cannot be scheduled on this device");
+  const void* fn = !cross ? (q.const_flag ? reinterpret_cast<const void*>(flash_attn768q_kernel<false, true>)
+                                          : reinterpret_cast<const void*>(flash_attn768q_kernel<false>))
+                          : reinterpret_cast<const void*>(flash_attn768q_kernel<true>);
+  DITTO_REQUIRE(max_active_clusters(fn, 4, Q7_THREADS, Q7_SMEM_BYTES) > 0, DITTO_E_UNSUPPORTED,
+                "flash768: four-CTA clusters cannot be scheduled on this device");
   TcOperand Q, K, V;
   Q.ptr = q.qkv; Q.rows = q.T; Q.cols = Q7_D; Q.ld = q.ld; Q.s_outer = static_cast<int64_t>(q.T) * q.ld;
   K = Q; K.ptr = q.qkv + Q7_D;
@@ -887,15 +797,8 @@ int launch_flash768_quad(const Flash768Params& q, cudaStream_t st) {
   const double rows = n_run * q.T;
   ProfScope prof(q.tag, st, 4.0 * q.T * static_cast<double>(p.Tk) * Q7_D * n_run,
                  rows * Q7_D * ((cross ? 2.0 : 6.0) + 8.0 + (q.u_out ? 2.0 : 0.0)) + (cross ? 4.0 * n_run * static_cast<double>(p.Tk) * Q7_D : 0.0));
-  const int clusters = static_cast<int>(std::min<int64_t>(max_clusters, items));
-  cfg.gridDim = dim3(static_cast<unsigned>(4 * clusters), 1, 1);
   void* args[4] = {&mq, &mk, &mv, &p};
-  const void* fn = cross ? reinterpret_cast<const void*>(flash_attn768q_kernel<true>)
-                 : q.const_flag ? reinterpret_cast<const void*>(flash_attn768q_kernel<false, true>)
-                                : reinterpret_cast<const void*>(flash_attn768q_kernel<false>);
-  DITTO_CUDA(cudaLaunchKernelExC(&cfg, fn, args));
-  count_launch();
-  return 0;
+  return launch_clusters(fn, 4, Q7_THREADS, Q7_SMEM_BYTES, items, args, st);
 }
 
 }  // namespace ditto

@@ -18,11 +18,6 @@
 // half of the B tile, 6-stage TMA ring, persistent over row blocks: cluster c takes row blocks c, c + #clusters, ...
 // Weight rows are packed in the `perm4` order (accumulator column 8 kb + 2 q + e of a 64-column block = output column
 // 16 (kb / 2) + 4 q + 2 (kb % 2) + e), so a thread owns four consecutive outputs: 16-byte residual accesses, 8-byte bf16 stores.
-#include <algorithm>
-#include <map>
-#include <mutex>
-#include <tuple>
-
 #include "common.cuh"
 #include "kernels.cuh"
 
@@ -55,29 +50,6 @@ struct RlDev {
   bf16* u; long long ldu;            // [M, N] bf16 output (may be nullptr when gamma == nullptr)
   float inv_n;
 };
-
-__device__ __forceinline__ void rl_tmem_st_16x64(uint32_t taddr, const uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.16x256b.x8.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-        "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]), "r"(r[18]), "r"(r[19]),
-        "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]), "r"(r[27]), "r"(r[28]), "r"(r[29]),
-        "r"(r[30]), "r"(r[31])
-      : "memory");
-}
-__device__ __forceinline__ void rl_tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ uint32_t rl_mapa(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void rl_st_async2(uint32_t remote_addr, float a, float b, uint32_t remote_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v2.b32 [%0], {%1, %2}, [%3];" ::"r"(remote_addr),
-               "r"(__float_as_uint(a)), "r"(__float_as_uint(b)), "r"(remote_bar)
-               : "memory");
-}
 
 __global__ void __launch_bounds__(RL_THREADS, 1)
     tc_gemm_resid_ln_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, const RlDev p) {
@@ -271,14 +243,14 @@ __global__ void __launch_bounds__(RL_THREADS, 1)
             if (okB) *reinterpret_cast<uint2*>(ua + 8 * p.ldu) = make_uint2(pack_bf16x2(vB.x, vB.y), pack_bf16x2(vB.z, vB.w));
           }
         }
-        if (norm) rl_tmem_st_16x64(t_lane + (static_cast<uint32_t>(16 * hh) << 16) + cb * 64, o);
+        if (norm) tmem_st_16x64(t_lane + (static_cast<uint32_t>(16 * hh) << 16) + cb * 64, o);
       };
       sweep1(0, 0, f0); load_res(1, 0, f0);
       sweep1(0, 1, f1); load_res(1, 1, f1);
       sweep1(1, 0, f0);
       sweep1(1, 1, f1);
       if (norm) {
-        rl_tmem_st_wait();
+        tmem_st_wait();
         // this warp's slab partials (mean, M2) of its 32 rows -> every CTA that holds columns of these rows (same a, every pair)
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
@@ -290,9 +262,9 @@ __global__ void __launch_bounds__(RL_THREADS, 1)
           const uint32_t bar = smem_u32(&stat_bar[par]);
           for (int pr = 0; pr < p.n_tiles; ++pr) {
             const uint32_t dst_rank = static_cast<uint32_t>(2 * pr + a);
-            const uint32_t rs = rl_mapa(slot, dst_rank), rb = rl_mapa(bar, dst_rank);
+            const uint32_t rs = mapa_shared(slot, dst_rank), rb = mapa_shared(bar, dst_rank);
 #pragma unroll
-            for (int i = 0; i < 4; ++i) rl_st_async2(rs + i * 8 * 8, sm[i], sq[i], rb);
+            for (int i = 0; i < 4; ++i) st_async_f32x2(rs + i * 8 * 8, sm[i], sq[i], rb);
           }
         }
         mbar_wait(&stat_bar[par], (it >> 1) & 1u);
@@ -369,9 +341,6 @@ __global__ void __launch_bounds__(RL_THREADS, 1)
   }
 }
 
-std::mutex g_rl_mutex;
-std::map<std::pair<int, int>, int> g_rl_clusters;   // (device, cluster size) -> co-resident clusters
-
 }  // namespace
 
 bool gemm_resid_ln_supported(int N, int K) { return N > 0 && N % RL_BN == 0 && N / RL_BN <= RL_MAX_NT && K > 0 && K % 8 == 0; }
@@ -383,38 +352,9 @@ int gemm_resid_ln_weight_row(int r) {
   return blk * 64 + 16 * (kb / 2) + 4 * q + 2 * (kb % 2) + e;
 }
 
-// co-resident clusters of `csize` CTAs on the current device (queried once per device and size); <= 0: cannot be scheduled
-static int rl_clusters(int csize) {
-  DeviceState* ds = device_state();
-  int dev_id = 0;
-  if (ds == nullptr || cudaGetDevice(&dev_id) != cudaSuccess) return -1;
-  std::lock_guard<std::mutex> lock(g_rl_mutex);
-  auto key = std::make_pair(dev_id, csize);
-  auto it = g_rl_clusters.find(key);
-  if (it == g_rl_clusters.end()) {
-    int n = 0;
-    if (cudaFuncSetAttribute(tc_gemm_resid_ln_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RL_SMEM_BYTES) == cudaSuccess) {
-      cudaLaunchConfig_t cfg = {};
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = static_cast<unsigned>(csize);
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.blockDim = dim3(RL_THREADS, 1, 1);
-      cfg.dynamicSmemBytes = RL_SMEM_BYTES;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      cfg.gridDim = dim3(static_cast<unsigned>(csize * std::max(ds->num_sms, 1)), 1, 1);
-      if (cudaOccupancyMaxActiveClusters(&n, tc_gemm_resid_ln_kernel, &cfg) != cudaSuccess) n = 0;
-    }
-    (void)cudaGetLastError();
-    it = g_rl_clusters.emplace(key, n > 0 ? n : -1).first;
-  }
-  return it->second;
-}
-
 bool gemm_resid_ln_schedulable(int N) {
-  return N > 0 && N % RL_BN == 0 && N / RL_BN <= RL_MAX_NT && tc_gemm_init() == 0 && rl_clusters(2 * (N / RL_BN)) > 0;
+  return N > 0 && N % RL_BN == 0 && N / RL_BN <= RL_MAX_NT && tc_gemm_init() == 0 &&
+         max_active_clusters(reinterpret_cast<const void*>(tc_gemm_resid_ln_kernel), 2 * (N / RL_BN), RL_THREADS, RL_SMEM_BYTES) > 0;
 }
 
 int launch_gemm_resid_ln(const GemmResidLnParams& q, cudaStream_t st) {
@@ -428,10 +368,6 @@ int launch_gemm_resid_ln(const GemmResidLnParams& q, cudaStream_t st) {
                     (reinterpret_cast<uintptr_t>(q.u) & 7) == 0 && (reinterpret_cast<uintptr_t>(q.bias) & 15) == 0 &&
                     (reinterpret_cast<uintptr_t>(q.gamma) & 15) == 0 && (reinterpret_cast<uintptr_t>(q.beta) & 15) == 0,
                 DITTO_E_BADARG, "gemm_resid_ln: h / bias / gamma / beta must be 16-byte aligned with strides that keep rows aligned");
-  DeviceState* ds = device_state();
-  if (ds == nullptr) return DITTO_E_CUDA;
-  int dev_id = 0;
-  DITTO_CUDA(cudaGetDevice(&dev_id));
   RlDev p;
   p.M = q.M; p.N = q.N; p.K = q.K;
   p.n_tiles = q.N / RL_BN;
@@ -441,19 +377,9 @@ int launch_gemm_resid_ln(const GemmResidLnParams& q, cudaStream_t st) {
   p.resid = q.resid; p.ldr = q.ldr; p.resid_mod = static_cast<int>(q.resid_mod);
   p.inv_n = 1.0f / static_cast<float>(q.N);
   const int csize = 2 * p.n_tiles;
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = static_cast<unsigned>(csize);
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.blockDim = dim3(RL_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = RL_SMEM_BYTES;
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  int clusters = rl_clusters(csize);
-  DITTO_REQUIRE(clusters > 0, DITTO_E_UNSUPPORTED, "gemm_resid_ln: this cluster size cannot be scheduled on the device");
+  const void* fn = reinterpret_cast<const void*>(tc_gemm_resid_ln_kernel);
+  DITTO_REQUIRE(max_active_clusters(fn, csize, RL_THREADS, RL_SMEM_BYTES) > 0, DITTO_E_UNSUPPORTED,
+                "gemm_resid_ln: this cluster size cannot be scheduled on the device");
   TcOperand A, B;
   A.ptr = q.A; A.rows = q.M; A.cols = q.K; A.ld = q.lda;
   B.ptr = q.W; B.rows = q.N; B.cols = q.K; B.ld = q.ldw;
@@ -463,12 +389,8 @@ int launch_gemm_resid_ln(const GemmResidLnParams& q, cudaStream_t st) {
   const double rows = static_cast<double>(q.M);
   ProfScope prof(q.tag, st, 2.0 * rows * q.N * static_cast<double>(q.K),
                  rows * (2.0 * q.K + q.N * (8.0 + (q.u ? 2.0 : 0.0))) + 2.0 * q.N * static_cast<double>(q.K));
-  clusters = static_cast<int>(std::min<int64_t>(clusters, p.m_pairs));
-  cfg.gridDim = dim3(static_cast<unsigned>(csize * clusters), 1, 1);
   void* args[3] = {&ma, &mb, &p};
-  DITTO_CUDA(cudaLaunchKernelExC(&cfg, reinterpret_cast<const void*>(tc_gemm_resid_ln_kernel), args));
-  count_launch();
-  return 0;
+  return launch_clusters(fn, csize, RL_THREADS, RL_SMEM_BYTES, p.m_pairs, args, st);
 }
 
 }  // namespace ditto

@@ -1075,11 +1075,6 @@ __device__ __forceinline__ void tma_load_4d_mc(const CUtensorMap* m, uint64_t* b
       "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(mask)
       : "memory");
 }
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
 
 // Register re-distribution between the warp roles (setmaxnreg, one instruction per warpgroup): warps 0-3 (TMA producer,
 // MMA issuer, TMEM allocator, idle) shrink to 56 registers, the two epilogue warpgroups grow from the launch-bound limit
@@ -1439,19 +1434,6 @@ struct SmDev {
   const float2* ln_stat; int ln_parts; float ln_inv_h; const float* ln_c;
 };
 
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-// remote shared-memory store that signals the destination CTA's mbarrier with complete_tx (4 bytes): data and
-// notification travel together through the async proxy, so the sender needs no release fence (a release-scoped arrive
-// would first have to drain this thread's outstanding global stores of P).
-__device__ __forceinline__ void st_async_f32(uint32_t remote_addr, float v, uint32_t remote_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];"
-               ::"r"(remote_addr), "r"(__float_as_uint(v)), "r"(remote_bar)
-               : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_nctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
@@ -1813,6 +1795,7 @@ unsigned long long* g_dbg = nullptr;
 constexpr int kMaxDevices = 64;
 DeviceState g_dev_state[kMaxDevices];
 std::mutex g_dev_mutex;
+std::map<std::tuple<int, const void*, int>, int> g_max_clusters;  // (device, kernel, cluster size) -> max_active_clusters
 
 struct MapKey {
   uint64_t v[9];
@@ -1878,53 +1861,6 @@ int set_attr() {
 }
 
 
-// Launch a persistent 1-CTA kernel as clusters of `csize` CTAs (csize == 1: plain launch): grid = csize x min(work items,
-// co-resident clusters).  The co-residency query is cached per (kernel, cluster size).
-std::map<std::tuple<int, const void*, int>, int> g_max_clusters;  // (device, kernel, cluster size)
-template <typename Params>
-int launch_clustered(const void* func, int csize, int smem_bytes, int64_t num_work, const CUtensorMap& ma, const CUtensorMap& mb,
-                     const Params& p, cudaStream_t st) {
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[1];
-  cfg.blockDim = dim3(NUM_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = 0;
-  DeviceState* ds = device_state();
-  if (ds == nullptr) return DITTO_E_CUDA;
-  const int num_sms = ds->num_sms;
-  int dev_id = 0;
-  DITTO_CUDA(cudaGetDevice(&dev_id));
-  int clusters = num_sms;
-  if (csize > 1) {
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = static_cast<unsigned>(csize);
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.numAttrs = 1;
-    std::lock_guard<std::mutex> lock(g_dev_mutex);
-    auto key = std::make_tuple(dev_id, func, csize);
-    auto it = g_max_clusters.find(key);
-    if (it == g_max_clusters.end()) {
-      if (csize > 8) (void)cudaFuncSetAttribute(func, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-      cfg.gridDim = dim3(static_cast<unsigned>(csize * num_sms), 1, 1);
-      int n = 0;
-      cudaError_t e = cudaOccupancyMaxActiveClusters(&n, func, &cfg);
-      if (e != cudaSuccess) { (void)cudaGetLastError(); n = 0; }
-      it = g_max_clusters.emplace(key, n > 0 ? n : -1).first;
-    }
-    DITTO_REQUIRE(it->second > 0, DITTO_E_UNSUPPORTED, "tc_gemm: this cluster size cannot be scheduled on the device");
-    clusters = it->second;
-  }
-  clusters = static_cast<int>(std::min<int64_t>(clusters, num_work));
-  cfg.gridDim = dim3(static_cast<unsigned>(clusters * csize), 1, 1);
-  void* args[3] = {const_cast<CUtensorMap*>(&ma), const_cast<CUtensorMap*>(&mb), const_cast<Params*>(&p)};
-  DITTO_CUDA(cudaLaunchKernelExC(&cfg, func, args));
-  count_launch();
-  return 0;
-}
-
 }  // namespace
 
 void tc_gemm_set_debug_counters(unsigned long long* dev_ptr) { g_dbg = dev_ptr; }
@@ -1944,6 +1880,58 @@ DeviceState* device_state() {
     return nullptr;
   }
   return &g_dev_state[dev];
+}
+
+int max_active_clusters(const void* func, int csize, int threads, int smem_bytes) {
+  DeviceState* ds = device_state();
+  int dev = 0;
+  if (ds == nullptr || cudaGetDevice(&dev) != cudaSuccess) return -1;
+  std::lock_guard<std::mutex> lock(g_dev_mutex);
+  const auto key = std::make_tuple(dev, func, csize);
+  auto it = g_max_clusters.find(key);
+  if (it == g_max_clusters.end()) {
+    int n = 0;
+    if (cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes) == cudaSuccess &&
+        (csize <= 8 || cudaFuncSetAttribute(func, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess)) {
+      cudaLaunchAttribute attr;
+      attr.id = cudaLaunchAttributeClusterDimension;
+      attr.val.clusterDim.x = static_cast<unsigned>(csize);
+      attr.val.clusterDim.y = 1;
+      attr.val.clusterDim.z = 1;
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3(static_cast<unsigned>(csize * std::max(ds->num_sms, 1)), 1, 1);
+      cfg.blockDim = dim3(static_cast<unsigned>(threads), 1, 1);
+      cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
+      cfg.attrs = &attr;
+      cfg.numAttrs = 1;
+      if (cudaOccupancyMaxActiveClusters(&n, func, &cfg) != cudaSuccess) n = 0;
+    }
+    (void)cudaGetLastError();   // a failed set-up or query must not surface at the next launch check
+    it = g_max_clusters.emplace(key, n > 0 ? n : -1).first;
+  }
+  return it->second;
+}
+
+int launch_clusters(const void* func, int csize, int threads, int smem_bytes, int64_t work_items, void** args, cudaStream_t st) {
+  DeviceState* ds = device_state();
+  if (ds == nullptr) return DITTO_E_CUDA;
+  const int capacity = csize == 1 ? ds->num_sms : max_active_clusters(func, csize, threads, smem_bytes);
+  DITTO_REQUIRE(capacity > 0, DITTO_E_UNSUPPORTED, "tc_gemm: this cluster size cannot be scheduled on the device");
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = static_cast<unsigned>(csize);
+  attr.val.clusterDim.y = 1;
+  attr.val.clusterDim.z = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(static_cast<unsigned>(csize * std::min<int64_t>(capacity, work_items)), 1, 1);
+  cfg.blockDim = dim3(static_cast<unsigned>(threads), 1, 1);
+  cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
+  cfg.stream = st;
+  cfg.attrs = &attr;
+  cfg.numAttrs = csize > 1 ? 1 : 0;
+  DITTO_CUDA(cudaLaunchKernelExC(&cfg, func, args));
+  count_launch();
+  return 0;
 }
 
 // Per device: kernel attributes (dynamic shared memory opt-in, non-portable cluster sizes) and the SM count belong to the
@@ -2120,7 +2108,8 @@ int launch_tc_gemm(const TcGemmParams& q, cudaStream_t st) {
   }
   // no cluster: TMA multicast of the operands across CTAs of adjacent tiles was measured on B200 (profiles/README.md) and
   // lost -- for these epilogue-heavy batched attention GEMMs the lock-step coupling costs more than the saved L2 traffic
-  return launch_clustered(func, 1, SMEM_BYTES, tiles, ma, mb, p, st);
+  void* args[3] = {&ma, &mb, &p};
+  return launch_clusters(func, 1, NUM_THREADS, SMEM_BYTES, tiles, args, st);
 }
 #undef DITTO_LAUNCH_PAIR
 #undef DITTO_FUNC_1CTA
@@ -2171,7 +2160,8 @@ int launch_tc_scores_softmax(const TcScoresSoftmaxParams& q, cudaStream_t st) {
   ProfScope prof(q.tag, st, 2.0 * q.M * q.N * q.K * q.batch_inner * q.batch_outer, 0.0);
   const void* func = q.bias != nullptr ? reinterpret_cast<const void*>(&tc_scores_softmax_kernel<true>)
                                        : reinterpret_cast<const void*>(&tc_scores_softmax_kernel<false>);
-  return launch_clustered(func, csize, SM_SMEM_BYTES, items, ma, mb, p, st);
+  void* args[3] = {&ma, &mb, &p};
+  return launch_clusters(func, csize, NUM_THREADS, SM_SMEM_BYTES, items, args, st);
 }
 
 }  // namespace ditto

@@ -29,9 +29,15 @@ extern DebugOptions g_opt;
 struct DeviceState {
   bool tc_init = false, xf_attr = false, fa_attr = false, f768_attr = false;
   int num_sms = 0;
-  int f768q_clusters = 0;   // co-resident four-CTA clusters of flash_attn768q_kernel (0: not queried yet, -1: cannot be scheduled)
 };
 DeviceState* device_state();  // state of the CURRENT device (nullptr + error set when cudaGetDevice fails)
+// Co-resident clusters of `csize` CTAs (`threads` threads, `smem_bytes` of dynamic shared memory each) of the kernel `func`
+// on the current device, queried once per (device, kernel, cluster size); sets the kernel's shared-memory attribute.
+// <= 0: clusters of this size cannot be scheduled.
+int max_active_clusters(const void* func, int csize, int threads, int smem_bytes);
+// Persistent launch of `func` (the kernel strides over its work items by the number of clusters): grid = csize x
+// min(co-resident clusters, work_items); csize == 1 is a plain launch of one CTA per SM.  args: the kernel's parameters.
+int launch_clusters(const void* func, int csize, int threads, int smem_bytes, int64_t work_items, void** args, cudaStream_t st);
 
 // ---- elementwise.cu ----------------------------------------------------------------------------------
 int launch_cast_bf16(const float* x, bf16* y, int64_t n, cudaStream_t st);
