@@ -54,6 +54,7 @@ SIGNATURES = {
     "ditto_text_context_bytes": (_I64, [_P, _I64, _I64]),
     "ditto_workspace_bytes": (_I64, [_P, _I64, _I64, _I64]),
     "ditto_text_context": (_I32, [_P, _P, _I64, _I64, _P, _P, _I64, _P]),
+    "ditto_text_context_masked": (_I32, [_P, _P, _I64, _I64, C.POINTER(_I64), _P, _P, _I64, _P]),
     "ditto_forward": (_I32, [_P, _P, _I64, _P, _P, _I64, _I64, _I64, _P, _P, _I64, _P]),
     "ditto_cfg_ddpm_update": (_I32, [_P, _P, _P, _P, _P, _P, _F, _P, _I64, _I64, _P]),
     "ditto_p_sample": (_I32, [_P, _P, _P, _P, _P, _I32, _F, _I64, _I64, _I64, _P, _P, _P, _I64, _P]),

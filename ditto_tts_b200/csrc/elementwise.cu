@@ -35,6 +35,50 @@ int launch_cast_bf16(const float* x, bf16* y, int64_t n, cudaStream_t st) {
   return 0;
 }
 
+// masked text staging: text [n, S, D] fp32 -> y (bf16 or fp32) with the rows s >= len[seq] zeroed, so that whatever the caller
+// left in them (NaN / Inf included) gives finite K / V rows, which the zero probabilities of the masked keys then cancel
+template <typename OutT>
+__global__ void stage_text_kernel(const float* __restrict__ x, OutT* __restrict__ y, const int* __restrict__ len, int S, int D,
+                                  int64_t n) {
+  for (int64_t i = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) * 4; i < n;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x * 4) {
+    const int64_t row = i / D;
+    const bool keep = static_cast<int>(row % S) < __ldg(len + row / S);
+    const float4 v = keep ? *reinterpret_cast<const float4*>(x + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+    if constexpr (sizeof(OutT) == 2) {
+      uint2 o;
+      o.x = pack_bf16x2(v.x, v.y);
+      o.y = pack_bf16x2(v.z, v.w);
+      *reinterpret_cast<uint2*>(y + i) = o;
+    } else {
+      *reinterpret_cast<float4*>(y + i) = v;
+    }
+  }
+}
+
+int launch_stage_text(const float* x, void* y, bool y_bf16, const int* len, int64_t n_seq, int S, int D, cudaStream_t st) {
+  DITTO_REQUIRE(D % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(y) & 15) == 0,
+                DITTO_E_BADARG, "stage_text: needs D % 4 == 0 and 16-byte aligned buffers");
+  const int64_t n = n_seq * S * D;
+  if (n <= 0) return 0;
+  const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(ceil_div(n, 4 * 256), 148 * 16));
+  if (y_bf16) stage_text_kernel<bf16><<<blocks, 256, 0, st>>>(x, static_cast<bf16*>(y), len, S, D, n);
+  else stage_text_kernel<float><<<blocks, 256, 0, st>>>(x, static_cast<float*>(y), len, S, D, n);
+  DITTO_LAUNCH_CHECK();
+  return 0;
+}
+
+__global__ void fill_i32_kernel(int* __restrict__ y, int v, int64_t n) {
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += static_cast<int64_t>(gridDim.x) * blockDim.x)
+    y[i] = v;
+}
+int launch_fill_i32(int* y, int v, int64_t n, cudaStream_t st) {
+  if (n <= 0) return 0;
+  fill_i32_kernel<<<static_cast<unsigned>(std::min<int64_t>(ceil_div(n, 256), 148)), 256, 0, st>>>(y, v, n);
+  DITTO_LAUNCH_CHECK();
+  return 0;
+}
+
 // rows [rows, K] fp32 -> bf16 with an output-row permutation: y[r] = x[perm(r)]  (perm built on the host: GLU interleave
 // of [fc1 16 | gate 16] row blocks, RoPE pairing of the q and k thirds of in_proj -- see engine.cu)
 // With gamma / beta (deferred LayerNorm folded into the weight, see gemm_tc.cu DevParams):
@@ -419,13 +463,17 @@ int launch_rope(void* qkv, bool is_bf16, int64_t ld, const float* cos_t, const f
 
 // =====================================================================================================
 // row softmax over fp32 scores -> P (bf16 or fp32, may alias the input when fp32).  One warp per row.
+// col_len (optional): row r has min(cols, col_len[r / rows_per_len]) valid columns (masked text: the keys past a sequence's
+// text length); the others get probability 0 like the padding columns
 // =====================================================================================================
 template <typename OutT, bool kFast>
 __global__ void __launch_bounds__(256) softmax_kernel(const float* __restrict__ s, int64_t lds, OutT* __restrict__ p,
-                                                      int64_t ldp, int64_t rows, int cols) {
+                                                      int64_t ldp, int64_t rows, int cols, const int* __restrict__ col_len,
+                                                      int64_t rows_per_len) {
   const int lane = threadIdx.x & 31;
   const int64_t row = static_cast<int64_t>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
+  if (col_len != nullptr) cols = min(cols, __ldg(col_len + row / rows_per_len));
   const float* sr = s + row * lds;
   OutT* pr = p + row * ldp;
   float m = -INFINITY;
@@ -446,10 +494,12 @@ __global__ void __launch_bounds__(256) softmax_kernel(const float* __restrict__ 
 // single-pass variant for rows of at most 32 * kMaxV columns: the row lives in registers (one HBM read, one write)
 template <typename OutT, bool kFast, int kMaxV>
 __global__ void __launch_bounds__(256) softmax_reg_kernel(const float* __restrict__ s, int64_t lds, OutT* __restrict__ p,
-                                                          int64_t ldp, int64_t rows, int cols) {
+                                                          int64_t ldp, int64_t rows, int cols, const int* __restrict__ col_len,
+                                                          int64_t rows_per_len) {
   const int lane = threadIdx.x & 31;
   const int64_t row = static_cast<int64_t>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
+  if (col_len != nullptr) cols = min(cols, __ldg(col_len + row / rows_per_len));
   const float* sr = s + row * lds;
   OutT* pr = p + row * ldp;
   float v[kMaxV];
@@ -476,23 +526,25 @@ __global__ void __launch_bounds__(256) softmax_reg_kernel(const float* __restric
   }
 }
 
-int launch_softmax(const float* s, int64_t lds, void* p, bool p_bf16, int64_t ldp, int64_t rows, int cols, cudaStream_t st) {
+int launch_softmax(const float* s, int64_t lds, void* p, bool p_bf16, int64_t ldp, int64_t rows, int cols, cudaStream_t st,
+                   const int* col_len, int64_t rows_per_len) {
+  DITTO_REQUIRE(col_len == nullptr || rows_per_len > 0, DITTO_E_BADARG, "softmax: rows_per_len");
   if (rows <= 0) return 0;
   const unsigned blocks = static_cast<unsigned>(ceil_div(rows, 8));
   ProfScope prof(PC_SOFTMAX, st, 0.0, static_cast<double>(rows) * cols * (p_bf16 ? 6 : 8));
   const bool reg_ok = ldp <= 1024;
   if (p_bf16) {
     bf16* pp = static_cast<bf16*>(p);
-    if (reg_ok && ldp <= 128) softmax_reg_kernel<bf16, true, 4><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
-    else if (reg_ok && ldp <= 256) softmax_reg_kernel<bf16, true, 8><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
-    else if (reg_ok && ldp <= 768) softmax_reg_kernel<bf16, true, 24><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
-    else if (reg_ok) softmax_reg_kernel<bf16, true, 32><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
-    else softmax_kernel<bf16, true><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
+    if (reg_ok && ldp <= 128) softmax_reg_kernel<bf16, true, 4><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
+    else if (reg_ok && ldp <= 256) softmax_reg_kernel<bf16, true, 8><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
+    else if (reg_ok && ldp <= 768) softmax_reg_kernel<bf16, true, 24><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
+    else if (reg_ok) softmax_reg_kernel<bf16, true, 32><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
+    else softmax_kernel<bf16, true><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
   } else {
     float* pp = static_cast<float*>(p);
-    if (reg_ok && ldp <= 256) softmax_reg_kernel<float, false, 8><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
-    else if (reg_ok) softmax_reg_kernel<float, false, 32><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
-    else softmax_kernel<float, false><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols);
+    if (reg_ok && ldp <= 256) softmax_reg_kernel<float, false, 8><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
+    else if (reg_ok) softmax_reg_kernel<float, false, 32><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
+    else softmax_kernel<float, false><<<blocks, 256, 0, st>>>(s, lds, pp, ldp, rows, cols, col_len, rows_per_len);
   }
   DITTO_LAUNCH_CHECK();
   return 0;
@@ -536,26 +588,30 @@ int launch_silu(float* x, int64_t n, cudaStream_t st) {
 }
 
 // silu(mean_S(text)) : text [n, S, D] -> out [n, D]   (DiT.py:27 + the SiLU of text_mlp, DiT.py:19)
-__global__ void mean_silu_kernel(const float* __restrict__ text, float* __restrict__ out, int S, int D) {
+// len (optional): the mean of sequence seq runs over its first len[seq] rows only (masked text)
+__global__ void mean_silu_kernel(const float* __restrict__ text, float* __restrict__ out, int S, int D, const int* __restrict__ len) {
   const int seq = blockIdx.y;
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= D) return;
+  const int rows = len != nullptr ? __ldg(len + seq) : S;
   const float* p = text + static_cast<int64_t>(seq) * S * D + c;
   float acc = 0.f;
-  for (int s = 0; s < S; ++s) acc += p[static_cast<int64_t>(s) * D];
-  const float m = acc / static_cast<float>(S);
+  for (int s = 0; s < rows; ++s) acc += p[static_cast<int64_t>(s) * D];
+  const float m = acc / static_cast<float>(rows);
   out[static_cast<int64_t>(seq) * D + c] = m / (1.0f + expf(-m));
 }
-int launch_mean_silu(const float* text, float* out, int64_t n, int S, int D, cudaStream_t st) {
+int launch_mean_silu(const float* text, float* out, int64_t n, int S, int D, cudaStream_t st, const int* len) {
   dim3 grid(static_cast<unsigned>(ceil_div(D, 128)), static_cast<unsigned>(n));
-  mean_silu_kernel<<<grid, 128, 0, st>>>(text, out, S, D);
+  mean_silu_kernel<<<grid, 128, 0, st>>>(text, out, S, D, len);
   DITTO_LAUNCH_CHECK();
   return 0;
 }
 
-// folded cross-attention score bias: sb[seq, head, s] = scale * sum_i K[seq*S + s, head*d + i] * bq[head*d + i]; zero pad
+// folded cross-attention score bias: sb[seq, head, s] = scale * sum_i K[seq*S + s, head*d + i] * bq[head*d + i]; zero pad.
+// len (optional, masked text): sb = -inf for len[seq] <= s < S.  Every folded kernel adds this bias to its scores, so a masked
+// key gets probability exp(-inf) = 0 there; key 0 is always valid (len >= 1), so each row's maximum stays finite.
 __global__ void fold_bias_kernel(const bf16* __restrict__ kv, int64_t ld, const float* __restrict__ bq, float* __restrict__ sb,
-                                 int64_t total, int S, int Sp, int heads, int d, float scale) {
+                                 int64_t total, int S, int Sp, int heads, int d, float scale, const int* __restrict__ len) {
   const int lane = threadIdx.x & 31;
   const int64_t o = static_cast<int64_t>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);  // (seq, head, s in [0, Sp))
   if (o >= total) return;
@@ -568,12 +624,15 @@ __global__ void fold_bias_kernel(const bf16* __restrict__ kv, int64_t ld, const 
     for (int i = lane; i < d; i += 32) acc += __bfloat162float(row[i]) * bq[head * d + i];
   }
   acc = warp_sum(acc);
-  if (lane == 0) sb[o] = s_idx < S ? scale * acc : 0.f;
+  if (lane == 0) {
+    const bool masked = len != nullptr && s_idx < S && s_idx >= __ldg(len + seq);
+    sb[o] = masked ? -INFINITY : s_idx < S ? scale * acc : 0.f;
+  }
 }
 int launch_fold_bias(const bf16* kv, int64_t ld, const float* bq, float* sb, int64_t n, int S, int Sp, int heads, int d, float scale,
-                     cudaStream_t st) {
+                     cudaStream_t st, const int* len) {
   const int64_t total = n * heads * Sp;
-  fold_bias_kernel<<<static_cast<unsigned>(ceil_div(total, 8)), 256, 0, st>>>(kv, ld, bq, sb, total, S, Sp, heads, d, scale);
+  fold_bias_kernel<<<static_cast<unsigned>(ceil_div(total, 8)), 256, 0, st>>>(kv, ld, bq, sb, total, S, Sp, heads, d, scale, len);
   DITTO_LAUNCH_CHECK();
   return 0;
 }
@@ -581,14 +640,17 @@ int launch_fold_bias(const bf16* kv, int64_t ld, const float* bq, float* sb, int
 // one block per sequence.  A sequence whose text rows are all equal has equal rows of V Wo^T, so its cross-attention output
 // softmax(scores) (V Wo^T) + bo is the row vfold[0] + bo whatever the scores are.  Bitwise equality of the inputs is what
 // makes the rows of the folded projections equal: the GEMMs that build them treat every row alike.
+// Masked text (len != nullptr): only the first len[seq] rows take part (the others have probability 0), so a one-token text
+// with padding is constant.
 __global__ void const_text_kernel(const float* __restrict__ text, int S, int D, const bf16* __restrict__ vfold, int64_t vf_seq,
                                   bool vf_perm4, const float* __restrict__ bo, uint8_t* __restrict__ flag, float* __restrict__ crow,
-                                  int H) {
+                                  int H, const int* __restrict__ len) {
   const int64_t seq = blockIdx.x;
   if (flag != nullptr) {
     const uint32_t* t = reinterpret_cast<const uint32_t*>(text) + seq * S * D;
+    const int rows = len != nullptr ? __ldg(len + seq) : S;
     int diff = 0;
-    for (int64_t i = D + threadIdx.x; i < static_cast<int64_t>(S) * D; i += blockDim.x) diff |= t[i] != t[i % D];
+    for (int64_t i = D + threadIdx.x; i < static_cast<int64_t>(rows) * D; i += blockDim.x) diff |= t[i] != t[i % D];
     diff = __syncthreads_or(diff);
     if (threadIdx.x == 0) flag[seq] = diff ? 0 : 1;
   }
@@ -601,9 +663,9 @@ __global__ void const_text_kernel(const float* __restrict__ text, int S, int D, 
   }
 }
 int launch_const_text(const float* text, int64_t n, int S, int D, const bf16* vfold, int64_t vf_seq, bool vf_perm4, const float* bo,
-                      uint8_t* flag, float* crow, int H, cudaStream_t st) {
+                      uint8_t* flag, float* crow, int H, cudaStream_t st, const int* len) {
   DITTO_REQUIRE(!vf_perm4 || H % 64 == 0, DITTO_E_BADARG, "const_text: perm4 column order needs H % 64 == 0");
-  const_text_kernel<<<static_cast<unsigned>(n), 256, 0, st>>>(text, S, D, vfold, vf_seq, vf_perm4, bo, flag, crow, H);
+  const_text_kernel<<<static_cast<unsigned>(n), 256, 0, st>>>(text, S, D, vfold, vf_seq, vf_perm4, bo, flag, crow, H, len);
   DITTO_LAUNCH_CHECK();
   return 0;
 }

@@ -204,9 +204,13 @@ struct CtxLayout {
   // and, single head only, for sequences whose S text rows are all equal (the unconditional CFG half, S = 1):
   //   cflag [n] u8             = 1 when they are (cross-attention output = vfold[0] + bo for every query row)
   //   crow  [n, H] f32         = vfold[seq][0] + bo, plain column order, per layer
+  // and for every context
+  //   tlen  [n] i32            = text rows sequence seq uses (ditto_text_context_masked; S for a plain context): the
+  //                              unfolded cross-attention softmax reads it, the folded paths see -inf in sbias instead
   bf16 *kfold0 = nullptr, *vfold0 = nullptr;
   float *sbias0 = nullptr, *cvec0 = nullptr, *crow0 = nullptr;
   uint8_t* cflag = nullptr;
+  int* tlen = nullptr;
   size_t kfold_stride = 0, vfold_stride = 0, sbias_stride = 0, crow_stride = 0;  // elements between layers
   size_t total = 0;
 };
@@ -248,6 +252,7 @@ static CtxLayout ctx_layout(const ditto_engine* e, void* base, int64_t n, int64_
       c.crow0 = a.take<float>(static_cast<int64_t>(c.crow_stride) * e->L);
     }
   }
+  c.tlen = a.take<int>(n);
   c.total = a.off + 256;
   return c;
 }
@@ -272,6 +277,7 @@ struct Workspace {
   int ln_parts_h = 0, ln_parts_attn = 0;  // parts written by an N = H producer / by the per-head P.V producer
   float* tmp_small = nullptr;             // [n, Xd] pooled text
   bf16* text16 = nullptr;                 // [n*S, Xd]
+  float* text32 = nullptr;                // [n*S, Xd] fp32 path: masked text with the padded rows zeroed
   int* row_pos = nullptr;                 // [M] position of each packed row inside its sequence (ragged batches: RoPE)
   int64_t M = 0;                          // packed rows: sum over groups of n * T
   size_t total = 0;
@@ -315,6 +321,7 @@ static Workspace ws_layout(const ditto_engine* e, void* base, SeqGroup* gs, int 
   if (e->defer_ln || e->defer_ln2) w.lnstat = a.take<float2>(M * std::max(w.ln_parts_h, w.ln_parts_attn));
   w.tmp_small = a.take<float>(n_tot * e->Xd);
   w.text16 = a.take<bf16>(text_el * e->Xd);
+  if (!e->bf16_mode) w.text32 = a.take<float>(text_el * e->Xd);
   if (ng > 1) w.row_pos = a.take<int>(M);
   w.total = a.off + 256;
   return w;
@@ -336,7 +343,9 @@ namespace ditto {
 static int attention_bf16(ditto_engine* e, const Workspace& w, const bf16* q, int64_t ldq, int64_t q_seq_stride, const bf16* k,
                           int64_t ldk, int64_t k_seq_stride, const bf16* v, int64_t ldv, int64_t v_seq_stride, int64_t n, int Tq,
                           int Tk, float alpha, void* out, bool out_bf16, int64_t ldo, int64_t o_seq_stride, const float* resid,
-                          cudaStream_t st, bool cross, bf16* out2 = nullptr, float2* stat_out = nullptr) {
+                          cudaStream_t st, bool cross, bf16* out2 = nullptr, float2* stat_out = nullptr,
+                          const int* col_len = nullptr) {
+  // col_len (cross-attention): valid keys of each of the n sequences (the context's text lengths)
   const int d = e->d, heads = e->heads;
   if (e->flash_attn && !cross && !out_bf16 && resid != nullptr && out2 == nullptr && stat_out == nullptr && flash_attn_supported(d, Tq, Tk)) {
     FlashAttnParams f;
@@ -361,6 +370,7 @@ static int attention_bf16(ditto_engine* e, const Workspace& w, const bf16* q, in
     f.sp_outer = static_cast<int64_t>(heads) * Tq * ldp; f.npad = static_cast<int>(ldp);
     f.lpart = w.lpart; f.sl_inner = static_cast<int64_t>(Tq) * csize; f.sl_outer = static_cast<int64_t>(heads) * Tq * csize;
     f.tag = cross ? PC_TC_CROSS_SCORES : PC_TC_SELF_SCORES;
+    f.col_len = col_len;
     DITTO_TRY(launch_tc_scores_softmax(f, st));
   } else {
     TcGemmParams g;
@@ -371,7 +381,7 @@ static int attention_bf16(ditto_engine* e, const Workspace& w, const bf16* q, in
     g.so_outer = static_cast<int64_t>(heads) * Tq * ldp;
     g.tag = cross ? PC_TC_CROSS_SCORES : PC_TC_SELF_SCORES;
     DITTO_TRY(launch_tc_gemm(g, st));
-    DITTO_TRY(launch_softmax(w.scores, ldp, w.P, true, ldp, n * heads * Tq, Tk, st));
+    DITTO_TRY(launch_softmax(w.scores, ldp, w.P, true, ldp, n * heads * Tq, Tk, st, col_len, static_cast<int64_t>(heads) * Tq));
   }
   TcGemmParams o;
   o.A.ptr = static_cast<const bf16*>(w.P); o.A.rows = Tq; o.A.cols = Tk; o.A.ld = ldp; o.A.s_inner = static_cast<int64_t>(Tq) * ldp;
@@ -395,7 +405,8 @@ static int attention_bf16(ditto_engine* e, const Workspace& w, const bf16* q, in
 
 static int attention_f32(ditto_engine* e, const Workspace& w, const float* q, int64_t ldq, int64_t q_seq_stride, const float* k,
                          int64_t ldk, int64_t k_seq_stride, const float* v, int64_t ldv, int64_t v_seq_stride, int64_t n, int Tq,
-                         int Tk, float alpha, float* out, int64_t ldo, int64_t o_seq_stride, const float* resid, cudaStream_t st) {
+                         int Tk, float alpha, float* out, int64_t ldo, int64_t o_seq_stride, const float* resid, cudaStream_t st,
+                         const int* col_len = nullptr) {
   const int d = e->d, heads = e->heads;
   const int64_t ldp = round_up(Tk, 8);
   SgemmParams g;
@@ -404,7 +415,7 @@ static int attention_f32(ditto_engine* e, const Workspace& w, const float* q, in
   g.C = w.scores; g.ldc = ldp; g.sC_inner = static_cast<int64_t>(Tq) * ldp; g.sC_outer = static_cast<int64_t>(heads) * Tq * ldp;
   g.alpha = alpha; g.M = Tq; g.N = Tk; g.K = d; g.batch_inner = heads; g.batch_outer = static_cast<int>(n);
   DITTO_TRY(launch_sgemm(g, st));
-  DITTO_TRY(launch_softmax(w.scores, ldp, w.scores, false, ldp, n * heads * Tq, Tk, st));
+  DITTO_TRY(launch_softmax(w.scores, ldp, w.scores, false, ldp, n * heads * Tq, Tk, st, col_len, static_cast<int64_t>(heads) * Tq));
   SgemmParams o;
   o.A = w.scores; o.lda = ldp; o.sA_inner = static_cast<int64_t>(Tq) * ldp; o.sA_outer = static_cast<int64_t>(heads) * Tq * ldp;
   o.B = v; o.ldb = ldv; o.sB_inner = d; o.sB_outer = v_seq_stride; o.b_is_nk = false;
@@ -659,7 +670,7 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
                           H, H, st, PC_TC_CROSS_Q));
           const bf16* kc = static_cast<const bf16*>(kv);
           DITTO_TRY(attention_bf16(e, wg, qc, H, T * H, kc, 2 * H, S * 2 * H, kc + H, 2 * H, S * 2 * H, n, static_cast<int>(T),
-                                   static_cast<int>(S), sqrt_inv_d, oc, true, H, T * H, nullptr, st, true));
+                                   static_cast<int>(S), sqrt_inv_d, oc, true, H, T * H, nullptr, st, true, nullptr, nullptr, c.tlen));
           if (e->fc2_ln && !dln) {
             // out_proj + bias + residual AND norm3 in one cluster kernel (gemm_resid_ln.cu)                 DiT.py:148-151
             GemmResidLnParams f;
@@ -735,7 +746,7 @@ static int forward_impl(ditto_engine* e, const float* x, const int64_t* t, SeqGr
         const float* kc = reinterpret_cast<const float*>(static_cast<const char*>(c.kv0) + c.kv_stride * i);
         const int64_t T = g.T, S = g.S;
         DITTO_TRY(attention_f32(e, wg, qc + g.row0 * H, H, T * H, kc, 2 * H, S * 2 * H, kc + H, 2 * H, S * 2 * H, g.n, static_cast<int>(T),
-                                static_cast<int>(S), sqrt_inv_d, oc + g.row0 * H, H, T * H, nullptr, st));
+                                static_cast<int>(S), sqrt_inv_d, oc + g.row0 * H, H, T * H, nullptr, st, c.tlen));
       }
       if (do_cross)
       DITTO_TRY(sgemm_nt(oc, H, e->LW(i, "cross_attn.out_proj.weight"), H, w.h, H, e->LW(i, "cross_attn.out_proj.bias"), w.h, H, 1.f,
@@ -1163,25 +1174,53 @@ int64_t ditto_workspace_bytes(const ditto_engine_t* e, int64_t n_seq, int64_t T,
   return static_cast<int64_t>(ws_layout(e, nullptr, n_seq, T, S).total);
 }
 
-int32_t ditto_text_context(ditto_engine_t* e, const float* text_emb, int64_t n, int64_t S, void* ctx, void* workspace,
-                           int64_t workspace_bytes, void* stream) {
+namespace ditto {
+// ditto_text_context(_masked).  text_len == nullptr: every sequence uses all S rows (the plain context, the kernels of
+// the unmasked build); otherwise sequence i uses rows [0, text_len[i]).
+static int text_context_impl(ditto_engine_t* e, const float* text_emb, int64_t n, int64_t S, const int64_t* text_len, void* ctx,
+                             void* workspace, int64_t workspace_bytes, cudaStream_t st) {
   DITTO_REQUIRE(e && text_emb && ctx && workspace, DITTO_E_BADARG, "text_context: null argument");
   DITTO_REQUIRE(e->finalized, DITTO_E_STATE, "text_context: engine not finalized");
   DITTO_REQUIRE(n > 0 && S > 0, DITTO_E_BADARG, "text_context: empty input");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  DITTO_REQUIRE(S < (1ll << 31), DITTO_E_UNSUPPORTED, "text_context: S too large");
+  std::vector<int> len;
+  if (text_len != nullptr) {
+    len.resize(static_cast<size_t>(n));
+    bool all_full = true;
+    for (int64_t i = 0; i < n; ++i) {
+      DITTO_REQUIRE(text_len[i] >= 1 && text_len[i] <= S, DITTO_E_BADARG, "text_context_masked: every text length must be in [1, S]");
+      len[static_cast<size_t>(i)] = static_cast<int>(text_len[i]);
+      all_full = all_full && text_len[i] == S;
+    }
+    if (all_full) len.clear();   // nothing masked: the plain context, bit for bit
+  }
+  const bool masked = !len.empty();
   const int H = e->H, Xd = e->Xd;
   // only the small tail of the workspace is needed here; lay it out with T = 1
   Workspace w = ws_layout(e, workspace, n, 1, S);
   DITTO_REQUIRE(static_cast<int64_t>(w.total) <= workspace_bytes, DITTO_E_WORKSPACE, "text_context: workspace too small");
   CtxLayout c = ctx_layout(e, ctx, n, S);
-  // text modulation: text_mlp(SiLU(mean_S(text)))  (DiT.py:27,31)
+  // the per-sequence lengths the step kernels read; `mlen` is what the build kernels below get (null: unmasked)
+  if (masked)
+    DITTO_CUDA(cudaMemcpyAsync(c.tlen, len.data(), len.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  else
+    DITTO_TRY(launch_fill_i32(c.tlen, static_cast<int>(S), n, st));
+  const int* mlen = masked ? c.tlen : nullptr;
+  // text modulation: text_mlp(SiLU(mean_S(text)))  (DiT.py:27,31), the mean over the valid rows
   if (!e->blocks_only) {
-    DITTO_TRY(launch_mean_silu(text_emb, w.tmp_small, n, static_cast<int>(S), Xd, st));
+    DITTO_TRY(launch_mean_silu(text_emb, w.tmp_small, n, static_cast<int>(S), Xd, st, mlen));
     DITTO_TRY(sgemm_nt(w.tmp_small, Xd, e->W("ada_ln.text_mlp.1.weight"), Xd, c.text_mod, 2 * H, e->W("ada_ln.text_mlp.1.bias"), nullptr,
                        0, 1.f, static_cast<int>(n), 2 * H, Xd, st));
   }
-  // per-layer K|V = text @ in_proj[H:3H]^T + b  (torch MHA packed in_proj, rows H..3H)
-  if (e->bf16_mode) DITTO_TRY(launch_cast_bf16(text_emb, w.text16, n * S * Xd, st));
+  // per-layer K|V = text @ in_proj[H:3H]^T + b  (torch MHA packed in_proj, rows H..3H), from the text with its masked rows
+  // zeroed: their K / V stay finite whatever the caller left there, and the zero probabilities of those keys cancel them
+  const float* text_f32 = text_emb;
+  if (e->bf16_mode && masked) DITTO_TRY(launch_stage_text(text_emb, w.text16, true, mlen, n, static_cast<int>(S), Xd, st));
+  else if (e->bf16_mode) DITTO_TRY(launch_cast_bf16(text_emb, w.text16, n * S * Xd, st));
+  else if (masked) {
+    DITTO_TRY(launch_stage_text(text_emb, w.text32, false, mlen, n, static_cast<int>(S), Xd, st));
+    text_f32 = w.text32;
+  }
   for (int i = 0; i < e->L; ++i) {
     void* kv = static_cast<char*>(c.kv0) + c.kv_stride * i;
     const float* bias = e->LW(i, "cross_attn.in_proj_bias") + H;
@@ -1218,19 +1257,32 @@ int32_t ditto_text_context(ditto_engine_t* e, const float* text_emb, int64_t n, 
         v.tag = PC_TC_TEXT_KV;
         DITTO_TRY(launch_tc_gemm(v, st));
         DITTO_TRY(launch_fold_bias(kvb, 2 * H, fln ? e->layers[i].bq_g : e->LW(i, "cross_attn.in_proj_bias"), sb, n,
-                                   static_cast<int>(S), static_cast<int>(Sp), heads, d, sqrtf(1.0f / static_cast<float>(d)), st));
+                                   static_cast<int>(S), static_cast<int>(Sp), heads, d, sqrtf(1.0f / static_cast<float>(d)), st, mlen));
         if (fln)
           DITTO_TRY(launch_rowsum_bf16(kf, c.cvec0 + c.sbias_stride * i, n * heads, static_cast<int>(S), static_cast<int>(Sp), H, st));
         if (c.cflag != nullptr)   // the flags once (layer 0), the constant rows of every layer
           DITTO_TRY(launch_const_text(text_emb, n, static_cast<int>(S), Xd, vf, Sp * H, cross_flash_active(e, S),
-                                      e->LW(i, "cross_attn.out_proj.bias"), i == 0 ? c.cflag : nullptr, c.crow0 + c.crow_stride * i, H, st));
+                                      e->LW(i, "cross_attn.out_proj.bias"), i == 0 ? c.cflag : nullptr, c.crow0 + c.crow_stride * i, H, st,
+                                      mlen));
       }
     } else {
-      DITTO_TRY(sgemm_nt(text_emb, Xd, e->LW(i, "cross_attn.in_proj_weight") + static_cast<int64_t>(H) * H, H, static_cast<float*>(kv),
+      DITTO_TRY(sgemm_nt(text_f32, Xd, e->LW(i, "cross_attn.in_proj_weight") + static_cast<int64_t>(H) * H, H, static_cast<float*>(kv),
                          2 * H, bias, nullptr, 0, 1.f, static_cast<int>(n * S), 2 * H, Xd, st));
     }
   }
   return 0;
+}
+}  // namespace ditto
+
+int32_t ditto_text_context(ditto_engine_t* e, const float* text_emb, int64_t n, int64_t S, void* ctx, void* workspace,
+                           int64_t workspace_bytes, void* stream) {
+  return text_context_impl(e, text_emb, n, S, nullptr, ctx, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
+int32_t ditto_text_context_masked(ditto_engine_t* e, const float* text_emb, int64_t n, int64_t S, const int64_t* text_len, void* ctx,
+                                  void* workspace, int64_t workspace_bytes, void* stream) {
+  DITTO_REQUIRE(text_len, DITTO_E_BADARG, "text_context_masked: null text_len");
+  return text_context_impl(e, text_emb, n, S, text_len, ctx, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
 int32_t ditto_forward(ditto_engine_t* e, const float* x, int64_t n_x, const void* ctx, const int64_t* t, int64_t n_seq, int64_t T,

@@ -1429,6 +1429,7 @@ struct SmDev {
   int npad;
   float* lpart; long long sl_inner, sl_outer;
   int csize;   // key tiles per row = CTAs per cluster
+  const int* col_len;   // optional [batch_outer] valid key columns of each outer batch item (masked text); null: N
   // deferred LayerNorm of the query operand (HAS_BIAS variant): s = alpha (rstd acc - rstd mean c[col]) + bias[col];
   // statistics row = outer batch index * M + query row; c has the layout / strides of bias
   const float2* ln_stat; int ln_parts; float ln_inv_h; const float* ln_c;
@@ -1563,6 +1564,10 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
       const int m_blk = item % p.m_tiles;
       const int b = item / p.m_tiles;
       const int bo = b / p.batch_inner, bi = b - bo * p.batch_inner;
+      // valid key columns of this item: columns [nv, N) are masked keys and get probability 0 like the padding.  Always >= 1
+      // (key 0 is valid), so rank 0 sees a finite row maximum; a CTA whose whole tile is masked contributes -inf to the
+      // exchange and a zero partial sum.  Full 64-column blocks below nv keep the lean path.
+      const int nv = p.col_len != nullptr ? min(p.N, __ldg(p.col_len + bo)) : p.N;
       // second row: rowA + 8
       const long long rowA = static_cast<long long>(m_blk) * BLOCK_M + trow + g;
       const bool okA = rowA < p.M, okB = rowA + 8 < p.M;
@@ -1585,10 +1590,10 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
 #pragma unroll 1
       for (int cbk = 0; cbk < 4; ++cbk) {
         const int col0 = col_base + cbk * 64 + q2;
-        if (col0 - q2 >= p.N) break;  // warp-uniform
+        if (col0 - q2 >= nv) break;  // warp-uniform
         uint32_t r[32];
         tmem_ld_16x64(t_row + cbk * 64, r);
-        if (!HAS_BIAS && col0 - q2 + 64 <= p.N) {
+        if (!HAS_BIAS && col0 - q2 + 64 <= nv) {
           // lean block (no bias, all 64 columns valid): s' = alpha2 acc with alpha2 > 0, so the maximum is taken on the raw
           // accumulators and scaled once -- 1 instruction per element instead of ~7 (the generic block below predicates and
           // rescales every element; ncu: 21 instructions per score made this epilogue, not the MMA, the pace of the kernel)
@@ -1609,11 +1614,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
           bb[kb] = cc[kb] = make_float2(0.f, 0.f);
           if (HAS_BIAS) {
             const int c = col0 + kb * 8;
-            if (c < p.N) bb[kb].x = __ldg(bias + c) * 1.4426950408889634f;
-            if (c + 1 < p.N) bb[kb].y = __ldg(bias + c + 1) * 1.4426950408889634f;
+            if (c < nv) bb[kb].x = __ldg(bias + c) * 1.4426950408889634f;
+            if (c + 1 < nv) bb[kb].y = __ldg(bias + c + 1) * 1.4426950408889634f;
             if (lnc != nullptr) {
-              if (c < p.N) cc[kb].x = __ldg(lnc + c);
-              if (c + 1 < p.N) cc[kb].y = __ldg(lnc + c + 1);
+              if (c < nv) cc[kb].x = __ldg(lnc + c);
+              if (c + 1 < nv) cc[kb].y = __ldg(lnc + c + 1);
             }
           }
         }
@@ -1621,11 +1626,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
 #pragma unroll
         for (int kb = 0; kb < 8; ++kb) {
           const int c = col0 + kb * 8;
-          if (c < p.N) {
+          if (c < nv) {
             mA = fmaxf(mA, fmaf(aA, __uint_as_float(r[4 * kb]), fmaf(nA, cc[kb].x, bb[kb].x)));
             mB = fmaxf(mB, fmaf(aB, __uint_as_float(r[4 * kb + 2]), fmaf(nB, cc[kb].x, bb[kb].x)));
           }
-          if (c + 1 < p.N) {
+          if (c + 1 < nv) {
             mA = fmaxf(mA, fmaf(aA, __uint_as_float(r[4 * kb + 1]), fmaf(nA, cc[kb].y, bb[kb].y)));
             mB = fmaxf(mB, fmaf(aB, __uint_as_float(r[4 * kb + 3]), fmaf(nB, cc[kb].y, bb[kb].y)));
           }
@@ -1669,7 +1674,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
         if (col0 - q2 >= p.npad) break;  // warp-uniform (npad >= N)
         uint32_t r[32];
         tmem_ld_16x64(t_row + cbk * 64, r);
-        if (!HAS_BIAS && store2 && col0 - q2 + 64 <= p.N) {
+        if (!HAS_BIAS && store2 && col0 - q2 + 64 <= nv) {
           // lean block: exp2(alpha2 acc - m) in one FMA + MUFU per element, packed row sums, unpredicated column logic
           tmem_ld_wait();
           float2 sA2 = make_float2(0.f, 0.f), sB2 = make_float2(0.f, 0.f);
@@ -1696,11 +1701,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
           bb[kb] = cc[kb] = make_float2(0.f, 0.f);
           if (HAS_BIAS) {
             const int c = col0 + kb * 8;
-            if (c < p.N) bb[kb].x = __ldg(bias + c) * 1.4426950408889634f;
-            if (c + 1 < p.N) bb[kb].y = __ldg(bias + c + 1) * 1.4426950408889634f;
+            if (c < nv) bb[kb].x = __ldg(bias + c) * 1.4426950408889634f;
+            if (c + 1 < nv) bb[kb].y = __ldg(bias + c + 1) * 1.4426950408889634f;
             if (lnc != nullptr) {
-              if (c < p.N) cc[kb].x = __ldg(lnc + c);
-              if (c + 1 < p.N) cc[kb].y = __ldg(lnc + c + 1);
+              if (c < nv) cc[kb].x = __ldg(lnc + c);
+              if (c + 1 < nv) cc[kb].y = __ldg(lnc + c + 1);
             }
           }
         }
@@ -1708,7 +1713,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
 #pragma unroll
         for (int kb = 0; kb < 8; ++kb) {
           const int c = col0 + kb * 8;
-          const bool v0 = c < p.N, v1 = c + 1 < p.N;
+          const bool v0 = c < nv, v1 = c + 1 < nv;
           const float a0 = v0 ? ex2_approx(fmaf(aA, __uint_as_float(r[4 * kb]), fmaf(nA, cc[kb].x, bb[kb].x)) - mA) : 0.f;
           const float a1 = v1 ? ex2_approx(fmaf(aA, __uint_as_float(r[4 * kb + 1]), fmaf(nA, cc[kb].y, bb[kb].y)) - mA) : 0.f;
           const float b0 = v0 ? ex2_approx(fmaf(aB, __uint_as_float(r[4 * kb + 2]), fmaf(nB, cc[kb].x, bb[kb].x)) - mB) : 0.f;
@@ -1744,11 +1749,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
             bb[kb] = cc[kb] = make_float2(0.f, 0.f);
             if (HAS_BIAS) {
               const int c = col0 + kb * 8;
-              if (c < p.N) bb[kb].x = __ldg(bias + c) * 1.4426950408889634f;
-              if (c + 1 < p.N) bb[kb].y = __ldg(bias + c + 1) * 1.4426950408889634f;
+              if (c < nv) bb[kb].x = __ldg(bias + c) * 1.4426950408889634f;
+              if (c + 1 < nv) bb[kb].y = __ldg(bias + c + 1) * 1.4426950408889634f;
               if (lnc != nullptr) {
-                if (c < p.N) cc[kb].x = __ldg(lnc + c);
-                if (c + 1 < p.N) cc[kb].y = __ldg(lnc + c + 1);
+                if (c < nv) cc[kb].x = __ldg(lnc + c);
+                if (c + 1 < nv) cc[kb].y = __ldg(lnc + c + 1);
               }
             }
           }
@@ -1757,7 +1762,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1)
           for (int kb = 0; kb < 8; ++kb) {
             const int c = col0 + kb * 8;
             if (c >= p.npad) continue;
-            const bool v0 = c < p.N, v1 = c + 1 < p.N;
+            const bool v0 = c < nv, v1 = c + 1 < nv;
             const float a0 = v0 ? ex2_approx(fmaf(aA, __uint_as_float(r[4 * kb]), fmaf(nA, cc[kb].x, bb[kb].x)) - mA) * iA : 0.f;
             const float a1 = v1 ? ex2_approx(fmaf(aA, __uint_as_float(r[4 * kb + 1]), fmaf(nA, cc[kb].y, bb[kb].y)) - mA) * iA : 0.f;
             const float b0 = v0 ? ex2_approx(fmaf(aB, __uint_as_float(r[4 * kb + 2]), fmaf(nB, cc[kb].x, bb[kb].x)) - mB) * iB : 0.f;
@@ -2152,6 +2157,7 @@ int launch_tc_scores_softmax(const TcScoresSoftmaxParams& q, cudaStream_t st) {
   p.npad = q.npad;
   p.lpart = q.lpart; p.sl_inner = q.sl_inner; p.sl_outer = q.sl_outer;
   p.csize = csize;
+  p.col_len = q.col_len;
   p.ln_stat = q.ln_stat; p.ln_parts = q.ln_parts; p.ln_inv_h = q.ln_width > 0 ? 1.0f / static_cast<float>(q.ln_width) : 0.f;
   p.ln_c = q.ln_c;
   if (q.ln_stat != nullptr)

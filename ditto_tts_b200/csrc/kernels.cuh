@@ -41,6 +41,9 @@ int launch_clusters(const void* func, int csize, int threads, int smem_bytes, in
 
 // ---- elementwise.cu ----------------------------------------------------------------------------------
 int launch_cast_bf16(const float* x, bf16* y, int64_t n, cudaStream_t st);
+// text [n_seq, S, D] fp32 -> y (bf16 when y_bf16, else fp32) with rows s >= len[seq] (device, [n_seq]) set to zero
+int launch_stage_text(const float* x, void* y, bool y_bf16, const int* len, int64_t n_seq, int S, int D, cudaStream_t st);
+int launch_fill_i32(int* y, int v, int64_t n, cudaStream_t st);
 int launch_pack_rows(const float* x, bf16* y, float* bias_out, const float* bias_in, const int* perm, int rows, int K,
                      cudaStream_t st, const float* gamma = nullptr, const float* beta = nullptr, float* csum = nullptr);
 int launch_rowsum_bf16(const bf16* x, float* out, int64_t groups, int S, int Sp, int K, cudaStream_t st);
@@ -54,16 +57,20 @@ int launch_rope_table(const float* inv_freq, float* cos_t, float* sin_t, float* 
                       cudaStream_t st);
 int launch_rope(void* qkv, bool is_bf16, int64_t ld, const float* cos_t, const float* sin_t, int64_t rows, int seq_T,
                 int H, int head_dim, cudaStream_t st);
-int launch_softmax(const float* s, int64_t lds, void* p, bool p_bf16, int64_t ldp, int64_t rows, int cols, cudaStream_t st);
+// col_len (optional): row r has min(cols, col_len[r / rows_per_len]) valid columns, the rest get probability 0
+int launch_softmax(const float* s, int64_t lds, void* p, bool p_bf16, int64_t ldp, int64_t rows, int cols, cudaStream_t st,
+                   const int* col_len = nullptr, int64_t rows_per_len = 1);
 int launch_geglu_f32(const float* a, const float* g, float* out, int64_t n, cudaStream_t st);
 int launch_silu(float* x, int64_t n, cudaStream_t st);
-int launch_mean_silu(const float* text, float* out, int64_t n, int S, int D, cudaStream_t st);
+// len (optional, device [n]): masked text, sequence seq uses its first len[seq] rows only (mean over them; score bias -inf
+// past them; constant flag from them)
+int launch_mean_silu(const float* text, float* out, int64_t n, int S, int D, cudaStream_t st, const int* len = nullptr);
 int launch_fold_bias(const bf16* kv, int64_t ld, const float* bq, float* sb, int64_t n, int S, int Sp, int heads, int d, float scale,
-                     cudaStream_t st);
+                     cudaStream_t st, const int* len = nullptr);
 // constant text (all S rows of a sequence's text_emb [n, S, D] bitwise equal): flag[seq] (written when flag != nullptr) and,
 // for every sequence, crow[seq] = vfold[seq][0] + bo in the plain column order (vf_perm4: vfold columns in the perm4 order)
 int launch_const_text(const float* text, int64_t n, int S, int D, const bf16* vfold, int64_t vf_seq, bool vf_perm4, const float* bo,
-                      uint8_t* flag, float* crow, int H, cudaStream_t st);
+                      uint8_t* flag, float* crow, int H, cudaStream_t st, const int* len = nullptr);
 // number of nonzero bytes of flags[0, n) for the profiler's byte counts; 0 without synchronising unless profiling (which
 // synchronises anyway and is never captured)
 int64_t profiled_nonzero(const uint8_t* flags, int64_t n, cudaStream_t st);
@@ -180,6 +187,8 @@ struct TcScoresSoftmaxParams {
   bf16* P = nullptr; int64_t ldp = 0, sp_inner = 0, sp_outer = 0;
   int npad = 0;                                 // zero-fill bound (multiple of 2, >= N)
   float* lpart = nullptr; int64_t sl_inner = 0, sl_outer = 0;  // [M, csize] per batch item; required when csize > 1
+  // optional [batch_outer] valid key count of each outer batch item (masked text): columns [col_len[b], N) get probability 0
+  const int* col_len = nullptr;
   // deferred LayerNorm of Q (needs bias): statistics row = outer batch index * M + query row; ln_c strided like bias
   const float2* ln_stat = nullptr; int ln_parts = 0; int ln_width = 0; const float* ln_c = nullptr;
   int tag = PC_TC_OTHER;

@@ -8,8 +8,9 @@ C-ABI of include/ditto_b200.h).  Inference only; no autograd; no CPU fallback (C
 from __future__ import annotations
 
 import ctypes as C
+import operator
 import weakref
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
 import torch
 import torch.nn as nn
@@ -44,6 +45,33 @@ def _need_cuda_f32(name: str, t: torch.Tensor) -> torch.Tensor:
     if t.dtype != torch.float32:
         raise DittoError(f"{name} must be float32 (the reference path is fp32 end to end), got {t.dtype}")
     return t.contiguous()
+
+
+def _check_text_lengths(text_lengths, widths: List[int]) -> Optional[List[int]]:
+    """None, or one integer text length per utterance with text_lengths[i] in [1, widths[i]], the text rows utterance i was
+    given.  Lengths are data of the text context (ditto_text_context_masked): any value in range reuses the same graphs."""
+    if text_lengths is None:
+        return None
+    try:
+        vals = text_lengths.tolist() if hasattr(text_lengths, "tolist") else list(text_lengths)
+    except TypeError:
+        vals = None
+    if isinstance(text_lengths, (str, bytes)) or not isinstance(vals, list):
+        raise DittoError("text_lengths must be a sequence of one integer per utterance")
+    if len(vals) != len(widths):
+        raise DittoError(f"text_lengths must hold one length per utterance: {len(widths)} expected, got {len(vals)}")
+    out = []
+    for i, (v, hi) in enumerate(zip(vals, widths)):
+        if isinstance(v, bool):
+            raise DittoError(f"text_lengths[{i}] must be an integer, got a bool")
+        try:
+            v = operator.index(v)
+        except TypeError:
+            raise DittoError(f"text_lengths[{i}] must be an integer, got {type(v).__name__}") from None
+        if not 1 <= v <= hi:
+            raise DittoError(f"text_lengths[{i}] = {v} is outside [1, {hi}] (the text rows that utterance was given)")
+        out.append(v)
+    return out
 
 
 class GlobalAdaLN(nn.Module):
@@ -254,19 +282,27 @@ class _EngineHost:
             raise DittoError("ditto_workspace_bytes: bad sizes")
         return self._bufs.get("ws", nbytes, self._device())
 
-    def text_context(self, text_emb: torch.Tensor, name: str = "ctx", T_hint: int = 1) -> torch.Tensor:
-        """Step-invariant text work (cross-attention K/V of every layer + text modulation) for a batch."""
+    def text_context(self, text_emb: torch.Tensor, name: str = "ctx", T_hint: int = 1, text_lengths=None) -> torch.Tensor:
+        """Step-invariant text work (cross-attention K/V of every layer + text modulation) for a batch.  ``text_lengths``
+        (one integer in [1, S] per sequence): sequence i uses text rows [0, text_lengths[i]) only (ditto_text_context_masked)."""
         eng = self.engine()
         lib = _lib.load()
         text_emb = _need_cuda_f32("text_emb", text_emb)
+        if text_emb.dim() != 3:
+            raise DittoError("text_emb must be [n, S, text_dim]")
         n, S, Xd = text_emb.shape
         if Xd != self.text_dim:
             raise DittoError(f"text_emb last dim {Xd} != text_dim {self.text_dim}")
+        lens = _check_text_lengths(text_lengths, [S] * n)
         with torch.cuda.device(text_emb.device):
             ctx = self._bufs.get(name, lib.ditto_text_context_bytes(eng, n, S), text_emb.device)
             ws = self.workspace(n, T_hint, S)
-            _lib.check(lib.ditto_text_context(eng, _ptr(text_emb), n, S, _ptr(ctx), _ptr(ws), ws.numel(), _stream()),
-                       "ditto_text_context")
+            if lens is None:
+                _lib.check(lib.ditto_text_context(eng, _ptr(text_emb), n, S, _ptr(ctx), _ptr(ws), ws.numel(), _stream()),
+                           "ditto_text_context")
+            else:
+                _lib.check(lib.ditto_text_context_masked(eng, _ptr(text_emb), n, S, (C.c_int64 * n)(*lens), _ptr(ctx), _ptr(ws),
+                                                         ws.numel(), _stream()), "ditto_text_context_masked")
         return ctx
 
     def _destroy_engine(self):
@@ -453,24 +489,26 @@ class DiTTO(nn.Module, _EngineHost):
         return out
 
     @torch.no_grad()
-    def forward(self, x, text_emb, t):
-        """eps_hat = DiTTO.forward(x, text_emb, t)  (reference: DiTTO.py:66-94)."""
+    def forward(self, x, text_emb, t, *, text_lengths=None):
+        """eps_hat = DiTTO.forward(x, text_emb, t)  (reference: DiTTO.py:66-94).  ``text_lengths`` (one integer in [1, S] per
+        sequence): texts of different lengths padded to one S; sequence i then equals its run with ``text_emb[i, :len]``."""
         x = _need_cuda_f32("x", x)
         text_emb = _need_cuda_f32("text_emb", text_emb)
         if x.dim() != 3 or text_emb.dim() != 3 or x.shape[0] != text_emb.shape[0]:
             raise DittoError("expected x [n,T,H] and text_emb [n,S,text_dim] with the same n")
         t = t.to(device=x.device, dtype=torch.int64)
         _check_t_range(t, self.diffusion_steps, "DiTTO.forward")
-        ctx = self.text_context(text_emb, T_hint=x.shape[1])
+        ctx = self.text_context(text_emb, T_hint=x.shape[1], text_lengths=text_lengths)
         return self.forward_with_context(x, ctx, t, x.shape[0], text_emb.shape[1])
 
     @torch.no_grad()
-    def forward_ragged(self, xs, texts, t):
+    def forward_ragged(self, xs, texts, t, *, text_lengths=None):
         """``DiTTO.forward`` on a mixed-length batch, every utterance at its own length (no padding, no masks -- the
         reference has none): xs[i] [T_i,H], texts[i] [S_i,text_dim], t [B] -> list of eps_hat [T_i,H].
-        Equals ``[forward(x[None], text[None], t[i:i+1])[0] for ...]`` of the reference (DiTTO.py:66-94)."""
+        Equals ``[forward(x[None], text[None], t[i:i+1])[0] for ...]`` of the reference (DiTTO.py:66-94).
+        ``text_lengths[i]`` in [1, S_i]: utterance i uses ``texts[i][:len]`` (padded texts that share a group)."""
         from .ragged import RaggedBatch
-        rb = RaggedBatch(self, texts, [int(x.shape[0]) for x in xs], guided=False)
+        rb = RaggedBatch(self, texts, [int(x.shape[0]) for x in xs], guided=False, text_lengths=text_lengths)
         out = rb.forward(rb.pack(xs), rb.seq_t(t))
         return rb.unpack(out)
 

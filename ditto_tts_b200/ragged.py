@@ -17,7 +17,7 @@ import torch
 
 from . import _lib
 from ._lib import DittoError
-from .model import DiTTO, _need_cuda_f32, _ptr, _stream
+from .model import DiTTO, _check_text_lengths, _need_cuda_f32, _ptr, _stream
 from .sampler import _CapturedStep
 
 __all__ = ["RaggedBatch", "RaggedStepGraph"]
@@ -28,7 +28,9 @@ class RaggedBatch:
 
     ``texts[i]`` is ``[S_i, text_dim]`` (CUDA fp32), ``lengths[i]`` the latent frame count T_i.  With ``guided`` each
     group holds its conditional sequences followed by the unconditional ones (zero text embedding unless
-    ``null_texts`` supplies them), sharing the group's latents."""
+    ``null_texts`` supplies them), sharing the group's latents.  ``text_lengths[i]`` in [1, S_i]: utterance i (and its
+    unconditional branch) uses text rows [0, text_lengths[i]) only.  Groups stay keyed on ``texts[i].shape[0]``: padding texts
+    to a few widths makes them share groups, and the lengths, being data in the group's context, change no graph."""
 
     @staticmethod
     def signature(texts, lengths, guided: bool):
@@ -38,7 +40,7 @@ class RaggedBatch:
 
     def __init__(self, model: DiTTO, texts: Sequence[torch.Tensor], lengths: Sequence[int], guided: bool = False,
                  null_texts: Optional[Sequence[torch.Tensor]] = None, name: str = "ragged",
-                 ctx_storage: Optional[List[torch.Tensor]] = None):
+                 ctx_storage: Optional[List[torch.Tensor]] = None, text_lengths=None):
         if len(texts) == 0 or len(texts) != len(lengths):
             raise DittoError("RaggedBatch needs one text embedding and one length per utterance")
         self.model, self.guided = model, guided
@@ -47,6 +49,7 @@ class RaggedBatch:
         for i, x in enumerate(texts):
             if x.dim() != 2 or x.shape[1] != model.text_dim or x.shape[0] < 1:
                 raise DittoError(f"texts[{i}] must be [S, {model.text_dim}] with S >= 1")
+        text_lengths = _check_text_lengths(text_lengths, [int(x.shape[0]) for x in texts])
         self.lengths = [int(v) for v in lengths]
         if min(self.lengths) < 1 or max(self.lengths) > model.max_seq_len:
             raise DittoError("every length must be in [1, max_seq_len]")
@@ -77,7 +80,10 @@ class RaggedBatch:
                 if null.shape != tg.shape:
                     raise DittoError("null_texts must match texts in shape")
                 tg = torch.cat([tg, null], dim=0)
-            ctx = model.text_context(tg, name="ragged_ctx", T_hint=1)
+            lens = None
+            if text_lengths is not None:
+                lens = [text_lengths[i] for i in idx] * (2 if guided else 1)
+            ctx = model.text_context(tg, name="ragged_ctx", T_hint=1, text_lengths=lens)
             if ctx_storage is not None:       # buffers a cached step graph reads (same batch signature): refill in place
                 store = ctx_storage[gi]
                 k = min(store.numel(), ctx.numel())   # both hold at least ditto_text_context_bytes of this group

@@ -14,6 +14,9 @@ device buffer ``hist`` that the update kernel reads and rewrites.
 ``sample_latents(..., seeds=[s_0, ...], guidance_scale=[w_0, ...])`` gives every utterance its own noise stream (x_T and every
 step's noise depend on its seed alone, not on its batch-mates: include/ditto_b200.h, ditto_p_sample_per_utt) and its own
 guidance scale; one captured step graph serves every scale.
+``text_lengths=[l_0, ...]`` lets texts of different token counts share one padded ``text_emb`` [B, S, text_dim]: utterance b
+(and its unconditional branch) uses text rows [0, l_b) only and samples as it would with ``text_emb[b, :l_b]``.  The lengths
+live in the text context, so one captured step graph serves every set of lengths.
 """
 from __future__ import annotations
 
@@ -28,7 +31,7 @@ import torch
 
 from . import _lib, schedules
 from ._lib import DittoError
-from .model import DiTTO, _check_t_range, _need_cuda_f32, _ptr, _stream
+from .model import DiTTO, _check_t_range, _check_text_lengths, _need_cuda_f32, _ptr, _stream
 
 __all__ = ["DiTTOSampler", "StepGraph", "randn_latents"]
 
@@ -290,14 +293,19 @@ class DiTTOSampler:
         return self._tau_dev
 
     # ------------------------------------------------------------------------------------------
-    def _context(self, text_emb: torch.Tensor, guided: bool, null_text_emb: Optional[torch.Tensor], T: int):
+    def _context(self, text_emb: torch.Tensor, guided: bool, null_text_emb: Optional[torch.Tensor], T: int, text_lengths=None):
         text_emb = _need_cuda_f32("text_emb", text_emb)
+        if text_emb.dim() != 3:
+            raise DittoError("text_emb must be [B, S, text_dim]")
+        lens = _check_text_lengths(text_lengths, [text_emb.shape[1]] * text_emb.shape[0])
         if guided:
             null = torch.zeros_like(text_emb) if null_text_emb is None else _need_cuda_f32("null_text_emb", null_text_emb)
             if null.shape != text_emb.shape:
                 raise DittoError("null_text_emb must have the shape of text_emb")
             text_emb = torch.cat([text_emb, null], dim=0)  # [cond(B); uncond(B)]
-        return self.model.text_context(text_emb, name="sampler_ctx", T_hint=T)
+            if lens is not None:
+                lens = lens + lens                         # the unconditional branch uses the same lengths
+        return self.model.text_context(text_emb, name="sampler_ctx", T_hint=T, text_lengths=lens)
 
     def _p_sample_raw(self, x, ctx, t_n, z, guided, w, S, eps, x_out, ws=None, hist=None, known=None, mask=None, rng=None,
                       seeds=None, w_dev=None, advance=None):
@@ -319,13 +327,13 @@ class DiTTOSampler:
 
     # ------------------------------------------------------------------------------------------
     @torch.no_grad()
-    def predict_noise(self, x, t, text_emb, guidance_scale=None, null_text_emb=None):
+    def predict_noise(self, x, t, text_emb, guidance_scale=None, null_text_emb=None, *, text_lengths=None):
         """eps_hat (guided when a scale is given): the call at SpeechGenerator.py:135 + CFG combine."""
         w = self.guidance_scale if guidance_scale is None else guidance_scale
         guided = w is not None
         x = _need_cuda_f32("x", x)
         B, T, H = x.shape
-        ctx = self._context(text_emb, guided, null_text_emb, T)
+        ctx = self._context(text_emb, guided, null_text_emb, T, text_lengths)
         t = t.to(device=x.device, dtype=torch.int64)
         t_n = torch.cat([t, t]) if guided else t
         eps = self.model.forward_with_context(x, ctx, t_n.contiguous(), t_n.numel(), text_emb.shape[1])
@@ -334,7 +342,7 @@ class DiTTOSampler:
         return eps[B:] + w * (eps[:B] - eps[B:])
 
     @torch.no_grad()
-    def p_sample(self, x, t, text_emb, noise=None, guidance_scale=None, null_text_emb=None):
+    def p_sample(self, x, t, text_emb, noise=None, guidance_scale=None, null_text_emb=None, *, text_lengths=None):
         """One reverse step (reference: __p_sample, SpeechGenerator.py:131-147).  ``noise`` replaces the
         reference's in-place ``torch.randn_like(x)``; when omitted it is drawn the same way.  Not for ``dpmpp_2m``: its
         update needs the previous step's x0 prediction, which only sample_latents(_ragged) carries from step to step."""
@@ -346,7 +354,7 @@ class DiTTOSampler:
         x = _need_cuda_f32("x", x)
         B, T, H = x.shape
         self._activate()
-        ctx = self._context(text_emb, guided, null_text_emb, T)
+        ctx = self._context(text_emb, guided, null_text_emb, T, text_lengths)
         t = t.to(device=x.device, dtype=torch.int64)
         _check_t_range(t, self.model.diffusion_steps, "p_sample")
         t_n = (torch.cat([t, t]) if guided else t).contiguous()
@@ -379,7 +387,8 @@ class DiTTOSampler:
     def sample_latents(self, text_emb, audio_emb=None, *, x_init=None, noise=None, guidance_scale=None,
                        null_text_emb=None, cond_by_audio=False, record: Optional[List[torch.Tensor]] = None,
                        generator: Optional[torch.Generator] = None, use_graph: bool = True,
-                       known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None, seeds=None):
+                       known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None, seeds=None,
+                       text_lengths=None):
         """All reverse steps (reference: __sample_latents, SpeechGenerator.py:150-164).
 
         text_emb [B,S,text_dim]; ``audio_emb`` [B,T,H] gives the latent shape (and the start point when
@@ -396,7 +405,10 @@ class DiTTOSampler:
         ``seeds`` (B integers in [0, 2^64)) gives utterance b a noise stream of its own: x_T (unless ``x_init`` /
         ``cond_by_audio`` supplies it) and every step's noise are functions of seeds[b] alone (include/ditto_b200.h), so an
         utterance samples the same whatever else is in the batch.  Not together with ``noise`` or ``generator``.
-        ``guidance_scale`` may hold one scale per utterance."""
+        ``guidance_scale`` may hold one scale per utterance.
+
+        ``text_lengths`` (B integers in [1, S]): utterance b uses ``text_emb[b, :text_lengths[b]]`` (and the same rows of
+        ``null_text_emb``); what the other rows hold never reaches its result."""
         m = self.model
         w = self.guidance_scale if guidance_scale is None else guidance_scale
         guided = w is not None
@@ -428,7 +440,7 @@ class DiTTOSampler:
         self._activate(known=has_known)
         taus = self.timesteps.tolist()
         consecutive = self.num_steps == m.diffusion_steps
-        ctx = self._context(text_emb, guided, null_text_emb, T)
+        ctx = self._context(text_emb, guided, null_text_emb, T, text_lengths)
         n = 2 * B if guided else B
         if has_known:
             x = self._known_start(x, known, known_mask)
@@ -470,14 +482,16 @@ class DiTTOSampler:
     @torch.no_grad()
     def sample_latents_ragged(self, texts, lengths, *, x_init=None, noise=None, guidance_scale=None, null_texts=None,
                               record: Optional[List[List[torch.Tensor]]] = None, use_graph: bool = True,
-                              known=None, known_mask=None, seeds=None):
+                              known=None, known_mask=None, seeds=None, text_lengths=None):
         """``__sample_latents`` (SpeechGenerator.py:150-164) for a mixed-length batch: utterance i has ``lengths[i]`` latent
         frames (what the speech-length predictor returns x 75 fps, SpeechGenerator.py:157-158) and text ``texts[i]``
         [S_i, text_dim].  Every utterance is sampled at its own length, unpadded (see ragged.py).  ``x_init`` /
         ``noise`` are per-utterance lists ([T_i,H] / [steps,T_i,H]) for parity runs.  ``known`` / ``known_mask`` are
         per-utterance lists ([T_i,H] fp32 / [T_i] bool) of frames to keep, as in ``sample_latents``.  ``seeds`` and a
         per-utterance ``guidance_scale`` (utterance order) as in ``sample_latents``: an utterance's result does not depend on
-        which utterances share its batch, beyond the forward's batch-dependent rounding.  Returns a list of [T_i,H]."""
+        which utterances share its batch, beyond the forward's batch-dependent rounding.  ``text_lengths[i]`` in [1, S_i]:
+        utterance i uses ``texts[i][:len]`` only; padding texts to a few widths lets them share groups (and graphs, which the
+        lengths do not key).  Returns a list of [T_i,H]."""
         from .ragged import RaggedBatch, RaggedStepGraph
         m = self.model
         w = self.guidance_scale if guidance_scale is None else guidance_scale
@@ -489,7 +503,7 @@ class DiTTOSampler:
         sig = RaggedBatch.signature(texts, lengths, guided)
         cached = self._ragged_graphs.get(sig) if (use_graph and record is None) else None
         rb = RaggedBatch(m, texts, lengths, guided=guided, null_texts=null_texts,
-                         ctx_storage=cached[0] if cached is not None else None)
+                         ctx_storage=cached[0] if cached is not None else None, text_lengths=text_lengths)
         dev, H, steps = rb.device, m.hidden_dim, m.diffusion_steps
         seeds_dev = None if seeds is None else rb.pack_seeds(seeds)
         w_dev = rb.pack_w(w) if isinstance(w, list) else None

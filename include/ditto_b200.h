@@ -140,6 +140,16 @@ int64_t ditto_workspace_bytes(const ditto_engine_t* e, int64_t n_seq, int64_t T,
  * text_emb [n_seq, S, text_dim].  ctx: caller buffer of ditto_text_context_bytes(). */
 int32_t ditto_text_context(ditto_engine_t* e, const float* text_emb, int64_t n_seq, int64_t S, void* ctx,
                            void* workspace, int64_t workspace_bytes, void* stream);
+/* ditto_text_context with a text length per sequence: texts of different token counts padded to one S.  text_len is a
+ * HOST array of n_seq values, each in [1, S] (else DITTO_E_BADARG); sequence i then uses text rows [0, text_len[i]) only:
+ * the text mean of the AdaLN modulation runs over them, and every cross-attention that reads this context (ditto_forward,
+ * every ditto_p_sample*, the ragged calls, ditto_dit_block, ditto_attn_cross) gives the keys past text_len[i] probability 0.
+ * The result equals that sequence's run with the unpadded text[:text_len[i]]; what the padded rows hold (NaN / Inf too)
+ * never reaches it.  The lengths are data in ctx, so a CUDA graph captured on one masked context serves another of the same
+ * (n_seq, S) with other lengths.  All lengths == S is ditto_text_context.  Copies text_len with cudaMemcpyAsync from
+ * pageable memory: the call returns once text_len has been read (not inside a stream capture). */
+int32_t ditto_text_context_masked(ditto_engine_t* e, const float* text_emb, int64_t n_seq, int64_t S, const int64_t* text_len,
+                                  void* ctx, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* eps_hat = DiTTO.forward(x, text_emb, t)   (src/model/DiTTO.py:66-94)
  * x [n_x, T, H]; sequence i of n_seq reads x[i % n_x] (n_seq % n_x == 0; CFG: n_seq = 2 n_x shares x
